@@ -2,7 +2,8 @@
 """bench.py -- queries/sec of the flat-search hot path on B200 (BASELINE.json metric).
 
 Headline workload at every N: BASELINE configs[1] -- synthetic 1M x 384 fp32 rows, flat L2, 1024 queries, k=10.
-A "step" is one index.search() over the whole query batch.
+A "step" is one index.search() over the whole query batch; every measurement below times --steps of them.  Inputs come
+from fixed seeds, so --dump-outputs DIR (the headline's last timed result) is comparable between builds and runs.
 
   value      device-resident: queries / results are CUDA tensors, timed with CUDA events
   e2e        the same search through the C-ABI with HOST (pinned) buffers: H2D of the queries and D2H of (D, I) are
@@ -168,6 +169,24 @@ class ClockSampler:
 
 L2_BYTES = 126e6
 FLUSH_BYTES = 256 << 20
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, D, I):
+    """--dump-outputs: one search result as out_dir/distances.npy (float32) and out_dir/labels.npy (float64, exact for
+    every label below 2**53), so that two builds can be compared output for output.  A result larger than DUMP_BYTES is
+    cut to a fixed, seeded sample of its query rows, whose indices go to out_dir/query_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    D = np.asarray(D, np.float32)
+    I = np.asarray(I).astype(np.float64)
+    nq, k = D.shape
+    row_bytes = k * (4 + 8) + 8
+    if nq * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(SEED_Q).choice(nq, DUMP_BYTES // row_bytes, replace=False))
+        D, I = D[rows], I[rows]
+        np.save(os.path.join(out_dir, "query_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "distances.npy"), D)
+    np.save(os.path.join(out_dir, "labels.npy"), I)
 
 
 def host_threads() -> int:
@@ -305,8 +324,10 @@ def run_reference(args, wl, rank, world):
         step()
     t = time.time()
     for _ in range(args.steps):
-        step()
+        D, I = step()
     dt = (time.time() - t) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, D, I)
     qps = nq_s / dt * (n_cpu / n)
     cores = threads if nq_s >= 20 else min(threads, nq_s)
     # the reference's own configuration: one thread; a smaller sample keeps it bounded
@@ -427,9 +448,10 @@ class Ctx:
         self.env["torch"].cuda.synchronize()
 
 
-def measure(ctx, nq, steps, warmup, do_e2e=True, parity="auto", nchk=4):
+def measure(ctx, nq, steps, warmup, do_e2e=True, parity="auto", nchk=4, dump_dir=None):
     """One batch size on one index: device-resident value, e2e through host buffers, roofline of the dominant kernel,
-    parity spot check.  Collective at world > 1.  Returns the record on rank 0 (None elsewhere)."""
+    parity spot check; with dump_dir, rank 0 writes the result of the last timed device step there.  Collective at
+    world > 1.  Returns the record on rank 0 (None elsewhere)."""
     env, wl, ix, sh = ctx.env, ctx.wl, ctx.ix, ctx.sh
     b2f, torch, dist = env["b2f"], env["torch"], env["dist"]
     from rag_faiss_embedding_b200.encoder import synth_rows
@@ -498,6 +520,8 @@ def measure(ctx, nq, steps, warmup, do_e2e=True, parity="auto", nchk=4):
     st0 = ix.stats()
     ms_step = timed(step_device, steps)
     st1 = ix.stats()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, D_dev.cpu().numpy(), I_dev.cpu().numpy())
     # per-launch time of the dominant kernel: CUDA events recorded by the library around every launch in the timed
     # region (running sums, read once so that the host loop stays tight)
     n_launch = max(st1["prof_main_launches"] - st0["prof_main_launches"], 1)
@@ -589,7 +613,7 @@ def brief(rec):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every measurement (headline, e2e, series, c4)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
@@ -602,7 +626,11 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=20.0)
     ap.add_argument("--nq", type=int, default=0, help="diagnostics: another batch size on the workload's rows")
     ap.add_argument("--cpu-baseline-only", action="store_true", help="internal: print the cpu_baseline record for --nq queries and exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the (distances, labels) of the headline's last timed step as DIR/*.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.cpu_baseline_only:
         w0 = WORKLOADS[args.workload]
         print(json.dumps(cpu_baseline(w0, args.nq if args.nq > 0 else w0["nq"], args.cpu_budget)), flush=True)
@@ -644,26 +672,26 @@ def main():
     if rank == 0:
         sampler.start()
     ctx = Ctx(env, wl, args.algo, args.slack)
-    rec = measure(ctx, nq, args.steps, args.warmup, do_e2e=True, parity=parity)
+    rec = measure(ctx, nq, args.steps, args.warmup, do_e2e=True, parity=parity, dump_dir=args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
 
     series, c4 = [], None
     sw = min(args.warmup, 3)
     if headline and world == 1 and not args.no_series:
         # the other batch sizes of configs[1] on the same index
-        for nq_s, steps_s, algo_s in ((1, 20, "auto"), (1, 20, "tensor"), (32, 20, "auto"), (128, 20, "auto"), (4096, 10, "auto")):
+        for nq_s, algo_s in ((1, "auto"), (1, "tensor"), (32, "auto"), (128, "auto"), (4096, "auto")):
             ctx.ix.set_search_params(algo={"auto": b2f.ALGO_AUTO, "tensor": b2f.ALGO_TENSOR}[algo_s])
-            r = measure(ctx, nq_s, steps_s, sw, do_e2e=False, parity=parity)
+            r = measure(ctx, nq_s, args.steps, sw, do_e2e=False, parity=parity)
             if r:
                 series.append(brief(r))
         ctx.close()
         ctx = None
         # BASELINE configs[2]: 10M x 768 inner product (normalized), k = 100, batch 1 / 32 / 4096
         c3 = Ctx(env, WORKLOADS["c3_nq4096"], "auto", 0)
-        for nq_s, steps_s in ((1, 10), (32, 10), (4096, 5)):
+        for nq_s in (1, 32, 4096):
             s2 = ClockSampler(local_rank)
             s2.start()
-            r = measure(c3, nq_s, steps_s, sw, do_e2e=False, parity=parity if nq_s == 4096 else "off")
+            r = measure(c3, nq_s, args.steps, sw, do_e2e=False, parity=parity if nq_s == 4096 else "off")
             ck = s2.stop()
             if r:
                 r["clocks"] = ck
@@ -678,7 +706,7 @@ def main():
         s4 = ClockSampler(local_rank)
         if rank == 0:
             s4.start()
-        r = measure(c4ctx, WORKLOADS["c4shard"]["nq"], 5, sw, do_e2e=False, parity=parity)
+        r = measure(c4ctx, WORKLOADS["c4shard"]["nq"], args.steps, sw, do_e2e=False, parity=parity)
         ck = s4.stop() if rank == 0 else None
         if r:
             r["clocks"] = ck
@@ -687,7 +715,7 @@ def main():
         # the north star's small-batch target on this configuration: batch 1 and 32 against the HBM roofline
         small = []
         for nq_s in (1, 32):
-            rs = measure(c4ctx, nq_s, 10, sw, do_e2e=False, parity="off")
+            rs = measure(c4ctx, nq_s, args.steps, sw, do_e2e=False, parity="off")
             if rs:
                 small.append(brief(rs))
         if c4 is not None and small:
