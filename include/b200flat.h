@@ -156,7 +156,7 @@ B2F_API int b2f_index_read(const char* path, int32_t storage, int32_t device, b2
 
 /* ---- multi-GPU: merge per-shard top-k lists after the all-gather (SURVEY 8e) -------------------
  * D_parts/I_parts: [nparts, nq, k] (the all_gather_into_tensor layout); out: [nq, k].
- * Keeps faiss ordering and -1 padding.  Device buffers only.                                    */
+ * Keeps faiss ordering and -1 padding.  Device buffers only.  1 <= nparts <= 32 (else B2F_EINVAL). */
 B2F_API int b2f_merge_topk(int32_t metric, int64_t nq, int64_t k, int32_t nparts, const float* D_parts,
                    const int64_t* I_parts, float* D, int64_t* I, int32_t device, void* stream);
 /* Same merge over parts that are `part_stride_bytes` apart (D_parts / I_parts point at part 0): lets each rank

@@ -538,8 +538,9 @@ int b2f_index_create(int32_t d, int32_t metric, int32_t storage, int32_t device,
     cudaError_t e = cudaStreamCreateWithFlags(&ix->stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaMalloc(&ix->stats, 2 * sizeof(float));
     if (e == cudaSuccess) e = cudaMemset(ix->stats, 0, 2 * sizeof(float));
-    // centre [d] floats, then (8-byte aligned) d 64-bit words: the fixed-point accumulators its mean is summed in
-    const size_t centre_bytes = (((size_t)d * sizeof(float) + 7) & ~(size_t)7) + (size_t)d * 8;
+    // centre [d] floats, then (8-byte aligned) d 64-bit words and d floats: the fixed-point accumulators its mean is summed
+    // in and the per-column magnitudes that choose their scale
+    const size_t centre_bytes = (((size_t)d * sizeof(float) + 7) & ~(size_t)7) + (size_t)d * 12;
     if (e == cudaSuccess) e = cudaMalloc(&ix->centre, centre_bytes);
     if (e == cudaSuccess) e = cudaMemset(ix->centre, 0, centre_bytes);
     if (e == cudaSuccess) e = cudaHostAlloc(reinterpret_cast<void**>(&ix->host_flag), 64, cudaHostAllocMapped | cudaHostAllocPortable);
@@ -704,7 +705,7 @@ static int add_device_rows(b2f_index* ix, const float* src_dev, int64_t n, cudaS
         unsigned long long* acc = reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(ix->centre) + (((size_t)ix->d * sizeof(float) + 7) & ~(size_t)7));
         B2F_TRY(launch_mean_rows(src_dev, n < 65536 ? n : 65536, ix->d, ix->centre, acc, st));
         ix->mu_set = true;
-        ix->st.launches += 2;
+        ix->st.launches += 3;
     }
     B2F_TRY(launch_ingest(src_dev, n, ix->d, rows_out, ix->scan + ix->ntotal * ix->dpad, ix->dpad,
                           ix->norms + ix->ntotal, ix->stats, ix->mu_set ? ix->centre : nullptr,

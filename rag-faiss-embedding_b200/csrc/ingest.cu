@@ -48,28 +48,53 @@ __device__ __forceinline__ void emit_elem(float x, int64_t row, int col, int d, 
 // give two indexes built from the same vectors rows that differ by a bf16 ulp here and there (float atomics did exactly
 // that).  Every block sums its 64 rows in a fixed order and adds the sum to a 64-bit FIXED-POINT accumulator: integer
 // addition is associative, the order in which the blocks arrive does not matter.
-constexpr double kMeanScale = 16777216.0;   // 2^24: 6e-8 absolute on a 64-row sum, |sum of all rows| up to 5e11
-__global__ void __launch_bounds__(256) mean_rows_kernel(const float* __restrict__ src, int64_t m, int d, unsigned long long* __restrict__ acc) {
+// The fixed-point scale is a power of two chosen PER COLUMN from the largest |block sum| of that column (a first pass;
+// integer atomicMax on the float bits is order independent too): 2^e with nblocks * max|block sum| * 2^e <= 2^62, so the
+// sum of every block fits the signed 64-bit word whatever the magnitude of the rows.  (A fixed 2^24 wrapped silently once
+// |sum of the rows| passed 5.5e11 -- a column mean above 8.4e6 over 65536 rows -- and left a garbage centre.)  Scaling the
+// rows by a power of two scales every block sum, the exponent and so the centre exactly: the centre is scale-equivariant.
+__device__ __forceinline__ float block_col_sum(const float* __restrict__ src, int64_t m, int d, int c) {
     const int64_t r0 = (int64_t)blockIdx.x * 64, r1 = r0 + 64 < m ? r0 + 64 : m;
+    float a = 0.f;
+    for (int64_t r = r0; r < r1; r++) a += src[r * d + c];
+    return a;
+}
+__device__ __forceinline__ int mean_scale_exp(float amax, int64_t nblocks) {
+    if (!(amax > 0.f)) return 0;   // every block sum of the column is 0 (or none is finite): any scale
+    int ex;
+    frexp((double)amax * (double)nblocks, &ex);   // exact product; nblocks * amax < 2^ex
+    return 62 - ex;
+}
+// pass 0: colmax[c] = max |block sum| of column c; pass 1: acc[c] += block sum * 2^e(c)
+__global__ void __launch_bounds__(256) mean_rows_kernel(const float* __restrict__ src, int64_t m, int d, float* __restrict__ colmax,
+                                                        unsigned long long* __restrict__ acc, int pass) {
+    const int64_t nblocks = (m + 63) / 64;
     for (int c = threadIdx.x; c < d; c += blockDim.x) {
-        float a = 0.f;
-        for (int64_t r = r0; r < r1; r++) a += src[r * d + c];
-        if (a == a && fabsf(a) < 1.0e11f)   // (NaN / inf rows do not move the centre)
-            atomicAdd(acc + c, (unsigned long long)__double2ll_rn((double)a * kMeanScale));   // two's complement: signed sums
+        const float a = block_col_sum(src, m, d, c);
+        if (!isfinite(a)) continue;   // (NaN / inf rows do not move the centre)
+        if (pass == 0)
+            atomic_max_nonneg(colmax + c, fabsf(a));
+        else   // two's complement: signed sums
+            atomicAdd(acc + c, (unsigned long long)__double2ll_rn(ldexp((double)a, mean_scale_exp(colmax[c], nblocks))));
     }
 }
-__global__ void mean_finish_kernel(const unsigned long long* __restrict__ acc, int64_t m, int d, float* __restrict__ mu) {
+__global__ void mean_finish_kernel(const unsigned long long* __restrict__ acc, const float* __restrict__ colmax, int64_t m, int d,
+                                   float* __restrict__ mu) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c < d) mu[c] = (float)((double)(long long)acc[c] / kMeanScale / (double)m);
+    if (c < d) mu[c] = (float)(ldexp((double)(long long)acc[c], -mean_scale_exp(colmax[c], (m + 63) / 64)) / (double)m);
 }
 
-// acc: d 64-bit words of device scratch
+// acc: d 64-bit words followed by d floats of device scratch
 int launch_mean_rows(const float* src, int64_t m, int d, float* mu, unsigned long long* acc, cudaStream_t st) {
     if (m <= 0) return B2F_OK;
-    B2F_CUDA(cudaMemsetAsync(acc, 0, (size_t)d * 8, st));
-    mean_rows_kernel<<<(unsigned)((m + 63) / 64), 256, 0, st>>>(src, m, d, acc);
+    float* colmax = reinterpret_cast<float*>(acc + d);
+    B2F_CUDA(cudaMemsetAsync(acc, 0, (size_t)d * 12, st));
+    const unsigned blocks = (unsigned)((m + 63) / 64);
+    mean_rows_kernel<<<blocks, 256, 0, st>>>(src, m, d, colmax, acc, 0);
     B2F_CUDA(cudaGetLastError());
-    mean_finish_kernel<<<(d + 255) / 256, 256, 0, st>>>(acc, m, d, mu);
+    mean_rows_kernel<<<blocks, 256, 0, st>>>(src, m, d, colmax, acc, 1);
+    B2F_CUDA(cudaGetLastError());
+    mean_finish_kernel<<<(d + 255) / 256, 256, 0, st>>>(acc, colmax, m, d, mu);
     B2F_CUDA(cudaGetLastError());
     return B2F_OK;
 }
