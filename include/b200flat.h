@@ -150,7 +150,9 @@ B2F_API int b2f_index_reconstruct(b2f_index* idx, int64_t i0, int64_t n, float* 
  * ---- faiss.read_index(path):         faiss_store.py:106, rag_datastore_manager.py:205 ----------
  * Byte-compatible with FAISS's IndexFlat serialisation ("IxF2"/"IxFI" | i32 d | i64 ntotal |
  * i64 2^20 | i64 2^20 | u8 is_trained | i32 metric | u64 nfloats | fp32 rows).  Streams through
- * pinned chunks, so a 100+ GB index never needs a host copy.                                     */
+ * pinned chunks, so a 100+ GB index never needs a host copy.  Reading into B2F_STORE_BF16
+ * re-ingests the file's fp32 rows as a first add would: a new centre from the file's first rows,
+ * each row rounded around it.                                                                    */
 B2F_API int b2f_index_write(b2f_index* idx, const char* path);
 B2F_API int b2f_index_read(const char* path, int32_t storage, int32_t device, b2f_index** out);
 

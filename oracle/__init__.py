@@ -7,6 +7,7 @@ status ("parity unpinned" for search results; on-disk layout pinned by the refer
 from .flat_oracle import (  # noqa: F401
     METRIC_INNER_PRODUCT,
     METRIC_L2,
+    CENTRE_ROWS,
     build,
     c_search,
     c_synth_rows,
@@ -17,6 +18,9 @@ from .flat_oracle import (  # noqa: F401
     np_search_blas,
     torch_search_blas,
     np_synth_rows,
+    np_centre,
+    np_bf16_rne,
+    np_bf16_rows,
     np_read_index,
     np_write_index,
     recall_and_errors,

@@ -276,6 +276,54 @@ def np_synth_rows(seed, row0, nrows, d, normalize=False):
     return out.astype(np.float32)
 
 
+CENTRE_ROWS = 65536   # the centre is the mean of the first min(n, CENTRE_ROWS) rows of the first add
+
+
+def np_centre(first_rows):
+    """Same bits as the device centre (ingest.cu mean_rows_kernel + mean_finish_kernel) of an index whose first add
+    call receives `first_rows`.  m = min(n, 65536) rows in 64-row blocks (the last may be partial); each block sums its
+    column in float32, row after row from 0; a block whose sum is not finite is skipped but still counts in m.  The
+    finite block sums go into a 64-bit fixed-point accumulator at 2^e(c), e = 62 - exponent(max |block sum| * nblocks),
+    each rounded half to even (__double2ll_rn); mu = fl32(acc * 2^-e / m) in float64."""
+    x = _f32(first_rows)
+    m = min(x.shape[0], CENTRE_ROWS)
+    d = x.shape[1]
+    if m == 0:
+        return np.zeros(d, np.float32)
+    x = x[:m]
+    nblocks = (m + 63) // 64
+    pad = np.zeros((nblocks * 64, d), np.float32)   # a partial last block is padded with zeros: a + 0 == a
+    pad[:m] = x
+    sums = np.empty((nblocks, d), np.float32)
+    with np.errstate(over="ignore", invalid="ignore"):
+        for b0 in range(0, nblocks, 64):
+            # np.cumsum adds sequentially (np.sum would add pairwise); the kernel's leading 0 + x0 only turns -0 into +0
+            sums[b0:b0 + 64] = np.cumsum(pad[64 * b0:64 * (b0 + 64)].reshape(-1, 64, d), 1, np.float32)[:, -1]
+    fin = np.isfinite(sums)
+    a = np.where(fin, sums, np.float32(0)).astype(np.float64)
+    colmax = np.abs(a).max(0)
+    _, ex = np.frexp(colmax * nblocks)
+    e = np.where(colmax > 0, 62 - ex, 0).astype(np.int64)
+    terms = np.rint(np.ldexp(a, e[None, :])).astype(np.int64)   # rint: half to even; |term| <= 2^62 / nblocks
+    acc = terms.sum(0)
+    return (np.ldexp(acc.astype(np.float64), -e) / np.float64(m)).astype(np.float32)
+
+
+def np_bf16_rne(x):
+    """float32 -> bfloat16 (round to nearest even, subnormals kept, overflow to inf) -> float32.  NaN stays NaN."""
+    u = _f32(x).view(np.uint32).astype(np.uint64)
+    r = ((u + np.uint64(0x7FFF) + ((u >> np.uint64(16)) & np.uint64(1))) & np.uint64(0xFFFF0000)).astype(np.uint32)
+    out = r.view(np.float32)
+    return np.where(np.isnan(x), np.float32(np.nan), out).astype(np.float32)
+
+
+def np_bf16_rows(x, mu):
+    """The authoritative rows of a bf16-storage index: r = fl32(mu + bf16_rne(fl32(x - mu)))."""
+    x, mu = _f32(x), _f32(mu)
+    with np.errstate(over="ignore", invalid="ignore"):
+        return (mu[None, :] + np_bf16_rne(x - mu[None, :])).astype(np.float32)
+
+
 def np_write_index(path, xb, metric=METRIC_L2):
     xb = _f32(xb)
     n, d = xb.shape

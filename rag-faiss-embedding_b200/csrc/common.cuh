@@ -249,8 +249,12 @@ int launch_merge_faiss(int metric, int64_t nq, int64_t k, int nparts, const floa
 // bf16_auth: bf16 storage -- the authoritative row is fl32(mu + scan row); the IP bias and stats[1] refer to it.
 int launch_ingest(const float* src, int64_t n, int d, float* rows_f32, __nv_bfloat16* scan, int64_t dpad,
                   float* norms, float* stats, const float* mu, int ip_bias, int bf16_auth, cudaStream_t st);
-// mu[c] = mean of column c over the m rows of src
-int launch_mean_rows(const float* src, int64_t m, int d, float* mu, unsigned long long* acc, cudaStream_t st);
+// mu[c] = mean of column c over m rows, which may arrive in pieces: begin; pass 0 over every piece; pass 1 over every
+// piece; finish.  src of a piece holds its `rows` rows from row row0 (a multiple of 64) on.  acc: d 64-bit words + d floats.
+int launch_mean_begin(int d, unsigned long long* acc, cudaStream_t st);
+int launch_mean_pass(const float* src, int64_t row0, int64_t rows, int64_t m, int d, unsigned long long* acc, int pass,
+                     cudaStream_t st);
+int launch_mean_finish(int64_t m, int d, float* mu, unsigned long long* acc, cudaStream_t st);
 // K7: pooling (+normalise) of encoder output, optionally fused with the ingest writes.
 int launch_pool(const float* hidden, const int64_t* mask, int64_t B, int64_t T, int d, int pool, int normalize,
                 float* out_f32, __nv_bfloat16* scan, int64_t dpad, float* norms, float* stats, cudaStream_t st);

@@ -690,22 +690,59 @@ static bool centring_enabled() {
     return v == 1;
 }
 
+// The scan copy is taken around the mean of the first rows the index sees, fixed from then on: any centre is correct, a
+// representative one makes the bf16 pass far more decisive on embeddings that share a large common component.  bf16
+// storage keeps the same centred copy as its ONLY copy: the authoritative row is then fl32(mu + bf16(x - mu)) -- closer
+// to x than bf16(x) on such data, and the tensor pass certifies as on fp32 storage.
+// Which rows: the first min(n, 65536) rows of the FIRST add call, on every route (device rows, host rows, pooled,
+// generated, read from a file), whatever the route's staging -- so that the same rows give the same centre, and the same
+// bf16-storage index, bit for bit.  Every route calls take_centre before it ingests its first rows.  A route that stages
+// its rows through a smaller buffer passes its piece size (>= 64 rows) and stage(r0, rows, &src), which puts rows
+// [r0, r0 + rows) of the call on the device in stream order; both passes of the mean walk every piece, so such a route
+// stages the first <= 65536 rows once more (they fit one piece) or twice more, once per index.
+static const int64_t kCentreRows = 65536;
+
+extern "C++" {   // (a template inside the extern "C" block)
+template <class Stage>
+static int take_centre(b2f_index* ix, int64_t n, int64_t piece, cudaStream_t st, Stage&& stage) {
+    if (ix->mu_set || ix->ntotal != 0 || n <= 0 || !centring_enabled()) return B2F_OK;
+    const int64_t m = n < kCentreRows ? n : kCentreRows;
+    piece = piece >= m ? m : piece / 64 * 64;
+    if (piece <= 0) {
+        set_error("centre: staging piece of %lld rows is below one 64-row block", (long long)piece);
+        return B2F_EINVAL;
+    }
+    unsigned long long* acc = reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(ix->centre) + (((size_t)ix->d * sizeof(float) + 7) & ~(size_t)7));
+    B2F_TRY(launch_mean_begin(ix->d, acc, st));
+    const float* src = nullptr;
+    for (int pass = 0; pass < 2; pass++)
+        for (int64_t r0 = 0; r0 < m; r0 += piece) {
+            const int64_t rows = m - r0 < piece ? m - r0 : piece;
+            if (pass == 0 || piece < m) B2F_TRY(stage(r0, rows, &src));   // (one piece: pass 1 reads it again in place)
+            B2F_TRY(launch_mean_pass(src, r0, rows, m, ix->d, acc, pass, st));
+            ix->st.launches++;
+        }
+    B2F_TRY(launch_mean_finish(m, ix->d, ix->centre, acc, st));
+    ix->st.launches++;
+    ix->mu_set = true;
+    return B2F_OK;
+}
+}  // extern "C++"
+
+// the first add's rows are all on the device already: one piece
+static int take_centre_device(b2f_index* ix, const float* src_dev, int64_t n, cudaStream_t st) {
+    return take_centre(ix, n, n, st, [&](int64_t r0, int64_t, const float** src) {
+        *src = src_dev + r0 * ix->d;
+        return B2F_OK;
+    });
+}
+
 static int add_device_rows(b2f_index* ix, const float* src_dev, int64_t n, cudaStream_t st) {
-    // src_dev: [n, d] fp32 on the device (may alias the tail of rows_f32)
+    // src_dev: [n, d] fp32 on the device (may alias the tail of rows_f32); the centre is set (take_centre) beforehand
     float* rows_out = nullptr;
     if (ix->storage == B2F_STORE_F32) {
         float* dst = ix->rows_f32 + ix->ntotal * ix->d;
         if (src_dev != dst) rows_out = dst;
-    }
-    // The scan copy is taken around the mean of the first rows the index sees (at most 65536), fixed from then on: any
-    // centre is correct, a representative one makes the bf16 pass far more decisive on embeddings that share a large
-    // common component.  bf16 storage keeps the same centred copy as its ONLY copy: the authoritative row is then
-    // fl32(mu + bf16(x - mu)) -- closer to x than bf16(x) on such data, and the tensor pass certifies as on fp32 storage.
-    if (!ix->mu_set && ix->ntotal == 0 && centring_enabled()) {
-        unsigned long long* acc = reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(ix->centre) + (((size_t)ix->d * sizeof(float) + 7) & ~(size_t)7));
-        B2F_TRY(launch_mean_rows(src_dev, n < 65536 ? n : 65536, ix->d, ix->centre, acc, st));
-        ix->mu_set = true;
-        ix->st.launches += 3;
     }
     B2F_TRY(launch_ingest(src_dev, n, ix->d, rows_out, ix->scan + ix->ntotal * ix->dpad, ix->dpad,
                           ix->norms + ix->ntotal, ix->stats, ix->mu_set ? ix->centre : nullptr,
@@ -731,18 +768,25 @@ int b2f_index_add(b2f_index* ix, int64_t n, const float* x, int32_t mem, void* s
     if (ix->search_recorded && ix->last_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_done, 0));
     B2F_TRY(wait_ingest(ix, st));
     if (mem == B2F_MEM_DEVICE) {
+        B2F_TRY(take_centre_device(ix, x, n, st));
         B2F_TRY(add_device_rows(ix, x, n, st));
         ix->ntotal += n;
     } else if (ix->storage == B2F_STORE_F32) {
         // host -> final location, then derive the scan copy in place
         float* dst = ix->rows_f32 + ix->ntotal * ix->d;
         B2F_CUDA(cudaMemcpyAsync(dst, x, (size_t)n * ix->d * sizeof(float), cudaMemcpyHostToDevice, st));
+        B2F_TRY(take_centre_device(ix, dst, n, st));
         B2F_TRY(add_device_rows(ix, dst, n, st));
         ix->ntotal += n;
     } else {
         // bf16 storage: stage fp32 chunks through the workspace
         const int64_t chunk = (64LL << 20) / ((int64_t)ix->d * 4) > 0 ? (64LL << 20) / ((int64_t)ix->d * 4) : 1;
         B2F_TRY(ensure_ws(ix, (size_t)chunk * ix->d * 4 + 4096));
+        B2F_TRY(take_centre(ix, n, chunk, st, [&](int64_t r0, int64_t m, const float** src) {
+            B2F_CUDA(cudaMemcpyAsync(ix->ws, x + r0 * ix->d, (size_t)m * ix->d * 4, cudaMemcpyHostToDevice, st));
+            *src = reinterpret_cast<const float*>(ix->ws);
+            return B2F_OK;
+        }));
         for (int64_t r0 = 0; r0 < n; r0 += chunk) {
             const int64_t m = n - r0 < chunk ? n - r0 : chunk;
             B2F_CUDA(cudaMemcpyAsync(ix->ws, x + r0 * ix->d, (size_t)m * ix->d * 4, cudaMemcpyHostToDevice, st));
@@ -771,12 +815,19 @@ int b2f_index_add_synth(b2f_index* ix, uint64_t seed, int64_t row0, int64_t nrow
     if (ix->storage == B2F_STORE_F32) {
         float* dst = ix->rows_f32 + ix->ntotal * ix->d;
         B2F_TRY(launch_synth(seed, row0, nrows, ix->d, normalize, dst, st));
+        B2F_TRY(take_centre_device(ix, dst, nrows, st));
         B2F_TRY(add_device_rows(ix, dst, nrows, st));
         ix->ntotal += nrows;
         ix->st.launches++;
     } else {
         const int64_t chunk = (256LL << 20) / ((int64_t)ix->d * 4) > 0 ? (256LL << 20) / ((int64_t)ix->d * 4) : 1;
         B2F_TRY(ensure_ws(ix, (size_t)chunk * ix->d * 4 + 4096));
+        B2F_TRY(take_centre(ix, nrows, chunk, st, [&](int64_t r0, int64_t m, const float** src) {
+            B2F_TRY(launch_synth(seed, row0 + r0, m, ix->d, normalize, reinterpret_cast<float*>(ix->ws), st));
+            ix->st.launches++;
+            *src = reinterpret_cast<const float*>(ix->ws);
+            return B2F_OK;
+        }));
         for (int64_t r0 = 0; r0 < nrows; r0 += chunk) {
             const int64_t m = nrows - r0 < chunk ? nrows - r0 : chunk;
             B2F_TRY(launch_synth(seed, row0 + r0, m, ix->d, normalize, reinterpret_cast<float*>(ix->ws), st));
@@ -811,12 +862,21 @@ int b2f_index_add_pooled(b2f_index* ix, const float* hidden, const int64_t* mask
         float* dst = ix->rows_f32 + ix->ntotal * ix->d;
         B2F_TRY(launch_pool(hidden, mask, B, T, ix->d, pool, normalize, dst, nullptr, 0, nullptr, nullptr, st));
         ix->st.launches++;
+        B2F_TRY(take_centre_device(ix, dst, B, st));
         B2F_TRY(add_device_rows(ix, dst, B, st));
         ix->ntotal += B;
     } else {
         // bf16 storage: pool fp32 chunks into the workspace, ingest from there
         const int64_t chunk = (64LL << 20) / ((int64_t)ix->d * 4) > 0 ? (64LL << 20) / ((int64_t)ix->d * 4) : 1;
         B2F_TRY(ensure_ws(ix, (size_t)(B < chunk ? B : chunk) * ix->d * 4 + 4096));
+        B2F_TRY(take_centre(ix, B, chunk, st, [&](int64_t b0, int64_t m, const float** src) {
+            float* tmp = reinterpret_cast<float*>(ix->ws);
+            B2F_TRY(launch_pool(hidden + b0 * T * ix->d, mask ? mask + b0 * T : nullptr, m, T, ix->d, pool, normalize, tmp, nullptr, 0,
+                                nullptr, nullptr, st));
+            ix->st.launches++;
+            *src = tmp;
+            return B2F_OK;
+        }));
         for (int64_t b0 = 0; b0 < B; b0 += chunk) {
             const int64_t m = B - b0 < chunk ? B - b0 : chunk;
             float* tmp = reinterpret_cast<float*>(ix->ws);
@@ -1461,6 +1521,26 @@ int b2f_index_read(const char* path, int32_t storage, int32_t device, b2f_index*
         const size_t cbytes = (size_t)rows_per * d32 * 4;
         if (rc == B2F_OK && nt > 0) rc = ensure_pinned(ix, 2 * cbytes);
         if (rc == B2F_OK && nt > 0 && storage == B2F_STORE_BF16) rc = ensure_ws(ix, 2 * cbytes + 4096);
+        // the centre of an index read from a file is the mean of the file's first rows, as if they were added: read
+        // them for the mean first (through pinned slot 0), then start over at the first row
+        const long payload = ftell(f);
+        if (rc == B2F_OK && nt > 0)
+            rc = take_centre(ix, nt, rows_per, ix->stream, [&](int64_t r0, int64_t m, const float** src) {
+                B2F_CUDA(cudaStreamSynchronize(ix->stream));   // the pinned slot may still be in flight
+                const size_t cnt = (size_t)m * d32;
+                if (fseek(f, payload + (long)((size_t)r0 * d32 * 4), SEEK_SET) != 0 || fread(ix->pinned, 4, cnt, f) != cnt) {
+                    set_error("%s: truncated payload", path);
+                    return B2F_EFORMAT;
+                }
+                float* dst = storage == B2F_STORE_F32 ? ix->rows_f32 + r0 * d32 : reinterpret_cast<float*>(ix->ws);
+                B2F_CUDA(cudaMemcpyAsync(dst, ix->pinned, cnt * 4, cudaMemcpyHostToDevice, ix->stream));
+                *src = dst;
+                return B2F_OK;
+            });
+        if (rc == B2F_OK && nt > 0 && (cudaStreamSynchronize(ix->stream) != cudaSuccess || fseek(f, payload, SEEK_SET) != 0)) {
+            set_error("read: %s: could not rewind after the centre", path);
+            rc = B2F_EIO;
+        }
         cudaEvent_t evs[2] = {get_event(ix, 1), get_event(ix, 2)};
         bool used[2] = {false, false};
         int slot = 0;

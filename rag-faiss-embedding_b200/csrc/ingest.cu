@@ -46,15 +46,19 @@ __device__ __forceinline__ void emit_elem(float x, int64_t row, int col, int d, 
 // mu[c] = (1/m) * sum of column c over rows [0, m): the centre the scan copy is taken around.  The same rows must give the
 // same centre bit for bit -- bf16 storage rounds the stored rows around it, so a centre that moved in its last bit would
 // give two indexes built from the same vectors rows that differ by a bf16 ulp here and there (float atomics did exactly
-// that).  Every block sums its 64 rows in a fixed order and adds the sum to a 64-bit FIXED-POINT accumulator: integer
-// addition is associative, the order in which the blocks arrive does not matter.
+// that).  Every 64-row block sums its column in float32 in a fixed order and adds the sum to a 64-bit FIXED-POINT
+// accumulator: integer addition is associative, the order in which the blocks arrive does not matter.
 // The fixed-point scale is a power of two chosen PER COLUMN from the largest |block sum| of that column (a first pass;
 // integer atomicMax on the float bits is order independent too): 2^e with nblocks * max|block sum| * 2^e <= 2^62, so the
 // sum of every block fits the signed 64-bit word whatever the magnitude of the rows.  (A fixed 2^24 wrapped silently once
 // |sum of the rows| passed 5.5e11 -- a column mean above 8.4e6 over 65536 rows -- and left a garbage centre.)  Scaling the
 // rows by a power of two scales every block sum, the exponent and so the centre exactly: the centre is scale-equivariant.
-__device__ __forceinline__ float block_col_sum(const float* __restrict__ src, int64_t m, int d, int c) {
-    const int64_t r0 = (int64_t)blockIdx.x * 64, r1 = r0 + 64 < m ? r0 + 64 : m;
+// A block whose float32 sum is not finite -- a NaN or inf entry, or 64 rows whose sum overflows (same-sign entries above
+// ~5e36) -- is left out of the sum of that column but still counts in m.
+// The rows may arrive in pieces (a caller that stages them through a smaller buffer): every piece starts at a multiple of
+// 64 rows, and the exponent uses the block count of all m rows, so the result does not depend on the staging.
+__device__ __forceinline__ float block_col_sum(const float* __restrict__ src, int64_t rows, int d, int c) {
+    const int64_t r0 = (int64_t)blockIdx.x * 64, r1 = r0 + 64 < rows ? r0 + 64 : rows;
     float a = 0.f;
     for (int64_t r = r0; r < r1; r++) a += src[r * d + c];
     return a;
@@ -65,13 +69,14 @@ __device__ __forceinline__ int mean_scale_exp(float amax, int64_t nblocks) {
     frexp((double)amax * (double)nblocks, &ex);   // exact product; nblocks * amax < 2^ex
     return 62 - ex;
 }
-// pass 0: colmax[c] = max |block sum| of column c; pass 1: acc[c] += block sum * 2^e(c)
-__global__ void __launch_bounds__(256) mean_rows_kernel(const float* __restrict__ src, int64_t m, int d, float* __restrict__ colmax,
-                                                        unsigned long long* __restrict__ acc, int pass) {
+// src: `rows` rows of the m; pass 0: colmax[c] = max |block sum| of column c; pass 1: acc[c] += block sum * 2^e(c)
+__global__ void __launch_bounds__(256) mean_rows_kernel(const float* __restrict__ src, int64_t rows, int64_t m, int d,
+                                                        float* __restrict__ colmax, unsigned long long* __restrict__ acc,
+                                                        int pass) {
     const int64_t nblocks = (m + 63) / 64;
     for (int c = threadIdx.x; c < d; c += blockDim.x) {
-        const float a = block_col_sum(src, m, d, c);
-        if (!isfinite(a)) continue;   // (NaN / inf rows do not move the centre)
+        const float a = block_col_sum(src, rows, d, c);
+        if (!isfinite(a)) continue;   // the whole block is left out of this column (it still counts in m)
         if (pass == 0)
             atomic_max_nonneg(colmax + c, fabsf(a));
         else   // two's complement: signed sums
@@ -85,16 +90,25 @@ __global__ void mean_finish_kernel(const unsigned long long* __restrict__ acc, c
 }
 
 // acc: d 64-bit words followed by d floats of device scratch
-int launch_mean_rows(const float* src, int64_t m, int d, float* mu, unsigned long long* acc, cudaStream_t st) {
-    if (m <= 0) return B2F_OK;
-    float* colmax = reinterpret_cast<float*>(acc + d);
+int launch_mean_begin(int d, unsigned long long* acc, cudaStream_t st) {
     B2F_CUDA(cudaMemsetAsync(acc, 0, (size_t)d * 12, st));
-    const unsigned blocks = (unsigned)((m + 63) / 64);
-    mean_rows_kernel<<<blocks, 256, 0, st>>>(src, m, d, colmax, acc, 0);
+    return B2F_OK;
+}
+int launch_mean_pass(const float* src, int64_t row0, int64_t rows, int64_t m, int d, unsigned long long* acc, int pass,
+                     cudaStream_t st) {
+    if (rows <= 0) return B2F_OK;
+    if (row0 % 64 != 0 || row0 + rows > m) {
+        set_error("mean pass: piece [%lld, %lld) of %lld rows does not start on a 64-row block", (long long)row0,
+                  (long long)(row0 + rows), (long long)m);
+        return B2F_EINVAL;
+    }
+    mean_rows_kernel<<<(unsigned)((rows + 63) / 64), 256, 0, st>>>(src, rows, m, d, reinterpret_cast<float*>(acc + d), acc, pass);
     B2F_CUDA(cudaGetLastError());
-    mean_rows_kernel<<<blocks, 256, 0, st>>>(src, m, d, colmax, acc, 1);
-    B2F_CUDA(cudaGetLastError());
-    mean_finish_kernel<<<(d + 255) / 256, 256, 0, st>>>(acc, colmax, m, d, mu);
+    return B2F_OK;
+}
+int launch_mean_finish(int64_t m, int d, float* mu, unsigned long long* acc, cudaStream_t st) {
+    if (m <= 0) return B2F_OK;
+    mean_finish_kernel<<<(d + 255) / 256, 256, 0, st>>>(acc, reinterpret_cast<const float*>(acc + d), m, d, mu);
     B2F_CUDA(cudaGetLastError());
     return B2F_OK;
 }
