@@ -35,6 +35,71 @@ std::mutex& launch_cache_mutex() {
 
 using namespace b2f;
 
+// What searches teach an index about its data.  It goes with the data: b2f_index_reset starts it over.
+struct Adapt {
+    int slack_boost = 0;           // extra candidates per query, raised when too many queries fail certification
+    bool range_mode = false;       // earlier batches left many queries uncertified: run the range pass (one host sync per search)
+    int32_t range_ran_seq = 0;     // the search (sequence number) whose range pass served range_ran_nfail queries
+    int range_ran_nfail = 0;
+    int range_futile = 0;          // consecutive range passes that left most of their queries to the exact scan anyway
+    int range_ban = 0;             // searches to wait before the range pass may be switched on again
+    int range_quiet = 0;           // consecutive range-mode searches whose first pass certified everything
+    // Order-robust mode.  A batch whose candidate lists overflowed en masse (rows stored so that a query's best rows sit in
+    // one or two lists: the shared thresholds never tighten) switches the index to per-thread heaps for the first pass
+    // (plan_force_heap) plus the range pass for what the heaps cannot certify; LIST mode is tried again after heap_span
+    // searches, and the span doubles every time it fails again.
+    int heap_left = 0;             // searches still to run in this mode
+    int heap_span = 64;
+
+    // Folds in what finished search s counted: c0 uncertified queries, c1 of them with an overflowed list, of a batch of nqb.
+    void learn(int32_t s, int c0, int c1, int nqb, int certify) {
+        // The slack that certification needs grows with the neighbour density at rank k (i.e. with the database
+        // size and the data distribution): when too many queries of a batch had to fall back, keep more candidates
+        // per query from now on.  "Too many" is where the exact scans cost more than the wider tensor pass would: the
+        // fallback walks the database once per four queries (F / 4 x n d 4 B at ~5.5 TB/s) while the batch's tensor
+        // pass costs 2 nq n d flop at ~1.3 PFLOP/s and grows by < 10 % with 32 more candidates -- break-even at
+        // F ~ nq / 1200; the boost waits for 0.5 % because the range pass below is cheaper still.  (Round 1 waited for 2 % of
+        // the batch: BASELINE config 5 on 2 GPUs spent 9 of its 34 ms per search in exact scans for 0.5 % of the queries.)
+        if (certify && c0 - c1 > (nqb / 200 > 2 ? nqb / 200 : 2) && slack_boost < 224) slack_boost += 32;
+        // Well before that (F > nq / 1000) the range pass takes over: a second TENSOR pass over the uncertified queries with a
+        // fixed threshold per query, one database pass for all of them instead of one exact scan per four (range_pass).
+        // ... unless it does not help: neighbourhoods so dense that the fixed-threshold lists overflow too (thousands of
+        // near-duplicates) leave its queries to the exact scan anyway; two such searches in a row switch it off for a while.
+        if (range_ban > 0) range_ban--;
+        if (range_mode && range_ran_seq == s) {
+            if (2 * c0 > range_ran_nfail) {
+                if (++range_futile >= 2) {
+                    range_mode = false;
+                    range_futile = 0;
+                    range_ban = 256;
+                }
+            } else {
+                range_futile = 0;
+            }
+        }
+        if (certify && c1 > (nqb / 8 > 8 ? nqb / 8 : 8) && heap_left == 0) {
+            heap_left = heap_span;
+            if (heap_span < 4096) heap_span *= 2;
+            if (range_ban == 0) {
+                range_mode = true;   // the heaps find the k' best whatever the row order; dense neighbourhoods still need the range pass
+                range_quiet = 0;
+            }
+        }
+        if (certify && !range_mode && range_ban == 0 && c0 - c1 > (nqb / 1000 > 2 ? nqb / 1000 : 2)) {
+            range_mode = true;
+            range_quiet = 0;
+        }
+    }
+    // A range-mode search whose first pass left nfail queries uncertified
+    void first_pass_failed(int nfail) {
+        if (nfail == 0) {
+            if (++range_quiet >= 8) range_mode = false;   // the data (or the adaptive slack) no longer needs it
+        } else {
+            range_quiet = 0;
+        }
+    }
+};
+
 struct b2f_index {
     int d = 0, metric = 1, storage = 0, device = 0;
     int64_t ntotal = 0, cap = 0, dpad = 0;
@@ -61,19 +126,7 @@ struct b2f_index {
     int32_t seq = 0;
     uint32_t scan_launches = 0;       // launch parity of the scan's cross-CTA bounds
     int32_t harvested_seq = 0;        // last seq whose counters were folded into the host-side statistics
-    int slack_boost = 0;              // extra candidates per query, raised when too many queries fail certification
-    bool range_mode = false;          // earlier batches left many queries uncertified: run the range pass (one host sync per search)
-    int32_t range_ran_seq = 0;        // the search (sequence number) whose range pass served range_ran_nfail queries
-    int range_ran_nfail = 0;
-    int range_futile = 0;             // consecutive range passes that left most of their queries to the exact scan anyway
-    int range_ban = 0;                // searches to wait before the range pass may be switched on again
-    int range_quiet = 0;              // consecutive range-mode searches whose first pass certified everything
-    // Order-robust mode.  A batch whose candidate lists overflowed en masse (rows stored so that a query's best rows sit in
-    // one or two lists: the shared thresholds never tighten) switches the index to per-thread heaps for the first pass
-    // (plan_force_heap) plus the range pass for what the heaps cannot certify; LIST mode is tried again after heap_span
-    // searches, and the span doubles every time it fails again.
-    int heap_left = 0;                // searches still to run in this mode
-    int heap_span = 64;
+    Adapt adapt;
     unsigned long long* totals = nullptr;  // device [4]: fallback queries, overflowed queries, rescued queries (running totals)
     cudaEvent_t ev_done = nullptr;    // recorded at the end of every search (searches return without synchronising)
     cudaStream_t last_stream = nullptr;
@@ -143,19 +196,28 @@ int check_device(int device) {
     return B2F_OK;
 }
 
-// simple bump allocator over the index workspace
+// Bump allocator over the index workspace of `size` bytes.  Over a null base it only measures: the same carve that lays
+// the buffers out then gives the bytes they need.  A carve that passes the end leaves fits() false.
 struct Bump {
     char* base;
+    size_t size;
     size_t off = 0;
-    explicit Bump(char* b) : base(b) {}
+    Bump(char* b, size_t n) : base(b), size(n) {}
     template <typename T>
     T* take(size_t count) {
         off = align_up(off, 256);
-        T* p = reinterpret_cast<T*>(base + off);
+        T* p = reinterpret_cast<T*>(reinterpret_cast<uintptr_t>(base) + off);
         off += count * sizeof(T);
         return p;
     }
+    bool fits() const { return off <= size; }
 };
+
+// rows of d floats that fit `bytes` (at least one)
+int64_t rows_in(size_t bytes, int d) {
+    const int64_t r = (int64_t)(bytes / ((size_t)d * 4));
+    return r > 0 ? r : 1;
+}
 
 int ensure_ws(b2f_index* ix, size_t bytes) {
     if (bytes <= ix->ws_bytes) return B2F_OK;
@@ -195,6 +257,34 @@ int ensure_pinned(b2f_index* ix, size_t bytes) {
     return B2F_OK;
 }
 
+// Adds are enqueued on the caller's stream (a device-tensor add / add_pooled runs behind the encoder on torch's
+// stream) and return without synchronising.  Everything that reads rows, norms, stats or the centre on ANOTHER
+// stream -- searches, write, reconstruct, the stats refresh, the growth copies -- first waits for the latest add.
+int wait_ingest(b2f_index* ix, cudaStream_t st) {
+    if (ix->add_recorded && ix->last_add_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_ingest, 0));
+    return B2F_OK;
+}
+int record_ingest(b2f_index* ix, cudaStream_t st) {
+    if (!ix->ev_ingest) B2F_CUDA(cudaEventCreateWithFlags(&ix->ev_ingest, cudaEventDisableTiming));
+    // an add on a new stream is ordered behind the previous add (both write stats / may share the workspace)
+    B2F_CUDA(cudaEventRecord(ix->ev_ingest, st));
+    ix->last_add_stream = st;
+    ix->add_recorded = true;
+    return B2F_OK;
+}
+
+// The start of every entry point that works on the index's buffers from stream st: the device must be usable, a search
+// still running on another stream must be done with the workspace (searches return without synchronising), and the
+// latest add must have landed.
+int enter_stream(b2f_index* ix, const DeviceGuard& g, cudaStream_t st) {
+    if (!g.ok) {
+        set_error("cudaSetDevice(%d) failed", ix->device);
+        return B2F_ENOGPU;
+    }
+    if (ix->search_recorded && ix->last_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_done, 0));
+    return wait_ingest(ix, st);
+}
+
 int ensure_capacity(b2f_index* ix, int64_t need) {
     if (need <= ix->cap) return B2F_OK;
     if (need > (int64_t)INT32_MAX - 64) {
@@ -222,11 +312,10 @@ int ensure_capacity(b2f_index* ix, int64_t need) {
     if (ix->ntotal > 0) {
         // an ingest may still be pending on a caller stream (e.g. behind an encoder forward): its rows must have landed
         // before they are copied into the new buffers
-        if (ix->add_recorded && ix->last_add_stream != ix->stream) B2F_CUDA(cudaStreamWaitEvent(ix->stream, ix->ev_ingest, 0));
+        B2F_TRY(wait_ingest(ix, ix->stream));
         if (nrows) B2F_CUDA(cudaMemcpyAsync(nrows, ix->rows_f32, (size_t)ix->ntotal * ix->d * sizeof(float), cudaMemcpyDeviceToDevice, ix->stream));
         B2F_CUDA(cudaMemcpyAsync(nscan, ix->scan, (size_t)ix->ntotal * ix->dpad * sizeof(__nv_bfloat16), cudaMemcpyDeviceToDevice, ix->stream));
         B2F_CUDA(cudaMemcpyAsync(nnorm, ix->norms, (size_t)ix->ntotal * sizeof(float), cudaMemcpyDeviceToDevice, ix->stream));
-        ix->st.launches += 0;
     }
     B2F_CUDA(cudaStreamSynchronize(ix->stream));
     B2F_CUDA(cudaDeviceSynchronize());  // other streams may still be searching the old buffers
@@ -274,22 +363,6 @@ int order_after(cudaStream_t waiter, cudaStream_t producer, b2f_index* ix) {
     }
     B2F_CUDA(cudaEventRecord(e, producer));
     B2F_CUDA(cudaStreamWaitEvent(waiter, e, 0));
-    return B2F_OK;
-}
-
-// Adds are enqueued on the caller's stream (a device-tensor add / add_pooled runs behind the encoder on torch's
-// stream) and return without synchronising.  Everything that reads rows, norms, stats or the centre on ANOTHER
-// stream -- searches, write, reconstruct, the stats refresh, the growth copies -- first waits for the latest add.
-int wait_ingest(b2f_index* ix, cudaStream_t st) {
-    if (ix->add_recorded && ix->last_add_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_ingest, 0));
-    return B2F_OK;
-}
-int record_ingest(b2f_index* ix, cudaStream_t st) {
-    if (!ix->ev_ingest) B2F_CUDA(cudaEventCreateWithFlags(&ix->ev_ingest, cudaEventDisableTiming));
-    // an add on a new stream is ordered behind the previous add (both write stats / may share the workspace)
-    B2F_CUDA(cudaEventRecord(ix->ev_ingest, st));
-    ix->last_add_stream = st;
-    ix->add_recorded = true;
     return B2F_OK;
 }
 
@@ -343,42 +416,7 @@ void harvest_flag(b2f_index* ix) {
     if (hf[4] != s) return;  // a later search is publishing right now: take that one next time
     ix->harvested_seq = s;
     ix->st.last_list_entries = (int64_t)(((uint64_t)(uint32_t)c3 << 32) | (uint32_t)c2);
-    // The slack that certification needs grows with the neighbour density at rank k (i.e. with the database
-    // size and the data distribution): when too many queries of a batch had to fall back, keep more candidates
-    // per query from now on.  "Too many" is where the exact scans cost more than the wider tensor pass would: the
-    // fallback walks the database once per four queries (F / 4 x n d 4 B at ~5.5 TB/s) while the batch's tensor
-    // pass costs 2 nq n d flop at ~1.3 PFLOP/s and grows by < 10 % with 32 more candidates -- break-even at
-    // F ~ nq / 1200; the boost waits for 0.5 % because the range pass below is cheaper still.  (Round 1 waited for 2 % of
-    // the batch: BASELINE config 5 on 2 GPUs spent 9 of its 34 ms per search in exact scans for 0.5 % of the queries.)
-    if (certify && c0 - c1 > (nqb / 200 > 2 ? nqb / 200 : 2) && ix->slack_boost < 224) ix->slack_boost += 32;
-    // Well before that (F > nq / 1000) the range pass takes over: a second TENSOR pass over the uncertified queries with a
-    // fixed threshold per query, one database pass for all of them instead of one exact scan per four (search_locked).
-    // ... unless it does not help: neighbourhoods so dense that the fixed-threshold lists overflow too (thousands of
-    // near-duplicates) leave its queries to the exact scan anyway; two such searches in a row switch it off for a while.
-    if (ix->range_ban > 0) ix->range_ban--;
-    if (ix->range_mode && ix->range_ran_seq == s) {
-        if (2 * c0 > ix->range_ran_nfail) {
-            if (++ix->range_futile >= 2) {
-                ix->range_mode = false;
-                ix->range_futile = 0;
-                ix->range_ban = 256;
-            }
-        } else {
-            ix->range_futile = 0;
-        }
-    }
-    if (certify && c1 > (nqb / 8 > 8 ? nqb / 8 : 8) && ix->heap_left == 0) {
-        ix->heap_left = ix->heap_span;
-        if (ix->heap_span < 4096) ix->heap_span *= 2;
-        if (ix->range_ban == 0) {
-            ix->range_mode = true;   // the heaps find the k' best whatever the row order; dense neighbourhoods still need the range pass
-            ix->range_quiet = 0;
-        }
-    }
-    if (certify && !ix->range_mode && ix->range_ban == 0 && c0 - c1 > (nqb / 1000 > 2 ? nqb / 1000 : 2)) {
-        ix->range_mode = true;
-        ix->range_quiet = 0;
-    }
+    ix->adapt.learn(s, c0, c1, nqb, certify);
 }
 
 void harvest_prof_slot(b2f_index* ix, b2f_index::ProfSlot& sl) {
@@ -593,12 +631,7 @@ int b2f_index_reset(b2f_index* ix) {
     DeviceGuard g(ix->device);
     ix->ntotal = 0;
     ix->mu_set = false;
-    // what earlier searches taught the index about its data goes with the data
-    ix->slack_boost = 0;
-    ix->range_mode = false;
-    ix->range_quiet = ix->range_futile = ix->range_ban = 0;
-    ix->heap_left = 0;
-    ix->heap_span = 64;
+    ix->adapt = {};
     if (ix->search_recorded) B2F_CUDA(cudaEventSynchronize(ix->ev_done));
     if (ix->add_recorded) B2F_CUDA(cudaEventSynchronize(ix->ev_ingest));
     B2F_CUDA(cudaMemsetAsync(ix->stats, 0, 2 * sizeof(float), ix->stream));
@@ -727,16 +760,6 @@ static int take_centre(b2f_index* ix, int64_t n, int64_t piece, cudaStream_t st,
     ix->mu_set = true;
     return B2F_OK;
 }
-}  // extern "C++"
-
-// the first add's rows are all on the device already: one piece
-static int take_centre_device(b2f_index* ix, const float* src_dev, int64_t n, cudaStream_t st) {
-    return take_centre(ix, n, n, st, [&](int64_t r0, int64_t, const float** src) {
-        *src = src_dev + r0 * ix->d;
-        return B2F_OK;
-    });
-}
-
 static int add_device_rows(b2f_index* ix, const float* src_dev, int64_t n, cudaStream_t st) {
     // src_dev: [n, d] fp32 on the device (may alias the tail of rows_f32); the centre is set (take_centre) beforehand
     float* rows_out = nullptr;
@@ -751,6 +774,49 @@ static int add_device_rows(b2f_index* ix, const float* src_dev, int64_t n, cudaS
     return B2F_OK;
 }
 
+// One add call of n rows, on every route.  Rows already on the device (dev) are ingested where they are.  Any other route
+// stages them in pieces of `piece` rows: stage(r0, rows, dst) puts rows [r0, r0 + rows) of the call into dst in stream
+// order -- their final place on fp32 storage (the ingest then derives the scan copy in place), the workspace on bf16
+// storage, whose only copy is the scan copy.  A call that fits one piece is staged once and gives the centre from those
+// rows; a longer one lets take_centre stage the centre's rows first.
+template <class Stage>
+static int ingest_call(b2f_index* ix, int64_t n, int64_t piece, const float* dev, cudaStream_t st, Stage&& stage) {
+    const int64_t base = ix->ntotal;
+    const bool via_ws = !dev && ix->storage == B2F_STORE_BF16;
+    if (via_ws) B2F_TRY(ensure_ws(ix, (size_t)(n < piece ? n : piece) * ix->d * 4 + 4096));
+    auto put = [&](int64_t r0, int64_t rows, const float** src) -> int {
+        if (dev) {
+            *src = dev + r0 * ix->d;
+            return B2F_OK;
+        }
+        float* dst = via_ws ? reinterpret_cast<float*>(ix->ws) : ix->rows_f32 + (base + r0) * ix->d;
+        *src = dst;
+        return stage(r0, rows, dst);
+    };
+    if (piece >= n) {
+        const float* src = nullptr;
+        B2F_TRY(put(0, n, &src));
+        B2F_TRY(take_centre(ix, n, n, st, [&](int64_t r0, int64_t, const float** s) {
+            *s = src + r0 * ix->d;
+            return B2F_OK;
+        }));
+        B2F_TRY(add_device_rows(ix, src, n, st));
+        ix->ntotal += n;
+    } else {
+        B2F_TRY(take_centre(ix, n, piece, st, put));
+        for (int64_t r0 = 0; r0 < n; r0 += piece) {
+            const int64_t rows = n - r0 < piece ? n - r0 : piece;
+            const float* src = nullptr;
+            B2F_TRY(put(r0, rows, &src));
+            B2F_TRY(add_device_rows(ix, src, rows, st));
+            ix->ntotal += rows;
+        }
+    }
+    ix->stats_dirty = true;
+    return record_ingest(ix, st);
+}
+}  // extern "C++"
+
 int b2f_index_add(b2f_index* ix, int64_t n, const float* x, int32_t mem, void* stream) {
     if (!ix || n < 0 || (n > 0 && !x)) {
         set_error("add: bad arguments");
@@ -759,44 +825,17 @@ int b2f_index_add(b2f_index* ix, int64_t n, const float* x, int32_t mem, void* s
     if (n == 0) return B2F_OK;
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
-    if (!g.ok) {
-        set_error("cudaSetDevice(%d) failed", ix->device);
-        return B2F_ENOGPU;
-    }
-    B2F_TRY(ensure_capacity(ix, ix->ntotal + n));
     cudaStream_t st = stream ? (cudaStream_t)stream : ix->stream;
-    if (ix->search_recorded && ix->last_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_done, 0));
-    B2F_TRY(wait_ingest(ix, st));
-    if (mem == B2F_MEM_DEVICE) {
-        B2F_TRY(take_centre_device(ix, x, n, st));
-        B2F_TRY(add_device_rows(ix, x, n, st));
-        ix->ntotal += n;
-    } else if (ix->storage == B2F_STORE_F32) {
-        // host -> final location, then derive the scan copy in place
-        float* dst = ix->rows_f32 + ix->ntotal * ix->d;
-        B2F_CUDA(cudaMemcpyAsync(dst, x, (size_t)n * ix->d * sizeof(float), cudaMemcpyHostToDevice, st));
-        B2F_TRY(take_centre_device(ix, dst, n, st));
-        B2F_TRY(add_device_rows(ix, dst, n, st));
-        ix->ntotal += n;
-    } else {
-        // bf16 storage: stage fp32 chunks through the workspace
-        const int64_t chunk = (64LL << 20) / ((int64_t)ix->d * 4) > 0 ? (64LL << 20) / ((int64_t)ix->d * 4) : 1;
-        B2F_TRY(ensure_ws(ix, (size_t)chunk * ix->d * 4 + 4096));
-        B2F_TRY(take_centre(ix, n, chunk, st, [&](int64_t r0, int64_t m, const float** src) {
-            B2F_CUDA(cudaMemcpyAsync(ix->ws, x + r0 * ix->d, (size_t)m * ix->d * 4, cudaMemcpyHostToDevice, st));
-            *src = reinterpret_cast<const float*>(ix->ws);
-            return B2F_OK;
-        }));
-        for (int64_t r0 = 0; r0 < n; r0 += chunk) {
-            const int64_t m = n - r0 < chunk ? n - r0 : chunk;
-            B2F_CUDA(cudaMemcpyAsync(ix->ws, x + r0 * ix->d, (size_t)m * ix->d * 4, cudaMemcpyHostToDevice, st));
-            B2F_TRY(add_device_rows(ix, reinterpret_cast<const float*>(ix->ws), m, st));
-            ix->ntotal += m;
-        }
-    }
-    ix->stats_dirty = true;
-    B2F_TRY(record_ingest(ix, st));
-    if (mem == B2F_MEM_HOST) B2F_CUDA(cudaStreamSynchronize(st));
+    B2F_TRY(enter_stream(ix, g, st));
+    B2F_TRY(ensure_capacity(ix, ix->ntotal + n));
+    if (mem == B2F_MEM_DEVICE) return ingest_call(ix, n, n, x, st, [](int64_t, int64_t, float*) { return B2F_OK; });
+    // host rows: one copy of all of them on fp32 storage, 64 MB pieces on bf16 storage
+    const int64_t piece = ix->storage == B2F_STORE_F32 ? n : rows_in(64u << 20, ix->d);
+    B2F_TRY(ingest_call(ix, n, piece, nullptr, st, [&](int64_t r0, int64_t m, float* dst) {
+        B2F_CUDA(cudaMemcpyAsync(dst, x + r0 * ix->d, (size_t)m * ix->d * 4, cudaMemcpyHostToDevice, st));
+        return B2F_OK;
+    }));
+    B2F_CUDA(cudaStreamSynchronize(st));
     return B2F_OK;
 }
 
@@ -808,36 +847,15 @@ int b2f_index_add_synth(b2f_index* ix, uint64_t seed, int64_t row0, int64_t nrow
     if (nrows == 0) return B2F_OK;
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
-    B2F_TRY(ensure_capacity(ix, ix->ntotal + nrows));
     cudaStream_t st = ix->stream;
-    if (ix->search_recorded && ix->last_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_done, 0));
-    B2F_TRY(wait_ingest(ix, st));
-    if (ix->storage == B2F_STORE_F32) {
-        float* dst = ix->rows_f32 + ix->ntotal * ix->d;
-        B2F_TRY(launch_synth(seed, row0, nrows, ix->d, normalize, dst, st));
-        B2F_TRY(take_centre_device(ix, dst, nrows, st));
-        B2F_TRY(add_device_rows(ix, dst, nrows, st));
-        ix->ntotal += nrows;
+    B2F_TRY(enter_stream(ix, g, st));
+    B2F_TRY(ensure_capacity(ix, ix->ntotal + nrows));
+    const int64_t piece = ix->storage == B2F_STORE_F32 ? nrows : rows_in(256u << 20, ix->d);
+    B2F_TRY(ingest_call(ix, nrows, piece, nullptr, st, [&](int64_t r0, int64_t m, float* dst) {
+        B2F_TRY(launch_synth(seed, row0 + r0, m, ix->d, normalize, dst, st));
         ix->st.launches++;
-    } else {
-        const int64_t chunk = (256LL << 20) / ((int64_t)ix->d * 4) > 0 ? (256LL << 20) / ((int64_t)ix->d * 4) : 1;
-        B2F_TRY(ensure_ws(ix, (size_t)chunk * ix->d * 4 + 4096));
-        B2F_TRY(take_centre(ix, nrows, chunk, st, [&](int64_t r0, int64_t m, const float** src) {
-            B2F_TRY(launch_synth(seed, row0 + r0, m, ix->d, normalize, reinterpret_cast<float*>(ix->ws), st));
-            ix->st.launches++;
-            *src = reinterpret_cast<const float*>(ix->ws);
-            return B2F_OK;
-        }));
-        for (int64_t r0 = 0; r0 < nrows; r0 += chunk) {
-            const int64_t m = nrows - r0 < chunk ? nrows - r0 : chunk;
-            B2F_TRY(launch_synth(seed, row0 + r0, m, ix->d, normalize, reinterpret_cast<float*>(ix->ws), st));
-            B2F_TRY(add_device_rows(ix, reinterpret_cast<const float*>(ix->ws), m, st));
-            ix->ntotal += m;
-            ix->st.launches++;
-        }
-    }
-    ix->stats_dirty = true;
-    B2F_TRY(record_ingest(ix, st));
+        return B2F_OK;
+    }));
     B2F_CUDA(cudaStreamSynchronize(st));
     return B2F_OK;
 }
@@ -851,45 +869,18 @@ int b2f_index_add_pooled(b2f_index* ix, const float* hidden, const int64_t* mask
     if (B == 0) return B2F_OK;
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
-    B2F_TRY(ensure_capacity(ix, ix->ntotal + B));
     cudaStream_t st = stream ? (cudaStream_t)stream : ix->stream;
-    if (ix->search_recorded && ix->last_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_done, 0));
-    B2F_TRY(wait_ingest(ix, st));
+    B2F_TRY(enter_stream(ix, g, st));
+    B2F_TRY(ensure_capacity(ix, ix->ntotal + B));
     // The pooled rows go through the SAME ingest kernel every other add uses: it derives the scan copy, the per-row
     // bias of the tensor pass (L2: |x~'|^2, IP: -mu.x -- NOT a norm) and the stats for either storage mode and metric.
-    if (ix->storage == B2F_STORE_F32) {
-        // pooled rows land in their final place
-        float* dst = ix->rows_f32 + ix->ntotal * ix->d;
-        B2F_TRY(launch_pool(hidden, mask, B, T, ix->d, pool, normalize, dst, nullptr, 0, nullptr, nullptr, st));
+    const int64_t piece = ix->storage == B2F_STORE_F32 ? B : rows_in(64u << 20, ix->d);
+    return ingest_call(ix, B, piece, nullptr, st, [&](int64_t b0, int64_t m, float* dst) {
+        B2F_TRY(launch_pool(hidden + b0 * T * ix->d, mask ? mask + b0 * T : nullptr, m, T, ix->d, pool, normalize, dst, nullptr, 0,
+                            nullptr, nullptr, st));
         ix->st.launches++;
-        B2F_TRY(take_centre_device(ix, dst, B, st));
-        B2F_TRY(add_device_rows(ix, dst, B, st));
-        ix->ntotal += B;
-    } else {
-        // bf16 storage: pool fp32 chunks into the workspace, ingest from there
-        const int64_t chunk = (64LL << 20) / ((int64_t)ix->d * 4) > 0 ? (64LL << 20) / ((int64_t)ix->d * 4) : 1;
-        B2F_TRY(ensure_ws(ix, (size_t)(B < chunk ? B : chunk) * ix->d * 4 + 4096));
-        B2F_TRY(take_centre(ix, B, chunk, st, [&](int64_t b0, int64_t m, const float** src) {
-            float* tmp = reinterpret_cast<float*>(ix->ws);
-            B2F_TRY(launch_pool(hidden + b0 * T * ix->d, mask ? mask + b0 * T : nullptr, m, T, ix->d, pool, normalize, tmp, nullptr, 0,
-                                nullptr, nullptr, st));
-            ix->st.launches++;
-            *src = tmp;
-            return B2F_OK;
-        }));
-        for (int64_t b0 = 0; b0 < B; b0 += chunk) {
-            const int64_t m = B - b0 < chunk ? B - b0 : chunk;
-            float* tmp = reinterpret_cast<float*>(ix->ws);
-            B2F_TRY(launch_pool(hidden + b0 * T * ix->d, mask ? mask + b0 * T : nullptr, m, T, ix->d, pool, normalize, tmp, nullptr, 0,
-                                nullptr, nullptr, st));
-            ix->st.launches++;
-            B2F_TRY(add_device_rows(ix, tmp, m, st));
-            ix->ntotal += m;
-        }
-    }
-    ix->stats_dirty = true;
-    B2F_TRY(record_ingest(ix, st));
-    return B2F_OK;
+        return B2F_OK;
+    });
 }
 
 int b2f_pool_normalize(const float* hidden, const int64_t* mask, int64_t B, int64_t T, int32_t d, int32_t pool,
@@ -938,6 +929,114 @@ int b2f_merge_topk(int32_t metric, int64_t nq, int64_t k, int32_t nparts, const 
 
 }  // extern "C"
 
+// ---- search workspace ------------------------------------------------------------------------------
+// The query side of one tensor pass: bf16 copy, |q~|^2, e_q and the per-query constant
+struct PassQueries {
+    __nv_bfloat16* qb;
+    float* qnorm;
+    float* qerr;
+    float* qconst;
+};
+static PassQueries take_queries(Bump& b, size_t rows, int64_t dpad) {
+    PassQueries p;
+    p.qb = b.take<__nv_bfloat16>(rows * dpad);
+    p.qnorm = b.take<float>(rows);
+    p.qerr = b.take<float>(rows);
+    p.qconst = b.take<float>(rows);
+    return p;
+}
+
+// LIST-mode scratch of a tensor pass planned as p
+static TensorScanLists take_lists(Bump& b, const TensorScanPlan& p) {
+    const size_t nq_pad = (size_t)p.nq_tiles * 128, words = nq_pad * p.nlists;
+    TensorScanLists l{};
+    l.shared_thr = b.take<float>(words);
+    l.counts = b.take<int32_t>(words);
+    l.final_thr = b.take<float>(words);
+    l.cand = b.take<uint2>(words * p.list_cap);
+    l.big_flag = b.take<uint8_t>(nq_pad);   // warp-merge pass-on flags
+    return l;
+}
+
+// What one search carves from the workspace, in one order.  search_locked carves it over a null base for the size, then
+// over the workspace.
+struct SearchWs {
+    float* q = nullptr;              // host buffers: device copies of the queries and the results
+    float* D = nullptr;
+    int64_t* I = nullptr;
+    void* scan_scratch = nullptr;
+    PassQueries pq{};                // tensor path from here on
+    TensorScanLists lists{};         // LIST mode
+    float* pk = nullptr;             // HEAP mode: partial lists, merged coarse candidates
+    int32_t* pi = nullptr;
+    float* ck = nullptr;
+    int32_t* ci = nullptr;
+    int32_t* fail_list = nullptr;
+    float* fail_tau = nullptr;       // range mode
+    // [0] uncertified queries, [1] of which list overflows, [2..3] u64 list entries, [4] rescued by the extended pass,
+    // [8..11] ticket counters of K2's die-aware unit assignment
+    int32_t* counters = nullptr;
+};
+
+static SearchWs carve_search(Bump& b, const b2f_index* ix, int nq, int k, bool host, bool tensor, const TensorScanPlan& plan,
+                             int chunk_nq, int kp) {
+    SearchWs w;
+    if (host) {
+        w.q = b.take<float>((size_t)nq * ix->d);
+        w.D = b.take<float>((size_t)nq * k);
+        w.I = b.take<int64_t>((size_t)nq * k);
+    }
+    w.scan_scratch = b.take<char>(scan_scratch_bytes(k));
+    if (!tensor) return w;
+    const size_t nq_pad = (size_t)plan.nq_tiles * 128;
+    w.pq = take_queries(b, nq_pad, ix->dpad);
+    if (plan.list_mode) {
+        w.lists = take_lists(b, plan);
+    } else {
+        w.pk = b.take<float>(nq_pad * plan.nsplits * kp);
+        w.pi = b.take<int32_t>(nq_pad * plan.nsplits * kp);
+        w.ck = b.take<float>((size_t)chunk_nq * kp);
+        w.ci = b.take<int32_t>((size_t)chunk_nq * kp);
+    }
+    w.fail_list = b.take<int32_t>(nq);
+    if (ix->adapt.range_mode) w.fail_tau = b.take<float>(nq);
+    w.counters = b.take<int32_t>(16);
+    w.lists.die_ctr = w.counters + 8;
+    return w;
+}
+
+// The re-rank of one tensor pass over the nq queries q (pq: their tensor-pass buffers): results go to D / I in faiss
+// layout, the queries it cannot certify to fail_list / fail_count
+static RerankArgs rerank_args(const b2f_index* ix, const float* q, const PassQueries& pq, int nq, int k, int kp, float* D,
+                              int64_t* I, int64_t id_offset, int32_t* fail_list, int32_t* fail_count) {
+    RerankArgs a{};
+    a.rows_f32 = ix->storage == B2F_STORE_F32 ? ix->rows_f32 : nullptr;
+    a.rows_bf16 = ix->scan;
+    a.pitch_bf16 = ix->dpad;
+    a.centre = (ix->storage == B2F_STORE_BF16 && ix->mu_set) ? ix->centre : nullptr;
+    a.q = q;
+    a.qnorm = pq.qnorm;
+    a.qerr = pq.qerr;
+    a.qconst = pq.qconst;
+    a.mu_norm = ix->mu_norm;
+    a.nq = nq;
+    a.kp = kp;
+    a.k = k;
+    a.d = ix->d;
+    a.metric = ix->metric;
+    a.ntotal = ix->ntotal;
+    a.max_row_norm = sqrtf(ix->host_stats[0]);
+    // fp32 storage: the bf16 rounding of the centred row; bf16 storage: what fl32(mu + x~') loses (0 uncentred)
+    a.max_row_err = sqrtf(ix->host_stats[1]);
+    a.certify = 1;
+    a.D = D;
+    a.I = I;
+    a.id_offset = id_offset;
+    a.fail_list = fail_list;
+    a.fail_count = fail_count;
+    return a;
+}
+
 // ---- range pass (second tensor pass over uncertified queries) -----------------------------------------
 constexpr int kRangeCap = 1024;   // failed queries one range pass holds; more go to the exact scan
 constexpr int kRangeListCap = 256;
@@ -947,19 +1046,94 @@ static int plan_range_pass(int nfail, int64_t n, int d, int kp, TensorScanPlan* 
     if (plan->list_cap < kRangeListCap) plan->list_cap = kRangeListCap;   // lists are not pruned: every row at or below the threshold
     return B2F_OK;
 }
-static size_t range_lists_bytes(const TensorScanPlan& p) {
-    const size_t nq_pad = (size_t)p.nq_tiles * 128;
-    return 3 * align_up(nq_pad * p.nlists * 4, 256) + align_up(nq_pad * p.nlists * (size_t)p.list_cap * 8, 256) + align_up(nq_pad, 256);
+
+// What a range pass carves behind the search's own buffers: its queries hold kRangeCap rows whatever the failed count,
+// its lists follow its plan
+struct RangeWs {
+    float* q;                        // the failed queries, gathered
+    PassQueries pq;
+    float* tau;
+    float* thr;
+    int32_t* out_map;
+    int32_t* fail_list;
+    int32_t* counters;               // [0..7] as SearchWs::counters, [8..11] K2's tickets, [16] compacted queries
+    TensorScanLists lists;
+};
+
+static RangeWs carve_range(Bump& b, const b2f_index* ix, int nq, const TensorScanPlan& rp) {
+    RangeWs r;
+    r.q = b.take<float>((size_t)kRangeCap * ix->d);
+    r.pq = take_queries(b, kRangeCap, ix->dpad);
+    r.tau = b.take<float>(kRangeCap);
+    r.thr = b.take<float>(kRangeCap);
+    r.out_map = b.take<int32_t>(kRangeCap);
+    r.fail_list = b.take<int32_t>(nq);
+    r.counters = b.take<int32_t>(32);
+    r.lists = take_lists(b, rp);
+    r.lists.die_ctr = r.counters + 8;
+    r.lists.range_thr = r.thr;
+    return r;
 }
-static size_t range_pass_bytes(const b2f_index* ix, int nq, int kp) {
-    size_t lists = 0;
-    for (int f = 128; f <= kRangeCap; f *= 2) {   // the list geometry depends on the number of failed queries: take the largest
+
+// Where a range pass carved behind `search` ends at most.  The list geometry depends on the number of failed queries,
+// known only after the host sync: take the largest over 128..kRangeCap of them.
+static size_t range_end(const Bump& search, const b2f_index* ix, int nq, int kp) {
+    size_t end = search.off;
+    for (int f = 128; f <= kRangeCap; f *= 2) {
         TensorScanPlan p{};
-        if (plan_range_pass(f, ix->ntotal, ix->d, kp, &p) == B2F_OK && range_lists_bytes(p) > lists) lists = range_lists_bytes(p);
+        if (plan_range_pass(f, ix->ntotal, ix->d, kp, &p) != B2F_OK) continue;
+        Bump b = search;
+        carve_range(b, ix, nq, p);
+        if (b.off > end) end = b.off;
     }
-    const size_t cap = kRangeCap;
-    return align_up(cap * ix->d * 4, 256) + align_up(cap * ix->dpad * 2, 256) + 7 * align_up(cap * 4, 256) +
-           2 * align_up((size_t)nq * 4, 256) + 8192 + lists;
+    return end;
+}
+
+// Range pass.  Earlier batches on this index left many queries uncertified (data denser than the bf16 band even after
+// centring): instead of one exact scan per four of them, ONE more tensor pass serves them all.  For a failed query the
+// first pass found an exact k-th key tau, an upper bound of the true one; every true top-k row therefore has a coarse key
+// <= thr(tau) (the certification bound, inverted), so a pass that lists EVERY row at or below that fixed threshold and
+// re-ranks all of them is exact.  The host must know how many queries failed to plan the pass: the one synchronisation
+// inside a search, paid only by indexes in this mode.
+// *served: the queries the pass served (0: it did not run); *scan_list / *scan_counters: what the closing scan reads.
+static int range_pass(b2f_index* ix, Bump& bump, const SearchWs& w, const float* q, int nq, int k, int kp, float* D, int64_t* I,
+                      int64_t id_offset, cudaStream_t st, int32_t** scan_list, int32_t** scan_counters, int* served) {
+    volatile int32_t* hf = ix->host_flag + 12;
+    B2F_CUDA(cudaMemcpyAsync(const_cast<int32_t*>(hf), w.counters, 4, cudaMemcpyDeviceToHost, st));
+    B2F_CUDA(cudaStreamSynchronize(st));
+    const int nfail = hf[0];
+    ix->adapt.first_pass_failed(nfail);
+    TensorScanPlan rp{};
+    const int nr = nfail < kRangeCap ? nfail : kRangeCap;
+    if (nfail < 8 || plan_range_pass(nr, ix->ntotal, ix->d, kp, &rp) != B2F_OK) return B2F_OK;
+    const RangeWs r = carve_range(bump, ix, nq, rp);
+    if (!bump.fits()) return B2F_OK;   // a layout the workspace was not sized for: the exact scan serves these queries
+    const int nq_pad = rp.nq_tiles * 128;
+    B2F_CUDA(cudaMemsetAsync(r.counters, 0, 32 * 4, st));
+    B2F_CUDA(cudaMemsetAsync(r.out_map, 0xff, (size_t)kRangeCap * 4, st));
+    B2F_CUDA(cudaMemsetAsync(r.q, 0, (size_t)nq_pad * ix->d * 4, st));
+    B2F_TRY(launch_gather_failed(q, ix->d, w.fail_list, w.fail_tau, w.counters, nfail, nr, r.q, r.tau, r.out_map, r.counters + 16,
+                                 r.fail_list, r.counters, st));
+    B2F_TRY(launch_prep_queries(r.q, nr, nq_pad, ix->d, r.pq.qb, ix->dpad, r.pq.qnorm, r.pq.qerr, r.pq.qconst,
+                                ix->mu_set ? ix->centre : nullptr, nullptr, 0, reinterpret_cast<uint32_t*>(r.lists.shared_thr),
+                                (int64_t)nq_pad * rp.nlists, st));
+    B2F_TRY(launch_range_thresholds(r.tau, r.out_map, nr, ix->d, ix->metric, r.pq.qnorm, r.pq.qerr, r.pq.qconst,
+                                    sqrtf(ix->host_stats[0]), sqrtf(ix->host_stats[1]), ix->mu_norm, r.thr, st));
+    B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, r.pq.qb, nr, nq_pad, rp, nullptr, nullptr,
+                               r.lists, st));
+    RerankArgs ra = rerank_args(ix, r.q, r.pq, nr, k, kp, D, I, id_offset, r.fail_list, r.counters);
+    ra.out_map = r.out_map;
+    ra.range = 1;
+    B2F_TRY(launch_merge_lists(r.lists, nr, rp, nullptr, ra, st));
+    // the statistics the closing kernel publishes: what the first pass counted, with the final fallback count
+    B2F_CUDA(cudaMemcpyAsync(r.counters + 1, w.counters + 1, 7 * 4, cudaMemcpyDeviceToDevice, st));
+    ix->st.launches += 5;
+    ix->st.last_launches += 5;
+    ix->st.range_queries += nr;
+    *served = nr;
+    *scan_list = r.fail_list;
+    *scan_counters = r.counters;
+    return B2F_OK;
 }
 
 // ---- search ----------------------------------------------------------------------------------------
@@ -984,19 +1158,14 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
     b2f_search_params P{};
     if (params) P = *params;
     DeviceGuard g(ix->device);
-    if (!g.ok) {
-        set_error("cudaSetDevice(%d) failed", ix->device);
-        return B2F_ENOGPU;
-    }
     cudaStream_t st = stream ? (cudaStream_t)stream : ix->stream;
+    B2F_TRY(enter_stream(ix, g, st));
     B2F_TRY(order_after(st, ix->stream, ix));
-    B2F_TRY(wait_ingest(ix, st));   // the latest add may sit on another stream (torch's, behind an encoder forward)
-    // searches return without synchronising: a search on another stream must not reuse the workspace early
-    if (ix->search_recorded && ix->last_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_done, 0));
     const bool host = mem == B2F_MEM_HOST;
     const bool profile = P.profile != 0;
     harvest_flag(ix);
 
+    // ---- plan ----------------------------------------------------------------------------------
     int algo = P.algo;
     // AUTO: fp32 storage serves the reference's own batch size (nq = 1) with the fp32 streaming scan -- the
     // reference's arithmetic, 90% of HBM on the fp32 rows.  bf16 storage has nothing to gain from it (both paths
@@ -1014,12 +1183,12 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
         }
         if (kp_env >= k + 2 && kp > 0) kp = kp_env;
     }
-    if (kp > 0 && P.slack <= 0 && ix->slack_boost > 0) {  // adaptive slack learned from earlier searches on this index
-        int boosted = ((kp + ix->slack_boost + 7) / 8) * 8;
+    if (kp > 0 && P.slack <= 0 && ix->adapt.slack_boost > 0) {  // adaptive slack learned from earlier searches on this index
+        int boosted = ((kp + ix->adapt.slack_boost + 7) / 8) * 8;
         if (boosted > 64) kp = boosted <= 256 ? boosted : 256;
     }
     TensorScanPlan plan{};
-    const bool heap_first = ix->heap_left > 0 && P.certify >= 0;
+    const bool heap_first = ix->adapt.heap_left > 0 && P.certify >= 0;
     plan_force_heap(heap_first);
     const int chunk_nq = (kp > 0 && ix->ntotal > 0) ? plan_tensor_chunked(nq, ix->ntotal, ix->d, kp, &plan) : 0;
     plan_force_heap(false);
@@ -1028,41 +1197,24 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
     // an explicit TENSOR request on a shape the tensor path cannot plan (k' > 256, or a database of a few rows with
     // k' other than 32 / 64) is served by the exact scan, like AUTO would; stats().last_algo tells
     if (algo == B2F_ALGO_TENSOR && !tensor_ok) algo = B2F_ALGO_SCAN;
+    const bool tensor = algo == B2F_ALGO_TENSOR;
     const int certify = P.certify >= 0 ? 1 : 0;
-    if (algo == B2F_ALGO_TENSOR && heap_first) ix->heap_left--;
+    if (tensor && heap_first) ix->adapt.heap_left--;
 
     // ---- workspace -----------------------------------------------------------------------------
-    size_t need = 8192;
-    if (host) need += align_up((size_t)nq * ix->d * 4, 256) + align_up((size_t)nq * k * 4, 256) + align_up((size_t)nq * k * 8, 256);
-    need += align_up(scan_scratch_bytes(k), 256) + 256;
-    if (algo == B2F_ALGO_TENSOR) {
-        const size_t nq_pad = (size_t)plan.nq_tiles * 128;
-        need += align_up(nq_pad * ix->dpad * 2, 256) + 3 * align_up(nq_pad * 4, 256);
-        if (plan.list_mode) {
-            need += align_up(nq_pad * plan.nlists * 4, 256) * 3;                       // shared thresholds + counts + final thresholds
-            need += align_up(nq_pad * plan.nlists * (size_t)plan.list_cap * 8, 256);   // candidate lists
-            need += align_up(nq_pad, 256);                                              // warp-merge pass-on flags
-        } else {
-            need += 2 * align_up(nq_pad * plan.nsplits * kp * 4, 256);  // partial lists
-            need += 2 * align_up((size_t)chunk_nq * kp * 4, 256);       // merged coarse
-        }
-        need += align_up((size_t)nq * 4, 256) + 256;                    // fail list + counters
-        if (ix->range_mode) need += range_pass_bytes(ix, nq, kp);
+    Bump layout(nullptr, SIZE_MAX);
+    carve_search(layout, ix, nq, k, host, tensor, plan, chunk_nq, kp);
+    B2F_TRY(ensure_ws(ix, tensor && ix->adapt.range_mode ? range_end(layout, ix, nq, kp) : layout.off));
+    Bump bump(ix->ws, ix->ws_bytes);
+    const SearchWs w = carve_search(bump, ix, nq, k, host, tensor, plan, chunk_nq, kp);
+    if (!bump.fits()) {
+        set_error("search workspace: the layout needs %zu bytes, the workspace has %zu", bump.off, bump.size);
+        return B2F_ECUDA;
     }
-    B2F_TRY(ensure_ws(ix, need));
-    Bump bump(ix->ws);
-
-    const float* qd = q;
-    float* Dd = D;
-    int64_t* Id = I;
-    if (host) {
-        float* qbuf = bump.take<float>((size_t)nq * ix->d);
-        Dd = bump.take<float>((size_t)nq * k);
-        Id = bump.take<int64_t>((size_t)nq * k);
-        B2F_CUDA(cudaMemcpyAsync(qbuf, q, (size_t)nq * ix->d * 4, cudaMemcpyHostToDevice, st));
-        qd = qbuf;
-    }
-    void* scan_scratch = bump.take<char>(scan_scratch_bytes(k));
+    const float* qd = host ? w.q : q;
+    float* Dd = host ? w.D : D;
+    int64_t* Id = host ? w.I : I;
+    if (host) B2F_CUDA(cudaMemcpyAsync(w.q, q, (size_t)nq * ix->d * 4, cudaMemcpyHostToDevice, st));
     ix->st.searches++;
     ix->st.last_launches = 0;
     ix->st.last_algo = algo;
@@ -1092,81 +1244,35 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
         B2F_TRY(launch_finalize(nullptr, nullptr, nq, 0, k, ix->metric, P.id_offset, nullptr, Dd, Id, st));
         ix->st.launches++;
         ix->st.last_launches++;
-    } else if (algo == B2F_ALGO_SCAN) {
+    } else if (!tensor) {
         B2F_TRY(main_event(0));
-        B2F_TRY(enqueue_scan(ix, qd, nullptr, nullptr, nq, k, Dd, Id, P.id_offset, scan_scratch, nullptr, 0, nq, 0, st));
+        B2F_TRY(enqueue_scan(ix, qd, nullptr, nullptr, nq, k, Dd, Id, P.id_offset, w.scan_scratch, nullptr, 0, nq, 0, st));
         B2F_TRY(main_event(1));
         n_main++;
     } else {
         const int nq_pad = plan.nq_tiles * 128;
         ix->st.last_kprime = kp;
-        __nv_bfloat16* qb = bump.take<__nv_bfloat16>((size_t)nq_pad * ix->dpad);
-        float* qnorm = bump.take<float>(nq_pad);
-        float* qerr = bump.take<float>(nq_pad);
-        float* qconst = bump.take<float>(nq_pad);
-        float* pk = nullptr;
-        int32_t* pi = nullptr;
-        float* ck = nullptr;
-        int32_t* ci = nullptr;
-        TensorScanLists lists{};
-        if (plan.list_mode) {
-            lists.shared_thr = bump.take<float>((size_t)nq_pad * plan.nlists);
-            lists.counts = bump.take<int32_t>((size_t)nq_pad * plan.nlists);
-            lists.final_thr = bump.take<float>((size_t)nq_pad * plan.nlists);
-            lists.cand = bump.take<uint2>((size_t)nq_pad * plan.nlists * plan.list_cap);
-            lists.big_flag = bump.take<uint8_t>((size_t)nq_pad);
-        } else {
-            pk = bump.take<float>((size_t)nq_pad * plan.nsplits * kp);
-            pi = bump.take<int32_t>((size_t)nq_pad * plan.nsplits * kp);
-            ck = bump.take<float>((size_t)chunk_nq * kp);
-            ci = bump.take<int32_t>((size_t)chunk_nq * kp);
-        }
-        int32_t* fail_list = bump.take<int32_t>(nq);
-        float* fail_tau = ix->range_mode ? bump.take<float>(nq) : nullptr;
-        // [0] uncertified queries, [1] of which list overflows, [2..3] u64 list entries, [4] rescued by the extended pass
-        int32_t* counters = bump.take<int32_t>(16);   // [8..11]: ticket counters of K2's die-aware unit assignment
-        lists.die_ctr = counters + 8;
         B2F_TRY(refresh_host_stats(ix, st));
         for (int c0 = 0; c0 < nq; c0 += chunk_nq) {
             const int cn = nq - c0 < chunk_nq ? nq - c0 : chunk_nq;  // queries in this pass (the plan covers chunk_nq)
             const float* qc = qd + (int64_t)c0 * ix->d;
             // one launch: bf16 copy / norms of the queries, reset the shared thresholds, clear the counters (first pass)
-            B2F_TRY(launch_prep_queries(qc, cn, nq_pad, ix->d, qb, ix->dpad, qnorm, qerr, qconst, ix->mu_set ? ix->centre : nullptr,
-                                        reinterpret_cast<uint32_t*>(counters),
-                                        c0 == 0 ? 16 : 0, reinterpret_cast<uint32_t*>(lists.shared_thr),
+            B2F_TRY(launch_prep_queries(qc, cn, nq_pad, ix->d, w.pq.qb, ix->dpad, w.pq.qnorm, w.pq.qerr, w.pq.qconst,
+                                        ix->mu_set ? ix->centre : nullptr, reinterpret_cast<uint32_t*>(w.counters),
+                                        c0 == 0 ? 16 : 0, reinterpret_cast<uint32_t*>(w.lists.shared_thr),
                                         plan.list_mode ? (int64_t)nq_pad * plan.nlists : 0, st));
             B2F_TRY(main_event(0));
-            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, qb, cn, nq_pad, plan, pk, pi, lists, st));
+            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, w.pq.qb, cn, nq_pad, plan, w.pk, w.pi,
+                                       w.lists, st));
             B2F_TRY(main_event(1));
             n_main++;
-            RerankArgs ra{};
-            ra.rows_f32 = ix->storage == B2F_STORE_F32 ? ix->rows_f32 : nullptr;
-            ra.rows_bf16 = ix->scan;
-            ra.pitch_bf16 = ix->dpad;
-            ra.centre = (ix->storage == B2F_STORE_BF16 && ix->mu_set) ? ix->centre : nullptr;
-            ra.q = qc;
-            ra.qnorm = qnorm;
-            ra.qerr = qerr;
-            ra.qconst = qconst;
-            ra.mu_norm = ix->mu_norm;
-            ra.cand_key = ck;
-            ra.cand_id = ci;
-            ra.nq = cn;
-            ra.kp = kp;
-            ra.k = k;
-            ra.d = ix->d;
-            ra.metric = ix->metric;
-            ra.ntotal = ix->ntotal;
-            ra.max_row_norm = sqrtf(ix->host_stats[0]);
-            // fp32 storage: the bf16 rounding of the centred row; bf16 storage: what fl32(mu + x~') loses (0 uncentred)
-            ra.max_row_err = sqrtf(ix->host_stats[1]);
+            // the re-rank writes faiss-formatted results directly (no finalize launch)
+            RerankArgs ra = rerank_args(ix, qc, w.pq, cn, k, kp, Dd + (int64_t)c0 * k, Id + (int64_t)c0 * k, P.id_offset,
+                                        w.fail_list, w.counters);
+            ra.cand_key = w.ck;
+            ra.cand_id = w.ci;
             ra.certify = certify;
-            ra.D = Dd + (int64_t)c0 * k;  // the re-rank writes faiss-formatted results directly (no finalize launch)
-            ra.I = Id + (int64_t)c0 * k;
-            ra.id_offset = P.id_offset;
-            ra.fail_list = fail_list;
-            ra.fail_tau = fail_tau;
-            ra.fail_count = counters;
+            ra.fail_tau = w.fail_tau;
             ra.q_base = c0;
             {   // First-stage re-rank (the best n candidates alone before the k' best): OFF.  Same-box A/B (r02n): no gain at
                 // 4096 / 8192 queries with k = 10 (the merge is not bound by the candidate row reads after all), and a loss
@@ -1180,112 +1286,29 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
             }
             if (plan.list_mode) {
                 // K3b + K4 + finalize fused: per query, merge the lists, re-rank exactly, certify, write (D, I)
-                B2F_TRY(launch_merge_lists(lists, cn, plan, reinterpret_cast<unsigned long long*>(counters + 2), ra, st));
+                B2F_TRY(launch_merge_lists(w.lists, cn, plan, reinterpret_cast<unsigned long long*>(w.counters + 2), ra, st));
                 ix->st.launches += 3;
                 ix->st.last_launches += 3;
             } else {
-                B2F_TRY(launch_merge_parts(pk, pi, cn, plan.nsplits, kp, kp, ck, ci, st));
+                B2F_TRY(launch_merge_parts(w.pk, w.pi, cn, plan.nsplits, kp, kp, w.ck, w.ci, st));
                 B2F_TRY(launch_rerank(ra, st));
                 ix->st.launches += 4;
                 ix->st.last_launches += 4;
             }
         }  // query chunks
-        int32_t* scan_list = fail_list;
-        int32_t* scan_counters = counters;
+        int32_t* scan_list = w.fail_list;
+        int32_t* scan_counters = w.counters;
         int range_served = 0;
-        if (ix->range_mode && certify && fail_tau) {
-            // Range pass.  Earlier batches on this index left many queries uncertified (data denser than the bf16 band even
-            // after centring): instead of one exact scan per four of them, ONE more tensor pass serves them all.  For a
-            // failed query the first pass found an exact k-th key tau, an upper bound of the true one; every true top-k row
-            // therefore has a coarse key <= thr(tau) (the certification bound, inverted), so a pass that lists EVERY row at
-            // or below that fixed threshold and re-ranks all of them is exact.  The host must know how many queries failed
-            // to plan the pass: the one synchronisation inside a search, paid only by indexes in this mode.
-            volatile int32_t* hf = ix->host_flag + 12;
-            B2F_CUDA(cudaMemcpyAsync(const_cast<int32_t*>(hf), counters, 4, cudaMemcpyDeviceToHost, st));
-            B2F_CUDA(cudaStreamSynchronize(st));
-            const int nfail = hf[0];
-            if (nfail == 0) {
-                if (++ix->range_quiet >= 8) ix->range_mode = false;   // the data (or the adaptive slack) no longer needs it
-            } else {
-                ix->range_quiet = 0;
-            }
-            TensorScanPlan rp{};
-            const int nr = nfail < kRangeCap ? nfail : kRangeCap;
-            if (nfail >= 8 && plan_range_pass(nr, ix->ntotal, ix->d, kp, &rp) == B2F_OK) {
-                const int nq_pad2 = rp.nq_tiles * 128;
-                float* qf = bump.take<float>((size_t)kRangeCap * ix->d);
-                __nv_bfloat16* qb2 = bump.take<__nv_bfloat16>((size_t)kRangeCap * ix->dpad);
-                float* qnorm2 = bump.take<float>(kRangeCap);
-                float* qerr2 = bump.take<float>(kRangeCap);
-                float* qconst2 = bump.take<float>(kRangeCap);
-                float* tau2 = bump.take<float>(kRangeCap);
-                float* thr2 = bump.take<float>(kRangeCap);
-                int32_t* out_map = bump.take<int32_t>(kRangeCap);
-                int32_t* fail_list2 = bump.take<int32_t>(nq);
-                int32_t* counters_b = bump.take<int32_t>(32);   // [0..7] as `counters`, [8..11] K2's tickets, [16] compacted queries
-                TensorScanLists l2{};
-                l2.shared_thr = bump.take<float>((size_t)nq_pad2 * rp.nlists);
-                l2.counts = bump.take<int32_t>((size_t)nq_pad2 * rp.nlists);
-                l2.final_thr = bump.take<float>((size_t)nq_pad2 * rp.nlists);
-                l2.cand = bump.take<uint2>((size_t)nq_pad2 * rp.nlists * rp.list_cap);
-                l2.big_flag = bump.take<uint8_t>((size_t)nq_pad2);
-                l2.die_ctr = counters_b + 8;
-                l2.range_thr = thr2;
-                B2F_CUDA(cudaMemsetAsync(counters_b, 0, 32 * 4, st));
-                B2F_CUDA(cudaMemsetAsync(out_map, 0xff, (size_t)kRangeCap * 4, st));
-                B2F_CUDA(cudaMemsetAsync(qf, 0, (size_t)nq_pad2 * ix->d * 4, st));
-                B2F_TRY(launch_gather_failed(qd, ix->d, fail_list, fail_tau, counters, nfail, nr, qf, tau2, out_map, counters_b + 16,
-                                             fail_list2, counters_b, st));
-                B2F_TRY(launch_prep_queries(qf, nr, nq_pad2, ix->d, qb2, ix->dpad, qnorm2, qerr2, qconst2, ix->mu_set ? ix->centre : nullptr,
-                                            nullptr, 0, reinterpret_cast<uint32_t*>(l2.shared_thr), (int64_t)nq_pad2 * rp.nlists, st));
-                B2F_TRY(launch_range_thresholds(tau2, out_map, nr, ix->d, ix->metric, qnorm2, qerr2, qconst2, sqrtf(ix->host_stats[0]),
-                                                sqrtf(ix->host_stats[1]), ix->mu_norm, thr2, st));
-                B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, qb2, nr, nq_pad2, rp, nullptr, nullptr, l2, st));
-                RerankArgs r2{};
-                r2.rows_f32 = ix->storage == B2F_STORE_F32 ? ix->rows_f32 : nullptr;
-                r2.rows_bf16 = ix->scan;
-                r2.pitch_bf16 = ix->dpad;
-                r2.centre = (ix->storage == B2F_STORE_BF16 && ix->mu_set) ? ix->centre : nullptr;
-                r2.q = qf;
-                r2.qnorm = qnorm2;
-                r2.qerr = qerr2;
-                r2.qconst = qconst2;
-                r2.mu_norm = ix->mu_norm;
-                r2.nq = nr;
-                r2.kp = kp;
-                r2.k = k;
-                r2.d = ix->d;
-                r2.metric = ix->metric;
-                r2.ntotal = ix->ntotal;
-                r2.max_row_norm = sqrtf(ix->host_stats[0]);
-                r2.max_row_err = sqrtf(ix->host_stats[1]);
-                r2.certify = 1;
-                r2.D = Dd;
-                r2.I = Id;
-                r2.id_offset = P.id_offset;
-                r2.fail_list = fail_list2;
-                r2.fail_count = counters_b;
-                r2.out_map = out_map;
-                r2.range = 1;
-                B2F_TRY(launch_merge_lists(l2, nr, rp, nullptr, r2, st));
-                // the statistics the closing kernel publishes: what the first pass counted, with the final fallback count
-                B2F_CUDA(cudaMemcpyAsync(counters_b + 1, counters + 1, 7 * 4, cudaMemcpyDeviceToDevice, st));
-                ix->st.launches += 5;
-                ix->st.last_launches += 5;
-                ix->st.range_queries += nr;
-                range_served = nr;
-                scan_list = fail_list2;
-                scan_counters = counters_b;
-            }
-        }
+        if (ix->adapt.range_mode && certify && w.fail_tau)
+            B2F_TRY(range_pass(ix, bump, w, qd, nq, k, kp, Dd, Id, P.id_offset, st, &scan_list, &scan_counters, &range_served));
         // Closing kernel: the exact scan over the queries that could not be certified.  The count lives on the
         // device -- with none (the usual case) the kernel publishes the counters and exits -- so the host never
         // waits inside a search and consecutive searches run back to back on the GPU.
-        B2F_TRY(enqueue_scan(ix, qd, scan_list, scan_counters, 0, k, Dd, Id, P.id_offset, scan_scratch, scan_counters, ++ix->seq, nq,
+        B2F_TRY(enqueue_scan(ix, qd, scan_list, scan_counters, 0, k, Dd, Id, P.id_offset, w.scan_scratch, scan_counters, ++ix->seq, nq,
                              certify, st));
         if (range_served) {
-            ix->range_ran_seq = ix->seq;
-            ix->range_ran_nfail = range_served;
+            ix->adapt.range_ran_seq = ix->seq;
+            ix->adapt.range_ran_nfail = range_served;
         }
     }
     if (slot) {
@@ -1331,10 +1354,8 @@ int b2f_index_search_pooled(b2f_index* ix, const float* hidden, const int64_t* m
     std::lock_guard<std::mutex> lk(ix->mu);   // held across pooling AND the search: the pooled queries live in ix->qpool
     {
         DeviceGuard g(ix->device);
-        if (!g.ok) {
-            set_error("cudaSetDevice(%d) failed", ix->device);
-            return B2F_ENOGPU;
-        }
+        cudaStream_t st = stream ? (cudaStream_t)stream : ix->stream;
+        B2F_TRY(enter_stream(ix, g, st));
         // pooled queries live in their own grow-only buffer (the search below carves the workspace itself)
         const size_t need = (size_t)B * ix->d * sizeof(float);
         if (need > ix->qpool_bytes) {
@@ -1350,8 +1371,6 @@ int b2f_index_search_pooled(b2f_index* ix, const float* hidden, const int64_t* m
             ix->qpool_bytes = need + (need >> 2);
         }
         qbuf = ix->qpool;
-        cudaStream_t st = stream ? (cudaStream_t)stream : ix->stream;
-        if (ix->search_recorded && ix->last_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_done, 0));
         B2F_TRY(launch_pool(hidden, mask, B, T, ix->d, pool, normalize, qbuf, nullptr, 0, nullptr, nullptr, st));
         ix->st.launches++;
     }
@@ -1371,9 +1390,8 @@ int b2f_index_reconstruct(b2f_index* ix, int64_t i0, int64_t n, float* out, int3
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
     cudaStream_t st = stream ? (cudaStream_t)stream : ix->stream;
+    B2F_TRY(enter_stream(ix, g, st));
     B2F_TRY(order_after(st, ix->stream, ix));
-    B2F_TRY(wait_ingest(ix, st));
-    if (ix->search_recorded && ix->last_stream != st) B2F_CUDA(cudaStreamWaitEvent(st, ix->ev_done, 0));  // shares the workspace
     const size_t bytes = (size_t)n * ix->d * 4;
     if (ix->storage == B2F_STORE_F32) {
         B2F_CUDA(cudaMemcpyAsync(out, ix->rows_f32 + i0 * ix->d, bytes, mem == B2F_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
@@ -1400,8 +1418,7 @@ int b2f_index_write(b2f_index* ix, const char* path) {
     }
     std::lock_guard<std::mutex> lk(ix->mu);
     DeviceGuard g(ix->device);
-    B2F_TRY(wait_ingest(ix, ix->stream));
-    if (ix->search_recorded && ix->last_stream != ix->stream) B2F_CUDA(cudaStreamWaitEvent(ix->stream, ix->ev_done, 0));
+    B2F_TRY(enter_stream(ix, g, ix->stream));
     FILE* f = fopen(path, "wb");
     if (!f) {
         set_error("could not open %s for writing", path);
@@ -1517,75 +1534,32 @@ int b2f_index_read(const char* path, int32_t storage, int32_t device, b2f_index*
     {
         DeviceGuard g(device);
         rc = ensure_capacity(ix, nt);
-        const int64_t rows_per = (int64_t)(kIoChunk / ((size_t)d32 * 4)) > 0 ? (int64_t)(kIoChunk / ((size_t)d32 * 4)) : 1;
-        const size_t cbytes = (size_t)rows_per * d32 * 4;
+        const int64_t piece = rows_in(kIoChunk, d32);
+        const size_t cbytes = (size_t)piece * d32 * 4;
         if (rc == B2F_OK && nt > 0) rc = ensure_pinned(ix, 2 * cbytes);
-        if (rc == B2F_OK && nt > 0 && storage == B2F_STORE_BF16) rc = ensure_ws(ix, 2 * cbytes + 4096);
-        // the centre of an index read from a file is the mean of the file's first rows, as if they were added: read
-        // them for the mean first (through pinned slot 0), then start over at the first row
+        // The rows are ingested as one add of nt rows, through two pinned slots: the fread of a piece overlaps the H2D and
+        // ingest of the one before.  The centre's rows are read once more first (take_centre), so every piece seeks to its rows.
         const long payload = ftell(f);
+        cudaEvent_t evs[2] = {get_event(ix, 1), get_event(ix, 2)};
+        int64_t pieces = 0;
         if (rc == B2F_OK && nt > 0)
-            rc = take_centre(ix, nt, rows_per, ix->stream, [&](int64_t r0, int64_t m, const float** src) {
-                B2F_CUDA(cudaStreamSynchronize(ix->stream));   // the pinned slot may still be in flight
+            rc = ingest_call(ix, nt, piece, nullptr, ix->stream, [&](int64_t r0, int64_t m, float* dst) {
+                const int slot = (int)(pieces++ & 1);
+                char* hbuf = ix->pinned + (size_t)slot * cbytes;
+                if (pieces > 2) B2F_CUDA(cudaEventSynchronize(evs[slot]));   // the slot's previous H2D has finished
                 const size_t cnt = (size_t)m * d32;
-                if (fseek(f, payload + (long)((size_t)r0 * d32 * 4), SEEK_SET) != 0 || fread(ix->pinned, 4, cnt, f) != cnt) {
+                if (fseek(f, payload + (long)((size_t)r0 * d32 * 4), SEEK_SET) != 0 || fread(hbuf, 4, cnt, f) != cnt) {
                     set_error("%s: truncated payload", path);
                     return B2F_EFORMAT;
                 }
-                float* dst = storage == B2F_STORE_F32 ? ix->rows_f32 + r0 * d32 : reinterpret_cast<float*>(ix->ws);
-                B2F_CUDA(cudaMemcpyAsync(dst, ix->pinned, cnt * 4, cudaMemcpyHostToDevice, ix->stream));
-                *src = dst;
+                B2F_CUDA(cudaMemcpyAsync(dst, hbuf, cnt * 4, cudaMemcpyHostToDevice, ix->stream));
+                B2F_CUDA(cudaEventRecord(evs[slot], ix->stream));
                 return B2F_OK;
             });
-        if (rc == B2F_OK && nt > 0 && (cudaStreamSynchronize(ix->stream) != cudaSuccess || fseek(f, payload, SEEK_SET) != 0)) {
-            set_error("read: %s: could not rewind after the centre", path);
-            rc = B2F_EIO;
-        }
-        cudaEvent_t evs[2] = {get_event(ix, 1), get_event(ix, 2)};
-        bool used[2] = {false, false};
-        int slot = 0;
-        // double-buffered: fread of chunk i+1 overlaps H2D + ingest of chunk i
-        for (int64_t r0 = 0; rc == B2F_OK && r0 < nt; r0 += rows_per, slot ^= 1) {
-            const int64_t m = nt - r0 < rows_per ? nt - r0 : rows_per;
-            char* hbuf = ix->pinned + (size_t)slot * cbytes;
-            if (used[slot] && cudaEventSynchronize(evs[slot]) != cudaSuccess) {
-                set_error("read: event sync failed");
-                rc = B2F_ECUDA;
-                break;
-            }
-            const size_t cnt = (size_t)m * d32;
-            if (fread(hbuf, 4, cnt, f) != cnt) {
-                set_error("%s: truncated payload", path);
-                rc = B2F_EFORMAT;
-                break;
-            }
-            cudaError_t e;
-            const float* src;
-            if (storage == B2F_STORE_F32) {
-                float* dst = ix->rows_f32 + ix->ntotal * d32;
-                e = cudaMemcpyAsync(dst, hbuf, cnt * 4, cudaMemcpyHostToDevice, ix->stream);
-                src = dst;
-            } else {
-                float* dbuf = reinterpret_cast<float*>(ix->ws + (size_t)slot * cbytes);
-                e = cudaMemcpyAsync(dbuf, hbuf, cnt * 4, cudaMemcpyHostToDevice, ix->stream);
-                src = dbuf;
-            }
-            if (e != cudaSuccess) {
-                set_error("read: H2D failed: %s", cudaGetErrorString(e));
-                rc = B2F_ECUDA;
-                break;
-            }
-            rc = add_device_rows(ix, src, m, ix->stream);
-            if (rc != B2F_OK) break;
-            cudaEventRecord(evs[slot], ix->stream);
-            used[slot] = true;
-            ix->ntotal += m;
-        }
         if (rc == B2F_OK && cudaStreamSynchronize(ix->stream) != cudaSuccess) {
             set_error("read: stream sync failed");
             rc = B2F_ECUDA;
         }
-        ix->stats_dirty = true;
     }
     fclose(f);
     if (rc != B2F_OK) {
