@@ -143,6 +143,34 @@ B2F_API int b2f_index_add(b2f_index* idx, int64_t n, const float* x, int32_t mem
 B2F_API int b2f_index_search(b2f_index* idx, int64_t nq, const float* q, int64_t k, float* D, int64_t* I,
                      int32_t mem, void* stream, const b2f_search_params* params);
 
+/* ---- index.range_search(q, radius): every row closer than a radius (faiss IndexFlat range search) ----------------
+ * L2: radius is on SQUARED distances, a row is a hit when dist < radius (strict); an L2 radius <= 0 returns nothing.
+ * IP: a row is a hit when ip > radius (strict).  NaN distances are never hits; a NaN radius is B2F_EINVAL.
+ * Distances are the engine's exact fp32 values -- L2 in the exact-difference form, IP the fp32 dot product, both to the
+ * authoritative rows (bf16 storage: fl32(mu + x~')) -- computed by the same code on every path, so a row's membership
+ * and its distance bits do not depend on the path that served the query, the batch size or the chunking.
+ * Within a query the hits are in ascending label order (label = row + params->id_offset).
+ * Layout of faiss's RangeSearchResult: lims [nq + 1] with lims[0] = 0, D [lims[nq]] fp32, I [lims[nq]] int64; query i
+ * owns [lims[i], lims[i+1]).
+ * params: algo AUTO / TENSOR use the tensor pass with a fixed per-query threshold wherever it can be planned (nq = 1
+ * included), SCAN forces the exact range scan; scan_max_nq > 0 sends AUTO batches of at most that many queries to the
+ * exact range scan (default: none); id_offset is added to every label; slack, certify and profile are ignored.
+ * A range search changes nothing top-k searches learn or report (b2f_stats: only `launches` grows).
+ * The result size is known only after the GPU has counted, so the library owns the result behind a handle. */
+typedef struct b2f_range_result b2f_range_result;
+/* index.range_search(x, radius): q [nq, d] fp32 in `mem`.  Returns once lims are known (host sync(s) inside); the
+ * hits may still be in flight on `stream`.  A result too large for device memory is B2F_ENOMEM. */
+B2F_API int b2f_index_range_search(b2f_index* idx, int64_t nq, const float* q, float radius, int32_t mem, void* stream,
+                                   const b2f_search_params* params, b2f_range_result** out);
+B2F_API int b2f_range_result_lims(const b2f_range_result* r, int64_t* lims /* host, nq + 1 */);
+/* D [lims[nq]] fp32, I [lims[nq]] int64 in `mem`; device: enqueued on `stream`, host: synchronous */
+B2F_API int b2f_range_result_fetch(b2f_range_result* r, float* D, int64_t* I, int32_t mem, void* stream);
+/* out[0] hits, [1] queries answered from tensor-pass lists, [2] queries answered by the exact range scan,
+ * [3] kernels launched, [4] host synchronisations */
+B2F_API int b2f_range_result_info(const b2f_range_result* r, int64_t out[5]);
+/* waits for the result's pending copies, then frees it */
+B2F_API int b2f_range_result_destroy(b2f_range_result* r);
+
 /* ---- index.reconstruct(i) / reconstruct_n(i0, n) (SURVEY 8b shim surface) ---------------------- */
 B2F_API int b2f_index_reconstruct(b2f_index* idx, int64_t i0, int64_t n, float* out, int32_t mem, void* stream);
 

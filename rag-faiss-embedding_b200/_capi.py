@@ -85,7 +85,13 @@ PROTOTYPES = {
     "b2f_index_device": (_i32, [_vp]),
     "b2f_index_add": (ctypes.c_int, [_vp, _i64, _vp, _i32, _vp]),
     "b2f_index_search": (ctypes.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i32, _vp, ctypes.POINTER(SearchParams)]),
-    "b2f_index_reconstruct": (ctypes.c_int, [_vp, _i64, _i64, _vp, _i32, _vp]),
+    "b2f_index_range_search": (ctypes.c_int, [_vp, _i64, _vp, ctypes.c_float, _i32, _vp, ctypes.POINTER(SearchParams),
+                                              ctypes.POINTER(_vp)]),
+    "b2f_range_result_lims": (ctypes.c_int, [_vp, ctypes.POINTER(_i64)]),
+    "b2f_range_result_fetch": (ctypes.c_int, [_vp, _vp, _vp, _i32, _vp]),
+    "b2f_range_result_info": (ctypes.c_int, [_vp, ctypes.POINTER(_i64)]),
+    "b2f_range_result_destroy": (ctypes.c_int, [_vp]),
+    "b2f_index_reconstruct":(ctypes.c_int, [_vp, _i64, _i64, _vp, _i32, _vp]),
     "b2f_index_write": (ctypes.c_int, [_vp, ctypes.c_char_p]),
     "b2f_index_read": (ctypes.c_int, [ctypes.c_char_p, _i32, _i32, ctypes.POINTER(_vp)]),
     "b2f_merge_topk": (ctypes.c_int, [_i32, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _vp]),

@@ -270,8 +270,10 @@ int launch_prep_queries(const float* q, int nq, int nq_pad, int d, __nv_bfloat16
 int launch_gather_failed(const float* q, int d, const int32_t* fail_list, const float* fail_tau, const int32_t* nfail, int nfail_host,
                          int cap, float* qf, float* tau2, int32_t* out_map, int32_t* range_count, int32_t* fail_list2,
                          int32_t* fail_count2, cudaStream_t st);
-int launch_range_thresholds(const float* tau2, const int32_t* out_map, int n, int d, int metric, const float* qnorm, const float* qerr,
-                            const float* qconst, float max_row_norm, float max_row_err, float mu_norm, float* thr, cudaStream_t st);
+// thr[i] for tau = tau2[i] (tau2 null: tau_all for every i); out_map (optional): slots with out_map[i] < 0 list nothing
+int launch_range_thresholds(const float* tau2, float tau_all, const int32_t* out_map, int n, int d, int metric, const float* qnorm,
+                            const float* qerr, const float* qconst, float max_row_norm, float max_row_err, float mu_norm, float* thr,
+                            cudaStream_t st);
 int launch_bf16_to_f32(const __nv_bfloat16* src, int64_t pitch, int64_t n, int d, const float* mu, float* dst, cudaStream_t st);
 
 // K4: exact fp32 re-rank of coarse candidates + certification.
@@ -342,5 +344,31 @@ int launch_tensor_scan(const __nv_bfloat16* scan, int64_t dpad, const float* nor
 // with every list entry when the first attempt fails), write (D, I); uncertified queries go to ra.fail_list
 int launch_merge_lists(const TensorScanLists& lists, int nq, const TensorScanPlan& plan, unsigned long long* total_entries,
                        const RerankArgs& ra, cudaStream_t st);
+
+// ---- range search (index.range_search(x, radius)): hit <=> exact key (ra: rows and queries, as K4) < tau ----------------
+constexpr int kRangeHitsMax = 4096;   // list entries one query of the tensor path filters (= the merge's MERGE_MAX)
+// The lists of a range-threshold tensor pass (lists.range_thr) -> each query's hits, sorted by row id, staged in
+// skey / sid [nq][kRangeHitsMax] with their number in staged[q] and count[q]; queries the lists cannot answer (overflow, more
+// than kRangeHitsMax entries, NaN threshold) get staged[q] = count[q] = 0 and are appended to scan_list / *scan_n.
+int launch_range_collect(const TensorScanLists& lists, int nq, const TensorScanPlan& plan, float tau, const RerankArgs& ra,
+                         float* skey, int32_t* sid, int32_t* staged, int32_t* count, int32_t* scan_list, int32_t* scan_n,
+                         cudaStream_t st);
+// The exact range scan's row tiles: the rows split into at most 2 x kNumSMs contiguous tiles
+struct RangeScanGeometry {
+    int64_t tile_rows;
+    int ntiles;
+};
+RangeScanGeometry range_scan_geometry(int64_t n);
+// Exact range scan of the listed queries (list null: 0..nlist_max-1; nlist_dev null: nlist_max of them) over all rows.
+// emit = false: hits per (list slot, tile) to tile_counts [nlist_max][ntiles], added to count[query].  emit = true: the same
+// hits, in row order, to D / I at base + lims[query] (+ the query's hits in earlier tiles).
+int launch_range_scan(const RerankArgs& a, float tau, const int32_t* list, const int32_t* nlist_dev, int nlist_max,
+                      int32_t* tile_counts, int32_t* count, const int64_t* lims, int64_t base, float* D, int64_t* I,
+                      int64_t id_offset, bool emit, cudaStream_t st);
+// lims[0..n]: exclusive prefix sums of count[0..n) (n <= 1024)
+int launch_range_offsets(const int32_t* count, int n, int64_t* lims, cudaStream_t st);
+// staged hits of queries 0..nq-1 to D / I at base + lims[q] in faiss format (L2: key, IP: -key; label = id + id_offset)
+int launch_range_emit(const float* skey, const int32_t* sid, const int32_t* staged, const int64_t* lims, int nq, int64_t base, int metric,
+                      float* D, int64_t* I, int64_t id_offset, cudaStream_t st);
 
 }  // namespace b2f

@@ -1123,6 +1123,7 @@ constexpr int MERGE_THREADS = kRerankThreads;  // 256
 constexpr int MERGE_MAX = 4096;   // composites held in shared memory (32 KB) at most; more -> the query falls back
 constexpr int RANK_MAX = 1024;    // direct ranking and extended certification up to this many list entries
 constexpr int KP_MAX = 256;
+static_assert(MERGE_MAX == kRangeHitsMax, "range search stages as many entries per query as the merge holds");
 
 __device__ __forceinline__ int block_count_le(const unsigned long long* comp, int M, unsigned long long bound, int* s_cnt,
                                               int it, int tid, int lane) {
@@ -1674,6 +1675,111 @@ static int launch_k2(const CUtensorMap& mq, const CUtensorMap& mx, const float* 
     return B2F_OK;
 }
 
+// ---- range search: filter the lists of a range-threshold pass down to the exact hits -----------------------------------
+// One CTA per query.  The pass listed every row whose coarse key is <= thr(tau), a proven superset of the rows whose exact
+// key is <= tau.  Each entry's exact key (exact_key_8lanes, as everywhere else) decides; the strict hits are sorted by row
+// id (bitonic over (id, key) composites; non-hits are all-ones and sort last) and staged in skey / sid [q][MERGE_MAX].
+// A query whose lists overflowed, that has more than MERGE_MAX entries or a NaN threshold goes to scan_list instead.
+__global__ void __launch_bounds__(MERGE_THREADS)
+range_collect_kernel(const uint2* __restrict__ cand, const int32_t* __restrict__ counts, const float* __restrict__ thr,
+                     int nl_stride, int tile_queries, int ntile_units, int total_units, int halves, int list_cap, float tau,
+                     const RerankArgs ra, float* __restrict__ skey, int32_t* __restrict__ sid, int32_t* __restrict__ staged,
+                     int32_t* __restrict__ count, int32_t* __restrict__ scan_list, int32_t* __restrict__ scan_n) {
+    __shared__ unsigned long long comp[MERGE_MAX];
+    __shared__ int s_off[2 * kNumSMs + 2];
+    __shared__ int s_ovf, s_hits;
+    const int q = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+    const TileInfo ti = tile_info(q / tile_queries, ntile_units, total_units, 0, halves);
+    const int nsplits = (ti.nfw + ti.nsw) * halves;
+    if (tid == 0) {
+        s_ovf = !(thr[q] == thr[q]);
+        s_hits = 0;
+    }
+    __syncthreads();
+    for (int s2 = tid; s2 < nsplits; s2 += MERGE_THREADS) {
+        const int c = counts[(int64_t)q * nl_stride + s2];
+        if (c > list_cap) s_ovf = 1;
+        s_off[s2 + 1] = c;
+    }
+    __syncthreads();
+    if (tid < 32) {
+        int run = 0;
+        for (int s0 = 0; s0 < nsplits; s0 += 32) {
+            const int s2 = s0 + lane;
+            int incl = s2 < nsplits ? s_off[s2 + 1] : 0;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const int up = __shfl_up_sync(kFull, incl, d);
+                if (lane >= d) incl += up;
+            }
+            __syncwarp();
+            if (s2 < nsplits) s_off[s2 + 1] = run + incl;
+            run += __shfl_sync(kFull, incl, 31);
+        }
+        if (lane == 0) {
+            s_off[0] = 0;
+            if (run > MERGE_MAX) s_ovf = 1;
+        }
+    }
+    __syncthreads();
+    if (s_ovf) {
+        if (tid == 0) {
+            scan_list[atomicAdd(scan_n, 1)] = q;
+            staged[q] = 0;
+            count[q] = 0;   // the exact range scan adds this query's hits
+        }
+        return;
+    }
+    const int M = s_off[nsplits];
+    for (int l = 0; l < nsplits; l++) {
+        const uint2* p = cand + ((int64_t)q * nl_stride + l) * list_cap;
+        for (int j = tid; j < s_off[l + 1] - s_off[l]; j += MERGE_THREADS) comp[s_off[l] + j] = (unsigned long long)p[j].y << 32;
+    }
+    __syncthreads();
+    const float* qv = ra.q + (int64_t)q * ra.d;
+    const bool l2 = ra.metric == B2F_METRIC_L2;
+    const int sl = lane & 7;
+    for (int c0 = 0; c0 < M; c0 += MERGE_THREADS / 8) {
+        const int c = c0 + (tid >> 3);
+        int32_t id = c < M ? (int32_t)(comp[c] >> 32) : -1;
+        if ((int64_t)id >= ra.ntotal) id = -1;
+        const float key = exact_key_8lanes(ra, qv, id, sl, l2);
+        if (sl == 0 && c < M) {
+            const bool hit = id >= 0 && key < tau;   // NaN is never a hit
+            comp[c] = hit ? (comp[c] | __float_as_uint(key)) : ~0ull;
+            if (hit) atomicAdd(&s_hits, 1);
+        }
+    }
+    int N = 1;
+    while (N < M) N <<= 1;
+    for (int i = M + tid; i < N; i += MERGE_THREADS) comp[i] = ~0ull;
+    __syncthreads();
+    for (int k = 2; k <= N; k <<= 1)
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < N; i += MERGE_THREADS) {
+                const int p = i ^ j;
+                if (p > i) {
+                    const unsigned long long a = comp[i], b = comp[p];
+                    if ((a > b) == ((i & k) == 0)) {
+                        comp[i] = b;
+                        comp[p] = a;
+                    }
+                }
+            }
+            __syncthreads();
+        }
+    const int H = s_hits;
+    for (int i = tid; i < H; i += MERGE_THREADS) {
+        const unsigned long long v = comp[i];
+        skey[(int64_t)q * MERGE_MAX + i] = __uint_as_float((uint32_t)v);
+        sid[(int64_t)q * MERGE_MAX + i] = (int32_t)(v >> 32);
+    }
+    if (tid == 0) {
+        staged[q] = H;
+        count[q] = H;
+    }
+}
+
 }  // namespace k2
 
 // Planning switch of the calling thread (index.cu sets it around the planning of one search): skip LIST mode.  An index
@@ -1943,6 +2049,22 @@ int launch_merge_lists(const TensorScanLists& lists, int nq, const TensorScanPla
                                                                plan.nlists, plan.pair_mode ? 2 * k2::BM : k2::BM, plan.tile_units, plan.units,
                                                                k2::EPI_WARPS_LIST / 4, plan.kp, plan.list_cap, cap_entries, total_entries,
                                                                only_flagged, ra);
+    B2F_CUDA(cudaGetLastError());
+    return B2F_OK;
+}
+
+int launch_range_collect(const TensorScanLists& lists, int nq, const TensorScanPlan& plan, float tau, const RerankArgs& ra,
+                         float* skey, int32_t* sid, int32_t* staged, int32_t* count, int32_t* scan_list, int32_t* scan_n,
+                         cudaStream_t st) {
+    if (nq <= 0) return B2F_OK;
+    if (!plan.list_mode || plan.nlists > 2 * kNumSMs) {
+        set_error("range collect: a LIST-mode plan of at most %d lists per query is required", 2 * kNumSMs);
+        return B2F_EINVAL;
+    }
+    k2::range_collect_kernel<<<nq, k2::MERGE_THREADS, 0, st>>>(reinterpret_cast<const uint2*>(lists.cand), lists.counts, lists.range_thr,
+                                                               plan.nlists, plan.pair_mode ? 2 * k2::BM : k2::BM, plan.tile_units,
+                                                               plan.units, k2::EPI_WARPS_LIST / 4, plan.list_cap, tau, ra, skey, sid,
+                                                               staged, count, scan_list, scan_n);
     B2F_CUDA(cudaGetLastError());
     return B2F_OK;
 }

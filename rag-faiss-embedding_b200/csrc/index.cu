@@ -1117,7 +1117,7 @@ static int range_pass(b2f_index* ix, Bump& bump, const SearchWs& w, const float*
     B2F_TRY(launch_prep_queries(r.q, nr, nq_pad, ix->d, r.pq.qb, ix->dpad, r.pq.qnorm, r.pq.qerr, r.pq.qconst,
                                 ix->mu_set ? ix->centre : nullptr, nullptr, 0, reinterpret_cast<uint32_t*>(r.lists.shared_thr),
                                 (int64_t)nq_pad * rp.nlists, st));
-    B2F_TRY(launch_range_thresholds(r.tau, r.out_map, nr, ix->d, ix->metric, r.pq.qnorm, r.pq.qerr, r.pq.qconst,
+    B2F_TRY(launch_range_thresholds(r.tau, 0.f, r.out_map, nr, ix->d, ix->metric, r.pq.qnorm, r.pq.qerr, r.pq.qconst,
                                     sqrtf(ix->host_stats[0]), sqrtf(ix->host_stats[1]), ix->mu_norm, r.thr, st));
     B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, r.pq.qb, nr, nq_pad, rp, nullptr, nullptr,
                                r.lists, st));
@@ -1330,6 +1330,315 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
     }
     return B2F_OK;
 }
+
+// ---- range search ----------------------------------------------------------------------------------
+// The result of one range search: lims on the host, the hits in buffers the library owns (faiss's RangeSearchResult).
+// D / I grow while the chunks are counted; a buffer they outgrow may still be read by copies in flight, so it is freed
+// with the others when the result is destroyed.
+struct b2f_range_result {
+    int device = 0;
+    std::vector<int64_t> lims;
+    float* D = nullptr;
+    int64_t* I = nullptr;
+    int64_t cap = 0;
+    std::vector<void*> retired;
+    cudaStream_t st = nullptr;       // the stream the search ran on
+    cudaEvent_t done = nullptr;      // recorded behind the last write to, or device copy from, D / I
+    int64_t info[5] = {0, 0, 0, 0, 0};
+};
+
+// A range search plans its tensor pass for the threshold alone: nothing is pruned or vouched for, so k' only sizes the
+// (unused) voucher state.  Every row at or below a query's threshold must fit its lists, and a query whose lists hold more
+// than kRangeHitsMax entries goes to the exact range scan anyway: lists of 2 x kRangeHitsMax / nlists entries, at least
+// kRangeListCap.
+constexpr int kRangeSearchKp = 32;
+
+static int plan_range_search(int nq, int64_t n, int d, TensorScanPlan* plan) {
+    if (plan_tensor_scan(nq, n, d, kRangeSearchKp, plan) != B2F_OK || !plan->list_mode) return B2F_EINVAL;
+    int cap = (int)align_up((size_t)(2 * kRangeHitsMax / plan->nlists), 64);
+    if (cap < kRangeListCap) cap = kRangeListCap;
+    plan->list_cap = cap < 1024 ? cap : 1024;
+    return B2F_OK;
+}
+
+// What one chunk of a range search carves from the workspace, in one order (measured over a null base first)
+struct RangeSearchWs {
+    float* q = nullptr;              // host queries: the chunk's device copy
+    int32_t* count = nullptr;        // [chunk] hits per query
+    int32_t* staged = nullptr;       // [chunk] hits the tensor path staged per query
+    int32_t* scan_list = nullptr;    // [chunk] queries left to the exact range scan
+    int64_t* lims = nullptr;         // [chunk + 1] chunk-local offsets
+    int32_t* tile_counts = nullptr;  // [chunk][ntiles] the exact range scan's hits per row tile
+    PassQueries pq{};                // tensor path from here on
+    float* thr = nullptr;
+    int32_t* counters = nullptr;     // [0] queries in scan_list, [8..11] K2's tickets
+    TensorScanLists lists{};
+    float* skey = nullptr;           // [chunk][kRangeHitsMax] staged hits: exact key, row id
+    int32_t* sid = nullptr;
+};
+
+static RangeSearchWs carve_range_search(Bump& b, const b2f_index* ix, int cn, bool host, bool tensor, const TensorScanPlan& plan,
+                                        int ntiles) {
+    RangeSearchWs w;
+    if (host) w.q = b.take<float>((size_t)cn * ix->d);
+    w.count = b.take<int32_t>(cn);
+    w.staged = b.take<int32_t>(cn);
+    w.scan_list = b.take<int32_t>(cn);
+    w.lims = b.take<int64_t>((size_t)cn + 1);
+    w.tile_counts = b.take<int32_t>((size_t)cn * ntiles);
+    if (!tensor) return w;
+    const size_t nq_pad = (size_t)plan.nq_tiles * 128;
+    w.pq = take_queries(b, nq_pad, ix->dpad);
+    w.thr = b.take<float>(nq_pad);
+    w.counters = b.take<int32_t>(16);
+    w.lists = take_lists(b, plan);
+    w.lists.die_ctr = w.counters + 8;
+    w.lists.range_thr = w.thr;
+    w.skey = b.take<float>((size_t)cn * kRangeHitsMax);
+    w.sid = b.take<int32_t>((size_t)cn * kRangeHitsMax);
+    return w;
+}
+
+// D / I of r hold at least `need` hits (contents kept)
+static int range_result_reserve(b2f_range_result* r, int64_t need, cudaStream_t st) {
+    if (need <= r->cap) return B2F_OK;
+    int64_t cap = 2 * r->cap > need ? 2 * r->cap : need;
+    float* D = nullptr;
+    int64_t* I = nullptr;
+    cudaError_t e = cudaMalloc(&D, (size_t)cap * sizeof(float));
+    if (e == cudaSuccess) e = cudaMalloc(&I, (size_t)cap * sizeof(int64_t));
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(D);
+        set_error("range search: %lld hits (%.2f GB of distances and labels) do not fit device memory: %s", (long long)need,
+                  (double)need * 12 / 1e9, cudaGetErrorString(e));
+        return B2F_ENOMEM;
+    }
+    if (r->cap > 0) {
+        B2F_CUDA(cudaMemcpyAsync(D, r->D, (size_t)r->cap * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        B2F_CUDA(cudaMemcpyAsync(I, r->I, (size_t)r->cap * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+    }
+    if (r->D) r->retired.push_back(r->D);
+    if (r->I) r->retired.push_back(r->I);
+    r->D = D;
+    r->I = I;
+    r->cap = cap;
+    return B2F_OK;
+}
+
+// The batch in chunks of at most kRangeCap queries.  A chunk goes to the tensor path when a LIST-mode pass can be planned
+// for it (halving the chunk until one can); with none even for one query, the chunk goes to the exact range scan.  Per chunk:
+// [tensor: prep, thresholds, K2 listing every row at or below thr(tau), collect] -> exact range scan count pass over what
+// the lists could not answer (or over the whole chunk) -> offsets -> ONE host sync for the chunk's lims -> emit.
+static int range_search_locked(b2f_index* ix, int nq, const float* q, float radius, int32_t mem, void* stream,
+                               const b2f_search_params* params, b2f_range_result* r) {
+    b2f_search_params P{};
+    if (params) P = *params;
+    const bool l2 = ix->metric == B2F_METRIC_L2;
+    r->lims.assign((size_t)nq + 1, 0);
+    if (nq == 0 || ix->ntotal == 0 || (l2 && !(radius > 0.f))) return B2F_OK;   // nothing can be a hit
+    DeviceGuard g(ix->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : ix->stream;
+    r->st = st;
+    B2F_TRY(enter_stream(ix, g, st));
+    B2F_TRY(order_after(st, ix->stream, ix));
+    const bool host = mem == B2F_MEM_HOST;
+    const float tau = l2 ? radius : -radius;   // hit <=> exact key < tau
+    int64_t launches = 0, syncs = ix->stats_dirty ? 1 : 0;
+    B2F_TRY(refresh_host_stats(ix, st));
+    const float max_row_norm = sqrtf(ix->host_stats[0]), max_row_err = sqrtf(ix->host_stats[1]);
+    // the threshold is the certification bound inverted: with a non-finite row in the index it bounds nothing
+    const bool bound_ok = isfinite(max_row_norm) && isfinite(max_row_err) && isfinite(ix->mu_norm);
+    const bool want_tensor = bound_ok && P.algo != B2F_ALGO_SCAN && !(P.algo == B2F_ALGO_AUTO && nq <= P.scan_max_nq);
+    RerankArgs a{};
+    a.rows_f32 = ix->storage == B2F_STORE_F32 ? ix->rows_f32 : nullptr;
+    a.rows_bf16 = ix->scan;
+    a.pitch_bf16 = ix->dpad;
+    a.centre = (ix->storage == B2F_STORE_BF16 && ix->mu_set) ? ix->centre : nullptr;
+    a.d = ix->d;
+    a.metric = ix->metric;
+    a.ntotal = ix->ntotal;
+    const RangeScanGeometry geo = range_scan_geometry(ix->ntotal);
+    B2F_TRY(ensure_pinned(ix, ((size_t)kRangeCap + 2) * sizeof(int64_t)));
+    int64_t* lims_h = reinterpret_cast<int64_t*>(ix->pinned);
+    int64_t base = 0;
+    for (int c0 = 0; c0 < nq;) {
+        int cn = nq - c0 < kRangeCap ? nq - c0 : kRangeCap;
+        TensorScanPlan plan{};
+        bool tensor = false;
+        for (int m = cn; want_tensor && !tensor; m = (m + 1) / 2) {
+            if (plan_range_search(m, ix->ntotal, ix->d, &plan) == B2F_OK) {
+                tensor = true;
+                cn = m;
+            } else if (m == 1) {
+                break;
+            }
+        }
+        Bump layout(nullptr, SIZE_MAX);
+        carve_range_search(layout, ix, cn, host, tensor, plan, geo.ntiles);
+        if (layout.off > ix->ws_bytes && ix->ws) syncs++;
+        B2F_TRY(ensure_ws(ix, layout.off));
+        Bump bump(ix->ws, ix->ws_bytes);
+        const RangeSearchWs w = carve_range_search(bump, ix, cn, host, tensor, plan, geo.ntiles);
+        if (!bump.fits()) {
+            set_error("range search workspace: the layout needs %zu bytes, the workspace has %zu", bump.off, bump.size);
+            return B2F_ECUDA;
+        }
+        const float* qc = host ? w.q : q + (int64_t)c0 * ix->d;
+        if (host) B2F_CUDA(cudaMemcpyAsync(w.q, q + (int64_t)c0 * ix->d, (size_t)cn * ix->d * 4, cudaMemcpyHostToDevice, st));
+        a.q = qc;
+        if (tensor) {
+            const int nq_pad = plan.nq_tiles * 128;
+            B2F_TRY(launch_prep_queries(qc, cn, nq_pad, ix->d, w.pq.qb, ix->dpad, w.pq.qnorm, w.pq.qerr, w.pq.qconst,
+                                        ix->mu_set ? ix->centre : nullptr, reinterpret_cast<uint32_t*>(w.counters), 16, nullptr, 0, st));
+            B2F_TRY(launch_range_thresholds(nullptr, tau, nullptr, cn, ix->d, ix->metric, w.pq.qnorm, w.pq.qerr, w.pq.qconst,
+                                            max_row_norm, max_row_err, ix->mu_norm, w.thr, st));
+            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, w.pq.qb, cn, nq_pad, plan, nullptr, nullptr,
+                                       w.lists, st));
+            B2F_TRY(launch_range_collect(w.lists, cn, plan, tau, a, w.skey, w.sid, w.staged, w.count, w.scan_list, w.counters, st));
+            launches += 4;
+        } else {
+            B2F_CUDA(cudaMemsetAsync(w.count, 0, (size_t)cn * 4, st));
+        }
+        const int32_t* list = tensor ? w.scan_list : nullptr;
+        const int32_t* nlist = tensor ? w.counters : nullptr;
+        B2F_TRY(launch_range_scan(a, tau, list, nlist, cn, w.tile_counts, w.count, nullptr, 0, nullptr, nullptr, 0, false, st));
+        B2F_TRY(launch_range_offsets(w.count, cn, w.lims, st));
+        launches += 2;
+        B2F_CUDA(cudaMemcpyAsync(lims_h, w.lims, ((size_t)cn + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        if (tensor) B2F_CUDA(cudaMemcpyAsync(lims_h + kRangeCap + 1, w.counters, 4, cudaMemcpyDeviceToHost, st));
+        B2F_CUDA(cudaStreamSynchronize(st));
+        syncs++;
+        const int64_t hits = lims_h[cn];
+        const int nscan = tensor ? *reinterpret_cast<const int32_t*>(lims_h + kRangeCap + 1) : cn;
+        for (int i = 0; i <= cn; i++) r->lims[(size_t)c0 + i] = base + lims_h[i];
+        if (hits > 0) {
+            B2F_TRY(range_result_reserve(r, base + hits, st));
+            if (tensor) {
+                B2F_TRY(launch_range_emit(w.skey, w.sid, w.staged, w.lims, cn, base, ix->metric, r->D, r->I, P.id_offset, st));
+                launches++;
+            }
+            if (nscan > 0) {
+                B2F_TRY(launch_range_scan(a, tau, list, nlist, cn, w.tile_counts, w.count, w.lims, base, r->D, r->I, P.id_offset, true, st));
+                launches++;
+            }
+        }
+        r->info[1] += cn - nscan;
+        r->info[2] += nscan;
+        base += hits;
+        c0 += cn;
+    }
+    r->info[0] = base;
+    r->info[3] = launches;
+    r->info[4] = syncs;
+    ix->st.launches += launches;
+    if (!r->done) B2F_CUDA(cudaEventCreateWithFlags(&r->done, cudaEventDisableTiming));
+    B2F_CUDA(cudaEventRecord(r->done, st));
+    if (!ix->ev_done) B2F_CUDA(cudaEventCreateWithFlags(&ix->ev_done, cudaEventDisableTiming));
+    B2F_CUDA(cudaEventRecord(ix->ev_done, st));
+    ix->last_stream = st;
+    ix->search_recorded = true;
+    return B2F_OK;
+}
+
+extern "C" {
+
+int b2f_range_result_destroy(b2f_range_result* r) {
+    if (!r) return B2F_OK;
+    DeviceGuard g(r->device);
+    if (r->done) {
+        cudaEventSynchronize(r->done);
+        cudaEventDestroy(r->done);
+    } else if (r->st) {
+        cudaStreamSynchronize(r->st);   // a search that failed half way may still write D / I
+    }
+    cudaGetLastError();
+    cudaFree(r->D);
+    cudaFree(r->I);
+    for (void* p : r->retired) cudaFree(p);
+    delete r;
+    return B2F_OK;
+}
+
+int b2f_index_range_search(b2f_index* ix, int64_t nq, const float* q, float radius, int32_t mem, void* stream,
+                           const b2f_search_params* params, b2f_range_result** out) {
+    if (!out) {
+        set_error("range_search: out is NULL");
+        return B2F_EINVAL;
+    }
+    *out = nullptr;
+    if (!ix) {
+        set_error("index is NULL");
+        return B2F_EINVAL;
+    }
+    if (nq < 0 || nq > (1 << 24) || (nq > 0 && !q)) {
+        set_error("range_search: bad arguments (nq=%lld)", (long long)nq);
+        return B2F_EINVAL;
+    }
+    if (radius != radius) {
+        set_error("range_search: radius is NaN");
+        return B2F_EINVAL;
+    }
+    b2f_range_result* r = new (std::nothrow) b2f_range_result();
+    if (!r) {
+        set_error("range_search: out of host memory");
+        return B2F_ENOMEM;
+    }
+    r->device = ix->device;
+    int rc;
+    {
+        std::lock_guard<std::mutex> lk(ix->mu);
+        rc = range_search_locked(ix, (int)nq, q, radius, mem, stream, params, r);
+    }
+    if (rc != B2F_OK) {
+        b2f_range_result_destroy(r);
+        return rc;
+    }
+    *out = r;
+    return B2F_OK;
+}
+
+int b2f_range_result_lims(const b2f_range_result* r, int64_t* lims) {
+    if (!r || !lims) {
+        set_error("range_result_lims: NULL argument");
+        return B2F_EINVAL;
+    }
+    memcpy(lims, r->lims.data(), r->lims.size() * sizeof(int64_t));
+    return B2F_OK;
+}
+
+int b2f_range_result_fetch(b2f_range_result* r, float* D, int64_t* I, int32_t mem, void* stream) {
+    const int64_t hits = r ? r->lims.back() : 0;
+    if (!r || (hits > 0 && (!D || !I))) {
+        set_error("range_result_fetch: NULL argument");
+        return B2F_EINVAL;
+    }
+    if (hits == 0) return B2F_OK;
+    DeviceGuard g(r->device);
+    if (mem == B2F_MEM_HOST) {
+        B2F_CUDA(cudaEventSynchronize(r->done));
+        B2F_CUDA(cudaMemcpy(D, r->D, (size_t)hits * sizeof(float), cudaMemcpyDeviceToHost));
+        B2F_CUDA(cudaMemcpy(I, r->I, (size_t)hits * sizeof(int64_t), cudaMemcpyDeviceToHost));
+        return B2F_OK;
+    }
+    cudaStream_t st = stream ? (cudaStream_t)stream : r->st;
+    B2F_CUDA(cudaStreamWaitEvent(st, r->done, 0));
+    B2F_CUDA(cudaMemcpyAsync(D, r->D, (size_t)hits * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    B2F_CUDA(cudaMemcpyAsync(I, r->I, (size_t)hits * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+    B2F_CUDA(cudaEventRecord(r->done, st));   // destroy waits for these copies
+    return B2F_OK;
+}
+
+int b2f_range_result_info(const b2f_range_result* r, int64_t out[5]) {
+    if (!r || !out) {
+        set_error("range_result_info: NULL argument");
+        return B2F_EINVAL;
+    }
+    for (int i = 0; i < 5; i++) out[i] = r->info[i];
+    return B2F_OK;
+}
+
+}  // extern "C"
 
 extern "C" {
 

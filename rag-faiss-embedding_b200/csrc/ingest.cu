@@ -470,17 +470,17 @@ int launch_gather_failed(const float* q, int d, const int32_t* fail_list, const 
 // The fixed threshold of a range query: every row whose exact key is <= tau (the k-th key already found, so: every true
 // top-k row) has a coarse key <= thr.  Inverse of the certification test (rerank_certified) with a 1e-6 margin on tau, so
 // that re-ranking everything at or below thr certifies by construction.
-__global__ void range_thresholds_kernel(const float* __restrict__ tau2, const int32_t* __restrict__ out_map, int n, int d, int l2,
+__global__ void range_thresholds_kernel(const float* __restrict__ tau2, float tau_all, const int32_t* __restrict__ out_map, int n, int d, int l2,
                                         const float* __restrict__ qnorm, const float* __restrict__ qerr,
                                         const float* __restrict__ qconst, float max_row_norm, float max_row_err, float mu_norm,
                                         float* __restrict__ thr) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    if (out_map[i] < 0) {
+    if (out_map && out_map[i] < 0) {
         thr[i] = -__int_as_float(0x7f800000);   // unused slot: nothing is listed
         return;
     }
-    const float tau = tau2[i];
+    const float tau = tau2 ? tau2[i] : tau_all;
     const float qn2 = qnorm[i], qn = sqrtf(qn2), eq = qerr[i];
     const float gam = 4.f * (float)(d + 16) * 5.9604645e-8f;
     if (l2) {
@@ -502,10 +502,11 @@ __global__ void range_thresholds_kernel(const float* __restrict__ tau2, const in
     }
 }
 
-int launch_range_thresholds(const float* tau2, const int32_t* out_map, int n, int d, int metric, const float* qnorm, const float* qerr,
-                            const float* qconst, float max_row_norm, float max_row_err, float mu_norm, float* thr, cudaStream_t st) {
+int launch_range_thresholds(const float* tau2, float tau_all, const int32_t* out_map, int n, int d, int metric, const float* qnorm,
+                            const float* qerr, const float* qconst, float max_row_norm, float max_row_err, float mu_norm, float* thr,
+                            cudaStream_t st) {
     if (n <= 0) return B2F_OK;
-    range_thresholds_kernel<<<(n + 255) / 256, 256, 0, st>>>(tau2, out_map, n, d, metric == B2F_METRIC_L2 ? 1 : 0, qnorm, qerr, qconst,
+    range_thresholds_kernel<<<(n + 255) / 256, 256, 0, st>>>(tau2, tau_all, out_map, n, d, metric == B2F_METRIC_L2 ? 1 : 0, qnorm, qerr, qconst,
                                                             max_row_norm, max_row_err, mu_norm, thr);
     B2F_CUDA(cudaGetLastError());
     return B2F_OK;

@@ -242,6 +242,52 @@ class IndexFlat:
         C.check(self._lib.b2f_index_search(self._h, x.shape[0], x.data_ptr(), k, D.data_ptr(), I.data_ptr(),
                                            C.MEM_DEVICE, _torch_stream(x), ctypes.byref(p)))
 
+    def range_search(self, x, radius: float, *, params: Optional[C.SearchParams] = None):
+        """index.range_search(x, radius) -> (lims, D, I), faiss's RangeSearchResult: query i owns
+        D[lims[i]:lims[i+1]] / I[lims[i]:lims[i+1]], ids ascending.  L2: squared distance < radius; IP: ip > radius.
+        numpy in: lims uint64, D float32, I int64 numpy arrays.  CUDA tensor in: int64 / float32 / int64 CUDA tensors
+        on the current torch stream.  The five numbers of b2f_range_result_info go to self.last_range_info."""
+        p = params if params is not None else self._params
+        dev = _is_torch(x) and x.is_cuda
+        if dev:
+            import torch
+
+            _assert(x.dim() == 2 and x.shape[1] == self.d, f"dimension mismatch: got {tuple(x.shape)}, d={self.d}")
+            self._check_tensor(x, "x")
+            x = x.to(torch.float32).contiguous()
+            stream = _torch_stream(x)
+            qptr, mem = x.data_ptr(), C.MEM_DEVICE
+        else:
+            if _is_torch(x):
+                x = x.detach().cpu().numpy()
+            x = self._coerce_host(x)
+            stream = None
+            qptr, mem = x.ctypes.data, C.MEM_HOST
+        n = x.shape[0]
+        h = ctypes.c_void_p()
+        C.check(self._lib.b2f_index_range_search(self._h, n, qptr, ctypes.c_float(radius), mem, stream, ctypes.byref(p),
+                                                 ctypes.byref(h)))
+        try:
+            lims = np.empty(n + 1, dtype=np.int64)
+            C.check(self._lib.b2f_range_result_lims(h, lims.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))))
+            total = int(lims[-1])
+            if dev:
+                D = torch.empty(total, dtype=torch.float32, device=x.device)
+                I = torch.empty(total, dtype=torch.int64, device=x.device)
+                C.check(self._lib.b2f_range_result_fetch(h, D.data_ptr(), I.data_ptr(), C.MEM_DEVICE, stream))
+                lims_out = torch.from_numpy(lims).to(x.device)
+            else:
+                D = np.empty(total, dtype=np.float32)
+                I = np.empty(total, dtype=np.int64)
+                C.check(self._lib.b2f_range_result_fetch(h, D.ctypes.data, I.ctypes.data, C.MEM_HOST, None))
+                lims_out = lims.astype(np.uint64)
+            info = (ctypes.c_int64 * 5)()
+            C.check(self._lib.b2f_range_result_info(h, info))
+            self.last_range_info = dict(zip(("hits", "tensor_queries", "scan_queries", "launches", "host_syncs"), list(info)))
+        finally:
+            self._lib.b2f_range_result_destroy(h)
+        return lims_out, D, I
+
     def search_into(self, x: np.ndarray, k: int, D: np.ndarray, I: np.ndarray):
         """Host-buffer search into caller-owned (ideally pinned) arrays: the raw C-ABI call."""
         C.check(self._lib.b2f_index_search(self._h, x.shape[0], x.ctypes.data, k, D.ctypes.data, I.ctypes.data,
