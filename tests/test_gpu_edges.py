@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 import oracle as orc
+from tests.exact_checks import check_structure
 
 pytestmark = pytest.mark.gpu
 
@@ -72,6 +73,7 @@ def m():
 
 
 def _check(D, I, D_ref, I_ref, metric, rel=REL, min_recall=1.0, abs_floor=1e-4):
+    check_structure(D, I, metric)
     r = orc.recall_and_errors(D, I, D_ref, I_ref, metric, rel_tol=rel, abs_floor=abs_floor)
     assert r["recall"] >= min_recall, r
     assert r["id_mismatch"] == 0, r

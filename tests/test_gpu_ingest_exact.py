@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 
 import oracle as orc
+from tests.exact_checks import check_structure
 
 pytestmark = pytest.mark.gpu
 
@@ -80,6 +81,7 @@ def _build(m, route, x, tmp_path, metric=1, seed=None):
 
 
 def _check_search(D, I, D_ref, I_ref, metric, min_recall=1.0):
+    check_structure(D, I, metric)
     r = orc.recall_and_errors(D, I, D_ref, I_ref, metric, rel_tol=1e-5)
     assert r["recall"] >= min_recall and r["id_mismatch"] == 0 and r["padding_ok"] and r["max_rel_err"] <= 1e-5, r
 

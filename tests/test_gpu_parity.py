@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import oracle as orc
+from tests.exact_checks import check_structure
 
 pytestmark = pytest.mark.gpu
 
@@ -24,6 +25,7 @@ def m():
 
 
 def _check(D, I, D_ref, I_ref, metric, rel=REL, min_recall=1.0):
+    check_structure(D, I, metric)
     r = orc.recall_and_errors(D, I, D_ref, I_ref, metric, rel_tol=rel)
     # min_recall < 1 only where fp32 keys of neighbouring rows differ by less than an ulp, so that the k-th and the
     # (k+1)-th neighbour of a float64 oracle are a tie in the reference's own fp32 arithmetic (id_mismatch still
