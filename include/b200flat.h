@@ -171,6 +171,19 @@ B2F_API int b2f_range_result_info(const b2f_range_result* r, int64_t out[5]);
 /* waits for the result's pending copies, then frees it */
 B2F_API int b2f_range_result_destroy(b2f_range_result* r);
 
+/* ---- index.remove_ids(sel): faiss IndexFlat::remove_ids (no reference call site) ---------------------------------
+ * Removes the named rows; the survivors keep their order and are renumbered 0 .. ntotal' - 1 (labels above a removed
+ * row shift down).  *nremoved (may be NULL) = rows removed.  Ids outside [0, ntotal) and duplicates are ignored; removing
+ * nothing launches nothing.  Every surviving row keeps its stored bits (fp32 rows; bf16 storage: fl32(mu + x~'), its
+ * scan copy and bias too), and the centre mu stays until reset -- removing every row is not a reset.  The certification
+ * bound is taken again over the survivors, so removing a non-finite row gives the tensor path back.  Synchronous on
+ * return; searches still in flight on any stream finish first.  The device work is an in-place compaction of the rows
+ * above the first removed one: each moved byte read once and written once, no second copy of the rows.             */
+/* ids: host int64 [n], any order */
+B2F_API int b2f_index_remove_ids(b2f_index* idx, int64_t n, const int64_t* ids, int64_t* nremoved);
+/* IDSelectorRange(imin, imax): rows imin <= i < imax */
+B2F_API int b2f_index_remove_range(b2f_index* idx, int64_t imin, int64_t imax, int64_t* nremoved);
+
 /* ---- index.reconstruct(i) / reconstruct_n(i0, n) (SURVEY 8b shim surface) ---------------------- */
 B2F_API int b2f_index_reconstruct(b2f_index* idx, int64_t i0, int64_t n, float* out, int32_t mem, void* stream);
 
@@ -257,6 +270,12 @@ B2F_API int b2f_plan_describe(int64_t nq, int64_t n, int32_t d, int64_t k, int32
  * first `cap` of which are written to tiles[s * cap ..] (tiles may be NULL).  Host logic only (tests).          */
 B2F_API int b2f_plan_unit_work(int32_t tile_units, int32_t units, int32_t round_tiles, int64_t db_tiles, int32_t kprime,
                        int32_t unit, int32_t seg_info[14], int64_t* tiles, int64_t cap, int32_t counts[2]);
+/* How b2f_index_remove_ids plans a removal of ids [n] from ntotal rows (host logic only, no GPU): the sorted disjoint
+ * runs it removes, runs[2 j] <= row < runs[2 j + 1] (*nruns of them; runs: room for 2 n, or NULL); the new row of every
+ * row, dest[ntotal] (-1: removed; or NULL); and the compaction tiles for rows of row_bytes bytes (*ntiles of them, the
+ * first cap written to tiles[3 t ..]: first source row, then [first, last + 1) of the tiles it waits for).           */
+B2F_API int b2f_remove_plan(int64_t ntotal, int64_t n, const int64_t* ids, int64_t row_bytes, int64_t* runs, int64_t* nruns,
+                            int64_t* dest, int64_t* tiles, int64_t cap, int64_t* ntiles);
 B2F_API int b2f_index_stats(const b2f_index* idx, b2f_stats* out);
 B2F_API const char* b2f_last_error(void);
 B2F_API int b2f_version(void);

@@ -16,6 +16,8 @@ from ._capi import (  # noqa: F401
 from .index import (  # noqa: F401
     METRIC_INNER_PRODUCT,
     METRIC_L2,
+    IDSelectorBatch,
+    IDSelectorRange,
     IndexFlat,
     IndexFlatIP,
     IndexFlatL2,

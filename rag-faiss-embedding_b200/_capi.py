@@ -91,6 +91,8 @@ PROTOTYPES = {
     "b2f_range_result_fetch": (ctypes.c_int, [_vp, _vp, _vp, _i32, _vp]),
     "b2f_range_result_info": (ctypes.c_int, [_vp, ctypes.POINTER(_i64)]),
     "b2f_range_result_destroy": (ctypes.c_int, [_vp]),
+    "b2f_index_remove_ids": (ctypes.c_int, [_vp, _i64, _vp, ctypes.POINTER(_i64)]),
+    "b2f_index_remove_range": (ctypes.c_int, [_vp, _i64, _i64, ctypes.POINTER(_i64)]),
     "b2f_index_reconstruct":(ctypes.c_int, [_vp, _i64, _i64, _vp, _i32, _vp]),
     "b2f_index_write": (ctypes.c_int, [_vp, ctypes.c_char_p]),
     "b2f_index_read": (ctypes.c_int, [ctypes.c_char_p, _i32, _i32, ctypes.POINTER(_vp)]),
@@ -110,6 +112,7 @@ PROTOTYPES = {
     "b2f_plan_describe": (ctypes.c_int, [_i64, _i64, _i32, _i64, _i32, ctypes.POINTER(_i32)]),
     "b2f_plan_unit_work": (ctypes.c_int, [_i32, _i32, _i32, _i64, _i32, _i32, ctypes.POINTER(_i32), ctypes.POINTER(_i64), _i64,
                                           ctypes.POINTER(_i32)]),
+    "b2f_remove_plan": (ctypes.c_int, [_i64, _i64, _vp, _i64, _vp, ctypes.POINTER(_i64), _vp, _vp, _i64, ctypes.POINTER(_i64)]),
     "b2f_index_stats": (ctypes.c_int, [_vp, ctypes.POINTER(Stats)]),
     "b2f_last_error": (ctypes.c_char_p, []),
     "b2f_version": (ctypes.c_int, []),

@@ -6,12 +6,13 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <mutex>
 #include <new>
 #include <vector>
 
-#include "common.cuh"
+#include "remove.cuh"
 
 namespace b2f {
 
@@ -131,9 +132,12 @@ struct b2f_index {
     cudaEvent_t ev_done = nullptr;    // recorded at the end of every search (searches return without synchronising)
     cudaStream_t last_stream = nullptr;
     bool search_recorded = false;
-    cudaEvent_t ev_ingest = nullptr;  // recorded behind every add on the stream it was enqueued on
+    cudaEvent_t ev_ingest = nullptr;  // recorded behind every add (and removal) on the stream it was enqueued on
     cudaStream_t last_add_stream = nullptr;
     bool add_recorded = false;
+    uint32_t* rm_flags = nullptr;     // device, grow-only, zeroed once: the compaction's ticket + per-tile "read" flags
+    int64_t rm_flag_words = 0;
+    uint32_t rm_epoch = 0;            // the flag value of the latest compaction launch (one new value per launch)
     // profiling: a ring of event sets so that timing never forces a host synchronisation inside a search
     struct ProfSlot {
         cudaEvent_t t0 = nullptr, t1 = nullptr;
@@ -609,6 +613,7 @@ int b2f_index_destroy(b2f_index* ix) {
     if (ix->pinned) cudaFreeHost(ix->pinned);
     if (ix->host_flag) cudaFreeHost(ix->host_flag);
     cudaFree(ix->totals);
+    cudaFree(ix->rm_flags);
     for (cudaEvent_t e : ix->ev) cudaEventDestroy(e);
     if (ix->ev_done) cudaEventDestroy(ix->ev_done);
     if (ix->ev_ingest) cudaEventDestroy(ix->ev_ingest);
@@ -1714,6 +1719,135 @@ int b2f_index_reconstruct(b2f_index* ix, int64_t i0, int64_t n, float* out, int3
         B2F_CUDA(cudaMemcpyAsync(out, ix->ws, bytes, cudaMemcpyDeviceToHost, st));
     }
     if (mem == B2F_MEM_HOST) B2F_CUDA(cudaStreamSynchronize(st));
+    return B2F_OK;
+}
+
+// ---- remove_ids -------------------------------------------------------------------------------------
+// faiss IndexFlatCodes::remove_ids: the rows of `runs` (sorted, disjoint, inside [0, ntotal)) go, the survivors keep their
+// order and are renumbered from 0.  Every surviving row keeps its bits in all three arrays; the centre stays; the stats are
+// taken again over the survivors, so a removed non-finite row no longer spoils certification; Adapt stays (speed only).
+static int remove_runs_locked(b2f_index* ix, const std::vector<int64_t>& runs, int64_t* nremoved) {
+    const int64_t nr = (int64_t)runs.size() / 2;
+    int64_t removed = 0;
+    for (int64_t j = 0; j < nr; j++) removed += runs[2 * j + 1] - runs[2 * j];
+    if (nremoved) *nremoved = removed;
+    if (removed == 0) return B2F_OK;
+    DeviceGuard g(ix->device);
+    cudaStream_t st = ix->stream;
+    B2F_TRY(enter_stream(ix, g, st));
+    // Until now rows were only ever appended.  A search, range search, device reconstruct or write may still be reading
+    // them on any stream: all of it finishes before a row is overwritten (as before ensure_capacity's copies).
+    B2F_CUDA(cudaDeviceSynchronize());
+    const int64_t first = runs[0], n_new = ix->ntotal - removed;
+    if (ix->ntotal - first > removed) {   // survivors above the first removed row: they move
+        struct Arr {
+            void* base;
+            int64_t row_bytes;
+        } arrs[3] = {{ix->rows_f32, (int64_t)ix->d * 4}, {ix->scan, ix->dpad * 2}, {ix->norms, 4}};
+        int64_t tiles = 0;
+        for (const Arr& a : arrs)
+            if (a.base) tiles = std::max(tiles, remove_tiles(first, ix->ntotal, a.row_bytes));
+        std::vector<int64_t> words;
+        remove_runs_layout(runs, words);
+        const auto carve = [&](Bump& b, int64_t** runs_dev, RemoveSpan** spans) {
+            *runs_dev = b.take<int64_t>(words.size());
+            *spans = b.take<RemoveSpan>((size_t)tiles);
+        };
+        int64_t* runs_dev = nullptr;
+        RemoveSpan* spans = nullptr;
+        Bump layout(nullptr, SIZE_MAX);
+        carve(layout, &runs_dev, &spans);
+        B2F_TRY(ensure_ws(ix, layout.off));
+        Bump bump(ix->ws, ix->ws_bytes);
+        carve(bump, &runs_dev, &spans);
+        B2F_CUDA(cudaMemcpyAsync(runs_dev, words.data(), words.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+        const RemoveRuns rr = remove_runs_view(runs_dev, nr);
+        const int64_t need = 1 + tiles;
+        if (need > ix->rm_flag_words) {
+            cudaFree(ix->rm_flags);
+            ix->rm_flags = nullptr;
+            ix->rm_flag_words = 0;
+            cudaError_t e = cudaMalloc(&ix->rm_flags, (size_t)need * 4);
+            if (e == cudaSuccess) e = cudaMemset(ix->rm_flags, 0, (size_t)need * 4);
+            if (e != cudaSuccess) {
+                cudaGetLastError();
+                set_error("remove: %lld flag words: %s", (long long)need, cudaGetErrorString(e));
+                return B2F_ENOMEM;
+            }
+            ix->rm_flag_words = need;
+            ix->rm_epoch = 0;
+        }
+        for (const Arr& a : arrs) {
+            if (!a.base) continue;   // bf16 storage keeps no fp32 rows
+            if (++ix->rm_epoch == 0) ix->rm_epoch = 1;   // 0 is what fresh flags hold
+            B2F_TRY(launch_remove_compact(a.base, a.row_bytes, rr, first, ix->ntotal, spans, ix->rm_flags, ix->rm_epoch, st));
+            ix->st.launches += 2;
+        }
+    }
+    B2F_CUDA(cudaMemsetAsync(ix->stats, 0, 2 * sizeof(float), st));
+    const float* mu = ix->mu_set ? ix->centre : nullptr;
+    if (n_new > 0) {
+        if (ix->storage == B2F_STORE_F32)   // ingest's own arithmetic over the fp32 rows, writing nothing but the stats
+            B2F_TRY(launch_ingest(ix->rows_f32, n_new, ix->d, nullptr, nullptr, ix->dpad, nullptr, ix->stats, mu, 0, 0, st));
+        else
+            B2F_TRY(launch_scan_stats(ix->scan, n_new, ix->d, ix->dpad, mu, ix->stats, st));
+        ix->st.launches++;
+    }
+    ix->ntotal = n_new;
+    ix->stats_dirty = true;
+    B2F_TRY(record_ingest(ix, st));
+    B2F_CUDA(cudaStreamSynchronize(st));   // faiss semantics: done on return
+    return B2F_OK;
+}
+
+int b2f_index_remove_ids(b2f_index* ix, int64_t n, const int64_t* ids, int64_t* nremoved) {
+    if (nremoved) *nremoved = 0;
+    if (!ix || n < 0 || (n > 0 && !ids)) {
+        set_error("remove_ids: bad arguments");
+        return B2F_EINVAL;
+    }
+    std::lock_guard<std::mutex> lk(ix->mu);
+    return remove_runs_locked(ix, remove_runs_from_ids(ix->ntotal, n, ids), nremoved);
+}
+
+int b2f_index_remove_range(b2f_index* ix, int64_t imin, int64_t imax, int64_t* nremoved) {
+    if (nremoved) *nremoved = 0;
+    if (!ix) {
+        set_error("index is NULL");
+        return B2F_EINVAL;
+    }
+    std::lock_guard<std::mutex> lk(ix->mu);
+    const int64_t a = imin > 0 ? imin : 0, b = imax < ix->ntotal ? imax : ix->ntotal;
+    std::vector<int64_t> runs;
+    if (a < b) runs = {a, b};
+    return remove_runs_locked(ix, runs, nremoved);
+}
+
+int b2f_remove_plan(int64_t ntotal, int64_t n, const int64_t* ids, int64_t row_bytes, int64_t* runs, int64_t* nruns, int64_t* dest,
+                    int64_t* tiles, int64_t cap, int64_t* ntiles) {
+    if (ntotal < 0 || n < 0 || (n > 0 && !ids) || row_bytes <= 0 || !nruns || !ntiles || cap < 0) {
+        set_error("remove_plan: bad arguments");
+        return B2F_EINVAL;
+    }
+    const std::vector<int64_t> r = remove_runs_from_ids(ntotal, n, ids);
+    const int64_t nr = (int64_t)r.size() / 2;
+    *nruns = nr;
+    if (runs) memcpy(runs, r.data(), r.size() * sizeof(int64_t));
+    std::vector<int64_t> words;
+    remove_runs_layout(r, words);
+    const RemoveRuns rr = remove_runs_view(words.data(), nr);
+    if (dest)
+        for (int64_t s = 0; s < ntotal; s++) dest[s] = remove_dest(rr, s, 0, nr);
+    *ntiles = 0;
+    if (nr == 0) return B2F_OK;
+    const int64_t first = r[0], tr = remove_tile_rows(row_bytes);
+    *ntiles = remove_tiles(first, ntotal, row_bytes);
+    for (int64_t t = 0; tiles && t < *ntiles && t < cap; t++) {
+        const RemoveSpan sp = remove_tile_span(rr, first, ntotal, tr, t);
+        tiles[3 * t] = sp.s0;
+        tiles[3 * t + 1] = sp.w0;
+        tiles[3 * t + 2] = sp.w1;
+    }
     return B2F_OK;
 }
 

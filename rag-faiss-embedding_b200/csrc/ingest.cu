@@ -2,7 +2,7 @@
 // K7 (fused encoder epilogue: CLS / masked-mean pool, optional L2 normalise, written straight into
 // index storage), query preparation for the tensor path, and the synthetic-row generator.
 // All HBM-bound elementwise / row-reduction work: one warp (or CTA) per row, 16-byte accesses.
-#include "common.cuh"
+#include "remove.cuh"
 
 namespace b2f {
 
@@ -22,6 +22,13 @@ __device__ __forceinline__ double warp_sum(double v) {
     return v;
 }
 
+// bf16 storage: the authoritative element r = fl32(m + xb) of a stored (centred, rounded) element xb, and what the fp32
+// addition loses, (r - m) - xb.  The ingest and the stats taken again after a removal (scan_stats_kernel) both use it.
+__device__ __forceinline__ float auth_loss(float m, float xb, float& r) {
+    r = m + xb;
+    return (float)((double)r - ((double)m + (double)xb));
+}
+
 // Writes one element group of a row to every derived store and returns (bf16(x)^2, (x-bf16(x))^2).
 // bf16_auth: the index keeps no fp32 rows -- the authoritative row IS r = fl32(m + bf16(x - m)); then the "rounding
 // error" of the scan copy is what the fp32 addition loses, (r - m) - bf16(x - m), and *r_out receives r.
@@ -36,8 +43,8 @@ __device__ __forceinline__ void emit_elem(float x, int64_t row, int col, int d, 
     nn = fmaf(xb, xb, nn);
     float e = xc - xb;
     if (bf16_auth) {
-        const float r = m + xb;
-        e = (float)((double)r - ((double)m + (double)xb));
+        float r;
+        e = auth_loss(m, xb, r);
         if (r_out) *r_out = r;
     }
     ee = fmaf(e, e, ee);
@@ -119,7 +126,8 @@ int launch_mean_finish(int64_t m, int d, float* mu, unsigned long long* acc, cud
 // IP: -mu.x).  Embeddings share a large common component (the reference's own index: |x| ~ 7.7 with relative
 // neighbour gaps of 1e-4; a random-init encoder: all cosines > 0.95), and bf16 rounding error scales with the
 // magnitude of what is rounded: centred, the certification bound is 5-30x tighter on such data.
-// stats[0] = max |x~'|^2, stats[1] = max |x' - x~'|^2 over every row ever ingested
+// stats[0] = max |x~'|^2, stats[1] = max |x' - x~'|^2 over every row ingested since the index was created or reset, or,
+// after a removal, over the rows that survived it (taken again with this per-row arithmetic)
 // bf16_auth (bf16 storage): there are no fp32 rows; the authoritative row is r = fl32(mu + x~'), so the IP bias is
 // -mu.r and stats[1] bounds |(r - mu) - x~'| (what the fp32 addition loses: ~1e-7 |r|), not the bf16 rounding.
 __global__ void __launch_bounds__(256)
@@ -156,9 +164,9 @@ ingest_kernel(const float* __restrict__ src, int64_t n, int d, float* __restrict
                 float e0 = x.x - b0, e1 = x.y - b1, e2 = x.z - b2, e3 = x.w - b3;
                 if (bf16_auth) {
                     // the authoritative row: r = fl32(mu + x~'); what matters is how far r - mu is from x~'
-                    const float r0 = m4.x + b0, r1 = m4.y + b1, r2 = m4.z + b2, r3 = m4.w + b3;
-                    e0 = (float)((double)r0 - ((double)m4.x + (double)b0)); e1 = (float)((double)r1 - ((double)m4.y + (double)b1));
-                    e2 = (float)((double)r2 - ((double)m4.z + (double)b2)); e3 = (float)((double)r3 - ((double)m4.w + (double)b3));
+                    float r0, r1, r2, r3;
+                    e0 = auth_loss(m4.x, b0, r0); e1 = auth_loss(m4.y, b1, r1);
+                    e2 = auth_loss(m4.z, b2, r2); e3 = auth_loss(m4.w, b3, r3);
                     if (ip_bias) mx += (double)m4.x * r0 + (double)m4.y * r1 + (double)m4.z * r2 + (double)m4.w * r3;
                 }
                 ee = fmaf(e0, e0, ee); ee = fmaf(e1, e1, ee); ee = fmaf(e2, e2, ee); ee = fmaf(e3, e3, ee);
@@ -193,6 +201,54 @@ int launch_ingest(const float* src, int64_t n, int d, float* rows_f32, __nv_bflo
     int64_t blocks = (n + wpb - 1) / wpb;
     if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
     ingest_kernel<<<(unsigned)blocks, wpb * 32, 0, st>>>(src, n, d, rows_f32, scan, dpad, norms, stats, mu, ip_bias, bf16_auth);
+    B2F_CUDA(cudaGetLastError());
+    return B2F_OK;
+}
+
+// stats over the survivors of a bf16-storage index, from its scan copy: the per-row arithmetic of ingest_kernel's
+// bf16_auth branch (same lanes, same fmaf order, the same auth_loss), so the maxima equal an ingest of the same rows
+__global__ void __launch_bounds__(256)
+scan_stats_kernel(const __nv_bfloat16* __restrict__ scan, int64_t n, int d, int64_t dpad, const float* __restrict__ mu,
+                  float* __restrict__ stats) {
+    const int lane = threadIdx.x & 31;
+    const int64_t wpg = (int64_t)gridDim.x * (blockDim.x >> 5);
+    float max_nn = 0.f, max_ee = 0.f;
+    for (int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); row < n; row += wpg) {
+        float nn = 0.f, ee = 0.f, r;
+        if ((d & 3) == 0) {
+            for (int c = lane * 4; c < d; c += 128) {
+                const uint2 pk = *reinterpret_cast<const uint2*>(scan + row * dpad + c);
+                const __nv_bfloat162 lo = *reinterpret_cast<const __nv_bfloat162*>(&pk.x), hi = *reinterpret_cast<const __nv_bfloat162*>(&pk.y);
+                const float4 m4 = mu ? __ldg(reinterpret_cast<const float4*>(mu + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                const float b0 = __low2float(lo), b1 = __high2float(lo), b2 = __low2float(hi), b3 = __high2float(hi);
+                nn = fmaf(b0, b0, nn); nn = fmaf(b1, b1, nn); nn = fmaf(b2, b2, nn); nn = fmaf(b3, b3, nn);
+                const float e0 = auth_loss(m4.x, b0, r), e1 = auth_loss(m4.y, b1, r), e2 = auth_loss(m4.z, b2, r), e3 = auth_loss(m4.w, b3, r);
+                ee = fmaf(e0, e0, ee); ee = fmaf(e1, e1, ee); ee = fmaf(e2, e2, ee); ee = fmaf(e3, e3, ee);
+            }
+        } else {
+            for (int c = lane; c < d; c += 32) {
+                const float xb = __bfloat162float(scan[row * dpad + c]);
+                nn = fmaf(xb, xb, nn);
+                const float e = auth_loss(mu ? mu[c] : 0.f, xb, r);
+                ee = fmaf(e, e, ee);
+            }
+        }
+        nn = warp_sum(nn);
+        ee = warp_sum(ee);
+        max_nn = fmaxf(max_nn, nn);
+        max_ee = fmaxf(max_ee, ee);
+    }
+    if (lane == 0) {
+        atomic_max_nonneg(stats, max_nn);
+        atomic_max_nonneg(stats + 1, max_ee);
+    }
+}
+
+int launch_scan_stats(const __nv_bfloat16* scan, int64_t n, int d, int64_t dpad, const float* mu, float* stats, cudaStream_t st) {
+    if (n <= 0) return B2F_OK;
+    int64_t blocks = (n + 7) / 8;
+    if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
+    scan_stats_kernel<<<(unsigned)blocks, 256, 0, st>>>(scan, n, d, dpad, mu, stats);
     B2F_CUDA(cudaGetLastError());
     return B2F_OK;
 }

@@ -53,6 +53,37 @@ def _torch_stream(t) -> int:
     return h if h != 0 else 1
 
 
+def _id_array(x) -> np.ndarray:
+    """A 1-D array of ids as faiss's wrapper takes it: any integer (or numeric) array, coerced to int64."""
+    if _is_torch(x):
+        x = x.detach().cpu().numpy()
+    x = np.asarray(x)
+    _assert(x.ndim == 1, f"expected a 1-D array of ids, got shape {x.shape}")
+    return np.ascontiguousarray(x, dtype=np.int64)
+
+
+class IDSelectorRange:
+    """faiss.IDSelectorRange(imin, imax): the ids imin <= i < imax."""
+
+    def __init__(self, imin: int, imax: int):
+        self.imin = int(imin)
+        self.imax = int(imax)
+
+
+class IDSelectorBatch:
+    """faiss.IDSelectorBatch(ids) or IDSelectorBatch(n, ids): the first n of ids (any order; duplicates allowed)."""
+
+    def __init__(self, *args):
+        if len(args) == 1:
+            self.ids = _id_array(args[0])
+        elif len(args) == 2:
+            n, ids = int(args[0]), _id_array(args[1])
+            _assert(0 <= n <= ids.shape[0], f"IDSelectorBatch: n={n} but {ids.shape[0]} ids given")
+            self.ids = ids[:n]
+        else:
+            raise TypeError("IDSelectorBatch(ids) or IDSelectorBatch(n, ids)")
+
+
 class IndexFlat:
     """Exact (brute-force) index with faiss.IndexFlat's surface."""
 
@@ -295,6 +326,18 @@ class IndexFlat:
 
     def reset(self):
         C.check(self._lib.b2f_index_reset(self._h))
+
+    def remove_ids(self, x) -> int:
+        """index.remove_ids(sel) (faiss IndexFlat::remove_ids): x is an IDSelectorRange, an IDSelectorBatch or a 1-D
+        integer array (numpy or torch).  The survivors keep their order and are renumbered from 0, so every label above
+        a removed row shifts down; ids outside [0, ntotal) are ignored.  Returns the number of rows removed."""
+        n = ctypes.c_int64(0)
+        if isinstance(x, IDSelectorRange):
+            C.check(self._lib.b2f_index_remove_range(self._h, x.imin, x.imax, ctypes.byref(n)))
+        else:
+            ids = x.ids if isinstance(x, IDSelectorBatch) else _id_array(x)
+            C.check(self._lib.b2f_index_remove_ids(self._h, ids.shape[0], ids.ctypes.data, ctypes.byref(n)))
+        return int(n.value)
 
     def reconstruct(self, key: int) -> np.ndarray:
         out = np.empty((self.d,), np.float32)

@@ -20,7 +20,7 @@ from typing import Callable, List, Optional, Tuple
 import numpy as np
 
 from . import _capi as C
-from .index import METRIC_L2, IndexFlat
+from .index import METRIC_L2, IDSelectorBatch, IDSelectorRange, IndexFlat, _id_array
 
 
 def partition_rows(n: int, world: int) -> List[Tuple[int, int]]:
@@ -51,6 +51,21 @@ class SegmentMap:
         if not self.local_starts:
             return 0
         return self.global_starts[0] if len(self.local_starts) == 1 else None
+
+    def remove(self, labels: np.ndarray) -> np.ndarray:
+        """Takes the sorted unique global labels `labels` out: returns the local rows of this shard that hold them, and
+        renumbers what is left as remove_ids does -- each segment's global start moves down by the labels removed below
+        it, its local start by the local rows removed below it; empty segments go, contiguous ones merge."""
+        starts = self.local_starts + [self.nlocal]
+        local = []
+        kept = SegmentMap()
+        for i, (ls, gs) in enumerate(zip(self.local_starts, self.global_starts)):
+            cnt = starts[i + 1] - ls
+            lo, hi = np.searchsorted(labels, [gs, gs + cnt])
+            local.append(labels[lo:hi] - gs + ls)
+            kept.append(gs - int(lo), cnt - int(hi - lo))
+        self.local_starts, self.global_starts, self.nlocal = kept.local_starts, kept.global_starts, kept.nlocal
+        return np.concatenate(local) if local else np.zeros(0, np.int64)
 
     def to_global_numpy(self, local_ids: np.ndarray) -> np.ndarray:
         out = local_ids.astype(np.int64, copy=True)
@@ -307,6 +322,22 @@ class ShardedIndexFlat:
         if was_numpy and not isinstance(Dm, np.ndarray):
             Dm, Im = Dm.cpu().numpy(), Im.cpu().numpy()
         return Dm, Im
+
+    def remove_ids(self, x) -> int:
+        """index.remove_ids(sel) over the whole sharded index: x (IDSelectorRange, IDSelectorBatch or 1-D integer array)
+        names global labels, the same on every rank.  Each rank removes the rows it holds and renumbers its segments;
+        the labels of the concatenated database shift down as on one index.  No communication.  Returns the number of
+        labels removed (the same on every rank)."""
+        if isinstance(x, IDSelectorRange):
+            labels = np.arange(max(x.imin, 0), min(x.imax, self.ntotal), dtype=np.int64)
+        else:
+            labels = x.ids if isinstance(x, IDSelectorBatch) else _id_array(x)
+            labels = np.unique(labels[(labels >= 0) & (labels < self.ntotal)])
+        local = self.segments.remove(labels)
+        if len(local):
+            self.local.remove_ids(local)
+        self.ntotal -= int(len(labels))
+        return int(len(labels))
 
     def reset(self):
         self.local.reset()

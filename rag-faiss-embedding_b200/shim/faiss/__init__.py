@@ -17,6 +17,8 @@ if "rag_faiss_embedding_b200" not in _sys.modules and _ilu.find_spec("rag_faiss_
 from rag_faiss_embedding_b200 import (  # noqa: E402,F401
     METRIC_INNER_PRODUCT,
     METRIC_L2,
+    IDSelectorBatch,
+    IDSelectorRange,
     IndexFlat,
     IndexFlatIP,
     IndexFlatL2,

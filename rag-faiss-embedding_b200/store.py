@@ -4,7 +4,7 @@ index), method names, argument meaning, return shapes and error behaviour, so da
 query.py:36 and initialize_rag.py:57-61 work against it as they do against the original.
 
 Differences, all additive: `search_many` (a batch of queries in one device call -- the reference
-forces nq=1 at faiss_store.py:61), `metric="ip"`, and the instance is not forced to be a process-wide
+forces nq=1 at faiss_store.py:61), `remove_documents`, `metric="ip"`, and the instance is not forced to be a process-wide
 singleton unless `singleton=True` is requested through `get_instance()`.
 """
 from __future__ import annotations
@@ -79,6 +79,19 @@ class FAISSVectorStore:
         dist, rows = self.index.search(q, k)
         mapped = [[self.doc_ids[r] for r in row if r != -1 and r < len(self.doc_ids)] for row in rows]
         return dist, mapped
+
+    def remove_documents(self, doc_ids: Sequence[int]) -> int:
+        """Removes every row whose document id is in doc_ids, and the same positions from self.doc_ids, so that rows and
+        ids stay aligned (and save_index writes a .mapping that matches the file).  Returns the number of rows removed."""
+        drop = set(doc_ids)
+        rows = [i for i, d in enumerate(self.doc_ids) if d in drop]
+        if not rows:
+            return 0
+        n = self.index.remove_ids(np.asarray(rows, dtype=np.int64))
+        gone = set(rows)
+        self.doc_ids = [d for i, d in enumerate(self.doc_ids) if i not in gone]
+        log.info("removed %d vectors", n)
+        return n
 
     # faiss_store.py:83-97
     def save_index(self, filepath: Optional[str] = None):
