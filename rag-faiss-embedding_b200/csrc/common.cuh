@@ -302,7 +302,6 @@ struct RerankArgs {
     int32_t* fail_list;             // queries that could not be certified (q + q_base), re-run by the closing exact scan
     int32_t* fail_count;            // [0] uncertified queries, [1] of which list overflows, [2..3] u64 list entries
     int32_t q_base;                 // first query of this pass within the whole batch (query chunks)
-    int32_t stage1;                 // LIST merge: candidates tried first on their own (0 = off; see merge_lists_kernel)
     float* fail_tau;                // optional [nq]: exact k-th key found for fail_list[i] (FLT_MAX: none) -- the range pass's input
     const int32_t* out_map;         // optional: query q of this launch writes row out_map[q] of D / I (< 0: skip) and is
                                     // recorded under that index when it fails (range pass over compacted failed queries)
@@ -334,8 +333,8 @@ struct TensorScanLists {  // LIST-mode scratch (device)
     uint8_t* big_flag;    // [nq_pad] big batches: queries the warp-per-query merge passes on to the block kernel
     const float* range_thr;  // optional [nq_pad]: range pass -- fixed per-query thresholds (no shared thresholds, no refresh)
 };
-int plan_tensor_scan(int nq, int64_t n, int d, int kp, TensorScanPlan* plan);
-void plan_force_heap(bool on);   // planning switch of the calling thread: per-thread heaps instead of LIST mode (k' = 32 / 64)
+// force_heap: per-thread heaps instead of LIST mode (k' = 32 / 64)
+int plan_tensor_scan(int nq, int64_t n, int d, int kp, bool force_heap, TensorScanPlan* plan);
 int plan_unit_work(int T, int U, int R, int64_t ntiles, int kp, int unit, int32_t* seg_info, int64_t* tiles, int64_t cap, int32_t* counts);
 int launch_tensor_scan(const __nv_bfloat16* scan, int64_t dpad, const float* norms, int64_t n, int metric,
                        const __nv_bfloat16* qb, int nq, int nq_pad, const TensorScanPlan& plan, float* pk,

@@ -132,19 +132,6 @@ __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 // TMA load issued by either CTA of the pair; the bytes are credited to the LEADER CTA's mbarrier
-// Same load with an L2 cache policy (database blocks that several units read: keep them, evict_last)
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ void tma_load_2d_pair_hint(void* dst, const CUtensorMap* map, int x, int y, uint64_t* bar, uint64_t policy) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(
-            smem_u32(dst)),
-        "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar) & kPeerBitMask), "r"(x), "r"(y), "l"(policy)
-        : "memory");
-}
 __device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* map, int x, int y, uint64_t* bar) {
     asm volatile(
         "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
@@ -241,10 +228,7 @@ struct ListArgs {
     int nl_stride;       // lists per query allocated (the largest per-tile list count)
     int cap;             // entries per list
     float* final_thr;    // [nq_pad * nsplits]  threshold the list was pruned against at the end of the stream
-    int early;           // 1: scheduled threshold refreshes happen before the wait for the tile's accumulator
-    int period_mask;     // refresh every (period_mask + 1) tiles after the first 32 (power of two - 1)
-    int l2_keep;         // 1: database blocks are loaded with an evict_last L2 policy (several units read each block)
-    int die_mode;        // > 0: die-aware unit assignment; the value selects the smid -> die guess
+    bool die_aware;      // die-aware unit assignment (takes tickets from die_ctr)
     int32_t* die_ctr;    // [4] ticket counters (zero between launches)
     int bal_T;           // balanced work split: query tile units (pair tiles when PAIR) ...
     int bal_U;           // ... shared evenly by this many units (CTAs / CTA pairs); T <= U
@@ -509,7 +493,7 @@ tensor_scan_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         // pulls every block across the die-to-die L2 fabric.  Logical units are therefore handed out in the order of
         // their position inside the tile (frac(u T / U)): the hardware units of die 0 take tickets from the front of
         // that order, those of die 1 from the back, so each die serves (about) one half of every round's tiles.
-        if (la.die_mode > 0) {
+        if (la.die_aware) {
             // (in the spare bytes behind the TMEM base holder: the pair variant has no room for static shared memory)
             int& s_unit = *reinterpret_cast<int*>(smem + L::tmem_off + 8);
             int& s_idx = *reinterpret_cast<int*>(smem + L::tmem_off + 12);
@@ -517,8 +501,7 @@ tensor_scan_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
             if (threadIdx.x == 0 && cta_rank == 0) {
                 uint32_t smid;
                 asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-                const int die = la.die_mode == 1 ? (smid >= (uint32_t)(kNumSMs / 2) ? 1 : 0)
-                              : la.die_mode == 2 ? (int)(smid & 1u) : (int)((smid >> 1) & 1u);
+                const int die = smid >= (uint32_t)(kNumSMs / 2) ? 1 : 0;
                 const int t = atomicAdd(la.die_ctr + die, 1);
                 s_idx = die == 0 ? t : U - 1 - t;   // front / back of the position order; U tickets in total, no collision
                 if (atomicAdd(la.die_ctr + 3, 1) == U - 1) {   // every unit has its ticket: re-arm the counters
@@ -655,7 +638,6 @@ tensor_scan_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         {
             int stage = 0;
             uint32_t phase = 0;
-            const uint64_t l2_keep_policy = (PAIR && la.l2_keep) ? l2_policy_evict_last() : 0ull;
 #pragma unroll 1
 #pragma unroll 1
         for (int sgi = 0; sgi < nseg; sgi++) {   // (never unrolled: two copies of the loops below thrash the instruction cache)
@@ -688,8 +670,7 @@ tensor_scan_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                             if constexpr (PAIR) {
                                 // this CTA's half of the 256-row block; the leader's full barrier collects both halves
                                 if (cta_rank == 0) mbar_expect_tx(&full_bar[ustage], 2 * kStageBytes);
-                                if (la.l2_keep) tma_load_2d_pair_hint(sa, &map_x, kb * BK, row0 + (int)cta_rank * (BN / 2), &full_bar[ustage], l2_keep_policy);
-                                else tma_load_2d_pair(sa, &map_x, kb * BK, row0 + (int)cta_rank * (BN / 2), &full_bar[ustage]);
+                                tma_load_2d_pair(sa, &map_x, kb * BK, row0 + (int)cta_rank * (BN / 2), &full_bar[ustage]);
                             } else {
                                 mbar_expect_tx(&full_bar[ustage], kStageBytes);
                                 if constexpr (!QRES) tma_load_2d(sa, &map_q, kb * BK, qt * BM, &full_bar[ustage]);
@@ -970,12 +951,11 @@ tensor_scan_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                 const uint32_t acc_phase = (gt >> 1) & 1;
                 // Scheduled refresh of the shared threshold BEFORE waiting for the tile's accumulator: the ~1.4 us
                 // of L2 round trips overlap the MMAs the thread would wait for anyway, and no accumulator registers
-                // are live yet (same-box A/B: the refreshes inside the tile cost 3-4% of the kernel).
-                if (la.early && active && t >= 2 && (t < 8 || (t < 32 && (t & 3) == 0) || (t & la.period_mask) == 0)) refresh(true);
-                // which chunks of this tile start with a refresh: all of tile 0, every other one of tile 1, then (only
-                // without the early refresh above) the first chunk of scheduled tiles
-                const uint32_t rmask = t == 0 ? 0xffffffffu : (t == 1 ? 0x55555555u
-                                     : ((!la.early && (t < 8 || (t < 32 && (t & 3) == 0) || (t & 15) == 0)) ? 1u : 0u));
+                // are live yet (same-box A/B: the refreshes inside the tile cost 3-4% of the kernel).  After the first 32
+                // tiles, every 32nd (same-box A/B over periods 4..128: 32 is the flat optimum, profiles/r01_j_ab_refresh.txt).
+                if (active && t >= 2 && (t < 8 || (t < 32 && (t & 3) == 0) || (t & 31) == 0)) refresh(true);
+                // which chunks of this tile start with a refresh: all of tile 0, every other one of tile 1
+                const uint32_t rmask = t == 0 ? 0xffffffffu : (t == 1 ? 0x55555555u : 0u);
                 mbar_wait(&bias_full[acc], acc_phase);
                 mbar_wait(&tmem_full[acc], acc_phase);
                 tc_fence_after();
@@ -1404,10 +1384,6 @@ merge_lists_kernel(const uint2* __restrict__ cand, const int32_t* __restrict__ c
     const float tc = dec_key(s_tc_enc);
     const int nc1 = M < kp ? M : kp;
     const float bound1 = (M > kp || big) ? fminf(sk[kp - 1], tc) : tc;   // big: rows beyond the kept entries have keys >= sk[k' - 1]
-    // Big batches are bound by the random row reads of the re-rank (8192 queries x 32 candidates x 1.5 KB = 400 MB), so
-    // they first try the best `stage1` coarse candidates alone: every other row has a coarse key >= sk[stage1], and on
-    // data the bf16 pass separates well that already certifies ~95% of the queries with half the rows read.  (Small
-    // batches are latency-bound: a failed first stage would cost them a dependent round trip, so they skip it.)
     __shared__ float s_tau_last;   // exact k-th key of the last re-rank (what a failed query hands to the range pass)
     bool cert = false;
     if (ra.range) {
@@ -1416,9 +1392,7 @@ merge_lists_kernel(const uint2* __restrict__ cand, const int32_t* __restrict__ c
         if (M <= RANK_MAX) cert = rerank_block(ra, q, sk, si, M, tc, false, ek, ei, &s_tau_last);
         else if (tid == 0) s_tau_last = FLT_MAX;
     } else {
-        if (ra.certify && ra.stage1 >= ra.k && ra.stage1 < nc1)
-            cert = rerank_block(ra, q, sk, si, ra.stage1, fminf(sk[ra.stage1], tc), false, ek, ei, &s_tau_last);
-        if (!cert) cert = rerank_block(ra, q, sk, si, nc1, bound1, M < kp, ek, ei, &s_tau_last);
+        cert = rerank_block(ra, q, sk, si, nc1, bound1, M < kp, ek, ei, &s_tau_last);
         if (!cert && ra.certify && !big && M > kp && M <= RANK_MAX) {
             // every list entry: rows outside the lists have coarse keys above T_c
             cert = rerank_block(ra, q, sk, si, M, tc, false, ek, ei, &s_tau_last);
@@ -1434,8 +1408,10 @@ merge_lists_kernel(const uint2* __restrict__ cand, const int32_t* __restrict__ c
 // end-of-stream pruning a query of a big batch has ~80 list entries, so one warp can do everything a CTA does: 64
 // queries in flight per SM instead of five.  Queries it cannot hold (more than WM_MAX entries, an overflowed list)
 // are flagged and answered by the block kernel launched right behind (it skips unflagged queries).  Measured gain:
-// 8 % of the merge at 8192 queries, a loss below that -- it is used from 8192 queries up.
+// 8 % of the merge at 8192 queries, a loss below that -- it is used from 8192 queries up (same-box A/B, r02n: 8192
+// queries 125 -> 114 us, 4096 queries 78 -> 82 us, 1024 queries 47 -> 73 us).
 constexpr int WM_WARPS = 8;      // queries per CTA
+constexpr int WM_MIN_NQ = 8192;  // batch size from which the warp kernel runs first
 constexpr int WM_MAX = 128;      // list entries per query
 constexpr int WM_LISTS = 64;     // lists per query
 
@@ -1558,14 +1534,11 @@ merge_lists_warp_kernel(const uint2* __restrict__ cand, const int32_t* __restric
         si[rank] = (int32_t)(uint32_t)(mine & 0xffffffffu);
     }
     __syncwarp();
-    // exact re-rank + certification: first stage, the k' best, every list entry (see merge_lists_kernel)
+    // exact re-rank + certification: the k' best, then every list entry (see merge_lists_kernel)
     const int nc1 = M < kp ? M : kp;
     const float bound1 = (M > kp) ? fminf(sk[kp - 1], tc) : tc;
-    bool cert = false;
     float tau = FLT_MAX;
-    if (ra.certify && ra.stage1 >= ra.k && ra.stage1 < nc1)
-        cert = warp_rerank(ra, q, sk, si, ra.stage1, fminf(sk[ra.stage1], tc), false, s_ek[warp], s_ei[warp], lane, tau);
-    if (!cert) cert = warp_rerank(ra, q, sk, si, nc1, bound1, M < kp, s_ek[warp], s_ei[warp], lane, tau);
+    bool cert = warp_rerank(ra, q, sk, si, nc1, bound1, M < kp, s_ek[warp], s_ei[warp], lane, tau);
     if (!cert && ra.certify && M > kp) {
         cert = warp_rerank(ra, q, sk, si, M, tc, false, s_ek[warp], s_ei[warp], lane, tau);
         if (lane == 0 && cert) atomicAdd(ra.fail_count + 4, 1);
@@ -1782,14 +1755,10 @@ range_collect_kernel(const uint2* __restrict__ cand, const int32_t* __restrict__
 
 }  // namespace k2
 
-// Planning switch of the calling thread (index.cu sets it around the planning of one search): skip LIST mode.  An index
-// whose data defeats the shared thresholds -- rows stored in an order that puts a query's best rows into one or two
-// lists, so that the thresholds never tighten and the lists overflow -- is searched with per-thread heaps instead (exact
-// top-k' of every split whatever the order, ~6x the epilogue cost), for k' = 32 / 64.
-static thread_local bool t_force_heap = false;
-void plan_force_heap(bool on) { t_force_heap = on; }
-
-int plan_tensor_scan(int nq, int64_t n, int d, int kp, TensorScanPlan* plan) {
+// force_heap: skip LIST mode.  An index whose data defeats the shared thresholds -- rows stored in an order that puts a
+// query's best rows into one or two lists, so that the thresholds never tighten and the lists overflow -- is searched
+// with per-thread heaps instead (exact top-k' of every split whatever the order, ~6x the epilogue cost), for k' = 32 / 64.
+int plan_tensor_scan(int nq, int64_t n, int d, int kp, bool force_heap, TensorScanPlan* plan) {
     if (kp < 8 || kp > 256 || n <= 0 || nq <= 0) return B2F_EINVAL;
     plan->kp = kp;
     plan->nq_tiles = (nq + k2::BM - 1) / k2::BM;
@@ -1804,10 +1773,6 @@ int plan_tensor_scan(int nq, int64_t n, int d, int kp, TensorScanPlan* plan) {
     // many units as query tile units, a few database tiles per unit, and j = ceil(k' / voucher lists of a tile) <=
     // JSLOTS for every tile.
     auto try_list = [&](int tiles, int max_units, int* units_out, int* nv_min_out, int* nseg_max_out) -> bool {
-        {
-            const char* e = getenv("B200FLAT_MAX_UNITS");   // diagnostics: cap the units of a pass
-            if (e && atoi(e) >= 1 && atoi(e) < max_units) max_units = atoi(e);
-        }
         if (tiles > max_units || ntiles < 2) return false;   // more than one wave; a single database tile
         int units = max_units;
         // >= 4 database tiles per unit: a voucher segment (at least half a share) then always has rows to vouch for;
@@ -1836,10 +1801,9 @@ int plan_tensor_scan(int nq, int64_t n, int d, int kp, TensorScanPlan* plan) {
     };
     // (1) CTA pairs halve the L2->SM traffic of the database blocks; worth it once the batch spans several
     //     128-query tiles (an odd tile count wastes half a pair on padding).
-    const bool heap_only = t_force_heap && (kp == 32 || kp == 64);
-    const char* no_pair = getenv("B200FLAT_NO_PAIR");
+    const bool heap_only = force_heap && (kp == 32 || kp == 64);
     int units = 0, nv_min = 1, nseg_max = 1;
-    if (!heap_only && !(no_pair && no_pair[0] == '1') && kblocks <= k2::QRES_MAX_KB && plan->nq_tiles >= 2 &&
+    if (!heap_only && kblocks <= k2::QRES_MAX_KB && plan->nq_tiles >= 2 &&
         (plan->nq_tiles % 2 == 0 || plan->nq_tiles >= 7) && try_list((plan->nq_tiles + 1) / 2, kNumSMs / 2, &units, &nv_min, &nseg_max)) {
         plan->pair_mode = 1;
         plan->list_mode = 1;
@@ -1875,8 +1839,6 @@ int plan_tensor_scan(int nq, int64_t n, int d, int kp, TensorScanPlan* plan) {
         int r = 2 * ((units + plan->tile_units - 1) / plan->tile_units);
         if (r < 2) r = 2;
         if (r > 512) r = 512;
-        const char* e = getenv("B200FLAT_ROUND_TILES");   // diagnostics: database tiles per round of the sweep
-        if (e && atoi(e) >= 1 && atoi(e) <= 4096) r = atoi(e);
         plan->round_tiles = r;
     }
     // expected list length ~ 32 (blind first chunk) + (j + spread) * ln(rows per list / 32); 2.5x headroom
@@ -1949,39 +1911,12 @@ int launch_tensor_scan(const __nv_bfloat16* scan, int64_t dpad, const float* nor
         la.nl_stride = plan.nlists;
         la.cap = plan.list_cap;
         la.final_thr = lists.final_thr;
-        {
-            static int early = -1;
-            if (early < 0) {
-                const char* e = getenv("B200FLAT_EARLY_REFRESH");
-                early = (e && e[0] == '0') ? 0 : 1;
-            }
-            la.early = early;
-            static int period = -1;
-            if (period < 0) {
-                const char* e = getenv("B200FLAT_REFRESH_PERIOD");
-                period = e ? atoi(e) : 32;   // same-box A/B over 4..128: 32 is the flat optimum (profiles/r01_j_ab_refresh.txt)
-                if (period != 2 && period != 4 && period != 8 && period != 16 && period != 32 && period != 64 && period != 128) period = 32;
-            }
-            la.period_mask = period - 1;
-            static int keep = -1;
-            if (keep < 0) {
-                const char* e = getenv("B200FLAT_L2_KEEP");
-                keep = (e && e[0] == '1') ? 1 : 0;
-            }
-            la.l2_keep = keep;
-            static int die_mode = -1;
-            if (die_mode < 0) {
-                const char* e = getenv("B200FLAT_DIE_MODE");
-                die_mode = e ? atoi(e) : 1;
-                if (die_mode < 0 || die_mode > 3) die_mode = 1;
-            }
-            la.die_mode = (lists.die_ctr && plan.tile_units > 1) ? die_mode : 0;   // one query tile: every block has one reader
-            la.die_ctr = lists.die_ctr;
-            la.bal_T = plan.tile_units;
-            la.bal_U = plan.units;
-            la.bal_R = plan.round_tiles;
-            la.range_thr = lists.range_thr;
-        }
+        la.die_aware = lists.die_ctr && plan.tile_units > 1;   // one query tile: every block has one reader
+        la.die_ctr = lists.die_ctr;
+        la.bal_T = plan.tile_units;
+        la.bal_U = plan.units;
+        la.bal_R = plan.round_tiles;
+        la.range_thr = lists.range_thr;
         // lists.shared_thr was filled with 0x7f7f7f7f (3.39e38, "no information yet") by the query-prep kernel
         if (plan.pair_mode)
             return l2 ? k2::launch_k2<0, true, true, true, true>(mq, mx, norms, n, nq, kblocks, plan, pk, pi, la, st)
@@ -2031,12 +1966,7 @@ int launch_merge_lists(const TensorScanLists& lists, int nq, const TensorScanPla
     }
     // big batches: one warp per query first; what it cannot hold is flagged for the block kernel behind it
     const uint8_t* only_flagged = nullptr;
-    static int warp_env = -1;
-    if (warp_env < 0) {
-        const char* e = getenv("B200FLAT_WARP_MERGE");   // diagnostics: 0 = off, n > 1 = batch size from which it is used
-        warp_env = e ? atoi(e) : 8192;   // same-box A/B (r02n): 8192 queries 125 -> 114 us, 4096 queries 78 -> 82 us, 1024: 47 -> 73 us
-    }
-    if (warp_env > 0 && nq >= warp_env && lists.big_flag && plan.nlists <= k2::WM_LISTS && plan.kp <= k2::WM_MAX / 2 && ra.D &&
+    if (nq >= k2::WM_MIN_NQ && lists.big_flag && plan.nlists <= k2::WM_LISTS && plan.kp <= k2::WM_MAX / 2 && ra.D &&
         !ra.range && !ra.out_map) {
         k2::merge_lists_warp_kernel<<<(nq + k2::WM_WARPS - 1) / k2::WM_WARPS, k2::WM_WARPS * 32, 0, st>>>(
             reinterpret_cast<const uint2*>(lists.cand), lists.counts, lists.final_thr, plan.nlists, plan.pair_mode ? 2 * k2::BM : k2::BM,

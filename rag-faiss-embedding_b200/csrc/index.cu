@@ -47,8 +47,8 @@ struct Adapt {
     int range_quiet = 0;           // consecutive range-mode searches whose first pass certified everything
     // Order-robust mode.  A batch whose candidate lists overflowed en masse (rows stored so that a query's best rows sit in
     // one or two lists: the shared thresholds never tighten) switches the index to per-thread heaps for the first pass
-    // (plan_force_heap) plus the range pass for what the heaps cannot certify; LIST mode is tried again after heap_span
-    // searches, and the span doubles every time it fails again.
+    // (plan_tensor_scan's force_heap) plus the range pass for what the heaps cannot certify; LIST mode is tried again after
+    // heap_span searches, and the span doubles every time it fails again.
     int heap_left = 0;             // searches still to run in this mode
     int heap_span = 64;
 
@@ -475,10 +475,11 @@ int tensor_kprime(int k, int slack) {
 // tiles got 4 or 5 whole units, and two passes of 8 tiles were cheaper than one of 16).
 // The planner still evaluates 1..8 equal passes and a few fixed pass sizes with a small cost model (tensor time per
 // unit, floored by the HBM time of one database pass, plus a fixed per-pass overhead) and returns the cheapest.
-int plan_tensor_chunked(int nq, int64_t n, int d, int kp, TensorScanPlan* plan) {
+// force_heap: as plan_tensor_scan's.
+int plan_tensor_chunked(int nq, int64_t n, int d, int kp, bool force_heap, TensorScanPlan* plan) {
     int feasible = nq;
     while (true) {
-        if (plan_tensor_scan(feasible, n, d, kp, plan) == B2F_OK) break;
+        if (plan_tensor_scan(feasible, n, d, kp, force_heap, plan) == B2F_OK) break;
         if (feasible <= 128) return 0;
         feasible = ((feasible / 2 + 127) / 128) * 128;
     }
@@ -487,29 +488,25 @@ int plan_tensor_chunked(int nq, int64_t n, int d, int kp, TensorScanPlan* plan) 
     const double t_hbm = (double)n * dpad * 2.0 / kHbm;
     int best_chunk = feasible;
     double best_cost = 1e30;
-    const char* nb = getenv("B200FLAT_NO_BALANCE");   // diagnostics: "1" = feasibility chunking only
-    const bool balance = !(nb && nb[0] == '1');
     // candidates: 1..8 equal passes, and the fixed pass sizes that fill one wave of pairs (74 / 37 pair tiles) or
     // give every tile many splits -- so that very large batches are cut into LIST-mode passes instead of falling
     // into the multi-wave HEAP selection (the first version of K2, ~6x slower per query)
     int cands[12];
     int nc = 0;
-    for (int m = 1; m <= (balance ? 8 : 1); m++) {
+    for (int m = 1; m <= 8; m++) {
         int chunk = (nq + m - 1) / m;
         chunk = (chunk + 255) / 256 * 256;   // whole pair tiles
         if (chunk > feasible) chunk = m == 1 ? feasible : 0;
         if (chunk >= 256 || m == 1) cands[nc++] = chunk;
     }
-    if (balance) {
-        const int fixed[4] = {74 * 256, 37 * 256, 4096, 2048};
-        for (int i = 0; i < 4; i++)
-            if (fixed[i] < nq && fixed[i] <= feasible) cands[nc++] = fixed[i];
-    }
+    const int fixed[4] = {74 * 256, 37 * 256, 4096, 2048};
+    for (int i = 0; i < 4; i++)
+        if (fixed[i] < nq && fixed[i] <= feasible) cands[nc++] = fixed[i];
     for (int i = 0; i < nc; i++) {
         const int chunk = cands[i];
         if (chunk <= 0) continue;
         TensorScanPlan p{};
-        if (plan_tensor_scan(chunk, n, d, kp, &p) != B2F_OK) continue;
+        if (plan_tensor_scan(chunk, n, d, kp, force_heap, &p) != B2F_OK) continue;
         const int passes = (nq + chunk - 1) / chunk;
         const double waves = p.list_mode ? 1.0 : (double)((p.units + kNumSMs - 1) / kNumSMs);
         // rows every unit streams: LIST mode shares the pass equally (tile_units / units of the database per unit,
@@ -523,7 +520,7 @@ int plan_tensor_chunked(int nq, int64_t n, int d, int kp, TensorScanPlan* plan) 
             best_chunk = chunk;
         }
     }
-    if (plan_tensor_scan(best_chunk, n, d, kp, plan) != B2F_OK) return 0;
+    if (plan_tensor_scan(best_chunk, n, d, kp, force_heap, plan) != B2F_OK) return 0;
     return best_chunk;
 }
 
@@ -670,7 +667,7 @@ int b2f_plan_describe(int64_t nq, int64_t n, int32_t d, int64_t k, int32_t slack
     const int kp = k <= 1024 ? tensor_kprime((int)k, slack) : 0;
     if (kp <= 0) return B2F_OK;
     TensorScanPlan plan{};
-    const int chunk = plan_tensor_chunked((int)nq, n, d, kp, &plan);
+    const int chunk = plan_tensor_chunked((int)nq, n, d, kp, false, &plan);
     if (chunk <= 0) return B2F_OK;
     out[0] = kp;
     out[1] = chunk;
@@ -719,15 +716,6 @@ int b2f_index_stats(const b2f_index* cix, b2f_stats* out) {
 }
 
 // ---- add -------------------------------------------------------------------------------------------
-static bool centring_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("B200FLAT_NO_CENTER");
-        v = (e && e[0] == '1') ? 0 : 1;
-    }
-    return v == 1;
-}
-
 // The scan copy is taken around the mean of the first rows the index sees, fixed from then on: any centre is correct, a
 // representative one makes the bf16 pass far more decisive on embeddings that share a large common component.  bf16
 // storage keeps the same centred copy as its ONLY copy: the authoritative row is then fl32(mu + bf16(x - mu)) -- closer
@@ -743,7 +731,7 @@ static const int64_t kCentreRows = 65536;
 extern "C++" {   // (a template inside the extern "C" block)
 template <class Stage>
 static int take_centre(b2f_index* ix, int64_t n, int64_t piece, cudaStream_t st, Stage&& stage) {
-    if (ix->mu_set || ix->ntotal != 0 || n <= 0 || !centring_enabled()) return B2F_OK;
+    if (ix->mu_set || ix->ntotal != 0 || n <= 0) return B2F_OK;
     const int64_t m = n < kCentreRows ? n : kCentreRows;
     piece = piece >= m ? m : piece / 64 * 64;
     if (piece <= 0) {
@@ -1047,7 +1035,7 @@ constexpr int kRangeCap = 1024;   // failed queries one range pass holds; more g
 constexpr int kRangeListCap = 256;
 
 static int plan_range_pass(int nfail, int64_t n, int d, int kp, TensorScanPlan* plan) {
-    if (plan_tensor_scan(nfail, n, d, kp, plan) != B2F_OK || !plan->list_mode) return B2F_EINVAL;
+    if (plan_tensor_scan(nfail, n, d, kp, false, plan) != B2F_OK || !plan->list_mode) return B2F_EINVAL;
     if (plan->list_cap < kRangeListCap) plan->list_cap = kRangeListCap;   // lists are not pruned: every row at or below the threshold
     return B2F_OK;
 }
@@ -1178,25 +1166,13 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
     // of it because of the unpacking), so every batch size goes to the tensor path there.
     const int scan_max = P.scan_max_nq > 0 ? P.scan_max_nq : (ix->storage == B2F_STORE_BF16 ? 0 : 1);
     int kp = tensor_kprime(k, P.slack);
-    {
-        // diagnostics: B200FLAT_KPRIME=<multiple of 8> forces k' (LIST-mode shapes; same-box A/B of the candidate count)
-        static int kp_env = -1;
-        if (kp_env < 0) {
-            const char* e = getenv("B200FLAT_KPRIME");
-            kp_env = e ? atoi(e) : 0;
-            if (kp_env < 0 || kp_env > 256 || (kp_env & 7)) kp_env = 0;
-        }
-        if (kp_env >= k + 2 && kp > 0) kp = kp_env;
-    }
     if (kp > 0 && P.slack <= 0 && ix->adapt.slack_boost > 0) {  // adaptive slack learned from earlier searches on this index
         int boosted = ((kp + ix->adapt.slack_boost + 7) / 8) * 8;
         if (boosted > 64) kp = boosted <= 256 ? boosted : 256;
     }
     TensorScanPlan plan{};
     const bool heap_first = ix->adapt.heap_left > 0 && P.certify >= 0;
-    plan_force_heap(heap_first);
-    const int chunk_nq = (kp > 0 && ix->ntotal > 0) ? plan_tensor_chunked(nq, ix->ntotal, ix->d, kp, &plan) : 0;
-    plan_force_heap(false);
+    const int chunk_nq = (kp > 0 && ix->ntotal > 0) ? plan_tensor_chunked(nq, ix->ntotal, ix->d, kp, heap_first, &plan) : 0;
     const bool tensor_ok = chunk_nq > 0;
     if (algo == B2F_ALGO_AUTO) algo = (nq <= scan_max || !tensor_ok) ? B2F_ALGO_SCAN : B2F_ALGO_TENSOR;
     // an explicit TENSOR request on a shape the tensor path cannot plan (k' > 256, or a database of a few rows with
@@ -1279,16 +1255,6 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
             ra.certify = certify;
             ra.fail_tau = w.fail_tau;
             ra.q_base = c0;
-            {   // First-stage re-rank (the best n candidates alone before the k' best): OFF.  Same-box A/B (r02n): no gain at
-                // 4096 / 8192 queries with k = 10 (the merge is not bound by the candidate row reads after all), and a loss
-                // at k = 100, k' = 192 (0.69 -> 0.93 ms per C3 search).  B200FLAT_STAGE1=<n> enables it for experiments.
-                static int s1_env = -2;
-                if (s1_env == -2) {
-                    const char* e = getenv("B200FLAT_STAGE1");
-                    s1_env = e ? atoi(e) : 0;
-                }
-                ra.stage1 = (s1_env >= k && s1_env < kp) ? s1_env : 0;
-            }
             if (plan.list_mode) {
                 // K3b + K4 + finalize fused: per query, merge the lists, re-rank exactly, certify, write (D, I)
                 B2F_TRY(launch_merge_lists(w.lists, cn, plan, reinterpret_cast<unsigned long long*>(w.counters + 2), ra, st));
@@ -1359,7 +1325,7 @@ struct b2f_range_result {
 constexpr int kRangeSearchKp = 32;
 
 static int plan_range_search(int nq, int64_t n, int d, TensorScanPlan* plan) {
-    if (plan_tensor_scan(nq, n, d, kRangeSearchKp, plan) != B2F_OK || !plan->list_mode) return B2F_EINVAL;
+    if (plan_tensor_scan(nq, n, d, kRangeSearchKp, false, plan) != B2F_OK || !plan->list_mode) return B2F_EINVAL;
     int cap = (int)align_up((size_t)(2 * kRangeHitsMax / plan->nlists), 64);
     if (cap < kRangeListCap) cap = kRangeListCap;
     plan->list_cap = cap < 1024 ? cap : 1024;

@@ -427,7 +427,7 @@ def test_near_duplicate_ip_results_are_consistent(m):
         check_structure(D, I, IP, len(xb))
         check_consistent(D, I, xb, xq, IP)
     assert st["range_queries"] > 0, st
-    # the warp-per-query merge's near-duplicate batch (test_big_batch_warp_merge_and_first_stage)
+    # the warp-per-query merge's near-duplicate batch (test_big_batch_warp_merge)
     d, nq = 128, 8192
     rng = np.random.default_rng(5)
     centres = rng.standard_normal((600, d)).astype(np.float32)

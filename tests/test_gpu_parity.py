@@ -385,10 +385,10 @@ def test_centred_bf16_storage_certifies_embedding_like_data(m, metric, tmp_path)
 
 
 @pytest.mark.parametrize("metric", [1, 0])
-def test_big_batch_warp_merge_and_first_stage(m, metric):
+def test_big_batch_warp_merge(m, metric):
     """Batches of >= 8192 queries take the warp-per-query list merge; queries it cannot hold are passed on to the block
     kernel.  Exact on benign data, and on data where the k' best cannot certify (near-duplicate rows: dozens of rows
-    within the bf16 band of the k-th neighbour), so that the extended stage and the exact scan must answer."""
+    within the bf16 band of the k-th neighbour), so that the re-rank of every list entry and the exact scan must answer."""
     n, d, nq, k = 60000, 128, 8192, 10
     xb = orc.c_synth_rows(1234, 0, n, d, metric == 0)
     xq = orc.c_synth_rows(5678, 0, nq, d, metric == 0)
@@ -398,7 +398,7 @@ def test_big_batch_warp_merge_and_first_stage(m, metric):
     st = ix.stats()
     assert st["last_algo"] == m.ALGO_TENSOR and st["fallback_queries"] == 0, st
     # clusters of 40 near-duplicates around 600 centres: the neighbours of a query near a centre are separated by far less
-    # than the bf16 rounding band, so the first stage (and often the k' stage) fails and the later stages must answer
+    # than the bf16 rounding band, so the k' stage often fails and the later stages must answer
     rng = np.random.default_rng(5)
     centres = rng.standard_normal((600, d)).astype(np.float32)
     xb2 = (np.repeat(centres, 40, axis=0) + rng.standard_normal((24000, d)).astype(np.float32) * 2e-3).astype(np.float32)
