@@ -207,6 +207,19 @@ B2F_API int b2f_merge_topk(int32_t metric, int64_t nq, int64_t k, int32_t nparts
 B2F_API int b2f_merge_topk_strided(int32_t metric, int64_t nq, int64_t k, int32_t nparts, const float* D_parts,
                    const int64_t* I_parts, int64_t part_stride_bytes, float* D, int64_t* I, int32_t device,
                    void* stream);
+/* Merge nparts per-shard range-search results into one, query by query, hits in ascending label order.
+ * lims_parts: device int64 [nparts][nq + 1], part p's own lims (any base: part p's hits of query q are its
+ * elements lims_parts[p][q] - lims_parts[p][0] .. lims_parts[p][q+1] - lims_parts[p][0]);
+ * part p's D (fp32) at D_parts + p * part_stride_bytes, its I (int64) at I_parts + p * part_stride_bytes
+ * (the packed all-gather layout [D | pad | I], as b2f_merge_topk_strided).
+ * Within a part and a query the labels must be strictly ascending; different parts hold disjoint labels.
+ * Output: D [total], I [total], total = sum over p of the parts' hit counts, query q at offset
+ * sum_p (lims_parts[p][q] - lims_parts[p][0]).  Distances are copied bit for bit.  1 <= nparts <= 32.
+ * Device buffers only; enqueued on `stream` without a host synchronisation (the hit count is read on the device), so
+ * with nq > 0 the hit pointers must not be NULL even when every part is empty.  part_stride_bytes: a multiple of 16. */
+B2F_API int b2f_merge_range_strided(int64_t nq, int32_t nparts, const int64_t* lims_parts, const float* D_parts,
+                                    const int64_t* I_parts, int64_t part_stride_bytes, float* D, int64_t* I,
+                                    int32_t device, void* stream);
 
 /* ---- multi-GPU over NVLink peer memory: the exchange + merge above as ONE kernel (no NCCL call, no second launch).
  * One process per GPU.  create() allocates this rank's receive buffers (two generations x world slots of

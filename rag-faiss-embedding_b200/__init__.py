@@ -25,7 +25,7 @@ from .index import (  # noqa: F401
     write_index,
 )
 from .store import FAISSVectorStore  # noqa: F401
-from .sharded import ShardedIndexFlat, merge_topk  # noqa: F401
+from .sharded import ShardedIndexFlat, merge_range, merge_topk  # noqa: F401
 
 _capi.load()
 

@@ -241,6 +241,10 @@ int launch_finalize(const float* keys, const int32_t* ids, int nq, int kin, int 
 // after part 0 (dense [nparts][nq][k] arrays, or one packed message per rank)
 int launch_merge_faiss(int metric, int64_t nq, int64_t k, int nparts, const float* Dp, const int64_t* Ip,
                        int64_t stride_d_bytes, int64_t stride_i_bytes, float* D, int64_t* I, cudaStream_t st);
+// multi-GPU merge of nparts range-search results (lims [nparts][nq + 1], any base; hits of part p stride * p bytes after
+// part 0) into one result in ascending label order per query
+int launch_merge_range(int64_t nq, int nparts, const int64_t* lims, const float* Dp, const int64_t* Ip, int64_t stride,
+                       float* D, int64_t* I, cudaStream_t st);
 
 // K5: ingest. src fp32 [n,d] (device) -> rows fp32 (optional), bf16 scan copy (pitch dpad), norms.
 // stats (device, 2 floats): running max |bf16(x)|^2 and max |x - bf16(x)|^2 (certification bound).

@@ -909,6 +909,21 @@ int b2f_merge_topk_strided(int32_t metric, int64_t nq, int64_t k, int32_t nparts
     return launch_merge_faiss(metric, nq, k, nparts, D_parts, I_parts, part_stride_bytes, part_stride_bytes, D, I, (cudaStream_t)stream);
 }
 
+int b2f_merge_range_strided(int64_t nq, int32_t nparts, const int64_t* lims_parts, const float* D_parts,
+                            const int64_t* I_parts, int64_t part_stride_bytes, float* D, int64_t* I, int32_t device,
+                            void* stream) {
+    // the hit count lives in the device lims, so with nq > 0 every hit pointer must be usable
+    const bool misaligned = ((uintptr_t)lims_parts | (uintptr_t)I_parts | (uintptr_t)I) & 7 || ((uintptr_t)D_parts | (uintptr_t)D) & 3;
+    if (nq < 0 || nparts < 1 || nparts > 32 || !lims_parts || part_stride_bytes <= 0 || (part_stride_bytes & 15) ||
+        (nq > 0 && (!D_parts || !I_parts || !D || !I)) || misaligned) {
+        set_error("merge_range: bad arguments");
+        return B2F_EINVAL;
+    }
+    B2F_TRY(check_device(device));
+    DeviceGuard g(device);
+    return launch_merge_range(nq, nparts, lims_parts, D_parts, I_parts, part_stride_bytes, D, I, (cudaStream_t)stream);
+}
+
 int b2f_merge_topk(int32_t metric, int64_t nq, int64_t k, int32_t nparts, const float* D_parts, const int64_t* I_parts,
                    float* D, int64_t* I, int32_t device, void* stream) {
     if (nq < 0 || k <= 0 || !D_parts || !I_parts || !D || !I) {

@@ -154,4 +154,80 @@ int launch_merge_faiss(int metric, int64_t nq, int64_t k, int nparts, const floa
     return B2F_OK;
 }
 
+// Range-search results of nparts shards -> one result, query by query in ascending label order.  Part p: lims
+// lims[p * (nq + 1) ..] (any base), hits at Dp / Ip + p * stride bytes.  One thread per input hit: it finds its query
+// by binary search over its part's lims, and its output slot as the query's output base + its index in its own list
+// + the labels below it in every other part's list of that query (one lower_bound per part).  Labels are disjoint
+// across parts, so the slots are a permutation: no thread waits for another, and a query with 10^5 hits is spread
+// over as many threads as it has hits.  The hit count is read from the device lims, so the grid strides over it.
+constexpr int kRangeMergeThreads = 256;
+
+__global__ void __launch_bounds__(kRangeMergeThreads)
+merge_range_kernel(int64_t nq, int nparts, const int64_t* __restrict__ lims, const char* __restrict__ Dp,
+                   const char* __restrict__ Ip, int64_t stride, float* __restrict__ D, int64_t* __restrict__ I) {
+    __shared__ int64_t base[kWarp];       // lims[p][0]
+    __shared__ int64_t first[kWarp + 1];  // hits of parts < p
+    if (threadIdx.x < kWarp) {
+        const int lane = threadIdx.x;
+        int64_t b = 0, inc = 0;
+        if (lane < nparts) {
+            b = lims[lane * (nq + 1)];
+            inc = lims[lane * (nq + 1) + nq] - b;
+        }
+#pragma unroll
+        for (int s = 1; s < kWarp; s <<= 1) {
+            const int64_t t = __shfl_up_sync(kFull, inc, s);
+            if (lane >= s) inc += t;
+        }
+        base[lane] = b;
+        first[lane + 1] = inc;
+        if (lane == 0) first[0] = 0;
+    }
+    __syncthreads();
+    const int64_t total = first[nparts];
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
+        int p = 0;
+        while (first[p + 1] <= t) p++;
+        const int64_t e = t - first[p];
+        const int64_t* lp = lims + p * (nq + 1);
+        const int64_t key = e + base[p];
+        int64_t lo = 0, hi = nq;   // the last query q with lp[q] <= key: the one whose list holds e
+        while (hi - lo > 1) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (lp[mid] <= key) lo = mid;
+            else hi = mid;
+        }
+        const int64_t q = lo;
+        const int64_t label = reinterpret_cast<const int64_t*>(Ip + p * stride)[e];
+        const float dist = reinterpret_cast<const float*>(Dp + p * stride)[e];
+        int64_t o = key - lp[q];
+        for (int r = 0; r < nparts; r++) {
+            const int64_t* lr = lims + r * (nq + 1);
+            const int64_t s = lr[q] - base[r];
+            o += s;
+            if (r == p) continue;
+            const int64_t* ir = reinterpret_cast<const int64_t*>(Ip + r * stride) + s;
+            int64_t a = 0, z = lr[q + 1] - lr[q];   // lower_bound of label in part r's list of query q
+            while (a < z) {
+                const int64_t mid = (a + z) >> 1;
+                if (ir[mid] < label) a = mid + 1;
+                else z = mid;
+            }
+            o += a;
+        }
+        D[o] = dist;
+        I[o] = label;
+    }
+}
+
+int launch_merge_range(int64_t nq, int nparts, const int64_t* lims, const float* Dp, const int64_t* Ip, int64_t stride,
+                       float* D, int64_t* I, cudaStream_t st) {
+    if (nq <= 0) return B2F_OK;
+    // enough resident threads to hide the dependent loads of the searches; the grid strides over the device's hit count
+    merge_range_kernel<<<kNumSMs * 8, kRangeMergeThreads, 0, st>>>(nq, nparts, lims, reinterpret_cast<const char*>(Dp),
+                                                                   reinterpret_cast<const char*>(Ip), stride, D, I);
+    B2F_CUDA(cudaGetLastError());
+    return B2F_OK;
+}
+
 }  // namespace b2f

@@ -20,7 +20,7 @@ from typing import Callable, List, Optional, Tuple
 import numpy as np
 
 from . import _capi as C
-from .index import METRIC_L2, IDSelectorBatch, IDSelectorRange, IndexFlat, _id_array
+from .index import METRIC_L2, IDSelectorBatch, IDSelectorRange, IndexFlat, _assert, _id_array, _is_torch
 
 
 def partition_rows(n: int, world: int) -> List[Tuple[int, int]]:
@@ -67,6 +67,14 @@ class SegmentMap:
         self.local_starts, self.global_starts, self.nlocal = kept.local_starts, kept.global_starts, kept.nlocal
         return np.concatenate(local) if local else np.zeros(0, np.int64)
 
+    def monotone(self) -> bool:
+        """True when local row order is global label order (each segment's labels above the previous segment's): then
+        mapping a label-sorted list of local rows gives a label-sorted list of global labels.  add, add_synthetic and
+        remove_ids keep it; add_local with a lower global_start than an earlier segment breaks it."""
+        ends = self.local_starts[1:] + [self.nlocal]
+        return all(self.global_starts[i] + (ends[i] - self.local_starts[i]) <= self.global_starts[i + 1]
+                   for i in range(len(self.local_starts) - 1))
+
     def to_global_numpy(self, local_ids: np.ndarray) -> np.ndarray:
         out = local_ids.astype(np.int64, copy=True)
         if not self.local_starts:
@@ -104,17 +112,65 @@ def merge_topk(metric: int, D_parts, I_parts):
     return D, I
 
 
+# a rank's packed range hits [D | pad | I] of one all-gather stay below this; a query with more hits gets a gather
+# of its own
+RANGE_PART_BYTES = 256 << 20
+
+
+def _range_layout(nhits: int) -> Tuple[int, int]:
+    """Packed [D fp32 | pad | I int64] of nhits hits: (byte offset of I, part bytes), both multiples of 16."""
+    off_i = (nhits * 4 + 15) // 16 * 16
+    return off_i, (off_i + nhits * 8 + 15) // 16 * 16
+
+
+def merge_range_strided(lims_parts, recv, part_bytes: int, off_i: int, D, I):
+    """b2f_merge_range_strided over an all-gathered buffer: lims_parts [G, nq + 1] int64 (any base), recv [G * part_bytes]
+    uint8 holding G packed parts [D | pad | I at off_i]; writes the label-ordered union into D / I [total] (CUDA
+    tensors on one device, enqueued on the current torch stream)."""
+    import torch
+
+    G, nq = int(lims_parts.shape[0]), int(lims_parts.shape[1]) - 1
+    lims_parts = lims_parts.contiguous()
+    stream = int(torch.cuda.current_stream(recv.device).cuda_stream) or 1  # 0x1 = cudaStreamLegacy
+    C.check(C.load().b2f_merge_range_strided(nq, G, lims_parts.data_ptr(), recv.data_ptr(), recv.data_ptr() + off_i,
+                                             part_bytes, D.data_ptr(), I.data_ptr(), recv.device.index or 0,
+                                             ctypes.c_void_p(stream)))
+
+
+def merge_range(parts):
+    """parts: G per-shard range results (lims [nq + 1], D [.], I [.]) as CUDA tensors on one device, labels disjoint
+    across parts -> one (lims, D, I) with each query's hits in ascending label order, via the CUDA merge kernel."""
+    import torch
+
+    dev = parts[0][1].device
+    lims_parts = torch.stack([p[0].to(device=dev, dtype=torch.int64) for p in parts])
+    lims = lims_parts.sum(0) - lims_parts[:, :1].sum()
+    nhits = [int(p[1].numel()) for p in parts]
+    total = sum(nhits)
+    D = torch.empty(total, dtype=torch.float32, device=dev)
+    I = torch.empty(total, dtype=torch.int64, device=dev)
+    if total == 0:
+        return lims, D, I
+    off_i, part = _range_layout(max(nhits))
+    recv = torch.zeros(len(parts) * part, dtype=torch.uint8, device=dev)
+    for g, (_, Dp, Ip) in enumerate(parts):
+        recv[g * part: g * part + 4 * nhits[g]].view(torch.float32).copy_(Dp)
+        recv[g * part + off_i: g * part + off_i + 8 * nhits[g]].view(torch.int64).copy_(Ip)
+    merge_range_strided(lims_parts, recv, part, off_i, D, I)
+    return lims, D, I
+
+
 class ShardedIndexFlat:
     """IndexFlat surface over a torch.distributed process group, one shard per rank.
 
-    `local_index` / `merge_fn` exist so the host logic (partitioning, label mapping, the collective)
-    can be exercised on CPU with the gloo backend in tests; the defaults are the CUDA index and the
-    CUDA merge kernel.
+    `local_index` / `merge_fn` / `range_merge_fn` exist so the host logic (partitioning, label mapping, the
+    collectives) can be exercised on CPU with the gloo backend in tests; the defaults are the CUDA index and the
+    CUDA merge kernels.  range_merge_fn has merge_range_strided's signature.
     """
 
     def __init__(self, d: int, metric: int = METRIC_L2, *, storage: Optional[int] = None,
                  device: Optional[int] = None, group=None, local_index=None,
-                 merge_fn: Optional[Callable] = None):
+                 merge_fn: Optional[Callable] = None, range_merge_fn: Optional[Callable] = None):
         import torch.distributed as dist
 
         self._dist = dist
@@ -125,6 +181,7 @@ class ShardedIndexFlat:
         self.metric_type = metric
         self.local = local_index if local_index is not None else IndexFlat(d, metric, storage=storage, device=device)
         self._merge = merge_fn if merge_fn is not None else merge_topk
+        self._range_merge = range_merge_fn if range_merge_fn is not None else merge_range_strided
         self.segments = SegmentMap()
         self.ntotal = 0
         self.is_trained = True
@@ -322,6 +379,105 @@ class ShardedIndexFlat:
         if was_numpy and not isinstance(Dm, np.ndarray):
             Dm, Im = Dm.cpu().numpy(), Im.cpu().numpy()
         return Dm, Im
+
+    def _all_gather(self, t):
+        """[world, *t.shape] all-gather of t (the same shape on every rank), returned on t's device.  An NCCL group
+        gathers device tensors; a gloo group gathers host copies (the CPU tier, or several ranks sharing one GPU)."""
+        import torch
+
+        host = not (t.is_cuda and "nccl" in str(self._dist.get_backend(self.group)))
+        src = (t.cpu() if host else t).contiguous().view(-1)
+        out = torch.empty(self.world * src.numel(), dtype=t.dtype, device=src.device)
+        self._dist.all_gather_into_tensor(out, src, group=self.group)
+        out = out.view((self.world,) + tuple(t.shape))
+        return out.to(t.device) if host else out
+
+    @staticmethod
+    def _range_chunks(lims_host: np.ndarray) -> List[Tuple[int, int]]:
+        """Query ranges [q0, q1) over which no rank's packed hits ([world, nq + 1] lims) exceed RANGE_PART_BYTES; a
+        query with more hits than that on some rank is a range of its own."""
+        budget = max((RANGE_PART_BYTES - 32) // 12, 0)   # _range_layout(budget)[1] <= RANGE_PART_BYTES
+        nq = lims_host.shape[1] - 1
+        chunks, q0 = [], 0
+        while q0 < nq:
+            q1 = min(int(np.searchsorted(lims, lims[q0] + budget, side="right")) - 1 for lims in lims_host)
+            q1 = min(max(q1, q0 + 1), nq)
+            chunks.append((q0, q1))
+            q0 = q1
+        return chunks
+
+    def range_search(self, x, radius: float, *, params: Optional[C.SearchParams] = None):
+        """index.range_search(x, radius) over the whole sharded index: replicated queries -> the same faiss
+        RangeSearchResult (lims, D, I) on every rank, each query's hits in ascending label order, as IndexFlat returns
+        it (numpy in: lims uint64, D float32, I int64 numpy arrays; CUDA tensor in: CUDA tensors).
+
+        Each rank range-searches its shard; one all-gather of every rank's lims settles all sizes; the hits then move
+        in all-gathers of at most RANGE_PART_BYTES per rank, each followed by the CUDA merge (b2f_merge_range_strided)
+        into its slice of the result.  last_range_info: the local search's five numbers, `chunks` (hit all-gathers) and
+        `gathered_bytes` (bytes this rank sent: its lims and its packed hits)."""
+        import torch
+
+        # checked on every rank before the first collective, so that a bad call leaves no rank waiting for another
+        radius = float(radius)
+        if radius != radius:
+            raise C.B200FlatError(C.EINVAL, "range_search: radius is NaN")
+        shape = tuple(x.shape)
+        _assert(len(shape) == 2 and int(shape[1]) == self.d, f"dimension mismatch: got {shape}, index has d={self.d}")
+        dev_in = _is_torch(x) and x.is_cuda
+        nq = int(shape[0])
+
+        off = self.segments.single_offset()
+        if hasattr(self.local, "set_search_params"):
+            self.local.set_search_params(id_offset=off if off is not None else 0)
+        if params is not None:
+            params = C.SearchParams.from_buffer_copy(params)
+            params.id_offset = off if off is not None else 0
+            lims, D, I = self.local.range_search(x, radius, params=params)
+        else:
+            lims, D, I = self.local.range_search(x, radius)
+        info = dict(getattr(self.local, "last_range_info", {}))
+        if isinstance(D, np.ndarray):
+            lims, D, I = (torch.from_numpy(np.asarray(lims).astype(np.int64)), torch.from_numpy(D), torch.from_numpy(I))
+        if off is None:
+            I = self.segments.to_global_torch(I)
+            if not self.segments.monotone():
+                # a segment added below an earlier one: order each query's hits by label again
+                qid = torch.repeat_interleave(torch.arange(nq, device=I.device), lims.diff(), output_size=I.numel())
+                order = torch.argsort(I, stable=True)
+                order = order[torch.argsort(qid[order], stable=True)]
+                D, I = D[order], I[order]
+
+        chunks, sent = 0, 0
+        if self.world > 1:
+            # the hits stay on the shard's GPU (a host-side stand-in for the local index keeps them on the host)
+            work = torch.device("cuda", self.local.device) if isinstance(self.local, IndexFlat) else torch.device("cpu")
+            lims, D, I = lims.to(work), D.to(work), I.to(work)
+            lims_all = self._all_gather(lims)      # [world, nq + 1]: every rank's local lims (base 0)
+            lims_host = lims_all.cpu().numpy()
+            sent = 8 * (nq + 1)
+            glims = lims_host.sum(0)
+            Dm = torch.empty(int(glims[-1]), dtype=torch.float32, device=work)
+            Im = torch.empty(int(glims[-1]), dtype=torch.int64, device=work)
+            a_own = lims_host[self.rank]
+            for q0, q1 in self._range_chunks(lims_host):
+                nmax = int((lims_host[:, q1] - lims_host[:, q0]).max())
+                if nmax == 0:   # decided from the gathered lims, so every rank skips the same gathers
+                    continue
+                off_i, part = _range_layout(nmax)
+                a, b = int(a_own[q0]), int(a_own[q1])
+                send = torch.empty(part, dtype=torch.uint8, device=work)
+                send[: 4 * (b - a)].view(torch.float32).copy_(D[a:b])
+                send[off_i: off_i + 8 * (b - a)].view(torch.int64).copy_(I[a:b])
+                recv = self._all_gather(send).view(-1)
+                g0, g1 = int(glims[q0]), int(glims[q1])
+                self._range_merge(lims_all[:, q0:q1 + 1], recv, part, off_i, Dm[g0:g1], Im[g0:g1])
+                chunks += 1
+                sent += part
+            lims, D, I = torch.from_numpy(glims), Dm, Im
+        self.last_range_info = dict(info, chunks=chunks, gathered_bytes=sent)
+        if dev_in:
+            return lims.to(x.device), D.to(x.device), I.to(x.device)
+        return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
 
     def remove_ids(self, x) -> int:
         """index.remove_ids(sel) over the whole sharded index: x (IDSelectorRange, IDSelectorBatch or 1-D integer array)
