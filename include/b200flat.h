@@ -198,12 +198,9 @@ B2F_API int b2f_index_write(b2f_index* idx, const char* path);
 B2F_API int b2f_index_read(const char* path, int32_t storage, int32_t device, b2f_index** out);
 
 /* ---- multi-GPU: merge per-shard top-k lists after the all-gather (SURVEY 8e) -------------------
- * D_parts/I_parts: [nparts, nq, k] (the all_gather_into_tensor layout); out: [nq, k].
+ * Part p's D [nq, k] (fp32) at D_parts + p * part_stride_bytes, its I [nq, k] (int64) at I_parts + p * part_stride_bytes:
+ * each rank ships its distances and labels in ONE packed all-gather message [D | pad | I]; out: [nq, k].
  * Keeps faiss ordering and -1 padding.  Device buffers only.  1 <= nparts <= 32 (else B2F_EINVAL). */
-B2F_API int b2f_merge_topk(int32_t metric, int64_t nq, int64_t k, int32_t nparts, const float* D_parts,
-                   const int64_t* I_parts, float* D, int64_t* I, int32_t device, void* stream);
-/* Same merge over parts that are `part_stride_bytes` apart (D_parts / I_parts point at part 0): lets each rank
- * ship its distances and labels in ONE packed all-gather message instead of two.                      */
 B2F_API int b2f_merge_topk_strided(int32_t metric, int64_t nq, int64_t k, int32_t nparts, const float* D_parts,
                    const int64_t* I_parts, int64_t part_stride_bytes, float* D, int64_t* I, int32_t device,
                    void* stream);

@@ -96,7 +96,6 @@ PROTOTYPES = {
     "b2f_index_reconstruct":(ctypes.c_int, [_vp, _i64, _i64, _vp, _i32, _vp]),
     "b2f_index_write": (ctypes.c_int, [_vp, ctypes.c_char_p]),
     "b2f_index_read": (ctypes.c_int, [ctypes.c_char_p, _i32, _i32, ctypes.POINTER(_vp)]),
-    "b2f_merge_topk": (ctypes.c_int, [_i32, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _i32, _vp]),
     "b2f_merge_topk_strided": (ctypes.c_int, [_i32, _i64, _i64, _i32, _vp, _vp, _i64, _vp, _vp, _i32, _vp]),
     "b2f_merge_range_strided": (ctypes.c_int, [_i64, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _i32, _vp]),
     "b2f_exchange_create": (ctypes.c_int, [_i32, _i32, _i32, _i64, ctypes.POINTER(_vp), _vp]),

@@ -139,6 +139,49 @@ __device__ __forceinline__ void warp_merge_lists(const float* keys, const int32_
     }
 }
 
+// Merge one query's per-shard top-k lists in faiss conventions (lane l < nparts walks list l: distances dl, labels il,
+// k entries each, -1 padded) into the k best, written by lane 0 to D / I [k].  One warp.  Ties go to the lower label,
+// then the lower lane; -1 padding loses to everything.
+// CG: read the lists with ld.global.cg (the peer exchange's are written by other GPUs while its kernel runs).
+template <bool CG = false>
+__device__ __forceinline__ void warp_merge_faiss(bool l2, bool have, const float* dl, const int64_t* il, int k, float* D,
+                                                 int64_t* I, int lane) {
+    int pos = 0;
+    float hk = FLT_MAX;
+    int64_t hi = -1;
+    if (have) {
+        hi = CG ? __ldcg(il) : il[0];
+        hk = hi < 0 ? FLT_MAX : (l2 ? (CG ? __ldcg(dl) : dl[0]) : -(CG ? __ldcg(dl) : dl[0]));
+    }
+    for (int o = 0; o < k; o++) {
+        float bk = hk;
+        int64_t bi = hi;
+        int bl = lane;
+#pragma unroll
+        for (int s = 16; s >= 1; s >>= 1) {
+            const float tk = __shfl_xor_sync(kFull, bk, s);
+            const int64_t ti = __shfl_xor_sync(kFull, bi, s);
+            const int tl = __shfl_xor_sync(kFull, bl, s);
+            const bool less = tk < bk || (tk == bk && ((uint64_t)ti < (uint64_t)bi || (ti == bi && tl < bl)));
+            if (less) { bk = tk; bi = ti; bl = tl; }
+        }
+        if (lane == 0) {
+            D[o] = bi < 0 ? (l2 ? FLT_MAX : -FLT_MAX) : (l2 ? bk : -bk);
+            I[o] = bi;
+        }
+        if (have && lane == bl) {
+            pos++;
+            if (pos < k) {
+                hi = CG ? __ldcg(il + pos) : il[pos];
+                hk = hi < 0 ? FLT_MAX : (l2 ? (CG ? __ldcg(dl + pos) : dl[pos]) : -(CG ? __ldcg(dl + pos) : dl[pos]));
+            } else {
+                hi = -1;
+                hk = FLT_MAX;
+            }
+        }
+    }
+}
+
 __device__ __forceinline__ float4 ldg_stream(const float4* p) {
     float4 r;
     asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
@@ -237,10 +280,10 @@ int launch_merge_parts(const float* pk, const int32_t* pi, int nq, int nparts, i
 // qsel (optional) scatters row r of the input to output row qsel[r].
 int launch_finalize(const float* keys, const int32_t* ids, int nq, int kin, int k, int metric, int64_t id_offset,
                     const int32_t* qsel, float* D, int64_t* I, cudaStream_t st);
-// multi-GPU merge of nparts faiss-formatted [nq][k] lists; part p of the distances / labels sits p * stride bytes
-// after part 0 (dense [nparts][nq][k] arrays, or one packed message per rank)
-int launch_merge_faiss(int metric, int64_t nq, int64_t k, int nparts, const float* Dp, const int64_t* Ip,
-                       int64_t stride_d_bytes, int64_t stride_i_bytes, float* D, int64_t* I, cudaStream_t st);
+// multi-GPU merge of nparts faiss-formatted [nq][k] lists; part p's distances / labels sit p * stride bytes after
+// part 0's (one packed message per rank)
+int launch_merge_faiss(int metric, int64_t nq, int64_t k, int nparts, const float* Dp, const int64_t* Ip, int64_t stride,
+                       float* D, int64_t* I, cudaStream_t st);
 // multi-GPU merge of nparts range-search results (lims [nparts][nq + 1], any base; hits of part p stride * p bytes after
 // part 0) into one result in ascending label order per query
 int launch_merge_range(int64_t nq, int nparts, const int64_t* lims, const float* Dp, const int64_t* Ip, int64_t stride,

@@ -115,42 +115,8 @@ __global__ void __launch_bounds__(256) exchange_merge_kernel(const ExArgs a) {
     for (int64_t q = (int64_t)blockIdx.x * wpb + (threadIdx.x >> 5); q < a.nq; q += (int64_t)gridDim.x * wpb) {
         const bool have = lane < a.world;
         const char* part = (have && lane != a.rank) ? base + (int64_t)lane * a.slot_bytes : a.src;   // own part: the message itself
-        const float* dl = reinterpret_cast<const float*>(part) + q * a.k;
-        const int64_t* il = reinterpret_cast<const int64_t*>(part + a.off_i) + q * a.k;
-        int pos = 0;
-        float hk = FLT_MAX;
-        int64_t hi = -1;
-        if (have) {
-            hi = __ldcg(il);
-            hk = hi < 0 ? FLT_MAX : (a.l2 ? __ldcg(dl) : -__ldcg(dl));
-        }
-        for (int o = 0; o < a.k; o++) {
-            float bk = hk;
-            int64_t bi = hi;
-            int bl = lane;
-#pragma unroll
-            for (int s = 16; s >= 1; s >>= 1) {
-                const float tk = __shfl_xor_sync(kFull, bk, s);
-                const int64_t ti = __shfl_xor_sync(kFull, bi, s);
-                const int tl = __shfl_xor_sync(kFull, bl, s);
-                const bool less = tk < bk || (tk == bk && ((uint64_t)ti < (uint64_t)bi || (ti == bi && tl < bl)));
-                if (less) { bk = tk; bi = ti; bl = tl; }
-            }
-            if (lane == 0) {
-                a.D[q * a.k + o] = bi < 0 ? (a.l2 ? FLT_MAX : -FLT_MAX) : (a.l2 ? bk : -bk);
-                a.I[q * a.k + o] = bi;
-            }
-            if (have && lane == bl) {
-                pos++;
-                if (pos < a.k) {
-                    hi = __ldcg(il + pos);
-                    hk = hi < 0 ? FLT_MAX : (a.l2 ? __ldcg(dl + pos) : -__ldcg(dl + pos));
-                } else {
-                    hi = -1;
-                    hk = FLT_MAX;
-                }
-            }
-        }
+        warp_merge_faiss<true>(a.l2, have, reinterpret_cast<const float*>(part) + q * a.k,
+                         reinterpret_cast<const int64_t*>(part + a.off_i) + q * a.k, a.k, a.D + q * a.k, a.I + q * a.k, lane);
     }
 }
 

@@ -906,7 +906,7 @@ int b2f_merge_topk_strided(int32_t metric, int64_t nq, int64_t k, int32_t nparts
     }
     B2F_TRY(check_device(device));
     DeviceGuard g(device);
-    return launch_merge_faiss(metric, nq, k, nparts, D_parts, I_parts, part_stride_bytes, part_stride_bytes, D, I, (cudaStream_t)stream);
+    return launch_merge_faiss(metric, nq, k, nparts, D_parts, I_parts, part_stride_bytes, D, I, (cudaStream_t)stream);
 }
 
 int b2f_merge_range_strided(int64_t nq, int32_t nparts, const int64_t* lims_parts, const float* D_parts,
@@ -922,17 +922,6 @@ int b2f_merge_range_strided(int64_t nq, int32_t nparts, const int64_t* lims_part
     B2F_TRY(check_device(device));
     DeviceGuard g(device);
     return launch_merge_range(nq, nparts, lims_parts, D_parts, I_parts, part_stride_bytes, D, I, (cudaStream_t)stream);
-}
-
-int b2f_merge_topk(int32_t metric, int64_t nq, int64_t k, int32_t nparts, const float* D_parts, const int64_t* I_parts,
-                   float* D, int64_t* I, int32_t device, void* stream) {
-    if (nq < 0 || k <= 0 || !D_parts || !I_parts || !D || !I) {
-        set_error("merge_topk: bad arguments");
-        return B2F_EINVAL;
-    }
-    B2F_TRY(check_device(device));
-    DeviceGuard g(device);
-    return launch_merge_faiss(metric, nq, k, nparts, D_parts, I_parts, nq * k * 4, nq * k * 8, D, I, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -93,63 +93,30 @@ int launch_finalize(const float* keys, const int32_t* ids, int nq, int kin, int 
     return B2F_OK;
 }
 
-// Dp/Ip: [nparts][nq][k] faiss-formatted per-shard results -> D/I [nq][k].  One warp per query,
-// lane l walks list l.  Ties go to the lower label, -1 padding loses to everything.
-__global__ void merge_faiss_kernel(int l2, int64_t nq, int k, int nparts, const float* __restrict__ Dp,
-                                   const int64_t* __restrict__ Ip, int64_t stride_d_bytes, int64_t stride_i_bytes,
-                                   float* __restrict__ D, int64_t* __restrict__ I) {
+// Part p's faiss-formatted [nq][k] results at Dp / Ip + p * stride bytes -> D/I [nq][k].  One warp per query.
+__global__ void merge_faiss_kernel(int l2, int64_t nq, int k, int nparts, const char* __restrict__ Dp,
+                                   const char* __restrict__ Ip, int64_t stride, float* __restrict__ D,
+                                   int64_t* __restrict__ I) {
     const int lane = threadIdx.x & 31;
     const int64_t q = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (q >= nq) return;
     const bool have = lane < nparts;
-    const float* dl = reinterpret_cast<const float*>(reinterpret_cast<const char*>(Dp) + (have ? lane : 0) * stride_d_bytes) + q * k;
-    const int64_t* il = reinterpret_cast<const int64_t*>(reinterpret_cast<const char*>(Ip) + (have ? lane : 0) * stride_i_bytes) + q * k;
-    int pos = 0;
-    float hk = FLT_MAX;
-    int64_t hi = -1;
-    if (have) {
-        hi = il[0];
-        hk = hi < 0 ? FLT_MAX : (l2 ? dl[0] : -dl[0]);
-    }
-    for (int o = 0; o < k; o++) {
-        float bk = hk;
-        int64_t bi = hi;
-        int bl = lane;
-#pragma unroll
-        for (int s = 16; s >= 1; s >>= 1) {
-            const float tk = __shfl_xor_sync(kFull, bk, s);
-            const int64_t ti = __shfl_xor_sync(kFull, bi, s);
-            const int tl = __shfl_xor_sync(kFull, bl, s);
-            const bool less = tk < bk || (tk == bk && ((uint64_t)ti < (uint64_t)bi || (ti == bi && tl < bl)));
-            if (less) { bk = tk; bi = ti; bl = tl; }
-        }
-        if (lane == 0) {
-            D[q * k + o] = bi < 0 ? (l2 ? FLT_MAX : -FLT_MAX) : (l2 ? bk : -bk);
-            I[q * k + o] = bi;
-        }
-        if (have && lane == bl) {
-            pos++;
-            if (pos < k) {
-                hi = il[pos];
-                hk = hi < 0 ? FLT_MAX : (l2 ? dl[pos] : -dl[pos]);
-            } else {
-                hi = -1;
-                hk = FLT_MAX;
-            }
-        }
-    }
+    const int64_t part = (have ? lane : 0) * stride;
+    warp_merge_faiss(l2, have, reinterpret_cast<const float*>(Dp + part) + q * k,
+                     reinterpret_cast<const int64_t*>(Ip + part) + q * k, k, D + q * k, I + q * k, lane);
 }
 
-int launch_merge_faiss(int metric, int64_t nq, int64_t k, int nparts, const float* Dp, const int64_t* Ip,
-                       int64_t stride_d_bytes, int64_t stride_i_bytes, float* D, int64_t* I, cudaStream_t st) {
+int launch_merge_faiss(int metric, int64_t nq, int64_t k, int nparts, const float* Dp, const int64_t* Ip, int64_t stride,
+                       float* D, int64_t* I, cudaStream_t st) {
     if (nq <= 0 || k <= 0) return B2F_OK;
     if (nparts < 1 || nparts > kWarp) {
         set_error("merge_topk: nparts %d not in [1,32]", nparts);
         return B2F_EINVAL;
     }
     const int wpb = 4;
-    merge_faiss_kernel<<<(unsigned)((nq + wpb - 1) / wpb), wpb * kWarp, 0, st>>>(metric == B2F_METRIC_L2, nq, (int)k,
-                                                                                nparts, Dp, Ip, stride_d_bytes, stride_i_bytes, D, I);
+    merge_faiss_kernel<<<(unsigned)((nq + wpb - 1) / wpb), wpb * kWarp, 0, st>>>(
+        metric == B2F_METRIC_L2, nq, (int)k, nparts, reinterpret_cast<const char*>(Dp), reinterpret_cast<const char*>(Ip),
+        stride, D, I);
     B2F_CUDA(cudaGetLastError());
     return B2F_OK;
 }

@@ -5,8 +5,9 @@ Every rank holds a contiguous range of the database rows in its own single-GPU I
 replicated; each rank searches its shard (global label = shard offset + local row) straight into a message
 buffer, and ONE kernel per rank pushes the message into every peer's receive buffer over NVLink peer memory,
 flags, waits for the peers' flags and merges the world parts (csrc/exchange.cu; the whole step is one C call,
-b2f_exchange_search).  B200FLAT_EXCHANGE=nccl (or a failed IPC set-up) selects the NCCL form of the same step:
-one all_gather_into_tensor of the packed messages + the CUDA merge kernel (b2f_merge_topk_strided).
+b2f_exchange_search).  B200FLAT_EXCHANGE=nccl, a failed IPC set-up, or host (numpy) queries select the all-gather
+form of the same step: one all_gather_into_tensor of the packed messages + the CUDA merge kernel
+(b2f_merge_topk_strided).
 Exact top-k over a partition = merge of per-part exact top-k, so results equal the single-GPU index.
 
 The reference has no multi-process code; its file order / .mapping list stay valid because global
@@ -97,30 +98,47 @@ class SegmentMap:
         return torch.where(local_ids >= 0, local_ids - ls[seg] + gs[seg], local_ids)
 
 
-def merge_topk(metric: int, D_parts, I_parts):
-    """[G, nq, k] per-shard results (CUDA tensors) -> merged [nq, k] via the CUDA merge kernel."""
-    import torch
-
-    G, nq, k = D_parts.shape
-    D_parts = D_parts.contiguous()
-    I_parts = I_parts.contiguous()
-    D = torch.empty((nq, k), dtype=torch.float32, device=D_parts.device)
-    I = torch.empty((nq, k), dtype=torch.int64, device=D_parts.device)
-    stream = int(torch.cuda.current_stream(D_parts.device).cuda_stream) or 1  # 0x1 = cudaStreamLegacy
-    C.check(C.load().b2f_merge_topk(int(metric), nq, k, G, D_parts.data_ptr(), I_parts.data_ptr(), D.data_ptr(),
-                                    I.data_ptr(), D_parts.device.index or 0, ctypes.c_void_p(stream)))
-    return D, I
-
-
 # a rank's packed range hits [D | pad | I] of one all-gather stay below this; a query with more hits gets a gather
 # of its own
 RANGE_PART_BYTES = 256 << 20
 
 
-def _range_layout(nhits: int) -> Tuple[int, int]:
-    """Packed [D fp32 | pad | I int64] of nhits hits: (byte offset of I, part bytes), both multiples of 16."""
-    off_i = (nhits * 4 + 15) // 16 * 16
-    return off_i, (off_i + nhits * 8 + 15) // 16 * 16
+def _packed_layout(n: int) -> Tuple[int, int]:
+    """One rank's packed message [D fp32 | pad | I int64] of n results (top-k: nq * k; range: hits): (byte offset of I,
+    part bytes), both multiples of 16."""
+    off_i = (n * 4 + 15) // 16 * 16
+    return off_i, (off_i + n * 8 + 15) // 16 * 16
+
+
+def merge_topk_strided(metric: int, recv, part_bytes: int, off_i: int, D, I):
+    """b2f_merge_topk_strided over an all-gathered buffer: recv [G * part_bytes] uint8 holding G packed parts [D | pad |
+    I at off_i] of [nq, k] results each; writes the merged top-k into D / I [nq, k] (CUDA tensors on recv's device,
+    enqueued on the current torch stream)."""
+    import torch
+
+    nq, k = int(D.shape[0]), int(D.shape[1])
+    stream = int(torch.cuda.current_stream(recv.device).cuda_stream) or 1  # 0x1 = cudaStreamLegacy
+    C.check(C.load().b2f_merge_topk_strided(int(metric), nq, k, recv.numel() // part_bytes, recv.data_ptr(),
+                                            recv.data_ptr() + off_i, part_bytes, D.data_ptr(), I.data_ptr(),
+                                            recv.device.index or 0, ctypes.c_void_p(stream)))
+
+
+def merge_topk(metric: int, D_parts, I_parts):
+    """[G, nq, k] per-shard results (CUDA tensors) -> merged [nq, k] via the CUDA merge kernel."""
+    import torch
+
+    G, nq, k = D_parts.shape
+    dev = D_parts.device
+    D = torch.empty((nq, k), dtype=torch.float32, device=dev)
+    I = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    if nq == 0:
+        return D, I
+    off_i, part = _packed_layout(nq * k)
+    recv = torch.empty((G, part), dtype=torch.uint8, device=dev)
+    recv[:, : 4 * nq * k].view(torch.float32).copy_(D_parts.reshape(G, -1))
+    recv[:, off_i: off_i + 8 * nq * k].view(torch.int64).copy_(I_parts.reshape(G, -1))
+    merge_topk_strided(metric, recv.view(-1), part, off_i, D, I)
+    return D, I
 
 
 def merge_range_strided(lims_parts, recv, part_bytes: int, off_i: int, D, I):
@@ -151,7 +169,7 @@ def merge_range(parts):
     I = torch.empty(total, dtype=torch.int64, device=dev)
     if total == 0:
         return lims, D, I
-    off_i, part = _range_layout(max(nhits))
+    off_i, part = _packed_layout(max(nhits))
     recv = torch.zeros(len(parts) * part, dtype=torch.uint8, device=dev)
     for g, (_, Dp, Ip) in enumerate(parts):
         recv[g * part: g * part + 4 * nhits[g]].view(torch.float32).copy_(Dp)
@@ -165,7 +183,7 @@ class ShardedIndexFlat:
 
     `local_index` / `merge_fn` / `range_merge_fn` exist so the host logic (partitioning, label mapping, the
     collectives) can be exercised on CPU with the gloo backend in tests; the defaults are the CUDA index and the
-    CUDA merge kernels.  range_merge_fn has merge_range_strided's signature.
+    CUDA merge kernels.  merge_fn has merge_topk_strided's signature, range_merge_fn merge_range_strided's.
     """
 
     def __init__(self, d: int, metric: int = METRIC_L2, *, storage: Optional[int] = None,
@@ -180,7 +198,7 @@ class ShardedIndexFlat:
         self.d = d
         self.metric_type = metric
         self.local = local_index if local_index is not None else IndexFlat(d, metric, storage=storage, device=device)
-        self._merge = merge_fn if merge_fn is not None else merge_topk
+        self._merge = merge_fn if merge_fn is not None else merge_topk_strided
         self._range_merge = range_merge_fn if range_merge_fn is not None else merge_range_strided
         self.segments = SegmentMap()
         self.ntotal = 0
@@ -222,18 +240,15 @@ class ShardedIndexFlat:
         self.ntotal = int(ntotal)
 
     # -- search -----------------------------------------------------------------------------------
-    def search_local(self, x, k: int):
+    def _local_offset(self) -> Optional[int]:
+        """Sets the local index's id_offset to this shard's single label offset and returns it; None when the caller
+        must map local rows to labels itself (a multi-segment shard, or a local index without id offsets)."""
+        if not hasattr(self.local, "set_search_params"):
+            return None
         off = self.segments.single_offset()
-        if hasattr(self.local, "set_search_params"):
-            # always set: an offset left behind by an earlier single-segment search must not leak into the
-            # multi-segment branch, whose labels are remapped below
-            self.local.set_search_params(id_offset=off if off is not None else 0)
-        if off is not None and hasattr(self.local, "set_search_params"):
-            return self.local.search(x, k)
-        D, I = self.local.search(x, k)
-        if isinstance(I, np.ndarray):
-            return D, self.segments.to_global_numpy(I)
-        return D, self.segments.to_global_torch(I)
+        # always set: an offset left behind by an earlier single-segment search must not leak into a remapped search
+        self.local.set_search_params(id_offset=off if off is not None else 0)
+        return off
 
     def _peer_exchange(self, need_bytes: int):
         """The NVLink peer-memory exchange (csrc/exchange.cu), created on first use and re-created when a search needs
@@ -273,61 +288,6 @@ class ShardedIndexFlat:
         self._ex = h
         return h
 
-    def _search_packed(self, x, k: int, out=None):
-        """CUDA path of search(): every rank writes its (D, I) into ONE message buffer (12 * nq * k bytes), one kernel
-        pushes it to the peers over NVLink and merges the world parts (or: one NCCL all-gather + the merge kernel).
-        out = (D [nq, k] float32, I [nq, k] int64) CUDA tensors to write into (else allocated here)."""
-        import torch
-
-        nq = int(x.shape[0])
-        if out is not None:
-            Dm, Im = out
-            if not (Dm.is_cuda and Im.is_cuda and Dm.dtype == torch.float32 and Im.dtype == torch.int64
-                    and Dm.is_contiguous() and Im.is_contiguous() and tuple(Dm.shape) == (nq, k) == tuple(Im.shape)):
-                raise AssertionError("out must be contiguous CUDA tensors (D [nq, k] float32, I [nq, k] int64)")
-        else:
-            Dm = torch.empty((nq, k), dtype=torch.float32, device=x.device)
-            Im = torch.empty((nq, k), dtype=torch.int64, device=x.device)
-        if nq == 0:
-            return Dm, Im
-        if x.device.index != self.local.device:
-            raise AssertionError("queries are on another GPU than this rank's shard")
-        off_i = (nq * k * 4 + 15) // 16 * 16
-        part = (off_i + nq * k * 8 + 15) // 16 * 16
-        stream = int(torch.cuda.current_stream(x.device).cuda_stream) or 1  # 0x1 = cudaStreamLegacy
-        off = self.segments.single_offset()
-        ex = self._peer_exchange(part)
-        if ex is not None and off is not None:
-            # the whole sharded step behind one C call: local search into the exchange's message buffer, then
-            # push over NVLink peer memory + flag + merge in one kernel -- no allocation, no second library call
-            x = x.to(torch.float32).contiguous()
-            p = C.SearchParams.from_buffer_copy(self.local._params)
-            p.id_offset = off
-            C.check(C.load().b2f_exchange_search(ex, self.local._h, nq, x.data_ptr(), k, Dm.data_ptr(), Im.data_ptr(),
-                                                 ctypes.c_void_p(stream), ctypes.byref(p)))
-            return Dm, Im
-        send = torch.empty(part, dtype=torch.uint8, device=x.device)
-        D = send[: nq * k * 4].view(torch.float32).view(nq, k)
-        I = send[off_i: off_i + nq * k * 8].view(torch.int64).view(nq, k)
-        self.local.set_search_params(id_offset=off if off is not None else 0)
-        if off is not None:
-            self.local.search_tensors_into(x, k, D, I)
-        else:
-            Dl, Il = self.local.search(x, k)
-            D.copy_(Dl)
-            I.copy_(self.segments.to_global_torch(Il))
-        if ex is not None:
-            # the one exchange step of the path, fused with the merge: push over NVLink peer memory, flag, merge
-            C.check(C.load().b2f_exchange_merge(ex, send.data_ptr(), part, int(self.metric_type), nq, k, off_i,
-                                                Dm.data_ptr(), Im.data_ptr(), ctypes.c_void_p(stream)))
-            return Dm, Im
-        recv = torch.empty(self.world * part, dtype=torch.uint8, device=x.device)
-        self._dist.all_gather_into_tensor(recv, send, group=self.group)   # NCCL form of the same exchange
-        C.check(C.load().b2f_merge_topk_strided(int(self.metric_type), nq, k, self.world, recv.data_ptr(),
-                                                recv.data_ptr() + off_i, part, Dm.data_ptr(), Im.data_ptr(),
-                                                x.device.index or 0, ctypes.c_void_p(stream)))
-        return Dm, Im
-
     def search_host(self, x_host, k: int, D_out=None, I_out=None):
         """Host-resident replicated queries (the same pinned [nq, d] float32 tensor on every rank) -> merged (D, I)
         in host tensors.  Every rank uploads only ITS 1/G slice of the batch over PCIe and the slices are
@@ -355,30 +315,72 @@ class ShardedIndexFlat:
         return D_out, I_out
 
     def search(self, x, k: int, out=None):
-        """Replicated queries -> identical merged (D, I) on every rank.  out: optional caller-owned CUDA result
-        tensors (CUDA path only), so that a serving loop allocates nothing per search."""
-        if (self.world > 1 and self._merge is merge_topk and hasattr(x, "is_cuda") and x.is_cuda
-                and hasattr(self.local, "search_tensors_into")):
-            return self._search_packed(x, k, out)
-        D, I = self.search_local(x, k)
-        if self.world == 1:
-            return D, I
+        """Replicated queries -> identical merged (D, I) on every rank (numpy in: numpy arrays; CUDA tensor in: CUDA
+        tensors).  out: optional caller-owned CUDA result tensors (CUDA queries only), so that a serving loop allocates
+        nothing per search.
+
+        Every rank searches its shard into one packed message [D | pad | I] (12 * nq * k bytes).  With CUDA queries on
+        an IndexFlat shard one kernel pushes it to the peers over NVLink peer memory and merges the world parts; without
+        the peer exchange (B200FLAT_EXCHANGE=nccl, a failed IPC set-up, host queries) one all-gather carries it and
+        merge_fn merges."""
         import torch
 
-        was_numpy = isinstance(D, np.ndarray)
-        if was_numpy:
-            D, I = torch.from_numpy(D), torch.from_numpy(I)
-        nq, kk = D.shape
-        # concatenated-along-dim-0 form ([G*nq, k]) is accepted by both NCCL and gloo
-        Dg = torch.empty((self.world * nq, kk), dtype=D.dtype, device=D.device)
-        Ig = torch.empty((self.world * nq, kk), dtype=I.dtype, device=I.device)
-        # the one exchange step of the path: 12 * nq * k bytes per rank
-        self._dist.all_gather_into_tensor(Dg, D.contiguous(), group=self.group)
-        self._dist.all_gather_into_tensor(Ig, I.contiguous(), group=self.group)
-        Dm, Im = self._merge(self.metric_type, Dg.view(self.world, nq, kk), Ig.view(self.world, nq, kk))
-        if was_numpy and not isinstance(Dm, np.ndarray):
-            Dm, Im = Dm.cpu().numpy(), Im.cpu().numpy()
-        return Dm, Im
+        off = self._local_offset()
+        if self.world == 1:
+            D, I = self.local.search(x, k)
+            if off is None:
+                I = self.segments.to_global_numpy(I) if isinstance(I, np.ndarray) else self.segments.to_global_torch(I)
+            return D, I
+        nq = int(x.shape[0])
+        dev_in = _is_torch(x) and x.is_cuda
+        flat = isinstance(self.local, IndexFlat)
+        # the results stay on the shard's GPU (a host-side stand-in for the local index keeps them on the host)
+        work = torch.device("cuda", self.local.device) if flat else torch.device("cpu")
+        if dev_in and out is not None:
+            Dm, Im = out
+            if not (Dm.is_cuda and Im.is_cuda and Dm.dtype == torch.float32 and Im.dtype == torch.int64
+                    and Dm.is_contiguous() and Im.is_contiguous() and tuple(Dm.shape) == (nq, k) == tuple(Im.shape)):
+                raise AssertionError("out must be contiguous CUDA tensors (D [nq, k] float32, I [nq, k] int64)")
+        else:
+            Dm = torch.empty((nq, k), dtype=torch.float32, device=work)
+            Im = torch.empty((nq, k), dtype=torch.int64, device=work)
+
+        def result():
+            return (Dm.to(x.device), Im.to(x.device)) if dev_in else (Dm.cpu().numpy(), Im.cpu().numpy())
+
+        if nq == 0:   # the same on every rank: no collective
+            return result()
+        off_i, part = _packed_layout(nq * k)
+        ex = None
+        if dev_in and flat:
+            if x.device.index != self.local.device:
+                raise AssertionError("queries are on another GPU than this rank's shard")
+            stream = ctypes.c_void_p(int(torch.cuda.current_stream(x.device).cuda_stream) or 1)  # 0x1 = cudaStreamLegacy
+            ex = self._peer_exchange(part)
+            if ex is not None and off is not None:
+                # the whole sharded step behind one C call: local search into the exchange's message buffer, then
+                # push over NVLink peer memory + flag + merge in one kernel -- no allocation, no second library call
+                x = x.to(torch.float32).contiguous()
+                C.check(C.load().b2f_exchange_search(ex, self.local._h, nq, x.data_ptr(), k, Dm.data_ptr(),
+                                                     Im.data_ptr(), stream, ctypes.byref(self.local._params)))
+                return Dm, Im
+        send = torch.empty(part, dtype=torch.uint8, device=work)
+        D = send[: nq * k * 4].view(torch.float32).view(nq, k)
+        I = send[off_i: off_i + nq * k * 8].view(torch.int64).view(nq, k)
+        if dev_in and flat and off is not None:
+            self.local.search_tensors_into(x, k, D, I)
+        else:
+            Dl, Il = self.local.search(x, k)
+            Il = torch.as_tensor(Il)
+            D.copy_(torch.as_tensor(Dl))
+            I.copy_(Il if off is not None else self.segments.to_global_torch(Il))
+        if ex is not None:
+            # the one exchange step of the path, fused with the merge: push over NVLink peer memory, flag, merge
+            C.check(C.load().b2f_exchange_merge(ex, send.data_ptr(), part, int(self.metric_type), nq, k, off_i,
+                                                Dm.data_ptr(), Im.data_ptr(), stream))
+        else:
+            self._merge(self.metric_type, self._all_gather(send).view(-1), part, off_i, Dm, Im)
+        return result()
 
     def _all_gather(self, t):
         """[world, *t.shape] all-gather of t (the same shape on every rank), returned on t's device.  An NCCL group
@@ -396,7 +398,7 @@ class ShardedIndexFlat:
     def _range_chunks(lims_host: np.ndarray) -> List[Tuple[int, int]]:
         """Query ranges [q0, q1) over which no rank's packed hits ([world, nq + 1] lims) exceed RANGE_PART_BYTES; a
         query with more hits than that on some rank is a range of its own."""
-        budget = max((RANGE_PART_BYTES - 32) // 12, 0)   # _range_layout(budget)[1] <= RANGE_PART_BYTES
+        budget = max((RANGE_PART_BYTES - 32) // 12, 0)   # _packed_layout(budget)[1] <= RANGE_PART_BYTES
         nq = lims_host.shape[1] - 1
         chunks, q0 = [], 0
         while q0 < nq:
@@ -426,9 +428,7 @@ class ShardedIndexFlat:
         dev_in = _is_torch(x) and x.is_cuda
         nq = int(shape[0])
 
-        off = self.segments.single_offset()
-        if hasattr(self.local, "set_search_params"):
-            self.local.set_search_params(id_offset=off if off is not None else 0)
+        off = self._local_offset()
         if params is not None:
             params = C.SearchParams.from_buffer_copy(params)
             params.id_offset = off if off is not None else 0
@@ -463,7 +463,7 @@ class ShardedIndexFlat:
                 nmax = int((lims_host[:, q1] - lims_host[:, q0]).max())
                 if nmax == 0:   # decided from the gathered lims, so every rank skips the same gathers
                     continue
-                off_i, part = _range_layout(nmax)
+                off_i, part = _packed_layout(nmax)
                 a, b = int(a_own[q0]), int(a_own[q1])
                 send = torch.empty(part, dtype=torch.uint8, device=work)
                 send[: 4 * (b - a)].view(torch.float32).copy_(D[a:b])

@@ -42,7 +42,8 @@ class OracleIndex:
 
 
 def np_merge(metric, Dg, Ig):
-    """numpy restatement of b2f_merge_topk for [G, nq, k] inputs (torch CPU tensors or arrays)."""
+    """numpy restatement of the top-k merge kernel (b2f_merge_topk_strided) for [G, nq, k] inputs (torch CPU tensors or
+    arrays)."""
     Dg = np.asarray(Dg)
     Ig = np.asarray(Ig)
     G, nq, k = Dg.shape
@@ -57,3 +58,13 @@ def np_merge(metric, Dg, Ig):
     fmax = np.finfo(np.float32).max
     D = np.where(I < 0, fmax if metric == orc.METRIC_L2 else -fmax, D).astype(np.float32)
     return D, I
+
+
+def np_topk_merge_fn(metric, recv, part_bytes, off_i, D, I):
+    """ShardedIndexFlat(merge_fn=...) stand-in for the CUDA merge: splits the all-gathered host buffer (uint8 [G *
+    part_bytes], part g = [D fp32 | pad | I int64 at off_i], [nq, k] each) and merges with np_merge into D / I."""
+    nq, k = D.shape
+    buf = recv.numpy().reshape(-1, part_bytes)
+    Dg = buf[:, : 4 * nq * k].copy().view(np.float32).reshape(-1, nq, k)
+    Ig = buf[:, off_i: off_i + 8 * nq * k].copy().view(np.int64).reshape(-1, nq, k)
+    D.numpy()[:], I.numpy()[:] = np_merge(metric, Dg, Ig)

@@ -48,11 +48,15 @@ def _worker(rank, world, port, out_dir):
             del os.environ["B200FLAT_EXCHANGE"]
             Dh, Ih = ix.search_host(xq.cpu().pin_memory(), k)
             De, Ie = ix.search(xq[:0], k)
+            Dnp, Inp = ix.search(xq.cpu().numpy(), k)             # host queries: one all-gather, numpy results
+            Dct, Ict = ix.search(xq.cpu(), k)
             torch.cuda.synchronize()
             same = all(torch.equal(Io, I[: Io.shape[0]]) and torch.equal(Do, D[: Do.shape[0]]) for Do, Io in outs)
             same = same and torch.equal(Ib[:nq], I) and torch.equal(Ib[-nq:], I) and torch.equal(Db[nq:2 * nq], D)
             same = same and torch.equal(In, I) and torch.equal(Dn, D)
             same = same and torch.equal(Ih.cuda(), I) and torch.equal(Dh.cuda(), D) and tuple(Ie.shape) == (0, k)
+            same = same and all(isinstance(Dx, np.ndarray) and np.array_equal(Ix, I.cpu().numpy())
+                                and np.array_equal(Dx, D.cpu().numpy()) for Dx, Ix in ((Dnp, Inp), (Dct, Ict)))
             # caller-owned result tensors (nothing allocated per search)
             Do, Io = torch.empty_like(D), torch.empty_like(I)
             ix.search(xq, k, out=(Do, Io))

@@ -1,6 +1,7 @@
 """GPU tier of ShardedIndexFlat.range_search: the merge kernel (b2f_merge_range_strided) bit for bit against its numpy
 restatement; per-shard IndexFlats on one GPU merged by it against one IndexFlat over every row; the whole sharded path
-with two processes sharing one GPU over gloo; and, on >= 2 GPUs, the NCCL path with one process per GPU.
+with two processes sharing one GPU over gloo (and top-k search with numpy queries there); and, on >= 2 GPUs, the NCCL
+path with one process per GPU.
 
 On fp32 storage a shard holds exactly the rows one index would hold, and a range hit's distance does not depend on the
 path or the batch (DESIGN 3.5), so merged results must equal one index's bit for bit."""
@@ -57,7 +58,7 @@ def test_merge_kernel_equals_restatement(nparts, nq):
     want = np_merge_range(lims, D, I)
     assert _same(want, np_union_range(lims, D, I))
     nmax = max(len(i) for i in I)
-    off_i, part = sharded._range_layout(max(nmax, 1))
+    off_i, part = sharded._packed_layout(max(nmax, 1))
     buf = np.zeros(nparts * part, np.uint8)
     for g in range(nparts):
         buf[g * part: g * part + 4 * len(D[g])] = D[g].view(np.uint8)
@@ -149,8 +150,11 @@ def test_shards_merged_exact_on_lattice(metric):
 
 
 # ---- two processes sharing one GPU, gloo ---------------------------------------------------------------------------
-# Only range_search, add and remove_ids run on these indexes: the top-k path's peer exchange spin-waits on the other
-# rank's flag, and two contexts time-slicing one GPU must not be put in that position.
+# Top-k search runs on these indexes with numpy queries only, which take no peer exchange: the exchange spin-waits on the
+# other rank's flag, and two contexts time-slicing one GPU must not be put in that position.
+TOPK = 10
+
+
 def _one_gpu_worker(rank, world, port, out_dir):
     import torch
     import torch.distributed as dist
@@ -172,11 +176,17 @@ def _one_gpu_worker(rank, world, port, out_dir):
             ix = m.ShardedIndexFlat(d, metric, storage=m.STORE_F32, device=0)
             ix.add(z["xb1"])
             res = {"a": ix.range_search(xq, r)}
+            topk = {"a": ix.search(z["xq"], TOPK)}
             ix.add(z["xb2"])
             res["b"] = ix.range_search(xq, r)
             res["b_np"] = ix.range_search(z["xq"], r)
+            topk["b"] = ix.search(z["xq"], TOPK)
             ix.remove_ids(m.IDSelectorRange(100, 900))
             res["c"] = ix.range_search(xq, r)
+            topk["c"] = ix.search(z["xq"], TOPK)
+            for k, (D, I) in topk.items():
+                assert isinstance(D, np.ndarray) and isinstance(I, np.ndarray)
+                out[f"{metric}_{k}_topk_D"], out[f"{metric}_{k}_topk_I"] = D, I
             sharded.RANGE_PART_BYTES = 4096
             res["c_chunked"] = ix.range_search(xq, r)
             out[f"chunks{metric}"] = ix.last_range_info["chunks"]
@@ -218,11 +228,14 @@ def test_two_processes_on_one_gpu(tmp_path):
             one.add(rows)
             want = one.range_search(torch.from_numpy(xq).cuda(), r)
             assert int(want[0][-1]) > 0
+            Dw, Iw = one.search(xq, TOPK)
             keys = [key] + {"b": ["b_np"], "c": ["c_chunked"]}.get(key, [])
             for z in zs:
                 for k in keys:
                     got = tuple(z[f"{metric}_{k}_{name}"] for name in ("lims", "D", "I"))
                     assert _same(got, want), (metric, k)
+                assert np.array_equal(z[f"{metric}_{key}_topk_I"], Iw), (metric, key)
+                assert np.allclose(z[f"{metric}_{key}_topk_D"], Dw, rtol=1e-5), (metric, key)
                 assert z[f"{metric}_b_np_lims"].dtype == np.uint64
                 assert int(z[f"chunks{metric}"]) > 1
                 assert z[f"{metric}_empty_lims"].tolist() == [0] and len(z[f"{metric}_empty_I"]) == 0

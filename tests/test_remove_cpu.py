@@ -13,7 +13,7 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 import oracle as orc
-from tests.helpers import OracleIndex, np_merge
+from tests.helpers import OracleIndex, np_topk_merge_fn
 
 TILE_BYTES = 32 << 10   # kRemoveTileBytes
 
@@ -219,11 +219,7 @@ def _sharded_worker(rank, world, port, metric, out_dir):
         xb3 = orc.np_synth_rows(21, 580, 90, D_)
         xq = orc.np_synth_rows(22, 0, 7, D_)
 
-        def merge(metric_, Dg, Ig):
-            D, I = np_merge(metric_, Dg.numpy(), Ig.numpy())
-            return torch.from_numpy(D), torch.from_numpy(I)
-
-        ix = ShardedIndexFlat(D_, metric, local_index=RemovableOracleIndex(D_, metric), merge_fn=merge)
+        ix = ShardedIndexFlat(D_, metric, local_index=RemovableOracleIndex(D_, metric), merge_fn=np_topk_merge_fn)
         ix.add(xb1)
         ix.add(xb2)
         n1 = ix.remove_ids(REMOVE1)

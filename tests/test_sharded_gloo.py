@@ -1,17 +1,16 @@
-"""CPU tier: the N>1 host path (partition -> per-rank search -> one all-gather -> merge) on the gloo
-backend with world_size 2 and 3, using oracle-backed local shards.  Results must equal a
-single-index search of the concatenated database."""
+"""CPU tier: the N>1 path without the peer exchange (partition -> per-rank search into one packed message -> one
+all-gather -> merge) on the gloo backend with world_size 2 and 3, using oracle-backed local shards and the numpy
+restatement of the merge kernel.  Results must equal a single-index search of the concatenated database."""
 import os
 import socket
 
 import numpy as np
 import pytest
-import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
 import oracle as orc
-from tests.helpers import OracleIndex, np_merge
+from tests.helpers import OracleIndex, np_topk_merge_fn
 
 
 def _free_port():
@@ -34,11 +33,7 @@ def _worker(rank, world, port, metric, out_dir):
         xb2 = orc.np_synth_rows(11, 501, 77, d)
         xq = orc.np_synth_rows(12, 0, 9, d)
 
-        def merge(metric_, Dg, Ig):
-            D, I = np_merge(metric_, Dg.numpy(), Ig.numpy())
-            return torch.from_numpy(D), torch.from_numpy(I)
-
-        ix = ShardedIndexFlat(d, metric, local_index=OracleIndex(d, metric), merge_fn=merge)
+        ix = ShardedIndexFlat(d, metric, local_index=OracleIndex(d, metric), merge_fn=np_topk_merge_fn)
         ix.add(xb1)
         D0, I0 = ix.search(xq, k)   # single segment: the shard offset is applied by the local index ...
         ix.add(xb2)   # second add: labels continue after the first, shard holds two segments

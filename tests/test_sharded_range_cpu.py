@@ -70,7 +70,7 @@ def test_range_chunks_cap_each_rank_and_isolate_big_queries(monkeypatch):
     for q0, q1 in chunks:
         n = lims[:, q1] - lims[:, q0]
         assert q1 - q0 == 1 or n.max() <= 10
-        assert sharded._range_layout(int(n.max()))[1] <= sharded.RANGE_PART_BYTES or q1 - q0 == 1
+        assert sharded._packed_layout(int(n.max()))[1] <= sharded.RANGE_PART_BYTES or q1 - q0 == 1
     assert sharded.ShardedIndexFlat._range_chunks(np.zeros((3, 1), np.int64)) == []
 
 

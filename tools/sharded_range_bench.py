@@ -127,7 +127,7 @@ def main():
                 lims_parts[g, 1:] = torch.bincount(qid[sel], minlength=NQ).cumsum(0)
                 parts.append((Do[sel], Io[sel]))
             nmax = max(int(p[0].numel()) for p in parts)
-            off_i, part = sharded._range_layout(nmax)
+            off_i, part = sharded._packed_layout(nmax)
             recv = torch.zeros(G * part, dtype=torch.uint8, device="cuda")
             for g, (dp, ip) in enumerate(parts):
                 recv[g * part: g * part + 4 * dp.numel()].view(torch.float32).copy_(dp)
