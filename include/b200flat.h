@@ -143,6 +143,32 @@ B2F_API int b2f_index_add(b2f_index* idx, int64_t n, const float* x, int32_t mem
 B2F_API int b2f_index_search(b2f_index* idx, int64_t nq, const float* q, int64_t k, float* D, int64_t* I,
                      int32_t mem, void* stream, const b2f_search_params* params);
 
+/* ---- filtered search: faiss's index.search(x, k, params=SearchParameters(sel=...)) and the same for range_search -------
+ * A row is searched only when the selector contains its label (row + params->id_offset, the id the call would return):
+ * faiss's sel->is_member(id).  Top-k returns the k best allowed rows in the unfiltered tie order, padded with label -1 and
+ * distance +FLT_MAX (L2) / -FLT_MAX (IP) when fewer than k rows are allowed; range search returns exactly the hits of the
+ * unfiltered call whose label is allowed, with the same distance bits and order.  sel = NULL is the unfiltered call, and
+ * an allow-everything selector gives bit-identical results to it.  Filtered searches count in b2f_stats like any search
+ * and feed the same adaptive state (b2f_search_params.certify); that state changes speed only, never results.
+ * Each call builds a one-bit-per-row allow bitmap (and, on the tensor path, a copy of the row biases with the excluded
+ * rows' set to NaN, which no threshold admits) in the search workspace on `stream`; a filtered search still reads every
+ * row.  kind B2F_SEL_*; a bad kind, n < 0 or a NULL data with n > 0 is B2F_EINVAL.                                      */
+#define B2F_SEL_RANGE 1   /* faiss IDSelectorRange(imin, imax): imin <= label < imax */
+#define B2F_SEL_BATCH 2   /* faiss IDSelectorBatch(ids): data = int64 ids [n]; duplicates, negative ids and ids with no row never match */
+#define B2F_SEL_BITMAP 3  /* faiss IDSelectorBitmap(n, bitmap): data = uint8 [n] (n counts BYTES); label i is bit i & 7 of byte
+                             i >> 3; labels past the bitmap are not members */
+typedef struct b2f_selector {
+    int32_t kind;        /* B2F_SEL_* */
+    int32_t negate;      /* IDSelectorNot: 1 = every label the selector does NOT contain */
+    int64_t imin, imax;  /* RANGE: imin <= label < imax */
+    int64_t n;           /* BATCH: number of ids; BITMAP: number of bytes */
+    const void* data;    /* BATCH: int64 ids; BITMAP: uint8 bytes; in the call's `mem`, like q (host data is copied up on
+                            `stream` and may be released when the call returns) */
+} b2f_selector;
+/* b2f_index_search restricted to the selector's labels (b2f_index_search = this call with sel = NULL) */
+B2F_API int b2f_index_search_filtered(b2f_index* idx, int64_t nq, const float* q, int64_t k, float* D, int64_t* I,
+                                      int32_t mem, void* stream, const b2f_search_params* params, const b2f_selector* sel);
+
 /* ---- index.range_search(q, radius): every row closer than a radius (faiss IndexFlat range search) ----------------
  * L2: radius is on SQUARED distances, a row is a hit when dist < radius (strict); an L2 radius <= 0 returns nothing.
  * IP: a row is a hit when ip > radius (strict).  NaN distances are never hits; a NaN radius is B2F_EINVAL.
@@ -162,6 +188,9 @@ typedef struct b2f_range_result b2f_range_result;
  * hits may still be in flight on `stream`.  A result too large for device memory is B2F_ENOMEM. */
 B2F_API int b2f_index_range_search(b2f_index* idx, int64_t nq, const float* q, float radius, int32_t mem, void* stream,
                                    const b2f_search_params* params, b2f_range_result** out);
+/* b2f_index_range_search restricted to the selector's labels (b2f_index_range_search = this call with sel = NULL) */
+B2F_API int b2f_index_range_search_filtered(b2f_index* idx, int64_t nq, const float* q, float radius, int32_t mem, void* stream,
+                                            const b2f_search_params* params, const b2f_selector* sel, b2f_range_result** out);
 B2F_API int b2f_range_result_lims(const b2f_range_result* r, int64_t* lims /* host, nq + 1 */);
 /* D [lims[nq]] fp32, I [lims[nq]] int64 in `mem`; device: enqueued on `stream`, host: synchronous */
 B2F_API int b2f_range_result_fetch(b2f_range_result* r, float* D, int64_t* I, int32_t mem, void* stream);

@@ -16,11 +16,18 @@ from ._capi import (  # noqa: F401
 from .index import (  # noqa: F401
     METRIC_INNER_PRODUCT,
     METRIC_L2,
+    IDSelectorAnd,
+    IDSelectorArray,
     IDSelectorBatch,
+    IDSelectorBitmap,
+    IDSelectorNot,
+    IDSelectorOr,
     IDSelectorRange,
+    IDSelectorXor,
     IndexFlat,
     IndexFlatIP,
     IndexFlatL2,
+    SearchParameters,
     read_index,
     write_index,
 )

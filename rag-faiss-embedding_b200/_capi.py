@@ -25,6 +25,8 @@ MEM_DEVICE = 1
 ALGO_AUTO, ALGO_SCAN, ALGO_TENSOR = 0, 1, 2
 POOL_CLS, POOL_MEAN = 0, 1
 
+SEL_RANGE, SEL_BATCH, SEL_BITMAP = 1, 2, 3
+
 OK, EINVAL, ENOGPU, ECUDA, EIO, EFORMAT, ENOMEM, ERANGE = 0, -1, -2, -3, -4, -5, -6, -7
 
 
@@ -37,6 +39,18 @@ class SearchParams(ctypes.Structure):
         ("id_offset", ctypes.c_int64),
         ("profile", ctypes.c_int32),
         ("reserved", ctypes.c_int32),
+    ]
+
+
+class Selector(ctypes.Structure):
+    """b2f_selector: a faiss ID selector as the filtered entry points take it."""
+    _fields_ = [
+        ("kind", ctypes.c_int32),
+        ("negate", ctypes.c_int32),
+        ("imin", ctypes.c_int64),
+        ("imax", ctypes.c_int64),
+        ("n", ctypes.c_int64),
+        ("data", ctypes.c_void_p),
     ]
 
 
@@ -85,8 +99,12 @@ PROTOTYPES = {
     "b2f_index_device": (_i32, [_vp]),
     "b2f_index_add": (ctypes.c_int, [_vp, _i64, _vp, _i32, _vp]),
     "b2f_index_search": (ctypes.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i32, _vp, ctypes.POINTER(SearchParams)]),
+    "b2f_index_search_filtered": (ctypes.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _i32, _vp, ctypes.POINTER(SearchParams),
+                                                 ctypes.POINTER(Selector)]),
     "b2f_index_range_search": (ctypes.c_int, [_vp, _i64, _vp, ctypes.c_float, _i32, _vp, ctypes.POINTER(SearchParams),
                                               ctypes.POINTER(_vp)]),
+    "b2f_index_range_search_filtered": (ctypes.c_int, [_vp, _i64, _vp, ctypes.c_float, _i32, _vp, ctypes.POINTER(SearchParams),
+                                                       ctypes.POINTER(Selector), ctypes.POINTER(_vp)]),
     "b2f_range_result_lims": (ctypes.c_int, [_vp, ctypes.POINTER(_i64)]),
     "b2f_range_result_fetch": (ctypes.c_int, [_vp, _vp, _vp, _i32, _vp]),
     "b2f_range_result_info": (ctypes.c_int, [_vp, ctypes.POINTER(_i64)]),

@@ -244,6 +244,7 @@ struct ScanFuse {                  // device-side view (kernel argument)
     uint32_t* tub;                 // persistent [2][3][8]: per-query upper bound of the k-th best key (min over CTAs), all-ones when idle
     int32_t parity;                // launch parity: this launch uses tub[parity] and re-arms tub[parity ^ 1]
     const float* mu;               // bf16 rows: centre added back to every stored row (null: none)
+    const uint32_t* allow;         // optional filtered search: bit r of word r / 32 set = row r may be returned
 };
 struct ScanArgs {                  // host-side launch description
     const float* rows_f32;         // fp32 rows, or
@@ -267,6 +268,7 @@ struct ScanArgs {                  // host-side launch description
     int32_t nq_batch, certify;
     uint32_t* tub;
     int32_t parity;
+    const uint32_t* allow;         // optional (device): the filtered search's allow bitmap
 };
 constexpr int kScanTubWords = 2 * 3 * 8;
 int scan_max_parts();
@@ -353,6 +355,7 @@ struct RerankArgs {
     const int32_t* out_map;         // optional: query q of this launch writes row out_map[q] of D / I (< 0: skip) and is
                                     // recorded under that index when it fails (range pass over compacted failed queries)
     int32_t range;                  // 1: range pass -- the lists hold EVERY row with coarse key <= the fixed threshold: re-rank all
+    const uint32_t* allow;          // optional: the filtered search's allow bitmap (the exact range scan skips other rows)
 };
 int launch_rerank(const RerankArgs& a, cudaStream_t st);
 
@@ -416,5 +419,22 @@ int launch_range_offsets(const int32_t* count, int n, int64_t* lims, cudaStream_
 // staged hits of queries 0..nq-1 to D / I at base + lims[q] in faiss format (L2: key, IP: -key; label = id + id_offset)
 int launch_range_emit(const float* skey, const int32_t* sid, const int32_t* staged, const int64_t* lims, int nq, int64_t base, int metric,
                       float* D, int64_t* I, int64_t id_offset, cudaStream_t st);
+
+// ---- filtered search (filter.cu) ---------------------------------------------------------------------------------------
+// B2F_EINVAL for a bad kind, n < 0 or null data with n > 0 (null sel: fine)
+int check_selector(const b2f_selector* sel);
+// the part of the selector's data a call reads: BATCH ids [lo, hi), BITMAP bytes [lo, hi) (those of the index's labels)
+struct FilterWindow {
+    int64_t lo, hi;
+};
+FilterWindow filter_window(const b2f_selector& sel, int64_t ntotal, int64_t id_offset);
+// device bytes a call with host-memory selector data stages that data in
+size_t filter_staged_bytes(const b2f_selector& sel, int64_t ntotal, int64_t id_offset);
+// allow [ceil(ntotal / 32)]: bit r set <=> the selector contains label r + id_offset.  Host data (mem) goes up to
+// `staged` with cudaMemcpyAsync first.  One launch, two for BATCH with ids.
+int launch_allow_bitmap(const b2f_selector& sel, int32_t mem, int64_t ntotal, int64_t id_offset, void* staged, uint32_t* allow,
+                        cudaStream_t st);
+// bias[r] = norms[r] for allowed rows, NaN for the others: the row bias the tensor pass reads in a filtered search
+int launch_masked_bias(const float* norms, const uint32_t* allow, int64_t ntotal, float* bias, cudaStream_t st);
 
 }  // namespace b2f

@@ -376,7 +376,7 @@ int order_after(cudaStream_t waiter, cudaStream_t producer, b2f_index* ix) {
 // tensor-path search: it also publishes the search's counters.
 int enqueue_scan(b2f_index* ix, const float* qd, const int32_t* qsel, const int32_t* nsel_dev, int nsel, int k, float* Dd,
                  int64_t* Id, int64_t id_offset, void* scratch, int32_t* counters, int32_t seq, int nq_batch, int certify,
-                 cudaStream_t st) {
+                 const uint32_t* allow, cudaStream_t st) {
     ScanArgs a{};
     a.rows_f32 = ix->storage == B2F_STORE_F32 ? ix->rows_f32 : nullptr;
     a.rows_bf16 = ix->scan;
@@ -402,6 +402,7 @@ int enqueue_scan(b2f_index* ix, const float* qd, const int32_t* qsel, const int3
     a.certify = certify;
     a.tub = reinterpret_cast<uint32_t*>(ix->totals + 4);
     a.parity = (int32_t)(ix->scan_launches++ & 1);
+    a.allow = allow;
     B2F_TRY(launch_scan(a, st));
     ix->st.launches += 1;
     ix->st.last_launches += 1;
@@ -955,6 +956,37 @@ static TensorScanLists take_lists(Bump& b, const TensorScanPlan& p) {
     return l;
 }
 
+// A filtered search's buffers: the allow bitmap, the masked row bias of the tensor pass, and the device copy of host-memory
+// selector data
+struct FilterWs {
+    uint32_t* allow = nullptr;
+    float* bias = nullptr;
+    void* staged = nullptr;
+};
+
+static FilterWs carve_filter(Bump& b, const b2f_index* ix, const b2f_selector* sel, int64_t id_offset, bool host, bool tensor) {
+    FilterWs f;
+    if (!sel || ix->ntotal == 0) return f;
+    f.allow = b.take<uint32_t>((size_t)(ix->ntotal + 31) / 32);
+    if (tensor) f.bias = b.take<float>((size_t)ix->ntotal);
+    if (host) f.staged = b.take<char>(filter_staged_bytes(*sel, ix->ntotal, id_offset));
+    return f;
+}
+
+// Builds a filtered call's allow bitmap (and, for the tensor pass, its masked bias) on st; *launches: kernels launched
+static int build_filter(const b2f_index* ix, const b2f_selector* sel, int32_t mem, int64_t id_offset, const FilterWs& f,
+                        cudaStream_t st, int* launches) {
+    *launches = 0;
+    if (!f.allow) return B2F_OK;
+    B2F_TRY(launch_allow_bitmap(*sel, mem, ix->ntotal, id_offset, f.staged, f.allow, st));
+    *launches = (sel->kind == B2F_SEL_BATCH && sel->n > 0) ? 2 : 1;
+    if (f.bias) {
+        B2F_TRY(launch_masked_bias(ix->norms, f.allow, ix->ntotal, f.bias, st));
+        ++*launches;
+    }
+    return B2F_OK;
+}
+
 // What one search carves from the workspace, in one order.  search_locked carves it over a null base for the size, then
 // over the workspace.
 struct SearchWs {
@@ -973,11 +1005,13 @@ struct SearchWs {
     // [0] uncertified queries, [1] of which list overflows, [2..3] u64 list entries, [4] rescued by the extended pass,
     // [8..11] ticket counters of K2's die-aware unit assignment
     int32_t* counters = nullptr;
+    FilterWs filter{};               // filtered search
 };
 
 static SearchWs carve_search(Bump& b, const b2f_index* ix, int nq, int k, bool host, bool tensor, const TensorScanPlan& plan,
-                             int chunk_nq, int kp) {
+                             int chunk_nq, int kp, const b2f_selector* sel, int64_t id_offset) {
     SearchWs w;
+    w.filter = carve_filter(b, ix, sel, id_offset, host, tensor);
     if (host) {
         w.q = b.take<float>((size_t)nq * ix->d);
         w.D = b.take<float>((size_t)nq * k);
@@ -1116,8 +1150,8 @@ static int range_pass(b2f_index* ix, Bump& bump, const SearchWs& w, const float*
                                 (int64_t)nq_pad * rp.nlists, st));
     B2F_TRY(launch_range_thresholds(r.tau, 0.f, r.out_map, nr, ix->d, ix->metric, r.pq.qnorm, r.pq.qerr, r.pq.qconst,
                                     sqrtf(ix->host_stats[0]), sqrtf(ix->host_stats[1]), ix->mu_norm, r.thr, st));
-    B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, r.pq.qb, nr, nq_pad, rp, nullptr, nullptr,
-                               r.lists, st));
+    B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, w.filter.bias ? w.filter.bias : ix->norms, ix->ntotal, ix->metric, r.pq.qb, nr,
+                               nq_pad, rp, nullptr, nullptr, r.lists, st));
     RerankArgs ra = rerank_args(ix, r.q, r.pq, nr, k, kp, D, I, id_offset, r.fail_list, r.counters);
     ra.out_map = r.out_map;
     ra.range = 1;
@@ -1137,7 +1171,7 @@ static int range_pass(b2f_index* ix, Bump& bump, const SearchWs& w, const float*
 // The caller holds ix->mu (search_pooled pools the queries into the index's buffer and searches them under ONE
 // lock, so a second thread cannot overwrite or re-allocate that buffer in between).
 static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k64, float* D, int64_t* I, int32_t mem,
-                         void* stream, const b2f_search_params* params) {
+                         void* stream, const b2f_search_params* params, const b2f_selector* sel) {
     if (k64 <= 0) {
         set_error("k must be > 0 (faiss asserts k > 0)");
         return B2F_EINVAL;
@@ -1188,10 +1222,10 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
 
     // ---- workspace -----------------------------------------------------------------------------
     Bump layout(nullptr, SIZE_MAX);
-    carve_search(layout, ix, nq, k, host, tensor, plan, chunk_nq, kp);
+    carve_search(layout, ix, nq, k, host, tensor, plan, chunk_nq, kp, sel, P.id_offset);
     B2F_TRY(ensure_ws(ix, tensor && ix->adapt.range_mode ? range_end(layout, ix, nq, kp) : layout.off));
     Bump bump(ix->ws, ix->ws_bytes);
-    const SearchWs w = carve_search(bump, ix, nq, k, host, tensor, plan, chunk_nq, kp);
+    const SearchWs w = carve_search(bump, ix, nq, k, host, tensor, plan, chunk_nq, kp, sel, P.id_offset);
     if (!bump.fits()) {
         set_error("search workspace: the layout needs %zu bytes, the workspace has %zu", bump.off, bump.size);
         return B2F_ECUDA;
@@ -1204,6 +1238,10 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
     ix->st.last_launches = 0;
     ix->st.last_algo = algo;
     ix->st.last_kprime = 0;
+    int filter_launches = 0;
+    B2F_TRY(build_filter(ix, sel, mem, P.id_offset, w.filter, st, &filter_launches));
+    ix->st.launches += filter_launches;
+    ix->st.last_launches += filter_launches;
     int n_main = 0;
     b2f_index::ProfSlot* slot = nullptr;
     if (profile) {
@@ -1231,7 +1269,8 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
         ix->st.last_launches++;
     } else if (!tensor) {
         B2F_TRY(main_event(0));
-        B2F_TRY(enqueue_scan(ix, qd, nullptr, nullptr, nq, k, Dd, Id, P.id_offset, w.scan_scratch, nullptr, 0, nq, 0, st));
+        B2F_TRY(enqueue_scan(ix, qd, nullptr, nullptr, nq, k, Dd, Id, P.id_offset, w.scan_scratch, nullptr, 0, nq, 0, w.filter.allow,
+                             st));
         B2F_TRY(main_event(1));
         n_main++;
     } else {
@@ -1247,8 +1286,8 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
                                         c0 == 0 ? 16 : 0, reinterpret_cast<uint32_t*>(w.lists.shared_thr),
                                         plan.list_mode ? (int64_t)nq_pad * plan.nlists : 0, st));
             B2F_TRY(main_event(0));
-            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, w.pq.qb, cn, nq_pad, plan, w.pk, w.pi,
-                                       w.lists, st));
+            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, w.filter.bias ? w.filter.bias : ix->norms, ix->ntotal, ix->metric, w.pq.qb,
+                                       cn, nq_pad, plan, w.pk, w.pi, w.lists, st));
             B2F_TRY(main_event(1));
             n_main++;
             // the re-rank writes faiss-formatted results directly (no finalize launch)
@@ -1280,7 +1319,7 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
         // device -- with none (the usual case) the kernel publishes the counters and exits -- so the host never
         // waits inside a search and consecutive searches run back to back on the GPU.
         B2F_TRY(enqueue_scan(ix, qd, scan_list, scan_counters, 0, k, Dd, Id, P.id_offset, w.scan_scratch, scan_counters, ++ix->seq, nq,
-                             certify, st));
+                             certify, w.filter.allow, st));
         if (range_served) {
             ix->adapt.range_ran_seq = ix->seq;
             ix->adapt.range_ran_nfail = range_served;
@@ -1350,11 +1389,13 @@ struct RangeSearchWs {
     TensorScanLists lists{};
     float* skey = nullptr;           // [chunk][kRangeHitsMax] staged hits: exact key, row id
     int32_t* sid = nullptr;
+    FilterWs filter{};               // filtered search
 };
 
 static RangeSearchWs carve_range_search(Bump& b, const b2f_index* ix, int cn, bool host, bool tensor, const TensorScanPlan& plan,
-                                        int ntiles) {
+                                        int ntiles, const b2f_selector* sel, int64_t id_offset) {
     RangeSearchWs w;
+    w.filter = carve_filter(b, ix, sel, id_offset, host, tensor);
     if (host) w.q = b.take<float>((size_t)cn * ix->d);
     w.count = b.take<int32_t>(cn);
     w.staged = b.take<int32_t>(cn);
@@ -1406,7 +1447,7 @@ static int range_result_reserve(b2f_range_result* r, int64_t need, cudaStream_t 
 // [tensor: prep, thresholds, K2 listing every row at or below thr(tau), collect] -> exact range scan count pass over what
 // the lists could not answer (or over the whole chunk) -> offsets -> ONE host sync for the chunk's lims -> emit.
 static int range_search_locked(b2f_index* ix, int nq, const float* q, float radius, int32_t mem, void* stream,
-                               const b2f_search_params* params, b2f_range_result* r) {
+                               const b2f_search_params* params, const b2f_selector* sel, b2f_range_result* r) {
     b2f_search_params P{};
     if (params) P = *params;
     const bool l2 = ix->metric == B2F_METRIC_L2;
@@ -1450,11 +1491,11 @@ static int range_search_locked(b2f_index* ix, int nq, const float* q, float radi
             }
         }
         Bump layout(nullptr, SIZE_MAX);
-        carve_range_search(layout, ix, cn, host, tensor, plan, geo.ntiles);
+        carve_range_search(layout, ix, cn, host, tensor, plan, geo.ntiles, sel, P.id_offset);
         if (layout.off > ix->ws_bytes && ix->ws) syncs++;
         B2F_TRY(ensure_ws(ix, layout.off));
         Bump bump(ix->ws, ix->ws_bytes);
-        const RangeSearchWs w = carve_range_search(bump, ix, cn, host, tensor, plan, geo.ntiles);
+        const RangeSearchWs w = carve_range_search(bump, ix, cn, host, tensor, plan, geo.ntiles, sel, P.id_offset);
         if (!bump.fits()) {
             set_error("range search workspace: the layout needs %zu bytes, the workspace has %zu", bump.off, bump.size);
             return B2F_ECUDA;
@@ -1462,14 +1503,19 @@ static int range_search_locked(b2f_index* ix, int nq, const float* q, float radi
         const float* qc = host ? w.q : q + (int64_t)c0 * ix->d;
         if (host) B2F_CUDA(cudaMemcpyAsync(w.q, q + (int64_t)c0 * ix->d, (size_t)cn * ix->d * 4, cudaMemcpyHostToDevice, st));
         a.q = qc;
+        // (built per chunk: a later chunk may re-allocate the workspace)
+        int filter_launches = 0;
+        B2F_TRY(build_filter(ix, sel, mem, P.id_offset, w.filter, st, &filter_launches));
+        launches += filter_launches;
+        a.allow = w.filter.allow;
         if (tensor) {
             const int nq_pad = plan.nq_tiles * 128;
             B2F_TRY(launch_prep_queries(qc, cn, nq_pad, ix->d, w.pq.qb, ix->dpad, w.pq.qnorm, w.pq.qerr, w.pq.qconst,
                                         ix->mu_set ? ix->centre : nullptr, reinterpret_cast<uint32_t*>(w.counters), 16, nullptr, 0, st));
             B2F_TRY(launch_range_thresholds(nullptr, tau, nullptr, cn, ix->d, ix->metric, w.pq.qnorm, w.pq.qerr, w.pq.qconst,
                                             max_row_norm, max_row_err, ix->mu_norm, w.thr, st));
-            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, ix->norms, ix->ntotal, ix->metric, w.pq.qb, cn, nq_pad, plan, nullptr, nullptr,
-                                       w.lists, st));
+            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, w.filter.bias ? w.filter.bias : ix->norms, ix->ntotal, ix->metric, w.pq.qb,
+                                       cn, nq_pad, plan, nullptr, nullptr, w.lists, st));
             B2F_TRY(launch_range_collect(w.lists, cn, plan, tau, a, w.skey, w.sid, w.staged, w.count, w.scan_list, w.counters, st));
             launches += 4;
         } else {
@@ -1537,11 +1583,17 @@ int b2f_range_result_destroy(b2f_range_result* r) {
 
 int b2f_index_range_search(b2f_index* ix, int64_t nq, const float* q, float radius, int32_t mem, void* stream,
                            const b2f_search_params* params, b2f_range_result** out) {
+    return b2f_index_range_search_filtered(ix, nq, q, radius, mem, stream, params, nullptr, out);
+}
+
+int b2f_index_range_search_filtered(b2f_index* ix, int64_t nq, const float* q, float radius, int32_t mem, void* stream,
+                                    const b2f_search_params* params, const b2f_selector* sel, b2f_range_result** out) {
     if (!out) {
         set_error("range_search: out is NULL");
         return B2F_EINVAL;
     }
     *out = nullptr;
+    B2F_TRY(check_selector(sel));
     if (!ix) {
         set_error("index is NULL");
         return B2F_EINVAL;
@@ -1563,7 +1615,7 @@ int b2f_index_range_search(b2f_index* ix, int64_t nq, const float* q, float radi
     int rc;
     {
         std::lock_guard<std::mutex> lk(ix->mu);
-        rc = range_search_locked(ix, (int)nq, q, radius, mem, stream, params, r);
+        rc = range_search_locked(ix, (int)nq, q, radius, mem, stream, params, sel, r);
     }
     if (rc != B2F_OK) {
         b2f_range_result_destroy(r);
@@ -1619,12 +1671,18 @@ extern "C" {
 
 int b2f_index_search(b2f_index* ix, int64_t nq, const float* q, int64_t k, float* D, int64_t* I, int32_t mem, void* stream,
                      const b2f_search_params* params) {
+    return b2f_index_search_filtered(ix, nq, q, k, D, I, mem, stream, params, nullptr);
+}
+
+int b2f_index_search_filtered(b2f_index* ix, int64_t nq, const float* q, int64_t k, float* D, int64_t* I, int32_t mem,
+                              void* stream, const b2f_search_params* params, const b2f_selector* sel) {
+    B2F_TRY(check_selector(sel));
     if (!ix) {
         set_error("index is NULL");
         return B2F_EINVAL;
     }
     std::lock_guard<std::mutex> lk(ix->mu);
-    return search_locked(ix, nq, q, k, D, I, mem, stream, params);
+    return search_locked(ix, nq, q, k, D, I, mem, stream, params, sel);
 }
 
 int b2f_index_search_pooled(b2f_index* ix, const float* hidden, const int64_t* mask, int64_t B, int64_t T, int32_t pool,
@@ -1658,7 +1716,7 @@ int b2f_index_search_pooled(b2f_index* ix, const float* hidden, const int64_t* m
         B2F_TRY(launch_pool(hidden, mask, B, T, ix->d, pool, normalize, qbuf, nullptr, 0, nullptr, nullptr, st));
         ix->st.launches++;
     }
-    return search_locked(ix, B, qbuf, k, D, I, B2F_MEM_DEVICE, stream, params);
+    return search_locked(ix, B, qbuf, k, D, I, B2F_MEM_DEVICE, stream, params, nullptr);
 }
 
 int b2f_index_reconstruct(b2f_index* ix, int64_t i0, int64_t n, float* out, int32_t mem, void* stream) {

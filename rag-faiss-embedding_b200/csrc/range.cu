@@ -49,7 +49,8 @@ range_scan_kernel(const RerankArgs a, float tau, const int32_t* __restrict__ lis
         __syncthreads();
         for (int64_t r0 = r_lo; r0 < r_hi; r0 += kScanThreads / 8) {
             const int64_t row = r0 + rg;
-            const bool valid = row < r_hi;
+            // filtered search: an excluded row is neither read nor counted
+            const bool valid = row < r_hi && (!a.allow || ((__ldg(a.allow + (row >> 5)) >> (row & 31)) & 1u));
 #pragma unroll 1
             for (int i = 0; i < nqg; i++) {
                 const int32_t qi = list ? list[s0 + i] : s0 + i;

@@ -230,7 +230,9 @@ scan_kernel(const RowT* __restrict__ rows, int64_t pitch, int64_t n, int d, int 
         const float key = L2 ? acc[0] : -acc[0];
         const int v = lane & (V - 1);
         const int64_t row = row0 + v / NQ;
-        const bool pass = lane < V && row < n && (v % NQ) < nq_valid && cand_less(key, (int32_t)row, thr_k, thr_i);
+        // filtered search: a row is looked up in the allow bitmap only when it would otherwise enter a list
+        const bool pass = lane < V && row < n && (v % NQ) < nq_valid && cand_less(key, (int32_t)row, thr_k, thr_i) &&
+                          (!f.allow || ((__ldg(f.allow + (row >> 5)) >> (row & 31)) & 1u));
         unsigned m = __ballot_sync(kFull, pass);
         if (m) {
             while (m) {
@@ -426,6 +428,7 @@ static int launch_one(const RowT* rows, int64_t pitch, const ScanArgs& a, cudaSt
     f.tub = a.tub;
     f.parity = a.parity;
     f.mu = a.mu;
+    f.allow = a.allow;
     const RowT* rows_ = rows;
     int64_t pitch_ = pitch, n_ = a.n;
     int d_ = a.d, dq_ = dq, k_ = a.k;

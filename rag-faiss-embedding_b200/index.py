@@ -70,18 +70,130 @@ class IDSelectorRange:
         self.imax = int(imax)
 
 
+def _device_or_host_array(x, dtype, what: str):
+    """A 1-D selector array: a CUDA tensor stays on its device (contiguous, as dtype); anything else becomes numpy."""
+    if _is_torch(x) and x.is_cuda:
+        import torch
+
+        _assert(x.dim() == 1, f"{what}: expected a 1-D array, got shape {tuple(x.shape)}")
+        return x.to({np.int64: torch.int64, np.uint8: torch.uint8}[dtype]).contiguous()
+    if _is_torch(x):
+        x = x.detach().cpu().numpy()
+    x = np.asarray(x)
+    _assert(x.ndim == 1, f"{what}: expected a 1-D array, got shape {x.shape}")
+    return np.ascontiguousarray(x, dtype=dtype)
+
+
 class IDSelectorBatch:
-    """faiss.IDSelectorBatch(ids) or IDSelectorBatch(n, ids): the first n of ids (any order; duplicates allowed)."""
+    """faiss.IDSelectorBatch(ids) or IDSelectorBatch(n, ids): the first n of ids (any order; duplicates allowed).  ids
+    may be a CUDA tensor: a search with CUDA queries then reads it where it is."""
 
     def __init__(self, *args):
         if len(args) == 1:
-            self.ids = _id_array(args[0])
+            self.ids = _device_or_host_array(args[0], np.int64, "IDSelectorBatch")
         elif len(args) == 2:
-            n, ids = int(args[0]), _id_array(args[1])
+            n, ids = int(args[0]), _device_or_host_array(args[1], np.int64, "IDSelectorBatch")
             _assert(0 <= n <= ids.shape[0], f"IDSelectorBatch: n={n} but {ids.shape[0]} ids given")
             self.ids = ids[:n]
         else:
             raise TypeError("IDSelectorBatch(ids) or IDSelectorBatch(n, ids)")
+
+
+class IDSelectorBitmap:
+    """faiss.IDSelectorBitmap(bitmap) or IDSelectorBitmap(n, bitmap): label i is a member when bit i & 7 of byte i >> 3
+    is set.  As in faiss, n counts BYTES (the first n of bitmap); labels past the bitmap are not members.  bitmap: uint8
+    array (numpy, or a CUDA tensor that a search with CUDA queries reads where it is)."""
+
+    def __init__(self, *args):
+        if len(args) == 1:
+            self.bitmap = _device_or_host_array(args[0], np.uint8, "IDSelectorBitmap")
+        elif len(args) == 2:
+            n, bm = int(args[0]), _device_or_host_array(args[1], np.uint8, "IDSelectorBitmap")
+            _assert(0 <= n <= bm.shape[0], f"IDSelectorBitmap: n={n} bytes but {bm.shape[0]} given")
+            self.bitmap = bm[:n]
+        else:
+            raise TypeError("IDSelectorBitmap(bitmap) or IDSelectorBitmap(n, bitmap)")
+
+
+class IDSelectorNot:
+    """faiss.IDSelectorNot(sel): every id sel does not contain.  sel: an IDSelectorRange, IDSelectorBatch,
+    IDSelectorBitmap or IDSelectorNot (a chain of Nots folds to one negation)."""
+
+    def __init__(self, sel):
+        _selector_base(sel)   # TypeError for what the engine cannot evaluate
+        self.sel = sel
+
+
+def _unsupported(name):
+    def __init__(self, *args, **kwargs):
+        raise TypeError(f"{name} is not supported by this engine: filtered search takes IDSelectorRange, IDSelectorBatch, "
+                        f"IDSelectorBitmap, or IDSelectorNot over one of them")
+    return type(name, (), {"__init__": __init__, "__doc__": f"faiss.{name}: not supported (raises TypeError)."})
+
+
+IDSelectorAnd = _unsupported("IDSelectorAnd")
+IDSelectorOr = _unsupported("IDSelectorOr")
+IDSelectorXor = _unsupported("IDSelectorXor")
+IDSelectorArray = _unsupported("IDSelectorArray")
+
+
+def _selector_base(sel):
+    """(base selector, negate): sel with its chain of IDSelectorNot folded into one flag."""
+    negate = False
+    while isinstance(sel, IDSelectorNot):
+        sel, negate = sel.sel, not negate
+    if not isinstance(sel, (IDSelectorRange, IDSelectorBatch, IDSelectorBitmap)):
+        raise TypeError(f"unsupported selector {type(sel).__name__}: filtered search takes IDSelectorRange, IDSelectorBatch, "
+                        f"IDSelectorBitmap, or IDSelectorNot over one of them")
+    return sel, negate
+
+
+def selector_contains(sel, labels) -> np.ndarray:
+    """Host-side membership of each of the int64 labels in sel (faiss's sel.is_member): a bool array."""
+    base, negate = _selector_base(sel)
+    labels = np.asarray(labels, np.int64)
+    if isinstance(base, IDSelectorRange):
+        m = (labels >= base.imin) & (labels < base.imax)
+    elif isinstance(base, IDSelectorBatch):
+        m = np.isin(labels, _id_array(base.ids))
+    else:
+        bm = base.bitmap.cpu().numpy() if _is_torch(base.bitmap) else base.bitmap
+        byte = labels >> 3
+        ok = (labels >= 0) & (byte < bm.shape[0])
+        m = np.zeros(labels.shape, bool)
+        m[ok] = (bm[byte[ok]] >> (labels[ok] & 7)) & 1 == 1
+    return m != negate
+
+
+class SearchParameters:
+    """faiss.SearchParameters(sel=...): restricts search / range_search to the ids the selector contains.  Tuning comes
+    from IndexFlat.set_search_params."""
+
+    def __init__(self, sel=None):
+        self.sel = sel
+
+
+def _c_selector(sel, device=None):
+    """(C.Selector, keep-alive) for sel: with device (a torch.device) the ids / bytes are on that GPU (moved there on the
+    current torch stream when they are not), else in host memory."""
+    base, negate = _selector_base(sel)
+    c = C.Selector()
+    c.negate = 1 if negate else 0
+    if isinstance(base, IDSelectorRange):
+        c.kind, c.imin, c.imax = C.SEL_RANGE, base.imin, base.imax
+        return c, None
+    c.kind, arr = (C.SEL_BATCH, base.ids) if isinstance(base, IDSelectorBatch) else (C.SEL_BITMAP, base.bitmap)
+    if device is not None:
+        import torch
+
+        arr = torch.as_tensor(arr).to(device, non_blocking=False).contiguous()
+        ptr = arr.data_ptr()
+    else:
+        arr = arr.cpu().numpy() if _is_torch(arr) else arr
+        ptr = arr.ctypes.data
+    c.n = int(arr.shape[0])
+    c.data = ptr if c.n > 0 else None
+    return c, arr
 
 
 class IndexFlat:
@@ -151,6 +263,22 @@ class IndexFlat:
         if profile is not None:
             p.profile = 1 if profile else 0
         return self
+
+    def _split_params(self, params):
+        """params (a C.SearchParams, a SearchParameters, or None) -> (C.SearchParams, selector or None).  With a
+        SearchParameters the tuning comes from set_search_params."""
+        if isinstance(params, SearchParameters):
+            return self._params, params.sel
+        return (params if params is not None else self._params), None
+
+    def _search_call(self, n, qptr, k, Dptr, Iptr, mem, stream, p, sel, device=None):
+        if sel is None:
+            C.check(self._lib.b2f_index_search(self._h, n, qptr, k, Dptr, Iptr, mem, stream, ctypes.byref(p)))
+            return
+        c, keep = _c_selector(sel, device)
+        C.check(self._lib.b2f_index_search_filtered(self._h, n, qptr, k, Dptr, Iptr, mem, stream, ctypes.byref(p),
+                                                    ctypes.byref(c)))
+        del keep
 
     def _check_tensor(self, t, what: str):
         # a CUDA pointer of another GPU would be dereferenced on the index's device (illegal address, sticky error)
@@ -230,11 +358,12 @@ class IndexFlat:
                                                   D.data_ptr(), I.data_ptr(), _torch_stream(hidden), ctypes.byref(self._params)))
         return D, I
 
-    def search(self, x, k: int, *, params: Optional[C.SearchParams] = None):
+    def search(self, x, k: int, *, params=None):
         """index.search(x, k) -> (D float32 [n,k], I int64 [n,k]): faiss_store.py:64,
-        rag_datastore_manager.py:218."""
+        rag_datastore_manager.py:218.  params: a C.SearchParams (tuning), or faiss's SearchParameters(sel=...) to search
+        only the ids the selector contains (tuning from set_search_params)."""
         _assert(k > 0, "k must be > 0")
-        p = params if params is not None else self._params
+        p, sel = self._split_params(params)
         if _is_torch(x) and x.is_cuda:
             import torch
 
@@ -243,8 +372,8 @@ class IndexFlat:
             x = x.to(torch.float32).contiguous()
             D = torch.empty((x.shape[0], k), dtype=torch.float32, device=x.device)
             I = torch.empty((x.shape[0], k), dtype=torch.int64, device=x.device)
-            C.check(self._lib.b2f_index_search(self._h, x.shape[0], x.data_ptr(), k, D.data_ptr(), I.data_ptr(),
-                                               C.MEM_DEVICE, _torch_stream(x), ctypes.byref(p)))
+            self._search_call(x.shape[0], x.data_ptr(), k, D.data_ptr(), I.data_ptr(), C.MEM_DEVICE, _torch_stream(x), p, sel,
+                              x.device)
             return D, I
         if _is_torch(x):
             x = x.detach().cpu().numpy()
@@ -252,13 +381,12 @@ class IndexFlat:
         n = x.shape[0]
         D = np.empty((n, k), dtype=np.float32)
         I = np.empty((n, k), dtype=np.int64)
-        C.check(self._lib.b2f_index_search(self._h, n, x.ctypes.data, k, D.ctypes.data, I.ctypes.data,
-                                           C.MEM_HOST, None, ctypes.byref(p)))
+        self._search_call(n, x.ctypes.data, k, D.ctypes.data, I.ctypes.data, C.MEM_HOST, None, p, sel)
         return D, I
 
-    def search_tensors_into(self, x, k: int, D, I, *, params: Optional[C.SearchParams] = None):
+    def search_tensors_into(self, x, k: int, D, I, *, params=None):
         """Device-buffer search into caller-owned CUDA tensors D [n,k] float32 / I [n,k] int64 (contiguous); lets a
-        caller place both results inside one message buffer.  Enqueued on the current torch stream."""
+        caller place both results inside one message buffer.  Enqueued on the current torch stream.  params as search."""
         import torch
 
         _assert(k > 0, "k must be > 0")
@@ -269,16 +397,16 @@ class IndexFlat:
         for t, what in ((x, "x"), (D, "D"), (I, "I")):
             self._check_tensor(t, what)
         x = x.to(torch.float32).contiguous()
-        p = params if params is not None else self._params
-        C.check(self._lib.b2f_index_search(self._h, x.shape[0], x.data_ptr(), k, D.data_ptr(), I.data_ptr(),
-                                           C.MEM_DEVICE, _torch_stream(x), ctypes.byref(p)))
+        p, sel = self._split_params(params)
+        self._search_call(x.shape[0], x.data_ptr(), k, D.data_ptr(), I.data_ptr(), C.MEM_DEVICE, _torch_stream(x), p, sel, x.device)
 
-    def range_search(self, x, radius: float, *, params: Optional[C.SearchParams] = None):
+    def range_search(self, x, radius: float, *, params=None):
         """index.range_search(x, radius) -> (lims, D, I), faiss's RangeSearchResult: query i owns
         D[lims[i]:lims[i+1]] / I[lims[i]:lims[i+1]], ids ascending.  L2: squared distance < radius; IP: ip > radius.
         numpy in: lims uint64, D float32, I int64 numpy arrays.  CUDA tensor in: int64 / float32 / int64 CUDA tensors
-        on the current torch stream.  The five numbers of b2f_range_result_info go to self.last_range_info."""
-        p = params if params is not None else self._params
+        on the current torch stream.  The five numbers of b2f_range_result_info go to self.last_range_info.  params as
+        search: SearchParameters(sel=...) keeps exactly the hits whose label the selector contains."""
+        p, sel = self._split_params(params)
         dev = _is_torch(x) and x.is_cuda
         if dev:
             import torch
@@ -296,8 +424,14 @@ class IndexFlat:
             qptr, mem = x.ctypes.data, C.MEM_HOST
         n = x.shape[0]
         h = ctypes.c_void_p()
-        C.check(self._lib.b2f_index_range_search(self._h, n, qptr, ctypes.c_float(radius), mem, stream, ctypes.byref(p),
-                                                 ctypes.byref(h)))
+        if sel is None:
+            C.check(self._lib.b2f_index_range_search(self._h, n, qptr, ctypes.c_float(radius), mem, stream, ctypes.byref(p),
+                                                     ctypes.byref(h)))
+        else:
+            c, keep = _c_selector(sel, x.device if dev else None)
+            C.check(self._lib.b2f_index_range_search_filtered(self._h, n, qptr, ctypes.c_float(radius), mem, stream,
+                                                              ctypes.byref(p), ctypes.byref(c), ctypes.byref(h)))
+            del keep
         try:
             lims = np.empty(n + 1, dtype=np.int64)
             C.check(self._lib.b2f_range_result_lims(h, lims.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))))
@@ -335,7 +469,7 @@ class IndexFlat:
         if isinstance(x, IDSelectorRange):
             C.check(self._lib.b2f_index_remove_range(self._h, x.imin, x.imax, ctypes.byref(n)))
         else:
-            ids = x.ids if isinstance(x, IDSelectorBatch) else _id_array(x)
+            ids = _id_array(x.ids if isinstance(x, IDSelectorBatch) else x)
             C.check(self._lib.b2f_index_remove_ids(self._h, ids.shape[0], ids.ctypes.data, ctypes.byref(n)))
         return int(n.value)
 

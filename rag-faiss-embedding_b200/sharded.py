@@ -21,7 +21,8 @@ from typing import Callable, List, Optional, Tuple
 import numpy as np
 
 from . import _capi as C
-from .index import METRIC_L2, IDSelectorBatch, IDSelectorRange, IndexFlat, _assert, _id_array, _is_torch
+from .index import (METRIC_L2, IDSelectorBatch, IDSelectorBitmap, IDSelectorRange, IndexFlat, SearchParameters, _assert,
+                    _id_array, _is_torch, selector_contains)
 
 
 def partition_rows(n: int, world: int) -> List[Tuple[int, int]]:
@@ -250,6 +251,17 @@ class ShardedIndexFlat:
         self.local.set_search_params(id_offset=off if off is not None else 0)
         return off
 
+    def _local_params(self, params, off: Optional[int]):
+        """The local search's params for a SearchParameters holding global labels: a single-offset shard passes the
+        selector through (the C side adds the label offset before it tests membership); a multi-segment shard evaluates
+        membership of its rows' labels on the host and passes an IDSelectorBitmap over its local rows.  None: unfiltered."""
+        if not isinstance(params, SearchParameters) or params.sel is None:
+            return None
+        if off is not None:
+            return params
+        labels = self.segments.to_global_numpy(np.arange(self.local.ntotal, dtype=np.int64))
+        return SearchParameters(sel=IDSelectorBitmap(np.packbits(selector_contains(params.sel, labels), bitorder="little")))
+
     def _peer_exchange(self, need_bytes: int):
         """The NVLink peer-memory exchange (csrc/exchange.cu), created on first use and re-created when a search needs
         bigger slots.  Collective: every rank takes the same decisions (same need_bytes on every rank).  Returns None
@@ -314,10 +326,10 @@ class ShardedIndexFlat:
         torch.cuda.current_stream(dev).synchronize()
         return D_out, I_out
 
-    def search(self, x, k: int, out=None):
+    def search(self, x, k: int, out=None, *, params=None):
         """Replicated queries -> identical merged (D, I) on every rank (numpy in: numpy arrays; CUDA tensor in: CUDA
         tensors).  out: optional caller-owned CUDA result tensors (CUDA queries only), so that a serving loop allocates
-        nothing per search.
+        nothing per search.  params: SearchParameters(sel=...) over global labels searches only the labels sel contains.
 
         Every rank searches its shard into one packed message [D | pad | I] (12 * nq * k bytes).  With CUDA queries on
         an IndexFlat shard one kernel pushes it to the peers over NVLink peer memory and merges the world parts; without
@@ -326,8 +338,10 @@ class ShardedIndexFlat:
         import torch
 
         off = self._local_offset()
+        lp = self._local_params(params, off)
+        kw = {} if lp is None else {"params": lp}
         if self.world == 1:
-            D, I = self.local.search(x, k)
+            D, I = self.local.search(x, k, **kw)
             if off is None:
                 I = self.segments.to_global_numpy(I) if isinstance(I, np.ndarray) else self.segments.to_global_torch(I)
             return D, I
@@ -357,7 +371,7 @@ class ShardedIndexFlat:
                 raise AssertionError("queries are on another GPU than this rank's shard")
             stream = ctypes.c_void_p(int(torch.cuda.current_stream(x.device).cuda_stream) or 1)  # 0x1 = cudaStreamLegacy
             ex = self._peer_exchange(part)
-            if ex is not None and off is not None:
+            if ex is not None and off is not None and lp is None:
                 # the whole sharded step behind one C call: local search into the exchange's message buffer, then
                 # push over NVLink peer memory + flag + merge in one kernel -- no allocation, no second library call
                 x = x.to(torch.float32).contiguous()
@@ -368,9 +382,9 @@ class ShardedIndexFlat:
         D = send[: nq * k * 4].view(torch.float32).view(nq, k)
         I = send[off_i: off_i + nq * k * 8].view(torch.int64).view(nq, k)
         if dev_in and flat and off is not None:
-            self.local.search_tensors_into(x, k, D, I)
+            self.local.search_tensors_into(x, k, D, I, **kw)
         else:
-            Dl, Il = self.local.search(x, k)
+            Dl, Il = self.local.search(x, k, **kw)
             Il = torch.as_tensor(Il)
             D.copy_(torch.as_tensor(Dl))
             I.copy_(Il if off is not None else self.segments.to_global_torch(Il))
@@ -416,7 +430,8 @@ class ShardedIndexFlat:
         Each rank range-searches its shard; one all-gather of every rank's lims settles all sizes; the hits then move
         in all-gathers of at most RANGE_PART_BYTES per rank, each followed by the CUDA merge (b2f_merge_range_strided)
         into its slice of the result.  last_range_info: the local search's five numbers, `chunks` (hit all-gathers) and
-        `gathered_bytes` (bytes this rank sent: its lims and its packed hits)."""
+        `gathered_bytes` (bytes this rank sent: its lims and its packed hits).  params: a C.SearchParams (tuning), or
+        SearchParameters(sel=...) over global labels to keep only the hits whose label sel contains."""
         import torch
 
         # checked on every rank before the first collective, so that a bad call leaves no rank waiting for another
@@ -429,7 +444,10 @@ class ShardedIndexFlat:
         nq = int(shape[0])
 
         off = self._local_offset()
-        if params is not None:
+        lp = self._local_params(params, off)
+        if lp is not None:
+            lims, D, I = self.local.range_search(x, radius, params=lp)
+        elif params is not None and not isinstance(params, SearchParameters):
             params = C.SearchParams.from_buffer_copy(params)
             params.id_offset = off if off is not None else 0
             lims, D, I = self.local.range_search(x, radius, params=params)
@@ -487,7 +505,7 @@ class ShardedIndexFlat:
         if isinstance(x, IDSelectorRange):
             labels = np.arange(max(x.imin, 0), min(x.imax, self.ntotal), dtype=np.int64)
         else:
-            labels = x.ids if isinstance(x, IDSelectorBatch) else _id_array(x)
+            labels = _id_array(x.ids if isinstance(x, IDSelectorBatch) else x)
             labels = np.unique(labels[(labels >= 0) & (labels < self.ntotal)])
         local = self.segments.remove(labels)
         if len(local):

@@ -17,11 +17,18 @@ if "rag_faiss_embedding_b200" not in _sys.modules and _ilu.find_spec("rag_faiss_
 from rag_faiss_embedding_b200 import (  # noqa: E402,F401
     METRIC_INNER_PRODUCT,
     METRIC_L2,
+    IDSelectorAnd,
+    IDSelectorArray,
     IDSelectorBatch,
+    IDSelectorBitmap,
+    IDSelectorNot,
+    IDSelectorOr,
     IDSelectorRange,
+    IDSelectorXor,
     IndexFlat,
     IndexFlatIP,
     IndexFlatL2,
+    SearchParameters,
     read_index,
     write_index,
 )

@@ -16,7 +16,7 @@ from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 
-from .index import IndexFlatIP, IndexFlatL2, read_index, write_index
+from .index import IDSelectorBatch, IndexFlatIP, IndexFlatL2, SearchParameters, read_index, write_index
 
 log = logging.getLogger("b200flat.store")
 
@@ -56,11 +56,20 @@ class FAISSVectorStore:
         self.index.add(arr)
         log.info("added %d vectors", len(ids))
 
-    # faiss_store.py:49-81 -- nq is forced to 1, padding rows are dropped, every failure is swallowed
-    def search(self, query_vector, k: int = 5) -> Tuple[np.ndarray, List[int]]:
+    def _doc_params(self, doc_ids) -> dict:
+        """search() keywords restricting a search to the rows of the documents doc_ids (None: every row)."""
+        if doc_ids is None:
+            return {}
+        want = set(doc_ids)
+        rows = np.asarray([i for i, d in enumerate(self.doc_ids) if d in want], dtype=np.int64)
+        return {"params": SearchParameters(sel=IDSelectorBatch(rows))}
+
+    # faiss_store.py:49-81 -- nq is forced to 1, padding rows are dropped, every failure is swallowed.
+    # doc_ids (keyword only, no reference counterpart): search only the rows of those documents.
+    def search(self, query_vector, k: int = 5, *, doc_ids: Optional[Sequence[int]] = None) -> Tuple[np.ndarray, List[int]]:
         try:
             q = np.asarray(query_vector, dtype=np.float32).reshape(1, -1)
-            dist, rows = self.index.search(q, k)
+            dist, rows = self.index.search(q, k, **self._doc_params(doc_ids))
             kept_d, kept_ids = [], []
             for pos, row in enumerate(rows[0]):
                 if row != -1 and row < len(self.doc_ids):
@@ -71,12 +80,14 @@ class FAISSVectorStore:
             log.error("search failed: %s", exc)
             return np.array([]), []
 
-    def search_many(self, query_vectors, k: int = 5) -> Tuple[np.ndarray, List[List[int]]]:
-        """Batched variant (SURVEY 8f rank 3): [nq, d] queries -> (D [nq, k], doc ids per query)."""
+    def search_many(self, query_vectors, k: int = 5, *, doc_ids: Optional[Sequence[int]] = None
+                    ) -> Tuple[np.ndarray, List[List[int]]]:
+        """Batched variant (SURVEY 8f rank 3): [nq, d] queries -> (D [nq, k], doc ids per query).  doc_ids: search
+        only the rows of those documents."""
         q = np.asarray(query_vectors, dtype=np.float32)
         if q.ndim == 1:
             q = q[None, :]
-        dist, rows = self.index.search(q, k)
+        dist, rows = self.index.search(q, k, **self._doc_params(doc_ids))
         mapped = [[self.doc_ids[r] for r in row if r != -1 and r < len(self.doc_ids)] for row in rows]
         return dist, mapped
 
