@@ -223,6 +223,18 @@ void set_error(const char* fmt, ...);
 
 // ---- kernel launchers (one per .cu file) -------------------------------------------------------
 
+// The index's rows as every kernel that reads them sees them.  fp32 storage: f32 holds the authoritative rows and centre
+// is null (the bf16 copy is not authoritative there).  bf16 storage: f32 is null and the authoritative row is
+// fl32(centre + x~') of the stored row x~' (bf16, a row every pitch elements); centre is null for an uncentred index.
+struct StoredRows {
+    const float* f32;
+    const __nv_bfloat16* bf16;
+    int64_t pitch;
+    const float* centre;
+    int64_t n;
+    int d, metric;
+};
+
 // K1: fp32 exact-difference streaming scan + fused merge + faiss formatting, ONE cooperative launch for any
 // number of queries (walked in groups of <= 8 inside the kernel).
 struct ScanFuse {                  // device-side view (kernel argument)
@@ -247,12 +259,8 @@ struct ScanFuse {                  // device-side view (kernel argument)
     const uint32_t* allow;         // optional filtered search: bit r of word r / 32 set = row r may be returned
 };
 struct ScanArgs {                  // host-side launch description
-    const float* rows_f32;         // fp32 rows, or
-    const __nv_bfloat16* rows_bf16;
-    int64_t pitch_bf16;
-    const float* mu;               // bf16 rows: the centre added back to every stored row (null: none)
-    int64_t n;
-    int d, metric, k;
+    StoredRows rows;
+    int k;
     const float* q;                // [*, d] device fp32
     const int32_t* qsel;           // optional (device)
     const int32_t* nsel_dev;       // optional (device)
@@ -278,10 +286,8 @@ int launch_scan(const ScanArgs& a, cudaStream_t st);
 // K3: merge nparts sorted lists per query into the best kout: pk/pi [nq][nparts][klist] -> ok/oi [nq][kout]
 int launch_merge_parts(const float* pk, const int32_t* pi, int nq, int nparts, int klist, int kout, float* ok,
                        int32_t* oi, cudaStream_t st);
-// final formatting: keys -> faiss distances, int32 local ids -> int64 labels (+offset), padding.
-// qsel (optional) scatters row r of the input to output row qsel[r].
-int launch_finalize(const float* keys, const int32_t* ids, int nq, int kin, int k, int metric, int64_t id_offset,
-                    const int32_t* qsel, float* D, int64_t* I, cudaStream_t st);
+// the result of a search with no rows: every one of the nq x k slots is faiss's padding (+-FLT_MAX, -1)
+int launch_fill_empty(int nq, int k, int metric, float* D, int64_t* I, cudaStream_t st);
 // multi-GPU merge of nparts faiss-formatted [nq][k] lists; part p's distances / labels sit p * stride bytes after
 // part 0's (one packed message per rank)
 int launch_merge_faiss(int metric, int64_t nq, int64_t k, int nparts, const float* Dp, const int64_t* Ip, int64_t stride,
@@ -304,9 +310,9 @@ int launch_mean_begin(int d, unsigned long long* acc, cudaStream_t st);
 int launch_mean_pass(const float* src, int64_t row0, int64_t rows, int64_t m, int d, unsigned long long* acc, int pass,
                      cudaStream_t st);
 int launch_mean_finish(int64_t m, int d, float* mu, unsigned long long* acc, cudaStream_t st);
-// K7: pooling (+normalise) of encoder output, optionally fused with the ingest writes.
+// K7: pooling (+normalise) of encoder output into out_f32 [B, d].
 int launch_pool(const float* hidden, const int64_t* mask, int64_t B, int64_t T, int d, int pool, int normalize,
-                float* out_f32, __nv_bfloat16* scan, int64_t dpad, float* norms, float* stats, cudaStream_t st);
+                float* out_f32, cudaStream_t st);
 int launch_synth(uint64_t seed, int64_t row0, int64_t nrows, int d, int normalize, float* out, cudaStream_t st);
 // query preparation for the tensor path: bf16 copy (pitch dpad, rows padded to nq_pad with zeros),
 // |q|^2 in fp32 and the norm of the bf16 rounding error of each query.
@@ -327,10 +333,7 @@ int launch_bf16_to_f32(const __nv_bfloat16* src, int64_t pitch, int64_t n, int d
 
 // K4: exact fp32 re-rank of coarse candidates + certification.
 struct RerankArgs {
-    const float* rows_f32;          // authoritative fp32 rows (or null)
-    const __nv_bfloat16* rows_bf16; // bf16 storage: the stored rows x~'; the authoritative row is fl32(centre + x~')
-    int64_t pitch_bf16;
-    const float* centre;            // bf16 storage: the index's centre mu [d] (null: mu = 0)
+    StoredRows rows;
     const float* q;                 // [nq, d] fp32
     const float* qnorm;             // |q|^2
     const float* qerr;              // |q' - bf16(q')|   (q' = q - mu)
@@ -338,15 +341,12 @@ struct RerankArgs {
     float mu_norm;                  // |mu|
     const float* cand_key;          // [nq, kp] coarse keys (sorted ascending)
     const int32_t* cand_id;         // [nq, kp]
-    int nq, kp, k, d, metric;
-    int64_t ntotal;
+    int nq, kp, k;
     float max_row_norm;             // max |x~| over the index (bf16 copy)
     float max_row_err;              // max |x - bf16(x)| over the index (0 for bf16 storage)
     int certify;
-    float* out_key;                 // [nq, k] exact keys   (used when D == nullptr)
-    int32_t* out_id;                // [nq, k]
-    float* D;                       // optional fused finalize: faiss-formatted distances [nq, k]
-    int64_t* I;                     //                          labels [nq, k] (+ id_offset)
+    float* D;                       // faiss-formatted distances [nq, k]
+    int64_t* I;                     // labels [nq, k] (+ id_offset)
     int64_t id_offset;
     int32_t* fail_list;             // queries that could not be certified (q + q_base), re-run by the closing exact scan
     int32_t* fail_count;            // [0] uncertified queries, [1] of which list overflows, [2..3] u64 list entries

@@ -1419,14 +1419,14 @@ constexpr int WM_LISTS = 64;     // lists per query
 // conventions, returns whether the result is certified (warp-uniform).  ek / ei: nc floats / ints of scratch.
 __device__ __forceinline__ bool warp_rerank(const RerankArgs& a, int q, const float* sk, const int32_t* si, int nc, float bound,
                                             bool all_rows, float* ek, int32_t* ei, int lane, float& tau_out) {
-    const float* qv = a.q + (int64_t)q * a.d;
-    const bool l2 = a.metric == B2F_METRIC_L2;
+    const float* qv = a.q + (int64_t)q * a.rows.d;
+    const bool l2 = a.rows.metric == B2F_METRIC_L2;
     const int sl = lane & 7;
     for (int c0 = 0; c0 < nc; c0 += 4) {   // 8 lanes per candidate, 4 candidates per pass
         const int c = c0 + (lane >> 3);
         int32_t id = c < nc ? si[c] : -1;
-        if ((int64_t)id >= a.ntotal) id = -1;
-        const float key = exact_key_8lanes(a, qv, id, sl, l2);
+        if ((int64_t)id >= a.rows.n) id = -1;
+        const float key = exact_key_8lanes(a.rows, qv, id, sl, l2);
         if (sl == 0 && c < nc) {
             const bool ok = id >= 0 && !(key != key);
             ek[c] = ok ? key : FLT_MAX;
@@ -1709,14 +1709,14 @@ range_collect_kernel(const uint2* __restrict__ cand, const int32_t* __restrict__
         for (int j = tid; j < s_off[l + 1] - s_off[l]; j += MERGE_THREADS) comp[s_off[l] + j] = (unsigned long long)p[j].y << 32;
     }
     __syncthreads();
-    const float* qv = ra.q + (int64_t)q * ra.d;
-    const bool l2 = ra.metric == B2F_METRIC_L2;
+    const float* qv = ra.q + (int64_t)q * ra.rows.d;
+    const bool l2 = ra.rows.metric == B2F_METRIC_L2;
     const int sl = lane & 7;
     for (int c0 = 0; c0 < M; c0 += MERGE_THREADS / 8) {
         const int c = c0 + (tid >> 3);
         int32_t id = c < M ? (int32_t)(comp[c] >> 32) : -1;
-        if ((int64_t)id >= ra.ntotal) id = -1;
-        const float key = exact_key_8lanes(ra, qv, id, sl, l2);
+        if ((int64_t)id >= ra.rows.n) id = -1;
+        const float key = exact_key_8lanes(ra.rows, qv, id, sl, l2);
         if (sl == 0 && c < M) {
             const bool hit = id >= 0 && key < tau;   // NaN is never a hit
             comp[c] = hit ? (comp[c] | __float_as_uint(key)) : ~0ull;
@@ -1966,7 +1966,7 @@ int launch_merge_lists(const TensorScanLists& lists, int nq, const TensorScanPla
     }
     // big batches: one warp per query first; what it cannot hold is flagged for the block kernel behind it
     const uint8_t* only_flagged = nullptr;
-    if (nq >= k2::WM_MIN_NQ && lists.big_flag && plan.nlists <= k2::WM_LISTS && plan.kp <= k2::WM_MAX / 2 && ra.D &&
+    if (nq >= k2::WM_MIN_NQ && lists.big_flag && plan.nlists <= k2::WM_LISTS && plan.kp <= k2::WM_MAX / 2 &&
         !ra.range && !ra.out_map) {
         k2::merge_lists_warp_kernel<<<(nq + k2::WM_WARPS - 1) / k2::WM_WARPS, k2::WM_WARPS * 32, 0, st>>>(
             reinterpret_cast<const uint2*>(lists.cand), lists.counts, lists.final_thr, plan.nlists, plan.pair_mode ? 2 * k2::BM : k2::BM,

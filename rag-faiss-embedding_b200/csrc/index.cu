@@ -261,6 +261,41 @@ int ensure_pinned(b2f_index* ix, size_t bytes) {
     return B2F_OK;
 }
 
+// Lays one call's buffers out in the workspace.  carve(Bump&) takes them in one fixed order: over a null base it measures
+// them, then the workspace grows to max(measured, min_bytes) bytes and the same carve lays them out there.  *grew: a
+// workspace the call found had to be replaced (which waits for the device).
+template <class Carve>
+int carve_ws(b2f_index* ix, size_t min_bytes, Carve&& carve, const char* what, bool* grew = nullptr) {
+    Bump layout(nullptr, SIZE_MAX);
+    carve(layout);
+    const size_t need = std::max(layout.off, min_bytes);
+    if (grew) *grew = need > ix->ws_bytes && ix->ws;
+    B2F_TRY(ensure_ws(ix, need));
+    Bump bump(ix->ws, ix->ws_bytes);
+    carve(bump);
+    if (!bump.fits()) {
+        set_error("%s workspace: the layout needs %zu bytes, the workspace has %zu", what, bump.off, bump.size);
+        return B2F_ECUDA;
+    }
+    return B2F_OK;
+}
+
+// The centre of the scan copy (either storage; null before the first add): what ingest subtracts from a row and the query
+// preparation from a query before the bf16 rounding, and what bf16 storage adds back to a stored row.
+const float* scan_centre(const b2f_index* ix) { return ix->mu_set ? ix->centre : nullptr; }
+
+// The rows as the exact kernels read them.  Their centre is the one added back to a stored bf16 row: bf16 storage only.
+StoredRows stored_rows(const b2f_index* ix) {
+    const bool f32 = ix->storage == B2F_STORE_F32;
+    return StoredRows{f32 ? ix->rows_f32 : nullptr, ix->scan, ix->dpad, f32 ? nullptr : scan_centre(ix), ix->ntotal, ix->d, ix->metric};
+}
+
+// kernel launches of a search: the running total and the latest search's count
+void count_launches(b2f_index* ix, int n) {
+    ix->st.launches += n;
+    ix->st.last_launches += n;
+}
+
 // Adds are enqueued on the caller's stream (a device-tensor add / add_pooled runs behind the encoder on torch's
 // stream) and return without synchronising.  Everything that reads rows, norms, stats or the centre on ANOTHER
 // stream -- searches, write, reconstruct, the stats refresh, the growth copies -- first waits for the latest add.
@@ -274,6 +309,14 @@ int record_ingest(b2f_index* ix, cudaStream_t st) {
     B2F_CUDA(cudaEventRecord(ix->ev_ingest, st));
     ix->last_add_stream = st;
     ix->add_recorded = true;
+    return B2F_OK;
+}
+// recorded behind every search and range search on the stream it was enqueued on (they return without synchronising)
+int record_search(b2f_index* ix, cudaStream_t st) {
+    if (!ix->ev_done) B2F_CUDA(cudaEventCreateWithFlags(&ix->ev_done, cudaEventDisableTiming));
+    B2F_CUDA(cudaEventRecord(ix->ev_done, st));
+    ix->last_stream = st;
+    ix->search_recorded = true;
     return B2F_OK;
 }
 
@@ -348,7 +391,7 @@ int refresh_host_stats(b2f_index* ix, cudaStream_t st) {
     if (!ix->stats_dirty) return B2F_OK;
     B2F_CUDA(cudaMemcpyAsync(ix->host_stats, ix->stats, 2 * sizeof(float), cudaMemcpyDeviceToHost, st));
     std::vector<float> m((size_t)ix->d, 0.f);
-    if (ix->mu_set) B2F_CUDA(cudaMemcpyAsync(m.data(), ix->centre, (size_t)ix->d * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (const float* mu = scan_centre(ix)) B2F_CUDA(cudaMemcpyAsync(m.data(), mu, (size_t)ix->d * sizeof(float), cudaMemcpyDeviceToHost, st));
     B2F_CUDA(cudaStreamSynchronize(st));
     double s2 = 0.0;
     for (float v : m) s2 += (double)v * v;
@@ -378,13 +421,7 @@ int enqueue_scan(b2f_index* ix, const float* qd, const int32_t* qsel, const int3
                  int64_t* Id, int64_t id_offset, void* scratch, int32_t* counters, int32_t seq, int nq_batch, int certify,
                  const uint32_t* allow, cudaStream_t st) {
     ScanArgs a{};
-    a.rows_f32 = ix->storage == B2F_STORE_F32 ? ix->rows_f32 : nullptr;
-    a.rows_bf16 = ix->scan;
-    a.pitch_bf16 = ix->dpad;
-    a.mu = (ix->storage == B2F_STORE_BF16 && ix->mu_set) ? ix->centre : nullptr;
-    a.n = ix->ntotal;
-    a.d = ix->d;
-    a.metric = ix->metric;
+    a.rows = stored_rows(ix);
     a.k = k;
     a.q = qd;
     a.qsel = qsel;
@@ -404,8 +441,7 @@ int enqueue_scan(b2f_index* ix, const float* qd, const int32_t* qsel, const int3
     a.parity = (int32_t)(ix->scan_launches++ & 1);
     a.allow = allow;
     B2F_TRY(launch_scan(a, st));
-    ix->st.launches += 1;
-    ix->st.last_launches += 1;
+    count_launches(ix, 1);
     return B2F_OK;
 }
 
@@ -762,7 +798,7 @@ static int add_device_rows(b2f_index* ix, const float* src_dev, int64_t n, cudaS
         if (src_dev != dst) rows_out = dst;
     }
     B2F_TRY(launch_ingest(src_dev, n, ix->d, rows_out, ix->scan + ix->ntotal * ix->dpad, ix->dpad,
-                          ix->norms + ix->ntotal, ix->stats, ix->mu_set ? ix->centre : nullptr,
+                          ix->norms + ix->ntotal, ix->stats, scan_centre(ix),
                           ix->metric == B2F_METRIC_INNER_PRODUCT ? 1 : 0, ix->storage == B2F_STORE_BF16 ? 1 : 0, st));
     ix->st.launches++;
     return B2F_OK;
@@ -870,8 +906,7 @@ int b2f_index_add_pooled(b2f_index* ix, const float* hidden, const int64_t* mask
     // bias of the tensor pass (L2: |x~'|^2, IP: -mu.x -- NOT a norm) and the stats for either storage mode and metric.
     const int64_t piece = ix->storage == B2F_STORE_F32 ? B : rows_in(64u << 20, ix->d);
     return ingest_call(ix, B, piece, nullptr, st, [&](int64_t b0, int64_t m, float* dst) {
-        B2F_TRY(launch_pool(hidden + b0 * T * ix->d, mask ? mask + b0 * T : nullptr, m, T, ix->d, pool, normalize, dst, nullptr, 0,
-                            nullptr, nullptr, st));
+        B2F_TRY(launch_pool(hidden + b0 * T * ix->d, mask ? mask + b0 * T : nullptr, m, T, ix->d, pool, normalize, dst, st));
         ix->st.launches++;
         return B2F_OK;
     });
@@ -885,7 +920,7 @@ int b2f_pool_normalize(const float* hidden, const int64_t* mask, int64_t B, int6
     }
     B2F_TRY(check_device(device));
     DeviceGuard g(device);
-    return launch_pool(hidden, mask, B, T, d, pool, normalize, out, nullptr, 0, nullptr, nullptr, (cudaStream_t)stream);
+    return launch_pool(hidden, mask, B, T, d, pool, normalize, out, (cudaStream_t)stream);
 }
 
 int b2f_synth_rows(uint64_t seed, int64_t row0, int64_t nrows, int32_t d, int32_t normalize, float* out, int32_t device,
@@ -987,8 +1022,10 @@ static int build_filter(const b2f_index* ix, const b2f_selector* sel, int32_t me
     return B2F_OK;
 }
 
-// What one search carves from the workspace, in one order.  search_locked carves it over a null base for the size, then
-// over the workspace.
+// the row bias the tensor pass reads: a filtered search's masked copy, else the index's own
+static const float* tensor_bias(const b2f_index* ix, const FilterWs& f) { return f.bias ? f.bias : ix->norms; }
+
+// What one search carves from the workspace, in one order (carve_ws measures it, then lays it out).
 struct SearchWs {
     float* q = nullptr;              // host buffers: device copies of the queries and the results
     float* D = nullptr;
@@ -1041,10 +1078,7 @@ static SearchWs carve_search(Bump& b, const b2f_index* ix, int nq, int k, bool h
 static RerankArgs rerank_args(const b2f_index* ix, const float* q, const PassQueries& pq, int nq, int k, int kp, float* D,
                               int64_t* I, int64_t id_offset, int32_t* fail_list, int32_t* fail_count) {
     RerankArgs a{};
-    a.rows_f32 = ix->storage == B2F_STORE_F32 ? ix->rows_f32 : nullptr;
-    a.rows_bf16 = ix->scan;
-    a.pitch_bf16 = ix->dpad;
-    a.centre = (ix->storage == B2F_STORE_BF16 && ix->mu_set) ? ix->centre : nullptr;
+    a.rows = stored_rows(ix);
     a.q = q;
     a.qnorm = pq.qnorm;
     a.qerr = pq.qerr;
@@ -1053,9 +1087,6 @@ static RerankArgs rerank_args(const b2f_index* ix, const float* q, const PassQue
     a.nq = nq;
     a.kp = kp;
     a.k = k;
-    a.d = ix->d;
-    a.metric = ix->metric;
-    a.ntotal = ix->ntotal;
     a.max_row_norm = sqrtf(ix->host_stats[0]);
     // fp32 storage: the bf16 rounding of the centred row; bf16 storage: what fl32(mu + x~') loses (0 uncentred)
     a.max_row_err = sqrtf(ix->host_stats[1]);
@@ -1106,9 +1137,13 @@ static RangeWs carve_range(Bump& b, const b2f_index* ix, int nq, const TensorSca
     return r;
 }
 
-// Where a range pass carved behind `search` ends at most.  The list geometry depends on the number of failed queries,
-// known only after the host sync: take the largest over 128..kRangeCap of them.
-static size_t range_end(const Bump& search, const b2f_index* ix, int nq, int kp) {
+// Where a range pass carved behind the search's buffers (carve_search(Bump&) lays them out) ends at most.  The list
+// geometry depends on the number of failed queries, known only after the host sync: take the largest over 128..kRangeCap
+// of them.
+template <class Carve>
+static size_t range_end(Carve&& carve_search, const b2f_index* ix, int nq, int kp) {
+    Bump search(nullptr, SIZE_MAX);
+    carve_search(search);
     size_t end = search.off;
     for (int f = 128; f <= kRangeCap; f *= 2) {
         TensorScanPlan p{};
@@ -1145,21 +1180,19 @@ static int range_pass(b2f_index* ix, Bump& bump, const SearchWs& w, const float*
     B2F_CUDA(cudaMemsetAsync(r.q, 0, (size_t)nq_pad * ix->d * 4, st));
     B2F_TRY(launch_gather_failed(q, ix->d, w.fail_list, w.fail_tau, w.counters, nfail, nr, r.q, r.tau, r.out_map, r.counters + 16,
                                  r.fail_list, r.counters, st));
-    B2F_TRY(launch_prep_queries(r.q, nr, nq_pad, ix->d, r.pq.qb, ix->dpad, r.pq.qnorm, r.pq.qerr, r.pq.qconst,
-                                ix->mu_set ? ix->centre : nullptr, nullptr, 0, reinterpret_cast<uint32_t*>(r.lists.shared_thr),
-                                (int64_t)nq_pad * rp.nlists, st));
+    B2F_TRY(launch_prep_queries(r.q, nr, nq_pad, ix->d, r.pq.qb, ix->dpad, r.pq.qnorm, r.pq.qerr, r.pq.qconst, scan_centre(ix), nullptr,
+                                0, reinterpret_cast<uint32_t*>(r.lists.shared_thr), (int64_t)nq_pad * rp.nlists, st));
     B2F_TRY(launch_range_thresholds(r.tau, 0.f, r.out_map, nr, ix->d, ix->metric, r.pq.qnorm, r.pq.qerr, r.pq.qconst,
                                     sqrtf(ix->host_stats[0]), sqrtf(ix->host_stats[1]), ix->mu_norm, r.thr, st));
-    B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, w.filter.bias ? w.filter.bias : ix->norms, ix->ntotal, ix->metric, r.pq.qb, nr,
-                               nq_pad, rp, nullptr, nullptr, r.lists, st));
+    B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, tensor_bias(ix, w.filter), ix->ntotal, ix->metric, r.pq.qb, nr, nq_pad, rp, nullptr,
+                               nullptr, r.lists, st));
     RerankArgs ra = rerank_args(ix, r.q, r.pq, nr, k, kp, D, I, id_offset, r.fail_list, r.counters);
     ra.out_map = r.out_map;
     ra.range = 1;
     B2F_TRY(launch_merge_lists(r.lists, nr, rp, nullptr, ra, st));
     // the statistics the closing kernel publishes: what the first pass counted, with the final fallback count
     B2F_CUDA(cudaMemcpyAsync(r.counters + 1, w.counters + 1, 7 * 4, cudaMemcpyDeviceToDevice, st));
-    ix->st.launches += 5;
-    ix->st.last_launches += 5;
+    count_launches(ix, 5);
     ix->st.range_queries += nr;
     *served = nr;
     *scan_list = r.fail_list;
@@ -1221,15 +1254,13 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
     if (tensor && heap_first) ix->adapt.heap_left--;
 
     // ---- workspace -----------------------------------------------------------------------------
-    Bump layout(nullptr, SIZE_MAX);
-    carve_search(layout, ix, nq, k, host, tensor, plan, chunk_nq, kp, sel, P.id_offset);
-    B2F_TRY(ensure_ws(ix, tensor && ix->adapt.range_mode ? range_end(layout, ix, nq, kp) : layout.off));
-    Bump bump(ix->ws, ix->ws_bytes);
-    const SearchWs w = carve_search(bump, ix, nq, k, host, tensor, plan, chunk_nq, kp, sel, P.id_offset);
-    if (!bump.fits()) {
-        set_error("search workspace: the layout needs %zu bytes, the workspace has %zu", bump.off, bump.size);
-        return B2F_ECUDA;
-    }
+    SearchWs w;
+    Bump bump(nullptr, 0);   // the workspace behind w: a range pass carves its buffers there
+    const auto carve = [&](Bump& b) {
+        w = carve_search(b, ix, nq, k, host, tensor, plan, chunk_nq, kp, sel, P.id_offset);
+        bump = b;
+    };
+    B2F_TRY(carve_ws(ix, tensor && ix->adapt.range_mode ? range_end(carve, ix, nq, kp) : 0, carve, "search"));
     const float* qd = host ? w.q : q;
     float* Dd = host ? w.D : D;
     int64_t* Id = host ? w.I : I;
@@ -1240,8 +1271,7 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
     ix->st.last_kprime = 0;
     int filter_launches = 0;
     B2F_TRY(build_filter(ix, sel, mem, P.id_offset, w.filter, st, &filter_launches));
-    ix->st.launches += filter_launches;
-    ix->st.last_launches += filter_launches;
+    count_launches(ix, filter_launches);
     int n_main = 0;
     b2f_index::ProfSlot* slot = nullptr;
     if (profile) {
@@ -1264,9 +1294,8 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
     };
 
     if (ix->ntotal == 0) {
-        B2F_TRY(launch_finalize(nullptr, nullptr, nq, 0, k, ix->metric, P.id_offset, nullptr, Dd, Id, st));
-        ix->st.launches++;
-        ix->st.last_launches++;
+        B2F_TRY(launch_fill_empty(nq, k, ix->metric, Dd, Id, st));
+        count_launches(ix, 1);
     } else if (!tensor) {
         B2F_TRY(main_event(0));
         B2F_TRY(enqueue_scan(ix, qd, nullptr, nullptr, nq, k, Dd, Id, P.id_offset, w.scan_scratch, nullptr, 0, nq, 0, w.filter.allow,
@@ -1281,13 +1310,13 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
             const int cn = nq - c0 < chunk_nq ? nq - c0 : chunk_nq;  // queries in this pass (the plan covers chunk_nq)
             const float* qc = qd + (int64_t)c0 * ix->d;
             // one launch: bf16 copy / norms of the queries, reset the shared thresholds, clear the counters (first pass)
-            B2F_TRY(launch_prep_queries(qc, cn, nq_pad, ix->d, w.pq.qb, ix->dpad, w.pq.qnorm, w.pq.qerr, w.pq.qconst,
-                                        ix->mu_set ? ix->centre : nullptr, reinterpret_cast<uint32_t*>(w.counters),
-                                        c0 == 0 ? 16 : 0, reinterpret_cast<uint32_t*>(w.lists.shared_thr),
+            B2F_TRY(launch_prep_queries(qc, cn, nq_pad, ix->d, w.pq.qb, ix->dpad, w.pq.qnorm, w.pq.qerr, w.pq.qconst, scan_centre(ix),
+                                        reinterpret_cast<uint32_t*>(w.counters), c0 == 0 ? 16 : 0,
+                                        reinterpret_cast<uint32_t*>(w.lists.shared_thr),
                                         plan.list_mode ? (int64_t)nq_pad * plan.nlists : 0, st));
             B2F_TRY(main_event(0));
-            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, w.filter.bias ? w.filter.bias : ix->norms, ix->ntotal, ix->metric, w.pq.qb,
-                                       cn, nq_pad, plan, w.pk, w.pi, w.lists, st));
+            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, tensor_bias(ix, w.filter), ix->ntotal, ix->metric, w.pq.qb, cn, nq_pad, plan,
+                                       w.pk, w.pi, w.lists, st));
             B2F_TRY(main_event(1));
             n_main++;
             // the re-rank writes faiss-formatted results directly (no finalize launch)
@@ -1301,13 +1330,11 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
             if (plan.list_mode) {
                 // K3b + K4 + finalize fused: per query, merge the lists, re-rank exactly, certify, write (D, I)
                 B2F_TRY(launch_merge_lists(w.lists, cn, plan, reinterpret_cast<unsigned long long*>(w.counters + 2), ra, st));
-                ix->st.launches += 3;
-                ix->st.last_launches += 3;
+                count_launches(ix, 3);
             } else {
                 B2F_TRY(launch_merge_parts(w.pk, w.pi, cn, plan.nsplits, kp, kp, w.ck, w.ci, st));
                 B2F_TRY(launch_rerank(ra, st));
-                ix->st.launches += 4;
-                ix->st.last_launches += 4;
+                count_launches(ix, 4);
             }
         }  // query chunks
         int32_t* scan_list = w.fail_list;
@@ -1334,10 +1361,7 @@ static int search_locked(b2f_index* ix, int64_t nq64, const float* q, int64_t k6
         B2F_CUDA(cudaMemcpyAsync(D, Dd, (size_t)nq * k * 4, cudaMemcpyDeviceToHost, st));
         B2F_CUDA(cudaMemcpyAsync(I, Id, (size_t)nq * k * 8, cudaMemcpyDeviceToHost, st));
     }
-    if (!ix->ev_done) B2F_CUDA(cudaEventCreateWithFlags(&ix->ev_done, cudaEventDisableTiming));
-    B2F_CUDA(cudaEventRecord(ix->ev_done, st));
-    ix->last_stream = st;
-    ix->search_recorded = true;
+    B2F_TRY(record_search(ix, st));
     if (host) {
         B2F_CUDA(cudaStreamSynchronize(st));  // faiss semantics: results are in the caller's arrays on return
         harvest_flag(ix);
@@ -1467,13 +1491,7 @@ static int range_search_locked(b2f_index* ix, int nq, const float* q, float radi
     const bool bound_ok = isfinite(max_row_norm) && isfinite(max_row_err) && isfinite(ix->mu_norm);
     const bool want_tensor = bound_ok && P.algo != B2F_ALGO_SCAN && !(P.algo == B2F_ALGO_AUTO && nq <= P.scan_max_nq);
     RerankArgs a{};
-    a.rows_f32 = ix->storage == B2F_STORE_F32 ? ix->rows_f32 : nullptr;
-    a.rows_bf16 = ix->scan;
-    a.pitch_bf16 = ix->dpad;
-    a.centre = (ix->storage == B2F_STORE_BF16 && ix->mu_set) ? ix->centre : nullptr;
-    a.d = ix->d;
-    a.metric = ix->metric;
-    a.ntotal = ix->ntotal;
+    a.rows = stored_rows(ix);
     const RangeScanGeometry geo = range_scan_geometry(ix->ntotal);
     B2F_TRY(ensure_pinned(ix, ((size_t)kRangeCap + 2) * sizeof(int64_t)));
     int64_t* lims_h = reinterpret_cast<int64_t*>(ix->pinned);
@@ -1490,16 +1508,11 @@ static int range_search_locked(b2f_index* ix, int nq, const float* q, float radi
                 break;
             }
         }
-        Bump layout(nullptr, SIZE_MAX);
-        carve_range_search(layout, ix, cn, host, tensor, plan, geo.ntiles, sel, P.id_offset);
-        if (layout.off > ix->ws_bytes && ix->ws) syncs++;
-        B2F_TRY(ensure_ws(ix, layout.off));
-        Bump bump(ix->ws, ix->ws_bytes);
-        const RangeSearchWs w = carve_range_search(bump, ix, cn, host, tensor, plan, geo.ntiles, sel, P.id_offset);
-        if (!bump.fits()) {
-            set_error("range search workspace: the layout needs %zu bytes, the workspace has %zu", bump.off, bump.size);
-            return B2F_ECUDA;
-        }
+        RangeSearchWs w;
+        bool grew = false;
+        B2F_TRY(carve_ws(ix, 0, [&](Bump& b) { w = carve_range_search(b, ix, cn, host, tensor, plan, geo.ntiles, sel, P.id_offset); },
+                         "range search", &grew));
+        syncs += grew;
         const float* qc = host ? w.q : q + (int64_t)c0 * ix->d;
         if (host) B2F_CUDA(cudaMemcpyAsync(w.q, q + (int64_t)c0 * ix->d, (size_t)cn * ix->d * 4, cudaMemcpyHostToDevice, st));
         a.q = qc;
@@ -1510,12 +1523,12 @@ static int range_search_locked(b2f_index* ix, int nq, const float* q, float radi
         a.allow = w.filter.allow;
         if (tensor) {
             const int nq_pad = plan.nq_tiles * 128;
-            B2F_TRY(launch_prep_queries(qc, cn, nq_pad, ix->d, w.pq.qb, ix->dpad, w.pq.qnorm, w.pq.qerr, w.pq.qconst,
-                                        ix->mu_set ? ix->centre : nullptr, reinterpret_cast<uint32_t*>(w.counters), 16, nullptr, 0, st));
+            B2F_TRY(launch_prep_queries(qc, cn, nq_pad, ix->d, w.pq.qb, ix->dpad, w.pq.qnorm, w.pq.qerr, w.pq.qconst, scan_centre(ix),
+                                        reinterpret_cast<uint32_t*>(w.counters), 16, nullptr, 0, st));
             B2F_TRY(launch_range_thresholds(nullptr, tau, nullptr, cn, ix->d, ix->metric, w.pq.qnorm, w.pq.qerr, w.pq.qconst,
                                             max_row_norm, max_row_err, ix->mu_norm, w.thr, st));
-            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, w.filter.bias ? w.filter.bias : ix->norms, ix->ntotal, ix->metric, w.pq.qb,
-                                       cn, nq_pad, plan, nullptr, nullptr, w.lists, st));
+            B2F_TRY(launch_tensor_scan(ix->scan, ix->dpad, tensor_bias(ix, w.filter), ix->ntotal, ix->metric, w.pq.qb, cn, nq_pad, plan,
+                                       nullptr, nullptr, w.lists, st));
             B2F_TRY(launch_range_collect(w.lists, cn, plan, tau, a, w.skey, w.sid, w.staged, w.count, w.scan_list, w.counters, st));
             launches += 4;
         } else {
@@ -1555,11 +1568,7 @@ static int range_search_locked(b2f_index* ix, int nq, const float* q, float radi
     ix->st.launches += launches;
     if (!r->done) B2F_CUDA(cudaEventCreateWithFlags(&r->done, cudaEventDisableTiming));
     B2F_CUDA(cudaEventRecord(r->done, st));
-    if (!ix->ev_done) B2F_CUDA(cudaEventCreateWithFlags(&ix->ev_done, cudaEventDisableTiming));
-    B2F_CUDA(cudaEventRecord(ix->ev_done, st));
-    ix->last_stream = st;
-    ix->search_recorded = true;
-    return B2F_OK;
+    return record_search(ix, st);
 }
 
 extern "C" {
@@ -1713,7 +1722,7 @@ int b2f_index_search_pooled(b2f_index* ix, const float* hidden, const int64_t* m
             ix->qpool_bytes = need + (need >> 2);
         }
         qbuf = ix->qpool;
-        B2F_TRY(launch_pool(hidden, mask, B, T, ix->d, pool, normalize, qbuf, nullptr, 0, nullptr, nullptr, st));
+        B2F_TRY(launch_pool(hidden, mask, B, T, ix->d, pool, normalize, qbuf, st));
         ix->st.launches++;
     }
     return search_locked(ix, B, qbuf, k, D, I, B2F_MEM_DEVICE, stream, params, nullptr);
@@ -1738,11 +1747,11 @@ int b2f_index_reconstruct(b2f_index* ix, int64_t i0, int64_t n, float* out, int3
     if (ix->storage == B2F_STORE_F32) {
         B2F_CUDA(cudaMemcpyAsync(out, ix->rows_f32 + i0 * ix->d, bytes, mem == B2F_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
     } else if (mem == B2F_MEM_DEVICE) {
-        B2F_TRY(launch_bf16_to_f32(ix->scan + i0 * ix->dpad, ix->dpad, n, ix->d, ix->mu_set ? ix->centre : nullptr, out, st));
+        B2F_TRY(launch_bf16_to_f32(ix->scan + i0 * ix->dpad, ix->dpad, n, ix->d, scan_centre(ix), out, st));
         ix->st.launches++;
     } else {
         B2F_TRY(ensure_ws(ix, bytes + 4096));
-        B2F_TRY(launch_bf16_to_f32(ix->scan + i0 * ix->dpad, ix->dpad, n, ix->d, ix->mu_set ? ix->centre : nullptr, reinterpret_cast<float*>(ix->ws), st));
+        B2F_TRY(launch_bf16_to_f32(ix->scan + i0 * ix->dpad, ix->dpad, n, ix->d, scan_centre(ix), reinterpret_cast<float*>(ix->ws), st));
         ix->st.launches++;
         B2F_CUDA(cudaMemcpyAsync(out, ix->ws, bytes, cudaMemcpyDeviceToHost, st));
     }
@@ -1777,17 +1786,12 @@ static int remove_runs_locked(b2f_index* ix, const std::vector<int64_t>& runs, i
             if (a.base) tiles = std::max(tiles, remove_tiles(first, ix->ntotal, a.row_bytes));
         std::vector<int64_t> words;
         remove_runs_layout(runs, words);
-        const auto carve = [&](Bump& b, int64_t** runs_dev, RemoveSpan** spans) {
-            *runs_dev = b.take<int64_t>(words.size());
-            *spans = b.take<RemoveSpan>((size_t)tiles);
-        };
         int64_t* runs_dev = nullptr;
         RemoveSpan* spans = nullptr;
-        Bump layout(nullptr, SIZE_MAX);
-        carve(layout, &runs_dev, &spans);
-        B2F_TRY(ensure_ws(ix, layout.off));
-        Bump bump(ix->ws, ix->ws_bytes);
-        carve(bump, &runs_dev, &spans);
+        B2F_TRY(carve_ws(ix, 0, [&](Bump& b) {
+            runs_dev = b.take<int64_t>(words.size());
+            spans = b.take<RemoveSpan>((size_t)tiles);
+        }, "remove"));
         B2F_CUDA(cudaMemcpyAsync(runs_dev, words.data(), words.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
         const RemoveRuns rr = remove_runs_view(runs_dev, nr);
         const int64_t need = 1 + tiles;
@@ -1813,7 +1817,7 @@ static int remove_runs_locked(b2f_index* ix, const std::vector<int64_t>& runs, i
         }
     }
     B2F_CUDA(cudaMemsetAsync(ix->stats, 0, 2 * sizeof(float), st));
-    const float* mu = ix->mu_set ? ix->centre : nullptr;
+    const float* mu = scan_centre(ix);
     if (n_new > 0) {
         if (ix->storage == B2F_STORE_F32)   // ingest's own arithmetic over the fp32 rows, writing nothing but the stats
             B2F_TRY(launch_ingest(ix->rows_f32, n_new, ix->d, nullptr, nullptr, ix->dpad, nullptr, ix->stats, mu, 0, 0, st));
@@ -1922,7 +1926,7 @@ int b2f_index_write(b2f_index* ix, const char* path) {
                     e = cudaMemcpyAsync(hbuf, ix->rows_f32 + r0 * ix->d, (size_t)m * ix->d * 4, cudaMemcpyDeviceToHost, ix->stream);
                 } else {
                     float* dbuf = reinterpret_cast<float*>(ix->ws + (size_t)slot * cbytes);
-                    rc = launch_bf16_to_f32(ix->scan + r0 * ix->dpad, ix->dpad, m, ix->d, ix->mu_set ? ix->centre : nullptr, dbuf, ix->stream);
+                    rc = launch_bf16_to_f32(ix->scan + r0 * ix->dpad, ix->dpad, m, ix->d, scan_centre(ix), dbuf, ix->stream);
                     ix->st.launches++;
                     e = cudaMemcpyAsync(hbuf, dbuf, (size_t)m * ix->d * 4, cudaMemcpyDeviceToHost, ix->stream);
                 }

@@ -31,10 +31,10 @@ __device__ __forceinline__ float auth_loss(float m, float xb, float& r) {
 
 // Writes one element group of a row to every derived store and returns (bf16(x)^2, (x-bf16(x))^2).
 // bf16_auth: the index keeps no fp32 rows -- the authoritative row IS r = fl32(m + bf16(x - m)); then the "rounding
-// error" of the scan copy is what the fp32 addition loses, (r - m) - bf16(x - m), and *r_out receives r.
+// error" of the scan copy is what the fp32 addition loses, (r - m) - bf16(x - m), and r_out receives r.
 __device__ __forceinline__ void emit_elem(float x, int64_t row, int col, int d, float* rows_f32,
-                                          __nv_bfloat16* scan, int64_t dpad, float& nn, float& ee, float m = 0.f,
-                                          bool bf16_auth = false, float* r_out = nullptr) {
+                                          __nv_bfloat16* scan, int64_t dpad, float& nn, float& ee, float m,
+                                          bool bf16_auth, float& r_out) {
     if (rows_f32) rows_f32[row * d + col] = x;
     const float xc = x - m;  // the scan copy holds the CENTRED row (see ingest_kernel)
     const __nv_bfloat16 b = __float2bfloat16_rn(xc);
@@ -42,11 +42,7 @@ __device__ __forceinline__ void emit_elem(float x, int64_t row, int col, int d, 
     if (scan) scan[row * dpad + col] = b;
     nn = fmaf(xb, xb, nn);
     float e = xc - xb;
-    if (bf16_auth) {
-        float r;
-        e = auth_loss(m, xb, r);
-        if (r_out) *r_out = r;
-    }
+    if (bf16_auth) e = auth_loss(m, xb, r_out);
     ee = fmaf(e, e, ee);
 }
 
@@ -175,7 +171,7 @@ ingest_kernel(const float* __restrict__ src, int64_t n, int d, float* __restrict
             for (int c = lane; c < d; c += 32) {
                 const float x = src[row * d + c], m = mu ? mu[c] : 0.f;
                 float r = x;
-                emit_elem(x, row, c, d, rows_f32, scan, dpad, nn, ee, m, bf16_auth != 0, &r);
+                emit_elem(x, row, c, d, rows_f32, scan, dpad, nn, ee, m, bf16_auth != 0, r);
                 if (ip_bias) mx += (double)m * r;   // r = x (fp32 rows) or the authoritative rounded row (bf16 storage)
             }
         }
@@ -255,14 +251,13 @@ int launch_scan_stats(const __nv_bfloat16* scan, int64_t n, int d, int64_t dpad,
 
 // K7.  One CTA per sequence.  hidden [B,T,d] fp32, mask [B,T] int64 (may be null = all ones).
 // CLS: row = hidden[b,0,:] (vectorization.py:44).  MEAN: sum_t mask*h / max(sum_t mask, 1e-9).
-// normalize: row /= max(|row|, 1e-12).  The result goes to out_f32 [B,d] (index rows or a plain
-// output) and, when given, the bf16 scan copy / norms / stats of the index -- no host bounce.
+// normalize: row /= max(|row|, 1e-12).  The result goes to out_f32 [B,d]: staged index rows, which the ingest
+// kernel then takes like any other add's, or a plain output.
 __global__ void __launch_bounds__(256)
 pool_kernel(const float* __restrict__ hidden, const int64_t* __restrict__ mask, int64_t T, int d, int pool, int normalize,
-            float* __restrict__ out_f32, __nv_bfloat16* __restrict__ scan, int64_t dpad, float* __restrict__ norms,
-            float* __restrict__ stats) {
+            float* __restrict__ out_f32) {
     extern __shared__ float srow[];  // [d]
-    __shared__ float red[3][8];
+    __shared__ float red[8];
     const int64_t b = blockIdx.x;
     const float* h = hidden + b * T * d;
     float cnt = 1.f;
@@ -279,6 +274,7 @@ pool_kernel(const float* __restrict__ hidden, const int64_t* __restrict__ mask, 
         float* psum = srow + d;
         const int ncg = d / 4, nth = (int)blockDim.x / ncg;
         const int cg = (int)threadIdx.x % ncg, th = (int)threadIdx.x / ncg;
+        float4* const part = reinterpret_cast<float4*>(psum + th * d + cg * 4);   // this thread's partial sums
         if (th < nth) {
             float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
             for (int64_t t0 = th; t0 < T; t0 += 4 * nth) {
@@ -296,7 +292,7 @@ pool_kernel(const float* __restrict__ hidden, const int64_t* __restrict__ mask, 
                     acc.z = fmaf(mk[u], v[u].z, acc.z); acc.w = fmaf(mk[u], v[u].w, acc.w);
                 }
             }
-            *reinterpret_cast<float4*>(psum + th * d + cg * 4) = acc;
+            *part = acc;
         }
         __syncthreads();
         for (int c = threadIdx.x; c < d; c += blockDim.x) {
@@ -324,35 +320,16 @@ pool_kernel(const float* __restrict__ hidden, const int64_t* __restrict__ mask, 
         }
     }
     ss = warp_sum(ss);
-    if ((threadIdx.x & 31) == 0) red[0][threadIdx.x >> 5] = ss;
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = ss;
     __syncthreads();
     float tot = 0.f;
-    for (int w = 0; w < (int)(blockDim.x >> 5); w++) tot += red[0][w];
+    for (int w = 0; w < (int)(blockDim.x >> 5); w++) tot += red[w];
     const float scale = normalize ? 1.f / fmaxf(sqrtf(tot), 1e-12f) : 1.f;
-    float nn = 0.f, ee = 0.f;
-    for (int c = threadIdx.x; c < d; c += blockDim.x) emit_elem(srow[c] * scale, b, c, d, out_f32, scan, dpad, nn, ee);
-    if (scan)
-        for (int c = d + threadIdx.x; c < dpad; c += blockDim.x) scan[b * dpad + c] = __float2bfloat16_rn(0.f);
-    nn = warp_sum(nn);
-    ee = warp_sum(ee);
-    if ((threadIdx.x & 31) == 0) {
-        red[1][threadIdx.x >> 5] = nn;
-        red[2][threadIdx.x >> 5] = ee;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        float n2 = 0.f, e2 = 0.f;
-        for (int w = 0; w < (int)(blockDim.x >> 5); w++) { n2 += red[1][w]; e2 += red[2][w]; }
-        if (norms) norms[b] = n2;
-        if (stats) {
-            atomic_max_nonneg(stats, n2);
-            atomic_max_nonneg(stats + 1, e2);
-        }
-    }
+    for (int c = threadIdx.x; c < d; c += blockDim.x) out_f32[b * d + c] = srow[c] * scale;
 }
 
 int launch_pool(const float* hidden, const int64_t* mask, int64_t B, int64_t T, int d, int pool, int normalize,
-                float* out_f32, __nv_bfloat16* scan, int64_t dpad, float* norms, float* stats, cudaStream_t st) {
+                float* out_f32, cudaStream_t st) {
     if (B <= 0) return B2F_OK;
     if (T <= 0 || (pool != B2F_POOL_CLS && pool != B2F_POOL_MEAN)) {
         set_error("pool: bad T=%lld or pool mode %d", (long long)T, pool);
@@ -374,7 +351,7 @@ int launch_pool(const float* hidden, const int64_t* mask, int64_t B, int64_t T, 
             configured[dev] = 160 * 1024;
         }
     }
-    pool_kernel<<<(unsigned)B, 256, smem, st>>>(hidden, mask, T, d, pool, normalize, out_f32, scan, dpad, norms, stats);
+    pool_kernel<<<(unsigned)B, 256, smem, st>>>(hidden, mask, T, d, pool, normalize, out_f32);
     B2F_CUDA(cudaGetLastError());
     return B2F_OK;
 }

@@ -59,36 +59,18 @@ int launch_merge_parts(const float* pk, const int32_t* pi, int nq, int nparts, i
     return B2F_OK;
 }
 
-// keys/ids [nq][kin] (ascending, int32 local ids) -> D/I [.][k] in faiss conventions
-__global__ void finalize_kernel(const float* __restrict__ keys, const int32_t* __restrict__ ids, int nq, int kin, int k,
-                                int l2, int64_t id_offset, const int32_t* __restrict__ qsel, float* __restrict__ D,
-                                int64_t* __restrict__ I) {
+// D / I [nq][k] all padding: the result of a search over no rows
+__global__ void fill_empty_kernel(int64_t total, int l2, float* __restrict__ D, int64_t* __restrict__ I) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (int64_t)nq * k) return;
-    const int r = (int)(t / k), j = (int)(t % k);
-    const int orow = qsel ? qsel[r] : r;
-    float key = FLT_MAX;
-    int32_t id = -1;
-    if (j < kin) {
-        key = keys[(int64_t)r * kin + j];
-        id = ids[(int64_t)r * kin + j];
-    }
-    const int64_t o = (int64_t)orow * k + j;
-    if (id < 0) {
-        D[o] = l2 ? FLT_MAX : -FLT_MAX;
-        I[o] = -1;
-    } else {
-        D[o] = l2 ? key : -key;
-        I[o] = (int64_t)id + id_offset;
-    }
+    if (t >= total) return;
+    D[t] = l2 ? FLT_MAX : -FLT_MAX;
+    I[t] = -1;
 }
 
-int launch_finalize(const float* keys, const int32_t* ids, int nq, int kin, int k, int metric, int64_t id_offset,
-                    const int32_t* qsel, float* D, int64_t* I, cudaStream_t st) {
+int launch_fill_empty(int nq, int k, int metric, float* D, int64_t* I, cudaStream_t st) {
     const int64_t total = (int64_t)nq * k;
     if (total <= 0) return B2F_OK;
-    finalize_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(keys, ids, nq, kin, k, metric == B2F_METRIC_L2,
-                                                                      id_offset, qsel, D, I);
+    fill_empty_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(total, metric == B2F_METRIC_L2, D, I);
     B2F_CUDA(cudaGetLastError());
     return B2F_OK;
 }

@@ -24,7 +24,7 @@ range_scan_kernel(const RerankArgs a, float tau, const int32_t* __restrict__ lis
     __shared__ int s_hit[kScanGroup][32];
     __shared__ int s_cnt[kScanGroup];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, sl = lane & 7, rg = tid >> 3;
-    const bool l2 = a.metric == B2F_METRIC_L2;
+    const bool l2 = a.rows.metric == B2F_METRIC_L2;
     const int nl = nlist_dev ? *nlist_dev : nlist_host;
     const int ngroups = (nl + kScanGroup - 1) / kScanGroup;
     const int64_t items = (int64_t)ngroups * ntiles;
@@ -33,7 +33,7 @@ range_scan_kernel(const RerankArgs a, float tau, const int32_t* __restrict__ lis
         const int s0 = g * kScanGroup;
         const int nqg = nl - s0 < kScanGroup ? nl - s0 : kScanGroup;
         const int64_t r_lo = (int64_t)tile * tile_rows;
-        const int64_t r_hi = r_lo + tile_rows < a.ntotal ? r_lo + tile_rows : a.ntotal;
+        const int64_t r_hi = r_lo + tile_rows < a.rows.n ? r_lo + tile_rows : a.rows.n;
         int64_t off = 0;   // EMIT: where warp w's query writes next
         if (EMIT) {
             if (warp < nqg) {
@@ -54,7 +54,7 @@ range_scan_kernel(const RerankArgs a, float tau, const int32_t* __restrict__ lis
 #pragma unroll 1
             for (int i = 0; i < nqg; i++) {
                 const int32_t qi = list ? list[s0 + i] : s0 + i;
-                const float key = exact_key_8lanes(a, a.q + (int64_t)qi * a.d, valid ? (int32_t)row : -1, sl, l2);
+                const float key = exact_key_8lanes(a.rows, a.q + (int64_t)qi * a.rows.d, valid ? (int32_t)row : -1, sl, l2);
                 const bool hit = valid && key < tau;   // NaN is never a hit
                 if (EMIT) {
                     if (sl == 0) {
@@ -139,7 +139,7 @@ RangeScanGeometry range_scan_geometry(int64_t n) {
 int launch_range_scan(const RerankArgs& a, float tau, const int32_t* list, const int32_t* nlist_dev, int nlist_max,
                       int32_t* tile_counts, int32_t* count, const int64_t* lims, int64_t base, float* D, int64_t* I,
                       int64_t id_offset, bool emit, cudaStream_t st) {
-    const RangeScanGeometry g = range_scan_geometry(a.ntotal);
+    const RangeScanGeometry g = range_scan_geometry(a.rows.n);
     const int64_t items = (int64_t)((nlist_max + kScanGroup - 1) / kScanGroup) * g.ntiles;
     if (items <= 0) return B2F_OK;
     const int blocks = (int)(items < 4 * kNumSMs ? items : 4 * kNumSMs);

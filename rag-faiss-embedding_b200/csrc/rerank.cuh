@@ -10,11 +10,11 @@ constexpr int kRerankThreads = 256;
 // Exact fp32 key (L2: squared distance in exact-difference form; IP: negated dot product) of row `id` for the
 // query vector qv, computed by the 8 lanes of a lane group (sl = lane & 7); every lane returns the total.
 // The loads of a row are issued four 16-byte chunks at a time, so a lane group keeps 512 bytes in flight.
-__device__ __forceinline__ float exact_key_8lanes(const RerankArgs& a, const float* __restrict__ qv, int32_t id, int sl, bool l2) {
+__device__ __forceinline__ float exact_key_8lanes(const StoredRows& a, const float* __restrict__ qv, int32_t id, int sl, bool l2) {
     float acc = 0.f;
     if (id >= 0) {
-        if (a.rows_f32 && (a.d & 3) == 0) {
-            const float* x = a.rows_f32 + (int64_t)id * a.d;
+        if (a.f32 && (a.d & 3) == 0) {
+            const float* x = a.f32 + (int64_t)id * a.d;
             for (int j0 = sl * 4; j0 < a.d; j0 += 128) {
                 float4 xv[4], qq[4];
 #pragma unroll
@@ -38,8 +38,8 @@ __device__ __forceinline__ float exact_key_8lanes(const RerankArgs& a, const flo
                     }
                 }
             }
-        } else if (!a.rows_f32 && (a.d & 7) == 0) {
-            const __nv_bfloat16* x = a.rows_bf16 + (int64_t)id * a.pitch_bf16;
+        } else if (!a.f32 && (a.d & 7) == 0) {
+            const __nv_bfloat16* x = a.bf16 + (int64_t)id * a.pitch;
             for (int j0 = sl * 8; j0 < a.d; j0 += 128) {
                 uint4 w[2];
 #pragma unroll
@@ -76,8 +76,8 @@ __device__ __forceinline__ float exact_key_8lanes(const RerankArgs& a, const flo
             }
         } else {
             for (int j = sl; j < a.d; j += 8) {
-                const float xv = a.rows_f32 ? a.rows_f32[(int64_t)id * a.d + j]
-                                            : (a.centre ? a.centre[j] : 0.f) + __bfloat162float(a.rows_bf16[(int64_t)id * a.pitch_bf16 + j]);
+                const float xv = a.f32 ? a.f32[(int64_t)id * a.d + j]
+                                       : (a.centre ? a.centre[j] : 0.f) + __bfloat162float(a.bf16[(int64_t)id * a.pitch + j]);
                 if (l2) {
                     const float t = xv - qv[j];
                     acc = fmaf(t, t, acc);
@@ -97,13 +97,13 @@ __device__ __forceinline__ float exact_key_8lanes(const RerankArgs& a, const flo
 // valid); bound: a coarse key that every row OUTSIDE the candidates is known to reach or exceed.  True when the bf16 /
 // fp32 rounding bounds prove that no such row can beat tau.
 __device__ __forceinline__ bool rerank_certified(const RerankArgs& a, int q, float tau, float bound) {
-    const bool l2 = a.metric == B2F_METRIC_L2;
+    const bool l2 = a.rows.metric == B2F_METRIC_L2;
     const float qn2 = a.qnorm[q];
     const float qn = sqrtf(qn2);
     const float eq = a.qerr[q];
     // fp32 accumulation slack: gamma_n * sum|q_i x_i| <= n u |q||x| per inner product (n = d + 16 guards
     // the tensor core's chunked accumulation order, u = 2^-24), doubled for non-IEEE accumulator rounding
-    const float gam = 4.f * (float)(a.d + 16) * 5.9604645e-8f;
+    const float gam = 4.f * (float)(a.rows.d + 16) * 5.9604645e-8f;
     if (l2) {
         // c = |q~|^2 + |x~|^2 - 2<q~,x~>: the two norms are fp32 sums as well
         const float nu = gam * (2.f * qn * a.max_row_norm + qn2 + a.max_row_norm * a.max_row_norm);
@@ -135,8 +135,8 @@ __device__ __forceinline__ bool rerank_block(const RerankArgs& a, int q, const f
     __shared__ float s_tau;
     __shared__ int s_cert;
     const int lane = threadIdx.x & 31;
-    const float* qv = a.q + (int64_t)q * a.d;
-    const bool l2 = a.metric == B2F_METRIC_L2;
+    const float* qv = a.q + (int64_t)q * a.rows.d;
+    const bool l2 = a.rows.metric == B2F_METRIC_L2;
     const int64_t orow = a.out_map ? (int64_t)a.out_map[q] : (int64_t)q;   // row of D / I this query answers
     if (threadIdx.x == 0) s_tau = FLT_MAX;
     __syncthreads();
@@ -145,8 +145,8 @@ __device__ __forceinline__ bool rerank_block(const RerankArgs& a, int q, const f
     for (int c0 = 0; c0 < nc; c0 += kRerankThreads / 8) {
         const int c = c0 + (threadIdx.x >> 3);
         int32_t id = c < nc ? ci[c] : -1;
-        if ((int64_t)id >= a.ntotal) id = -1;  // never dereference a label outside the index
-        const float key = exact_key_8lanes(a, qv, id, sl, l2);
+        if ((int64_t)id >= a.rows.n) id = -1;  // never dereference a label outside the index
+        const float key = exact_key_8lanes(a.rows, qv, id, sl, l2);
         if (sl == 0 && c < nc) {
             const bool ok = id >= 0 && !(key != key);  // NaN never enters (faiss heap semantics)
             ek[c] = ok ? key : FLT_MAX;
@@ -164,27 +164,17 @@ __device__ __forceinline__ bool rerank_block(const RerankArgs& a, int q, const f
             const int32_t oi_ = ei[j];
             rank += (cand_less(ok_, oi_, mk, mi) || (ok_ == mk && oi_ == mi && j < t)) ? 1 : 0;
         }
-        if (rank < a.k) {
-            if (a.D) {  // fused finalize: faiss conventions straight to the caller's buffers
-                const int64_t o = orow * a.k + rank;
-                a.D[o] = mi < 0 ? (l2 ? FLT_MAX : -FLT_MAX) : (l2 ? mk : -mk);
-                a.I[o] = mi < 0 ? -1 : (int64_t)mi + a.id_offset;
-            } else {
-                a.out_key[(int64_t)q * a.k + rank] = mk;
-                a.out_id[(int64_t)q * a.k + rank] = mi;
-            }
+        if (rank < a.k) {   // faiss conventions straight to the caller's buffers
+            const int64_t o = orow * a.k + rank;
+            a.D[o] = mi < 0 ? (l2 ? FLT_MAX : -FLT_MAX) : (l2 ? mk : -mk);
+            a.I[o] = mi < 0 ? -1 : (int64_t)mi + a.id_offset;
         }
         if (rank == a.k - 1) s_tau = mk;
     }
     // fewer candidates than k: pad (faiss: label -1, distance +-FLT_MAX)
     for (int t = nc + threadIdx.x; t < a.k; t += kRerankThreads) {
-        if (a.D) {
-            a.D[orow * a.k + t] = l2 ? FLT_MAX : -FLT_MAX;
-            a.I[orow * a.k + t] = -1;
-        } else {
-            a.out_key[(int64_t)q * a.k + t] = FLT_MAX;
-            a.out_id[(int64_t)q * a.k + t] = -1;
-        }
+        a.D[orow * a.k + t] = l2 ? FLT_MAX : -FLT_MAX;
+        a.I[orow * a.k + t] = -1;
     }
     __syncthreads();
     if (threadIdx.x == 0) {

@@ -370,7 +370,7 @@ size_t scan_scratch_bytes(int k) {
 
 template <int NQ, bool L2, typename RowT, typename Vec>
 static int launch_one(const RowT* rows, int64_t pitch, const ScanArgs& a, cudaStream_t st) {
-    const int dq = ((a.d + Vec::N - 1) / Vec::N) * Vec::N;
+    const int dq = ((a.rows.d + Vec::N - 1) / Vec::N) * Vec::N;
     const size_t smem = (((size_t)NQ * dq + 2 * (size_t)kScanWarps * NQ * a.k + 1) & ~(size_t)1) * 4 + (size_t)kGatherCap * 8 +
                         (sizeof(RowT) == 2 ? (size_t)dq * 4 : 0);   // + the centre (bf16 rows)
     auto kern = scan_kernel<NQ, L2, RowT, Vec>;
@@ -402,7 +402,7 @@ static int launch_one(const RowT* rows, int64_t pitch, const ScanArgs& a, cudaSt
         return B2F_EINVAL;
     }
     const int use = occ > 4 ? 4 : occ;
-    const int64_t ngroups = (a.n + kRowsPerGroup - 1) / kRowsPerGroup;
+    const int64_t ngroups = (a.rows.n + kRowsPerGroup - 1) / kRowsPerGroup;
     int64_t want = (ngroups + kScanWarps - 1) / kScanWarps;
     int blocks = (int)(want < (int64_t)kNumSMs * use ? want : (int64_t)kNumSMs * use);
     if (blocks < 1) blocks = 1;
@@ -427,11 +427,11 @@ static int launch_one(const RowT* rows, int64_t pitch, const ScanArgs& a, cudaSt
     f.certify = a.certify;
     f.tub = a.tub;
     f.parity = a.parity;
-    f.mu = a.mu;
+    f.mu = a.rows.centre;
     f.allow = a.allow;
     const RowT* rows_ = rows;
-    int64_t pitch_ = pitch, n_ = a.n;
-    int d_ = a.d, dq_ = dq, k_ = a.k;
+    int64_t pitch_ = pitch, n_ = a.rows.n;
+    int d_ = a.rows.d, dq_ = dq, k_ = a.k;
     const float* q_ = a.q;
     void* args[] = {(void*)&rows_, (void*)&pitch_, (void*)&n_, (void*)&d_, (void*)&dq_, (void*)&q_, (void*)&k_, (void*)&f};
     // cooperative: every CTA is resident (the grid is sized from the occupancy query), so grid.sync() is legal
@@ -441,15 +441,15 @@ static int launch_one(const RowT* rows, int64_t pitch, const ScanArgs& a, cudaSt
 
 template <typename RowT, typename Vec>
 static int dispatch(const RowT* rows, int64_t pitch, const ScanArgs& a, cudaStream_t st) {
-    const bool l2 = a.metric == B2F_METRIC_L2;
+    const bool l2 = a.rows.metric == B2F_METRIC_L2;
     // queries per pass: bounded by the per-warp lists (8 warps x NQ x k x 8 bytes) and the query tile in smem
     int g = 8;
     auto pow2_le = [](int x) { int p = 1; while (p * 2 <= x) p *= 2; return p; };
     const int by_k = scan_nq_cap(a.k);
-    const int dq = ((a.d + Vec::N - 1) / Vec::N) * Vec::N;
+    const int dq = ((a.rows.d + Vec::N - 1) / Vec::N) * Vec::N;
     const int by_smem = 16384 / (dq > 0 ? dq : 1);
     if (by_smem < 1) {
-        set_error("d=%d too large for the streaming scan", a.d);
+        set_error("d=%d too large for the streaming scan", a.rows.d);
         return B2F_EINVAL;
     }
     if (g > by_k) g = by_k;
@@ -471,11 +471,12 @@ int launch_scan(const ScanArgs& a, cudaStream_t st) {
         set_error("scan: k=%d out of range", a.k);
         return B2F_EINVAL;
     }
-    if (a.rows_f32) {
-        if (a.d % 4 == 0) return dispatch<float, RowVec<float>>(a.rows_f32, a.d, a, st);
-        return dispatch<float, ScalarRow>(a.rows_f32, a.d, a, st);
+    const StoredRows& r = a.rows;
+    if (r.f32) {
+        if (r.d % 4 == 0) return dispatch<float, RowVec<float>>(r.f32, r.d, a, st);
+        return dispatch<float, ScalarRow>(r.f32, r.d, a, st);
     }
-    return dispatch<__nv_bfloat16, RowVec<__nv_bfloat16>>(a.rows_bf16, a.pitch_bf16, a, st);
+    return dispatch<__nv_bfloat16, RowVec<__nv_bfloat16>>(r.bf16, r.pitch, a, st);
 }
 
 }  // namespace b2f

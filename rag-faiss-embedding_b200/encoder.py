@@ -11,6 +11,7 @@ from __future__ import annotations
 import ctypes
 
 from . import _capi as C
+from .index import _torch_stream
 
 
 def pool_normalize(hidden, attention_mask=None, pool: str = "cls", normalize: bool = False):
@@ -26,10 +27,9 @@ def pool_normalize(hidden, attention_mask=None, pool: str = "cls", normalize: bo
     if attention_mask is not None:
         attention_mask = attention_mask.to(device=hidden.device, dtype=torch.int64).contiguous()
         mptr = attention_mask.data_ptr()
-    stream = int(torch.cuda.current_stream(hidden.device).cuda_stream) or 1  # 0x1 = cudaStreamLegacy
     C.check(C.load().b2f_pool_normalize(hidden.data_ptr(), mptr, B, T, d,
                                         C.POOL_MEAN if pool == "mean" else C.POOL_CLS, int(bool(normalize)),
-                                        out.data_ptr(), hidden.device.index or 0, ctypes.c_void_p(stream)))
+                                        out.data_ptr(), hidden.device.index or 0, ctypes.c_void_p(_torch_stream(hidden))))
     return out
 
 
@@ -38,7 +38,6 @@ def synth_rows(seed: int, row0: int, nrows: int, d: int, normalize: bool = False
     import torch
 
     out = torch.empty((nrows, d), dtype=torch.float32, device=f"cuda:{device}")
-    stream = int(torch.cuda.current_stream(out.device).cuda_stream) or 1  # 0x1 = cudaStreamLegacy
     C.check(C.load().b2f_synth_rows(int(seed), int(row0), int(nrows), int(d), int(bool(normalize)), out.data_ptr(),
-                                    device, ctypes.c_void_p(stream)))
+                                    device, ctypes.c_void_p(_torch_stream(out))))
     return out

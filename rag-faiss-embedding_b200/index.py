@@ -285,6 +285,38 @@ class IndexFlat:
         _assert(t.is_cuda and t.device.index == self.device,
                 f"{what} must be a CUDA tensor on the index's GPU (cuda:{self.device}), got {t.device}")
 
+    def _rows_in(self, x):
+        """Rows or queries x [n, d] -> (x as float32 and contiguous, pointer, mem kind, stream).  A CUDA tensor (on the
+        index's GPU) is read where it is, on the current torch stream; anything else becomes a host array."""
+        if _is_torch(x) and x.is_cuda:
+            import torch
+
+            _assert(x.dim() == 2 and x.shape[1] == self.d, f"dimension mismatch: got {tuple(x.shape)}, d={self.d}")
+            self._check_tensor(x, "x")
+            x = x.to(torch.float32).contiguous()
+            return x, x.data_ptr(), C.MEM_DEVICE, _torch_stream(x)
+        if _is_torch(x):
+            x = x.detach().cpu().numpy()
+        x = np.ascontiguousarray(x, dtype=np.float32)
+        _assert(x.ndim == 2, "expected a 2-D array [n, d]")
+        _assert(x.shape[1] == self.d, f"dimension mismatch: got {x.shape[1]}, index has d={self.d}")
+        return x, x.ctypes.data, C.MEM_HOST, None
+
+    def _hidden_in(self, hidden, attention_mask, what: str):
+        """Encoder output hidden [B, T, d] (a CUDA tensor on the index's GPU) and its optional attention mask [B, T] ->
+        (hidden as float32 and contiguous, the mask as int64 on hidden's device, its pointer); no mask: None, None.  The
+        caller holds on to the mask until the library call that reads it has been enqueued."""
+        import torch
+
+        _assert(_is_torch(hidden) and hidden.is_cuda and hidden.dim() == 3 and hidden.shape[2] == self.d,
+                f"{what} expects a CUDA tensor [B, T, d]")
+        self._check_tensor(hidden, "hidden")
+        hidden = hidden.to(torch.float32).contiguous()
+        if attention_mask is None:
+            return hidden, None, None
+        mask = attention_mask.to(device=hidden.device, dtype=torch.int64).contiguous()
+        return hidden, mask, mask.data_ptr()
+
     def stats(self) -> dict:
         s = C.Stats()
         C.check(self._lib.b2f_index_stats(self._h, ctypes.byref(s)))
@@ -294,27 +326,10 @@ class IndexFlat:
         C.check(self._lib.b2f_index_reserve(self._h, int(nrows)))
 
     # ---- faiss surface ----------------------------------------------------------------------
-    def _coerce_host(self, x) -> np.ndarray:
-        x = np.ascontiguousarray(x, dtype=np.float32)
-        _assert(x.ndim == 2, "expected a 2-D array [n, d]")
-        n, d = x.shape
-        _assert(d == self.d, f"dimension mismatch: got {d}, index has d={self.d}")
-        return x
-
     def add(self, x):
         """index.add(x): faiss_store.py:46, rag_datastore_manager.py:173."""
-        if _is_torch(x) and x.is_cuda:
-            import torch
-
-            _assert(x.dim() == 2 and x.shape[1] == self.d, f"dimension mismatch: got {tuple(x.shape)}, d={self.d}")
-            self._check_tensor(x, "x")
-            x = x.to(torch.float32).contiguous()
-            C.check(self._lib.b2f_index_add(self._h, x.shape[0], x.data_ptr(), C.MEM_DEVICE, _torch_stream(x)))
-            return
-        if _is_torch(x):
-            x = x.detach().cpu().numpy()
-        x = self._coerce_host(x)
-        C.check(self._lib.b2f_index_add(self._h, x.shape[0], x.ctypes.data, C.MEM_HOST, None))
+        x, ptr, mem, stream = self._rows_in(x)
+        C.check(self._lib.b2f_index_add(self._h, x.shape[0], ptr, mem, stream))
 
     def add_synthetic(self, seed: int, row0: int, nrows: int, normalize: bool = False):
         """Append rows of the counter-based synthetic matrix, generated on the device."""
@@ -322,16 +337,7 @@ class IndexFlat:
 
     def add_pooled(self, hidden, attention_mask=None, pool: str = "cls", normalize: bool = False):
         """Fused encoder epilogue (replaces vectorization.py:44-47): hidden [B,T,d] CUDA fp32 tensor."""
-        import torch
-
-        _assert(_is_torch(hidden) and hidden.is_cuda and hidden.dim() == 3 and hidden.shape[2] == self.d,
-                "add_pooled expects a CUDA tensor [B, T, d]")
-        self._check_tensor(hidden, "hidden")
-        hidden = hidden.to(torch.float32).contiguous()
-        mptr = None
-        if attention_mask is not None:
-            attention_mask = attention_mask.to(device=hidden.device, dtype=torch.int64).contiguous()
-            mptr = attention_mask.data_ptr()
+        hidden, mask, mptr = self._hidden_in(hidden, attention_mask, "add_pooled")
         C.check(self._lib.b2f_index_add_pooled(self._h, hidden.data_ptr(), mptr, hidden.shape[0], hidden.shape[1],
                                                C.POOL_MEAN if pool == "mean" else C.POOL_CLS, int(bool(normalize)),
                                                _torch_stream(hidden)))
@@ -342,14 +348,7 @@ class IndexFlat:
         import torch
 
         _assert(k > 0, "k must be > 0")
-        _assert(_is_torch(hidden) and hidden.is_cuda and hidden.dim() == 3 and hidden.shape[2] == self.d,
-                "search_pooled expects a CUDA tensor [B, T, d]")
-        self._check_tensor(hidden, "hidden")
-        hidden = hidden.to(torch.float32).contiguous()
-        mptr = None
-        if attention_mask is not None:
-            attention_mask = attention_mask.to(device=hidden.device, dtype=torch.int64).contiguous()
-            mptr = attention_mask.data_ptr()
+        hidden, mask, mptr = self._hidden_in(hidden, attention_mask, "search_pooled")
         B = hidden.shape[0]
         D = torch.empty((B, k), dtype=torch.float32, device=hidden.device)
         I = torch.empty((B, k), dtype=torch.int64, device=hidden.device)
@@ -364,24 +363,18 @@ class IndexFlat:
         only the ids the selector contains (tuning from set_search_params)."""
         _assert(k > 0, "k must be > 0")
         p, sel = self._split_params(params)
-        if _is_torch(x) and x.is_cuda:
+        x, ptr, mem, stream = self._rows_in(x)
+        n = x.shape[0]
+        if mem == C.MEM_DEVICE:
             import torch
 
-            _assert(x.dim() == 2 and x.shape[1] == self.d, f"dimension mismatch: got {tuple(x.shape)}, d={self.d}")
-            self._check_tensor(x, "x")
-            x = x.to(torch.float32).contiguous()
-            D = torch.empty((x.shape[0], k), dtype=torch.float32, device=x.device)
-            I = torch.empty((x.shape[0], k), dtype=torch.int64, device=x.device)
-            self._search_call(x.shape[0], x.data_ptr(), k, D.data_ptr(), I.data_ptr(), C.MEM_DEVICE, _torch_stream(x), p, sel,
-                              x.device)
+            D = torch.empty((n, k), dtype=torch.float32, device=x.device)
+            I = torch.empty((n, k), dtype=torch.int64, device=x.device)
+            self._search_call(n, ptr, k, D.data_ptr(), I.data_ptr(), mem, stream, p, sel, x.device)
             return D, I
-        if _is_torch(x):
-            x = x.detach().cpu().numpy()
-        x = self._coerce_host(x)
-        n = x.shape[0]
         D = np.empty((n, k), dtype=np.float32)
         I = np.empty((n, k), dtype=np.int64)
-        self._search_call(n, x.ctypes.data, k, D.ctypes.data, I.ctypes.data, C.MEM_HOST, None, p, sel)
+        self._search_call(n, ptr, k, D.ctypes.data, I.ctypes.data, mem, stream, p, sel)
         return D, I
 
     def search_tensors_into(self, x, k: int, D, I, *, params=None):
@@ -390,15 +383,15 @@ class IndexFlat:
         import torch
 
         _assert(k > 0, "k must be > 0")
-        _assert(x.is_cuda and x.dim() == 2 and x.shape[1] == self.d, f"dimension mismatch: got {tuple(x.shape)}, d={self.d}")
+        _assert(x.is_cuda, f"dimension mismatch: got {tuple(x.shape)}, d={self.d}")
+        x, ptr, mem, stream = self._rows_in(x)
         _assert(D.is_cuda and I.is_cuda and D.dtype == torch.float32 and I.dtype == torch.int64
                 and D.is_contiguous() and I.is_contiguous() and tuple(D.shape) == (x.shape[0], k) == tuple(I.shape),
                 "D / I must be contiguous CUDA tensors [n, k] of float32 / int64")
-        for t, what in ((x, "x"), (D, "D"), (I, "I")):
+        for t, what in ((D, "D"), (I, "I")):
             self._check_tensor(t, what)
-        x = x.to(torch.float32).contiguous()
         p, sel = self._split_params(params)
-        self._search_call(x.shape[0], x.data_ptr(), k, D.data_ptr(), I.data_ptr(), C.MEM_DEVICE, _torch_stream(x), p, sel, x.device)
+        self._search_call(x.shape[0], ptr, k, D.data_ptr(), I.data_ptr(), mem, stream, p, sel, x.device)
 
     def range_search(self, x, radius: float, *, params=None):
         """index.range_search(x, radius) -> (lims, D, I), faiss's RangeSearchResult: query i owns
@@ -407,21 +400,8 @@ class IndexFlat:
         on the current torch stream.  The five numbers of b2f_range_result_info go to self.last_range_info.  params as
         search: SearchParameters(sel=...) keeps exactly the hits whose label the selector contains."""
         p, sel = self._split_params(params)
-        dev = _is_torch(x) and x.is_cuda
-        if dev:
-            import torch
-
-            _assert(x.dim() == 2 and x.shape[1] == self.d, f"dimension mismatch: got {tuple(x.shape)}, d={self.d}")
-            self._check_tensor(x, "x")
-            x = x.to(torch.float32).contiguous()
-            stream = _torch_stream(x)
-            qptr, mem = x.data_ptr(), C.MEM_DEVICE
-        else:
-            if _is_torch(x):
-                x = x.detach().cpu().numpy()
-            x = self._coerce_host(x)
-            stream = None
-            qptr, mem = x.ctypes.data, C.MEM_HOST
+        x, qptr, mem, stream = self._rows_in(x)
+        dev = mem == C.MEM_DEVICE
         n = x.shape[0]
         h = ctypes.c_void_p()
         if sel is None:
@@ -437,6 +417,8 @@ class IndexFlat:
             C.check(self._lib.b2f_range_result_lims(h, lims.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))))
             total = int(lims[-1])
             if dev:
+                import torch
+
                 D = torch.empty(total, dtype=torch.float32, device=x.device)
                 I = torch.empty(total, dtype=torch.int64, device=x.device)
                 C.check(self._lib.b2f_range_result_fetch(h, D.data_ptr(), I.data_ptr(), C.MEM_DEVICE, stream))

@@ -22,7 +22,7 @@ import numpy as np
 
 from . import _capi as C
 from .index import (METRIC_L2, IDSelectorBatch, IDSelectorBitmap, IDSelectorRange, IndexFlat, SearchParameters, _assert,
-                    _id_array, _is_torch, selector_contains)
+                    _id_array, _is_torch, _torch_stream, selector_contains)
 
 
 def partition_rows(n: int, world: int) -> List[Tuple[int, int]]:
@@ -115,13 +115,10 @@ def merge_topk_strided(metric: int, recv, part_bytes: int, off_i: int, D, I):
     """b2f_merge_topk_strided over an all-gathered buffer: recv [G * part_bytes] uint8 holding G packed parts [D | pad |
     I at off_i] of [nq, k] results each; writes the merged top-k into D / I [nq, k] (CUDA tensors on recv's device,
     enqueued on the current torch stream)."""
-    import torch
-
     nq, k = int(D.shape[0]), int(D.shape[1])
-    stream = int(torch.cuda.current_stream(recv.device).cuda_stream) or 1  # 0x1 = cudaStreamLegacy
     C.check(C.load().b2f_merge_topk_strided(int(metric), nq, k, recv.numel() // part_bytes, recv.data_ptr(),
                                             recv.data_ptr() + off_i, part_bytes, D.data_ptr(), I.data_ptr(),
-                                            recv.device.index or 0, ctypes.c_void_p(stream)))
+                                            recv.device.index or 0, ctypes.c_void_p(_torch_stream(recv))))
 
 
 def merge_topk(metric: int, D_parts, I_parts):
@@ -146,14 +143,11 @@ def merge_range_strided(lims_parts, recv, part_bytes: int, off_i: int, D, I):
     """b2f_merge_range_strided over an all-gathered buffer: lims_parts [G, nq + 1] int64 (any base), recv [G * part_bytes]
     uint8 holding G packed parts [D | pad | I at off_i]; writes the label-ordered union into D / I [total] (CUDA
     tensors on one device, enqueued on the current torch stream)."""
-    import torch
-
     G, nq = int(lims_parts.shape[0]), int(lims_parts.shape[1]) - 1
     lims_parts = lims_parts.contiguous()
-    stream = int(torch.cuda.current_stream(recv.device).cuda_stream) or 1  # 0x1 = cudaStreamLegacy
     C.check(C.load().b2f_merge_range_strided(nq, G, lims_parts.data_ptr(), recv.data_ptr(), recv.data_ptr() + off_i,
                                              part_bytes, D.data_ptr(), I.data_ptr(), recv.device.index or 0,
-                                             ctypes.c_void_p(stream)))
+                                             ctypes.c_void_p(_torch_stream(recv))))
 
 
 def merge_range(parts):
@@ -262,6 +256,12 @@ class ShardedIndexFlat:
         labels = self.segments.to_global_numpy(np.arange(self.local.ntotal, dtype=np.int64))
         return SearchParameters(sel=IDSelectorBitmap(np.packbits(selector_contains(params.sel, labels), bitorder="little")))
 
+    def _work_device(self):
+        """Where the shard's results stay: its GPU (a host-side stand-in for the local index keeps them on the host)."""
+        import torch
+
+        return torch.device("cuda", self.local.device) if isinstance(self.local, IndexFlat) else torch.device("cpu")
+
     def _peer_exchange(self, need_bytes: int):
         """The NVLink peer-memory exchange (csrc/exchange.cu), created on first use and re-created when a search needs
         bigger slots.  Collective: every rank takes the same decisions (same need_bytes on every rank).  Returns None
@@ -348,8 +348,7 @@ class ShardedIndexFlat:
         nq = int(x.shape[0])
         dev_in = _is_torch(x) and x.is_cuda
         flat = isinstance(self.local, IndexFlat)
-        # the results stay on the shard's GPU (a host-side stand-in for the local index keeps them on the host)
-        work = torch.device("cuda", self.local.device) if flat else torch.device("cpu")
+        work = self._work_device()
         if dev_in and out is not None:
             Dm, Im = out
             if not (Dm.is_cuda and Im.is_cuda and Dm.dtype == torch.float32 and Im.dtype == torch.int64
@@ -369,7 +368,7 @@ class ShardedIndexFlat:
         if dev_in and flat:
             if x.device.index != self.local.device:
                 raise AssertionError("queries are on another GPU than this rank's shard")
-            stream = ctypes.c_void_p(int(torch.cuda.current_stream(x.device).cuda_stream) or 1)  # 0x1 = cudaStreamLegacy
+            stream = ctypes.c_void_p(_torch_stream(x))
             ex = self._peer_exchange(part)
             if ex is not None and off is not None and lp is None:
                 # the whole sharded step behind one C call: local search into the exchange's message buffer, then
@@ -467,8 +466,7 @@ class ShardedIndexFlat:
 
         chunks, sent = 0, 0
         if self.world > 1:
-            # the hits stay on the shard's GPU (a host-side stand-in for the local index keeps them on the host)
-            work = torch.device("cuda", self.local.device) if isinstance(self.local, IndexFlat) else torch.device("cpu")
+            work = self._work_device()
             lims, D, I = lims.to(work), D.to(work), I.to(work)
             lims_all = self._all_gather(lims)      # [world, nq + 1]: every rank's local lims (base 0)
             lims_host = lims_all.cpu().numpy()
